@@ -2,7 +2,7 @@
 """bench.py -- probit-ELBO fwd+bwd throughput (label-samples/s) on B200, BASELINE.json's metric.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload eurlex] [--z Z] [--scaling weak|strong]
-                    [--impl reference]
+                    [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch: draw the (S,B,Z) noise (Philox, on device), the forward of
 compute_loss (mpvae.py:145-210) and its full backward to logits / R / mu / logvar; at N > 1 the step ends with the sum
@@ -12,6 +12,11 @@ configs[4], SURVEY 8e); a run at N > 1 also reports the other mode as a short le
 `value` times the step with the inputs resident in HBM; `e2e` times the same call through the public
 `mpvae_b200.compute_loss` API starting from pinned HOST buffers (H2D of the step's inputs, D2H of the loss and of the
 step's eight metrics inside the timed region).  Prints ONE JSON line (rank 0).
+
+`--dump-outputs DIR` writes what the last step timed for `value` returned: compute_loss's eight outputs and, for a
+training workload, the gradients of the loss with respect to its seven differentiable inputs (`grad_<input>`), as
+DIR/<name>.npy.  Inputs and noise are seeded, so runs with the same arguments see the same inputs and two builds can be
+compared output for output.
 
 `--impl reference` times the reference's own CPU implementation instead: the UNMODIFIED compute_loss of
 /root/reference/mpvae.py, placed under oracle/_ref/ by oracle/make_ref.py (the oracle port when that copy is absent),
@@ -35,6 +40,10 @@ METRIC = "probit-ELBO fwd+bwd label-samples/s"
 UNIT = "label-samples/s"
 L2_BYTES = 126 * 1024 * 1024
 ROW_KEYS = ["y", "fe_out", "fe_mu", "fe_logvar", "fx_out", "fx_mu", "fx_logvar"]
+# compute_loss's 8-tuple, in order
+OUT_NAMES = ["total_loss", "nll_loss", "nll_loss_x", "c_loss", "c_loss_x", "kl_loss", "indiv_prob", "indiv_prob_label"]
+# per dumped array: 8 outputs + 7 gradients of at most 4 MB each keep a dump under 64 MB
+DUMP_MAX_BYTES = 4 << 20
 
 # dram__bytes_read.sum + dram__bytes_write.sum per launch of the dominant kernel, from the committed `ncu --set full`
 # captures under profiles/ ((L, Z, S*B rows, fused row forward) -> bytes)
@@ -74,7 +83,15 @@ def parse():
                     help="N>1: how g_R is summed over ranks (peer = inside the backward over NVLink peer memory, "
                          "mpvae_b200.peer.PeerRing, falling back to nccl if the ring cannot be set up on every rank; "
                          "nccl = all-reduce after the backward)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (loss terms, probabilities, gradients; rank 0's) as "
+                         "DIR/<name>.npy, arrays above %d MB as a fixed seeded sample" % (DUMP_MAX_BYTES >> 20))
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
+    return a
 
 
 def measured_peaks():
@@ -147,6 +164,26 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(smax) if smax else None,
                 "power_w_max": max(power) if power else None, "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def host_outputs(tensors):
+    """{name: device tensor} -> {name: float32/float64 numpy array}.  An array of more than DUMP_MAX_BYTES becomes a
+    sample of its flattened elements, as many as fit in DUMP_MAX_BYTES, taken at positions drawn from a fixed seed: the
+    same positions for the same shape and dtype, so two builds' dumps compare element for element."""
+    import numpy as np
+    import torch
+    host, positions = {}, {}
+    for name, t in tensors.items():
+        t = t.detach()
+        if t.dtype not in (torch.float32, torch.float64):
+            t = t.float()
+        n, cap = t.numel(), DUMP_MAX_BYTES // t.element_size()
+        if n > cap:
+            if (n, cap) not in positions:
+                positions[n, cap] = torch.from_numpy(np.sort(np.random.RandomState(0).choice(n, cap, replace=False)))
+            t = t.reshape(-1)[positions[n, cap].to(t.device)]
+        host[name] = t.cpu().numpy()
+    return host
 
 
 def workload(a):
@@ -380,7 +417,8 @@ def run_b200(a):
         if int(ok.item()) == 0 and ring is not None:
             ring = None                 # (its buffers stay allocated; the process is short-lived)
 
-    def one_step(leg, src, from_host, use_ring=True, noise=None):
+    def one_step(leg, src, from_host, use_ring=True, noise=None, keep=None):
+        """One step; `keep` (a dict), if given, receives what the step returns to its caller, by name."""
         args = leg.args
         args.noise_offset = step_no[0]
         args.peer_ring = ring if use_ring else None
@@ -404,6 +442,9 @@ def run_b200(a):
                     dist.all_reduce(r32.grad, op=dist.ReduceOp.AVG)   # the path's one exchange step: NCCL mean over NVLink
                 else:
                     r32.grad.div_(world)             # with the peer ring the backward already returned the sum
+            if keep is not None:
+                keep.update(("grad_" + k, t[k].grad) for k in ROW_KEYS if k != "y")
+                keep["grad_r_sqrt_sigma"] = r32.grad
             for k in ROW_KEYS:
                 if k != "y":
                     t[k].grad = None
@@ -413,6 +454,8 @@ def run_b200(a):
             # device, SURVEY 8f-N1: mpvae_b200.metrics.batch_metrics) come back to the host
             metrics_host.copy_(batch_metrics_tensor(out[6], t["y"], 0.5), non_blocking=True)
             loss_host.copy_(out[0].detach(), non_blocking=True)
+        if keep is not None:
+            keep.update(zip(OUT_NAMES, out))
         return out
 
     def timed_e2e(leg, n_steps):
@@ -434,13 +477,13 @@ def run_b200(a):
         torch.cuda.synchronize()
         return e0.elapsed_time(e1)
 
-    def timed(leg, n_steps, **kw):
+    def timed(leg, n_steps, keep=None, **kw):
         evs = []
-        for _ in range(n_steps):
+        for i in range(n_steps):
             flush.add_(1.0)                         # evict L2 between timed iterations (2 x 126 MB written)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            one_step(leg, leg.dev, False, **kw)
+            one_step(leg, leg.dev, False, keep=keep if i == n_steps - 1 else None, **kw)
             e1.record()
             evs.append((e0, e1))
         torch.cuda.synchronize()
@@ -468,8 +511,15 @@ def run_b200(a):
     barrier()
     sampler.mark_begin()            # clocks are reported for the two timed regions below only
     launches0 = _lib.launch_count()
-    ms = timed(main, a.steps)
+    last = {} if a.dump_outputs else None
+    ms = timed(main, a.steps, keep=last)
     launches = _lib.launch_count() - launches0
+    if last is not None and rank == 0:
+        # before any further step: with the peer ring, g_R lives in the ring's buffer, which the next step overwrites
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for name, arr in host_outputs(last).items():
+            np.save(os.path.join(a.dump_outputs, name + ".npy"), arr)
+    last = None
     barrier()
     total_ms = sum(ms)
     total_e2e = timed_e2e(main, a.steps)
