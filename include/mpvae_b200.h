@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MPVAE_ABI_VERSION 11
+#define MPVAE_ABI_VERSION 12
 
 /* flags */
 #define MPVAE_FLAG_SANITIZE_DEGENERATE 0x1u /* rows with n_pos*n_neg == 0 get zero ranking gradient instead of
@@ -169,6 +169,14 @@ uint64_t mpvae_workspace_bytes(int32_t S, int32_t B, int32_t L, int32_t Z, int32
 
 /* Forward: replaces the body of compute_loss (mpvae.py:145-210) given the noise tensor. */
 int mpvae_probit_forward(const mpvae_probit_params *p, void *cuda_stream);
+
+/* Prediction only: indiv_prob (B,L) = mean_s clamp(Phi(fx_out + noise.R^T)) (mpvae.py:170,180,203), the feature branch
+ * alone -- what scoring rows without labels needs.  Reads struct_bytes, flags, S, B, L, Z, fx_out, r, noise (or the
+ * library-noise fields noise_seed / noise_offset / noise_b_global / noise_row0 / noise_offset_dev), workspace /
+ * workspace_bytes (mpvae_workspace_bytes(S, B, L, Z, 0, flags) suffices) and writes indiv_prob only; every other field is
+ * ignored and may be NULL.  Takes the regime mpvae_probit_forward takes for the same (S, B, L, Z, flags) and returns
+ * the bits of its indiv_prob for the same fx_out, R and noise. */
+int mpvae_probit_predict(const mpvae_probit_params *p, void *cuda_stream);
 
 /* Backward: the autograd backward of compute_loss (implicit in the reference, train.py:125),
  * closed form in SURVEY.md 8(a-12).  Must follow a forward on the same workspace. */

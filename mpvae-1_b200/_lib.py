@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmpvae_b200.so")
 
-ABI_VERSION = 11
+ABI_VERSION = 12
 FLAG_SANITIZE_DEGENERATE = 0x1
 FLAG_CONTRACT_TENSOR = 0x2
 FLAG_CONTRACT_FMA = 0x4
@@ -25,7 +25,7 @@ PEER_TILE_BYTES = 65536
 
 # every symbol include/mpvae_b200.h declares
 EXPORTS = (
-    "mpvae_workspace_bytes", "mpvae_probit_forward", "mpvae_probit_backward", "mpvae_philox_normal",
+    "mpvae_workspace_bytes", "mpvae_probit_forward", "mpvae_probit_predict", "mpvae_probit_backward", "mpvae_philox_normal",
     "mpvae_contract_nt", "mpvae_contract_nt_pitched", "mpvae_contract_tn", "mpvae_grad_norm_workspace",
     "mpvae_grad_norm", "mpvae_adam_step", "mpvae_tc_planes_bytes", "mpvae_tc_tail_scratch_bytes", "mpvae_tc_split",
     "mpvae_tc_gemm_nt", "mpvae_tc_gemm_tn", "mpvae_peer_flag_bytes", "mpvae_peer_allreduce", "mpvae_peer_allreduce_dev", "mpvae_peer_allreduce_nvls", "mpvae_label_curves",
@@ -87,6 +87,8 @@ def _load():
     lib.mpvae_workspace_bytes.argtypes = [C.c_int32] * 5 + [C.c_uint32]
     lib.mpvae_probit_forward.restype = C.c_int
     lib.mpvae_probit_forward.argtypes = [C.POINTER(ProbitParams), C.c_void_p]
+    lib.mpvae_probit_predict.restype = C.c_int
+    lib.mpvae_probit_predict.argtypes = [C.POINTER(ProbitParams), C.c_void_p]
     lib.mpvae_probit_backward.restype = C.c_int
     lib.mpvae_probit_backward.argtypes = [C.POINTER(ProbitParams), C.c_void_p]
     lib.mpvae_philox_normal.restype = C.c_int

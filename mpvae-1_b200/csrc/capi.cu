@@ -168,6 +168,25 @@ const mpvae_probit_params* normalize(const mpvae_probit_params* p, mpvae_probit_
     return nullptr;
 }
 
+int check_noise_rows(const mpvae_probit_params* p) {
+    if (!p->noise && (p->noise_row0 < 0 || p->noise_b_global < p->noise_row0 + p->B)) {
+        set_error("library-side noise: rows [%d, %d) do not fit a global batch of %d", p->noise_row0, p->noise_row0 + p->B,
+                  p->noise_b_global);
+        return 1;
+    }
+    return 0;
+}
+
+int check_workspace(const mpvae_probit_params* p, bool backward) {
+    const uint64_t need = mpvae_workspace_bytes(p->S, p->B, p->L, p->Z, backward ? 1 : 0, p->flags);
+    if (p->workspace_bytes < need) {
+        set_error("workspace too small: %llu < %llu bytes", (unsigned long long)p->workspace_bytes, (unsigned long long)need);
+        return 1;
+    }
+    if ((reinterpret_cast<uintptr_t>(p->workspace) & 255u) != 0) { set_error("workspace must be 256-byte aligned"); return 1; }
+    return 0;
+}
+
 int validate(const mpvae_probit_params* p, bool backward) {
     if (p->S <= 0 || p->B <= 0 || p->L <= 0 || p->Z <= 0 || p->D < 0) {
         set_error("bad sizes S=%d B=%d L=%d Z=%d D=%d (empty batches are handled by the host wrapper)", p->S, p->B, p->L,
@@ -179,11 +198,7 @@ int validate(const mpvae_probit_params* p, bool backward) {
         set_error("NULL input pointer (y/fe_out/fx_out/r/workspace)");
         return 1;
     }
-    if (!p->noise && (p->noise_row0 < 0 || p->noise_b_global < p->noise_row0 + p->B)) {
-        set_error("library-side noise: rows [%d, %d) do not fit a global batch of %d", p->noise_row0, p->noise_row0 + p->B,
-                  p->noise_b_global);
-        return 1;
-    }
+    if (int rc = check_noise_rows(p)) return rc;
     if (p->D > 0 && (!p->fe_mu || !p->fe_logvar || !p->fx_mu || !p->fx_logvar)) { set_error("NULL mu/logvar pointer"); return 1; }
     if (!backward && (!p->scalars[0] || !p->scalars[1] || !p->scalars[2] || !p->scalars[3] || !p->scalars[4] ||
                       !p->scalars[5] || !p->indiv_prob || !p->indiv_prob_label)) { set_error("NULL forward output pointer"); return 1; }
@@ -191,15 +206,20 @@ int validate(const mpvae_probit_params* p, bool backward) {
         if (!p->g_fe_out || !p->g_fx_out) { set_error("NULL g_fe_out/g_fx_out"); return 1; }
         if (p->D > 0 && (!p->g_fe_mu || !p->g_fe_logvar || !p->g_fx_mu || !p->g_fx_logvar)) { set_error("NULL mu/logvar gradient pointer"); return 1; }
     }
-    const uint64_t need = mpvae_workspace_bytes(p->S, p->B, p->L, p->Z, 1, p->flags);
-    const uint64_t need_fwd = mpvae_workspace_bytes(p->S, p->B, p->L, p->Z, 0, p->flags);
-    if (p->workspace_bytes < (backward ? need : need_fwd)) {
-        set_error("workspace too small: %llu < %llu bytes", (unsigned long long)p->workspace_bytes,
-                  (unsigned long long)(backward ? need : need_fwd));
+    return check_workspace(p, backward);
+}
+
+// mpvae_probit_predict reads fx_out, r, the noise fields and indiv_prob only
+int validate_predict(const mpvae_probit_params* p) {
+    if (p->S <= 0 || p->B <= 0 || p->L <= 0 || p->Z <= 0) {
+        set_error("bad sizes S=%d B=%d L=%d Z=%d (empty batches are handled by the host wrapper)", p->S, p->B, p->L, p->Z);
         return 1;
     }
-    if ((reinterpret_cast<uintptr_t>(p->workspace) & 255u) != 0) { set_error("workspace must be 256-byte aligned"); return 1; }
-    return 0;
+    if ((long long)p->S * p->B > 0x7fffffffLL) { set_error("S*B overflows int32"); return 1; }
+    if (!p->fx_out || !p->r || !p->workspace) { set_error("NULL input pointer (fx_out/r/workspace)"); return 1; }
+    if (int rc = check_noise_rows(p)) return rc;
+    if (!p->indiv_prob) { set_error("NULL forward output pointer (indiv_prob)"); return 1; }
+    return check_workspace(p, false);
 }
 
 // side stream + events of the exchange that runs beside the g_R product (one process per GPU: created once per device,
@@ -269,6 +289,68 @@ RowArgs row_args(const mpvae_probit_params* p, const Workspace& w) {
     return a;
 }
 
+// Dense regime, up to and including the product: the noise operand (unless the product kernel draws it), the R split and
+// nr = noise . R^T on tcgen05.  fz: the fused row forward to run on the product kernel's math warps, or nullptr.  The
+// caller has zeroed the slots block.
+int dense_nt_product(const mpvae_probit_params* p, const Workspace& w, const FuseFwd* fz, cudaStream_t stream) {
+    char* base = static_cast<char*>(p->workspace);
+    float* nr = reinterpret_cast<float*>(base + w.nr);
+    uint32_t* slots = reinterpret_cast<uint32_t*>(base + w.slots);
+    const int M = p->S * p->B;
+    void* npl = base + w.noise_planes;
+    void* rpl = base + w.r_planes;
+    // library noise: drawn by the product kernel's own math warps just ahead of the tiles (unless those warps carry
+    // the fused row forward, or the caller asks for the separate kernel)
+    const bool jit_noise = !p->noise && !fz && !(p->flags & MPVAE_FLAG_SEPARATE_NOISE);
+    int rc = 0;
+    if (!jit_noise) {
+        ProfScope ps(MPVAE_PROF_NOISE, stream);
+        // operand rows are b-major (b * S + s): the S sample-rows of a batch row are neighbours
+        if (p->noise) rc = tc_split(p->noise, M, p->Z, npl, nullptr, 0, stream, 0, p->S, p->B);   // |N(0,1)| fits fp16 at scale 1
+        else rc = tc_philox_planes(npl, p->S, p->B, p->Z, p->noise_b_global, p->noise_row0, p->noise_seed, p->noise_offset, p->noise_offset_dev, stream);
+    }
+    if (rc) return rc;
+    {
+        ProfScope ps(MPVAE_PROF_SPLIT_R, stream);
+        rc = tc_split(p->r, p->L, p->Z, rpl, slots + SLOT_ABSMAX_R, 1, stream);
+    }
+    if (rc) return rc;
+    FuseNoise fnz{};
+    if (jit_noise) {
+        fnz.plane = static_cast<__half*>(npl);
+        fnz.S = p->S; fnz.B = p->B; fnz.Z = p->Z; fnz.pitch = tc_pitch(p->Z);
+        fnz.Bg = p->noise_b_global; fnz.row0 = p->noise_row0;
+        fnz.key = make_uint2((uint32_t)p->noise_seed, (uint32_t)(p->noise_seed >> 32));
+        fnz.off = make_uint2((uint32_t)p->noise_offset, (uint32_t)(p->noise_offset >> 32));
+        fnz.off_dev = reinterpret_cast<const unsigned long long*>(p->noise_offset_dev);
+        fnz.ready = slots + w.noise_counters / sizeof(uint32_t);
+        if ((long long)p->B * p->Z >= 0x7fffffffLL || p->Z < 4) { set_error("philox: B*Z=%lld, Z=%d out of range", (long long)p->B * p->Z, p->Z); return 6; }
+    }
+    ProfScope ps(MPVAE_PROF_PRODUCT_NT, stream);
+    // library noise sits on the fp16 grid: one plane, two MMA passes.
+    // No tail scratch here: K-slicing the last wave would make the summation order of x = noise.R^T depend on
+    // how many rows the call holds, and a row's predictions must not change with the shard it is computed in
+    return tc_gemm_nt(npl, rpl, nr, M, p->L, p->Z, nullptr, slots + SLOT_ABSMAX_R, stream, row_pitch(p->L), p->noise ? 0 : 1,
+                      nullptr, 0, fz, jit_noise ? &fnz : nullptr);
+}
+
+// CUDA-core regime, up to and including the product: the Philox normals (unless the caller gives the noise) and
+// nr = noise . R^T with the FMA engine
+int fma_nt_product(const mpvae_probit_params* p, const Workspace& w, cudaStream_t stream) {
+    char* base = static_cast<char*>(p->workspace);
+    const float* nz = p->noise;
+    if (!nz) {
+        ProfScope ps(MPVAE_PROF_NOISE, stream);
+        float* gen = reinterpret_cast<float*>(base + w.noise_f32);
+        if (int rc = launch_philox_normal(gen, p->S, p->B, p->Z, p->noise_b_global, p->noise_row0, p->noise_seed,
+                                          p->noise_offset, p->noise_offset_dev, stream)) return rc;
+        nz = gen;
+    }
+    ProfScope ps(MPVAE_PROF_PRODUCT_NT, stream);
+    return launch_contract_nt_fma(nz, p->r, reinterpret_cast<float*>(base + w.nr), p->S * p->B, p->L, p->Z, stream,
+                                  row_pitch(p->L));
+}
+
 }  // namespace
 }  // namespace mpv
 
@@ -336,7 +418,6 @@ int mpvae_probit_forward(const mpvae_probit_params* p_in, void* cuda_stream) {
     char* base = static_cast<char*>(p->workspace);
     float* nr = reinterpret_cast<float*>(base + w.nr);
     uint32_t* slots = reinterpret_cast<uint32_t*>(base + w.slots);
-    const int M = p->S * p->B;
     cudaError_t e = cudaMemsetAsync(slots, 0, w.slots_bytes, stream);   // last-CTA counter, absmax slots, tile counters
     if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
     int rc;
@@ -349,37 +430,8 @@ int mpvae_probit_forward(const mpvae_probit_params* p_in, void* cuda_stream) {
         a.E_x = reinterpret_cast<float*>(base + wb.e_x);
     }
     if (use_tensor(p->flags, p->S, p->B, p->L, p->Z)) {
-        void* npl = base + w.noise_planes;
-        void* rpl = base + w.r_planes;
         const bool fused = use_fused_forward(p->flags, p->S, p->B, p->L, p->Z);
-        // library noise: drawn by the product kernel's own math warps just ahead of the tiles (unless those warps carry
-        // the fused row forward, or the caller asks for the separate kernel)
-        const bool jit_noise = !p->noise && !fused && !(p->flags & MPVAE_FLAG_SEPARATE_NOISE);
-        rc = 0;
-        if (!jit_noise) {
-            ProfScope ps(MPVAE_PROF_NOISE, stream);
-            // operand rows are b-major (b * S + s): the S sample-rows of a batch row are neighbours
-            if (p->noise) rc = tc_split(p->noise, M, p->Z, npl, nullptr, 0, stream, 0, p->S, p->B);   // |N(0,1)| fits fp16 at scale 1
-            else rc = tc_philox_planes(npl, p->S, p->B, p->Z, p->noise_b_global, p->noise_row0, p->noise_seed, p->noise_offset, p->noise_offset_dev, stream);
-        }
-        if (rc) return rc;
-        {
-            ProfScope ps(MPVAE_PROF_SPLIT_R, stream);
-            rc = tc_split(p->r, p->L, p->Z, rpl, slots + SLOT_ABSMAX_R, 1, stream);
-        }
-        if (rc) return rc;
         FuseFwd fz{};
-        FuseNoise fnz{};
-        if (jit_noise) {
-            fnz.plane = static_cast<__half*>(npl);
-            fnz.S = p->S; fnz.B = p->B; fnz.Z = p->Z; fnz.pitch = tc_pitch(p->Z);
-            fnz.Bg = p->noise_b_global; fnz.row0 = p->noise_row0;
-            fnz.key = make_uint2((uint32_t)p->noise_seed, (uint32_t)(p->noise_seed >> 32));
-            fnz.off = make_uint2((uint32_t)p->noise_offset, (uint32_t)(p->noise_offset >> 32));
-            fnz.off_dev = reinterpret_cast<const unsigned long long*>(p->noise_offset_dev);
-            fnz.ready = slots + w.noise_counters / sizeof(uint32_t);
-            if ((long long)p->B * p->Z >= 0x7fffffffLL || p->Z < 4) { set_error("philox: B*Z=%lld, Z=%d out of range", (long long)p->B * p->Z, p->Z); return 6; }
-        }
         if (fused) {
             fz.S = p->S; fz.B = p->B; fz.L = p->L; fz.ldn = row_pitch(p->L);
             fz.stable = a.stable;
@@ -390,15 +442,7 @@ int mpvae_probit_forward(const mpvae_probit_params* p_in, void* cuda_stream) {
             fz.part = reinterpret_cast<FusePart*>(base + w.fuse_part);
             fz.done = slots + w.tile_counters / sizeof(uint32_t);
         }
-        {
-            ProfScope ps(MPVAE_PROF_PRODUCT_NT, stream);
-            // library noise sits on the fp16 grid: one plane, two MMA passes.
-            // No tail scratch here: K-slicing the last wave would make the summation order of x = noise.R^T depend on
-            // how many rows the call holds, and a row's predictions must not change with the shard it is computed in
-            rc = tc_gemm_nt(npl, rpl, nr, M, p->L, p->Z, nullptr, slots + SLOT_ABSMAX_R, stream, row_pitch(p->L), p->noise ? 0 : 1,
-                            nullptr, 0, fused ? &fz : nullptr, jit_noise ? &fnz : nullptr);
-        }
-        if (rc) return rc;
+        if ((rc = dense_nt_product(p, w, fused ? &fz : nullptr, stream))) return rc;
         ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
         if (fused) {
             a.part = fz.part;
@@ -420,21 +464,44 @@ int mpvae_probit_forward(const mpvae_probit_params* p_in, void* cuda_stream) {
         sn.seed = p->noise_seed; sn.offset = p->noise_offset; sn.offset_dev = p->noise_offset_dev;
         return launch_small_forward(a, sn, stream);
     }
-    const float* nz = p->noise;
-    if (!nz) {
-        ProfScope ps(MPVAE_PROF_NOISE, stream);
-        float* gen = reinterpret_cast<float*>(base + w.noise_f32);
-        if ((rc = launch_philox_normal(gen, p->S, p->B, p->Z, p->noise_b_global, p->noise_row0, p->noise_seed,
-                                       p->noise_offset, p->noise_offset_dev, stream))) return rc;
-        nz = gen;
-    }
-    {
-        ProfScope ps(MPVAE_PROF_PRODUCT_NT, stream);
-        rc = launch_contract_nt_fma(nz, p->r, nr, M, p->L, p->Z, stream, row_pitch(p->L));
-    }
-    if (rc) return rc;
+    if ((rc = fma_nt_product(p, w, stream))) return rc;
     ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
     return launch_row_forward(a, stream);
+}
+
+int mpvae_probit_predict(const mpvae_probit_params* p_in, void* cuda_stream) {
+    mpvae_probit_params tmp;
+    const mpvae_probit_params* p = normalize(p_in, &tmp);
+    if (!p) return 1;
+    if (int rc = validate_predict(p)) return rc;
+    cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
+    // the inference layout of mpvae_probit_forward; only nr, the noise / R operands and the slots are touched
+    const Workspace w = carve(p->S, p->B, p->L, p->Z, false, p->flags);
+    const RowArgs a = row_args(p, w);
+    int rc;
+    // the same regime as mpvae_probit_forward for the same (S, B, L, Z, flags)
+    if (use_tensor(p->flags, p->S, p->B, p->L, p->Z)) {
+        // absmax slot of R, per-block counters of the just-in-time noise
+        uint32_t* slots = reinterpret_cast<uint32_t*>(static_cast<char*>(p->workspace) + w.slots);
+        const cudaError_t e = cudaMemsetAsync(slots, 0, w.slots_bytes, stream);
+        if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
+        // the fused row forward (MPVAE_FLAG_FUSED_FORWARD) is loss work: predictions take the separate row kernel
+        if ((rc = dense_nt_product(p, w, nullptr, stream))) return rc;
+        ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
+        return launch_predict_rows(a, stream);
+    }
+    if (use_small(p->flags, p->S, p->B, p->L, p->Z)) {
+        ProfScope ps(MPVAE_PROF_FUSED_SMALL_FWD, stream);
+        SmallNoise sn{};
+        sn.r = p->r; sn.Z = p->Z;
+        sn.noise_ext = p->noise;
+        sn.Bg = p->noise_b_global; sn.row0 = p->noise_row0;
+        sn.seed = p->noise_seed; sn.offset = p->noise_offset; sn.offset_dev = p->noise_offset_dev;
+        return launch_small_predict(a, sn, stream);
+    }
+    if ((rc = fma_nt_product(p, w, stream))) return rc;
+    ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
+    return launch_predict_rows(a, stream);
 }
 
 int mpvae_probit_backward(const mpvae_probit_params* p_in, void* cuda_stream) {

@@ -19,6 +19,7 @@
 #include "philox.cuh"
 #include "probit_math.cuh"
 #include "rows.h"
+#include "small_rows.cuh"
 
 namespace mpv {
 
@@ -32,9 +33,6 @@ struct BlockCounts { int npos, nneg; };
 
 // One lane's inputs for one 32-label chunk and kST samples.
 struct RowChunk { float y, fe, fx, nr[kST]; };
-
-// row index of (s, b) in the scratch matrices (RowArgs::row_sb / row_ss)
-__device__ __forceinline__ size_t row_of(const RowArgs& a, int s, int b) { return (size_t)b * a.row_sb + (size_t)s * a.row_ss; }
 
 __device__ __forceinline__ void load_chunk(RowChunk& in, const RowArgs& a, const float* __restrict__ yrow,
                                            const float* __restrict__ ferow, const float* __restrict__ fxrow, int c, int lane,
@@ -567,25 +565,7 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
 //   tail            row_tail(): KL, log-mean-exp over samples, softmax weights, ranking sums, last-CTA batch means
 // The backward is one CTA per row as well (cell_backward_saved from the kept E and nr, logit gradients, KL gradients)
 // and leaves the row's contribution to g_R = gxs^T . noise in a scratch slab; a second, tiny kernel adds the slabs over
-// the batch in row order (deterministic).
-struct SmallArgs {
-    RowArgs a;
-    const float* r;            // (L, Z) fp32
-    int Z;
-    const float* noise_ext;    // (S, B, Z) caller's noise or nullptr
-    float* noise_out;          // (S, B, Z) fp32 copy kept for the backward, or nullptr (inference)
-    float* nr_out;             // (S*B, ldn) kept for the backward, or nullptr
-    int Bg, row0;
-    uint2 key, off;
-    const unsigned long long* off_dev;
-    float* partial;            // backward: (B, L*Z) per-row contributions to g_R
-};
-
-__device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-constexpr int kSmallThreads = 512;   // sixteen warps: a sample pair each per round
-constexpr int kSmallWarps = kSmallThreads / 32;
-
+// the batch in row order (deterministic).  R staging, the noise draw and the contraction are small_rows.cuh's.
 template <bool STABLE>
 __global__ void __launch_bounds__(kSmallThreads)
 probit_small_fwd_kernel(const SmallArgs p) {
@@ -599,22 +579,7 @@ probit_small_fwd_kernel(const SmallArgs p) {
     float* Rs = reinterpret_cast<float*>(s_raw);                           // [L][Z]
     float* nz = Rs + (((size_t)L * Z + 3) & ~(size_t)3);                   // [kSmallWarps][2][Z]
     float* ps = nz + (size_t)kSmallWarps * 2 * Z;                               // [npairs][2][L] pair sums of E
-    // ---- R -> shared memory: one TMA bulk copy for the 16-byte multiple, plain loads for the last few floats ----
-    const uint32_t bytes16 = ((uint32_t)(L * Z) * 4u) & ~15u;
-    const bool bulk = bytes16 != 0 && (reinterpret_cast<uintptr_t>(p.r) & 15u) == 0;
-    const uint32_t bar = smem_addr(&s_bar);
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    if (tid == 0 && bulk) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes16) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"(smem_addr(Rs)), "l"(p.r), "r"(bytes16), "r"(bar)
-                     : "memory");
-    }
-    for (int i = (bulk ? (int)(bytes16 >> 2) : 0) + tid; i < L * Z; i += kSmallThreads) Rs[i] = p.r[i];
+    const bool bulk = small_r_stage<kSmallThreads>(Rs, p.r, L, Z, &s_bar);
     // this lane's labels (L <= 128: at most four 32-label chunks)
     const int nch = (L + 31) >> 5;
     float yv[4], fev[4], fxv[4];
@@ -624,18 +589,7 @@ probit_small_fwd_kernel(const SmallArgs p) {
         yv[c] = fev[c] = fxv[c] = 0.f;
         if (c < nch && l < L) { yv[c] = a.y[(size_t)b * L + l]; fev[c] = a.fe_out[(size_t)b * L + l]; fxv[c] = a.fx_out[(size_t)b * L + l]; }
     }
-    if (bulk) {
-        uint32_t done = 0;
-        while (!done) {
-            asm volatile(
-                "{\n\t.reg .pred q;\n\t"
-                "mbarrier.try_wait.parity.shared::cta.b64 q, [%1], 0;\n\t"
-                "selp.u32 %0, 1, 0, q;\n\t}"
-                : "=r"(done)
-                : "r"(bar)
-                : "memory");
-        }
-    }
+    small_r_wait(bulk, &s_bar);
     __syncthreads();
     // ---- pairs of samples, a warp each ----
     const uint2 off = philox_offset(p.off, p.off_dev);
@@ -643,28 +597,7 @@ probit_small_fwd_kernel(const SmallArgs p) {
     for (int pair = warp; pair < npairs; pair += kSmallWarps) {
         const int s0 = pair << 1;
         const bool two = s0 + 1 < S;
-#pragma unroll
-        for (int i = 0; i < 2; ++i) {
-            const int s = s0 + i;
-            if (s >= S) break;
-            if (p.noise_ext) {
-                const float* src = p.noise_ext + ((size_t)s * B + b) * Z;
-                for (int z = lane; z < Z; z += 32) nzw[i * Z + z] = src[z];
-            } else {
-                // the normals of (s, global row, 0 .. Z): counters flat0 / 4 .. (flat0 + Z - 1) / 4 of the global tensor
-                const unsigned long long flat0 = ((unsigned long long)s * p.Bg + p.row0 + b) * Z;
-                const unsigned long long c0 = flat0 >> 2, c1 = (flat0 + Z - 1) >> 2;
-                for (unsigned long long c = c0 + lane; c <= c1; c += 32) {
-                    float n[4];
-                    philox_normal4(c, p.key, off, n);
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const long long z = (long long)(c << 2) + j - (long long)flat0;
-                        if (z >= 0 && z < Z) nzw[i * Z + z] = n[j];
-                    }
-                }
-            }
-        }
+        small_noise_pair(nzw, p, s0, b, off, lane);
         __syncwarp();
         if (p.noise_out) {
             for (int i = 0; i < (two ? 2 : 1); ++i)
@@ -676,14 +609,8 @@ probit_small_fwd_kernel(const SmallArgs p) {
         for (int c = 0; c < 4; ++c) {
             const int l = (c << 5) + lane;
             if (c >= nch || l >= L) continue;
-            // warp-level FMA chain in k order (the chain of contract_fma.cu: bit-equal results)
-            float acc0 = 0.f, acc1 = 0.f;
-            const float* rl = Rs + (size_t)l * Z;
-            for (int z = 0; z < Z; ++z) {
-                const float r = rl[z];
-                acc0 = fmaf(nzw[z], r, acc0);
-                acc1 = fmaf(nzw[Z + z], r, acc1);
-            }
+            float acc0, acc1;
+            small_nr_pair(Rs + (size_t)l * Z, nzw, Z, acc0, acc1);
             float pl = 0.f, px = 0.f;
 #pragma unroll
             for (int i = 0; i < 2; ++i) {
@@ -839,9 +766,6 @@ size_t row_smem_bytes(int L) {
     return (size_t)(kWarps / nwl) * 2 * (size_t)L * sizeof(float);
 }
 
-// cudaFuncAttributeMaxDynamicSharedMemorySize is per device: set once per device, to the cap, so that later launches
-// (e.g. under CUDA-graph capture) make no driver calls
-constexpr int kMaxDevices = 64;
 int device_slot() {
     int d = 0;
     cudaGetDevice(&d);
@@ -860,19 +784,6 @@ bool small_regime_fits(int S, int B, int L, int Z) {
     return small_fwd_smem(S, L, Z) <= 160 * 1024 && small_bwd_smem(S, L, Z) <= 160 * 1024;
 }
 size_t small_partial_bytes(int B, int L, int Z) { return (size_t)B * L * Z * sizeof(float); }
-
-static SmallArgs small_args(const RowArgs& a, const SmallNoise& n) {
-    SmallArgs p{};
-    p.a = a;
-    p.r = n.r; p.Z = n.Z;
-    p.noise_ext = n.noise_ext; p.noise_out = n.noise_out; p.nr_out = n.nr_out;
-    p.Bg = n.Bg; p.row0 = n.row0;
-    p.key = make_uint2((uint32_t)n.seed, (uint32_t)(n.seed >> 32));
-    p.off = make_uint2((uint32_t)n.offset, (uint32_t)(n.offset >> 32));
-    p.off_dev = reinterpret_cast<const unsigned long long*>(n.offset_dev);
-    p.partial = n.partial;
-    return p;
-}
 
 int launch_small_forward(RowArgs a, const SmallNoise& n, cudaStream_t stream) {
     const size_t smem = small_fwd_smem(a.S, a.L, n.Z);

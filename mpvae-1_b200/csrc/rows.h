@@ -54,6 +54,10 @@ struct RowArgs {
 };
 
 size_t row_smem_bytes(int L);
+// cudaFuncAttributeMaxDynamicSharedMemorySize is per device: launchers set it once per device (device_slot() <
+// kMaxDevices), so that later launches (e.g. under CUDA-graph capture) make no driver calls
+constexpr int kMaxDevices = 64;
+int device_slot();
 // Small regime (L, Z <= 128, L * Z <= 8192): the whole forward of a batch row in one CTA of one launch (probit_rows.cu).
 struct SmallNoise {
     const float* r;            // (L, Z) fp32
@@ -81,6 +85,11 @@ int launch_row_backward(RowArgs a, cudaStream_t stream);
 // from the saved per-(row, sample) statistics and the upstream cotangents; gp_absmax: two slots holding max |g_indiv_prob|
 // and max |g_indiv_prob_label| as fp32 bits (zero when absent)
 int launch_gxs_bound(RowArgs a, const unsigned int* gp_absmax, unsigned int* out_bits, cudaStream_t stream);
+
+// Prediction only (predict.cu): a.indiv_prob = mean_s E(nr + fx_out), the feature branch alone -- no labels, no
+// log-likelihoods, no ranking factors, no per-row tail.  Same E and the same sample order as the forward kernels.
+int launch_predict_rows(RowArgs a, cudaStream_t stream);                           // after the nt product (a.nr)
+int launch_small_predict(RowArgs a, const SmallNoise& n, cudaStream_t stream);     // small regime, one launch
 
 // CUDA-core contraction (contract_fma.cu)
 //   nt: C[M,N] = A[M,K] . B[N,K]^T

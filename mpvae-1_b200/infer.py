@@ -16,10 +16,17 @@ from .train import shard_rows
 
 
 @torch.no_grad()
-def predict_proba(model, feats: torch.Tensor, labels: torch.Tensor, args, batch_size: Optional[int] = None,
-                  loss_fn=None, gather: bool = True, group=None):
-    """Returns (indiv_prob (N, L), summed-loss dict).  `feats` / `labels` are device tensors for ALL N rows."""
-    if loss_fn is None:
+def predict_proba(model, feats: torch.Tensor, labels: Optional[torch.Tensor], args, batch_size: Optional[int] = None,
+                  loss_fn=None, gather: bool = True, group=None, predict_fn=None):
+    """Returns (indiv_prob (N, L), summed-loss dict).  `feats` / `labels` are device tensors for ALL N rows.
+
+    `labels=None` scores rows that have no labels: each batch runs only the feature branch (`model.feat_forward`) and
+    `mpvae.predict` (or `predict_fn`, same signature), and the loss dict is None.  With labels, `VAE.forward` draws the
+    label branch's reparameterisation noise first, so under the same torch seed the feature branch -- and hence the
+    predictions -- differ from the label-free call; on the same fx_out the two give the same bits."""
+    if labels is None and predict_fn is None:
+        from .mpvae import predict as predict_fn
+    if labels is not None and loss_fn is None:
         from .mpvae import compute_loss as loss_fn
     args = copy.copy(args)
     args.mode = "test"
@@ -34,18 +41,26 @@ def predict_proba(model, feats: torch.Tensor, labels: torch.Tensor, args, batch_
     n_batches = (hi - lo - 1) // bs + 1 if hi > lo else 0                            # test.py:43
     for i in range(n_batches):
         a, b = lo + bs * i, min(lo + bs * (i + 1), hi)
-        x, y = feats[a:b], labels[a:b].float()
+        x = feats[a:b]
         args.dp_global_batch, args.dp_row0 = n, a
         # one Philox offset for the whole pass: a row's noise is keyed by its GLOBAL row index (dp_row0 + local row), so
         # predictions do not depend on the world size or on how the rows are batched
         args.noise_offset = getattr(args, "noise_offset_base", 0)
+        if labels is None:
+            feat_out, _, _ = model.feat_forward(x)
+            probs.append(predict_fn(feat_out, model.r_sqrt_sigma, args))
+            continue
+        y = labels[a:b].float()
         label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar = model(y, x)
         out = loss_fn(y, label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar, model.r_sqrt_sigma, args)
         probs.append(out[6])
         sums["total_loss"] = sums["total_loss"] + out[0] * (b - a)                   # test.py:67-70
         sums["nll_loss"] = sums["nll_loss"] + out[1] * (b - a)
         sums["c_loss"] = sums["c_loss"] + out[3] * (b - a)
-    local = torch.cat(probs, 0) if probs else feats.new_empty((0, labels.shape[1]))
+    width = labels.shape[1] if labels is not None else model.r_sqrt_sigma.shape[0]
+    if labels is None:
+        sums = None
+    local = torch.cat(probs, 0) if probs else feats.new_empty((0, width))
     if was_training:
         model.train()
     if world == 1 or not gather:

@@ -25,7 +25,7 @@ import torch.nn.functional as F
 
 from . import _lib
 from .dense import linear
-from .probit import ProbitELBO, philox_normal
+from .probit import ProbitELBO, philox_normal, probit_predict
 
 _state = {"seed": 0x5EED_B200, "offset": 0}
 
@@ -168,6 +168,28 @@ def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar
     # args.peer_ring (peer.PeerRing, data-parallel runs): g_R comes back already summed over the ranks
     return ProbitELBO.apply(input_label.float(), fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise,
                             float(args.nll_coeff), float(args.c_coeff), flags, spec, getattr(args, "peer_ring", None))
+
+
+def predict(fx_out, r_sqrt_sigma, args, noise=None):
+    """The prediction `indiv_prob` (B, L) of compute_loss in test mode (mpvae.py:170,180,203) from the feature branch
+    alone (`VAE.feat_forward(feature)[0]`): no labels, no label branch, no loss.  Same S (args.n_test_sample), same
+    noise (`noise_plan`: a call without args.noise_offset consumes one offset, as compute_loss does), same flags, and
+    bit for bit the indiv_prob compute_loss returns for the same fx_out.  Inference only: it builds no autograd graph."""
+    if torch.is_grad_enabled() and (fx_out.requires_grad or r_sqrt_sigma.requires_grad):
+        raise RuntimeError("mpvae_b200.predict is inference only and returns no gradient: call it under torch.no_grad() "
+                           "(or detach its inputs); compute_loss is the differentiable path")
+    device = fx_out.device
+    if device.type != "cuda":
+        raise RuntimeError("mpvae_b200.predict needs CUDA tensors: the probit prediction is implemented as sm_100a "
+                           "kernels only (no CPU fallback)")
+    n_sample = args.n_test_sample
+    n_batch = fx_out.shape[0]
+    if n_batch == 0:
+        return fx_out.new_empty((0, fx_out.shape[1]))
+    r32 = r_sqrt_sigma.to(device).float()
+    noise, spec = noise_plan(args, n_sample, n_batch, device, noise)
+    flags = int(getattr(args, "mpvae_flags", 0))
+    return probit_predict(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags)
 
 
 probit_elbo = compute_loss

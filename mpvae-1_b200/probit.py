@@ -21,10 +21,9 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
-def _check_inputs(y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise, noise_spec):
-    tensors = (y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise)
-    dev = y.device
-    for name, t in zip(_NAMES, tensors):
+def _check_tensors(names, tensors):
+    dev = tensors[0].device
+    for name, t in zip(names, tensors):
         if t is None:
             continue
         if not t.is_cuda:
@@ -34,6 +33,10 @@ def _check_inputs(y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, no
             raise RuntimeError(f"mpvae_b200: {name} is on {t.device}, expected {dev}")
         if t.dtype != torch.float32:
             raise TypeError(f"mpvae_b200: {name} must be float32, got {t.dtype}")
+
+
+def _check_inputs(y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise, noise_spec):
+    _check_tensors(_NAMES, (y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise))
     B, L = fe_out.shape
     D = fe_mu.shape[1]
     if noise is not None:
@@ -181,6 +184,50 @@ class ProbitELBO(torch.autograd.Function):
         #       y     fe_out    fe_mu      fe_logvar  fx_out    fx_mu      fx_logvar  r32  noise nll_c c_c flags spec
         return (None, g_fe_out, g_mulv[0], g_mulv[1], g_fx_out, g_mulv[2], g_mulv[3], g_r, None, None, None, None, None,
                 None)
+
+
+def probit_predict(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0):
+    """indiv_prob (B, L) = mean over S samples of clamp(Phi(fx_out + noise.R^T)) (mpvae.py:170,180,203): the prediction
+    of the feature branch, without labels and without the loss.  Bit-equal to `ProbitELBO`'s indiv_prob on the same
+    fx_out, R and noise.  `noise` / `noise_spec` as for `ProbitELBO`; inference only (no autograd graph)."""
+    if noise is None and noise_spec is None:
+        raise ValueError("probit_predict needs either a noise tensor or a noise_spec")
+    if fx_out.dim() != 2:
+        raise ValueError(f"fx_out must be (batch, label_dim), got {tuple(fx_out.shape)}")
+    B, L = fx_out.shape
+    S = int(S)
+    if S < 1:
+        raise ValueError(f"n_sample must be positive, got {S}")
+    if r32.dim() != 2 or r32.shape[0] != L:
+        raise ValueError(f"r_sqrt_sigma has shape {tuple(r32.shape)}, expected ({L}, z_dim)")
+    Z = r32.shape[1]
+    if noise is not None and noise.shape != (S, B, Z):
+        raise ValueError(f"noise has shape {tuple(noise.shape)}, expected {(S, B, Z)} (n_sample, batch, z_dim)")
+    _check_tensors(("fx_out", "r_sqrt_sigma", "noise"), (fx_out, r32, noise))
+    lib = _lib.lib()
+    fx_out, r32 = fx_out.contiguous(), r32.contiguous()
+    if noise is not None:
+        noise = noise.contiguous()
+    dev = fx_out.device
+    with torch.cuda.device(dev):
+        ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 0, flags))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        prob = torch.empty((B, L), dtype=torch.float32, device=dev)
+        if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
+            # test hook: see ProbitELBO.forward
+            ws.fill_(255)
+            prob.fill_(float("nan"))
+        p = _lib.ProbitParams()
+        p.struct_bytes = C.sizeof(_lib.ProbitParams)
+        p.flags = flags
+        p.S, p.B, p.L, p.Z = S, B, L, Z
+        p.fx_out, p.r, p.noise = _ptr(fx_out), _ptr(r32), _ptr(noise)
+        _set_noise_spec(p, noise_spec, B)
+        p.indiv_prob = _ptr(prob)
+        p.workspace, p.workspace_bytes = _ptr(ws), ws_bytes
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(lib.mpvae_probit_predict(C.byref(p), stream), "mpvae_probit_predict")
+    return prob
 
 
 def philox_normal(S, B, Z, *, seed, offset=0, device="cuda", global_batch=None, row0=0):
