@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define MPVAE_ABI_VERSION 12
+#define MPVAE_ABI_VERSION 13
 
 /* flags */
 #define MPVAE_FLAG_SANITIZE_DEGENERATE 0x1u /* rows with n_pos*n_neg == 0 get zero ranking gradient instead of
@@ -234,6 +234,29 @@ enum { MPVAE_M_ACC = 0, MPVAE_M_HA, MPVAE_M_EBF1, MPVAE_M_MIF1, MPVAE_M_MAF1, MP
 uint64_t mpvae_batch_metrics_workspace(int32_t B, int32_t L);
 int mpvae_batch_metrics(const float *indiv_prob, const float *input_label, int32_t B, int32_t L, float threshold,
                         double *out, void *workspace, uint64_t workspace_bytes, void *cuda_stream);
+
+/* Closed-form prediction: the S -> infinity limit of mpvae_probit_predict, and the pairwise label co-occurrence of the
+ * same predictive distribution.  The noise n = R eps enters linearly, so with h_l = fx_out[b, l] * scale_l,
+ * scale_l = 1 / sqrt(1 + sum_z R[l, z]^2) and rho_ij = R_i . R_j * scale_i * scale_j:
+ *   P(y_l = 1)          = c + k Phi(h_l)
+ *   P(y_i = 1, y_j = 1) = c^2 + c k (Phi(h_i) + Phi(h_j)) + k^2 Phi2(h_i, h_j; rho_ij)
+ * where E = c + k Phi is the clamp of mpvae.py:177 (c = eps1 / 2, k = 1 - eps1, eps1 = fp32(1e-6)) and Phi2 the standard
+ * bivariate normal CDF (Genz's BVND, fp64).  r = (L, Z) fp32 R; pairs = (P, 2) int32, 8-byte aligned; scale (L) and rho
+ * (P) are fp64 buffers the caller keeps between calls.  A pair index outside [0, L) yields NaN.
+ *   mpvae_predictive_scale  scale_out[l] = scale_l (fp64 sums over z in a fixed order)
+ *   mpvae_predictive_rho    rho_out[p] = rho of pair p
+ *   mpvae_predict_exact     indiv_prob (B, L) = E(x') with x' = fp32(fx_out * scale) rounded once, through the same
+ *                           probit_E (probit_E_stable under MPVAE_FLAG_STABLE_CDF) as every other entry point
+ *   mpvae_predict_pairs     out (B, P) = P(y_i = 1, y_j = 1) in fp64, rounded once to fp32; a pair (i, i) gives the bits
+ *                           of mpvae_predict_exact's P(y_i = 1) under the same flags
+ * Flags other than MPVAE_FLAG_STABLE_CDF are ignored.  B = 0 or P = 0 launches nothing. */
+int mpvae_predictive_scale(const float *r, int32_t L, int32_t Z, double *scale_out, void *cuda_stream);
+int mpvae_predictive_rho(const float *r, int32_t L, int32_t Z, const double *scale, const int32_t *pairs, int32_t P,
+                         double *rho_out, void *cuda_stream);
+int mpvae_predict_exact(const float *fx_out, int32_t B, int32_t L, const double *scale, uint32_t flags, float *indiv_prob,
+                        void *cuda_stream);
+int mpvae_predict_pairs(const float *fx_out, int32_t B, int32_t L, const double *scale, const int32_t *pairs,
+                        const double *rho, int32_t P, uint32_t flags, float *out, void *cuda_stream);
 
 /* The tail of the training step, train.py:126-128 (clip_grad_norm_(params, max_norm); optimizer.step() with
  * torch.optim.Adam(lr, weight_decay)), over flat device buffers.

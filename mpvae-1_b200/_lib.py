@@ -12,7 +12,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libmpvae_b200.so")
 
-ABI_VERSION = 12
+ABI_VERSION = 13
 FLAG_SANITIZE_DEGENERATE = 0x1
 FLAG_CONTRACT_TENSOR = 0x2
 FLAG_CONTRACT_FMA = 0x4
@@ -32,6 +32,7 @@ EXPORTS = (
     "mpvae_peer_alloc", "mpvae_peer_open", "mpvae_peer_close", "mpvae_peer_free", "mpvae_contract_workspace_bytes", "mpvae_last_error",
     "mpvae_abi_version", "mpvae_launch_count", "mpvae_batch_metrics", "mpvae_batch_metrics_workspace",
     "mpvae_peer_error", "mpvae_profile", "mpvae_profile_read", "mpvae_profile_name", "mpvae_test_log_normal",
+    "mpvae_predictive_scale", "mpvae_predictive_rho", "mpvae_predict_exact", "mpvae_predict_pairs",
 )
 
 _f = C.c_void_p  # device pointer
@@ -100,6 +101,16 @@ def _load():
     lib.mpvae_batch_metrics.restype = C.c_int
     lib.mpvae_batch_metrics.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_void_p, C.c_void_p,
                                         C.c_uint64, C.c_void_p]
+    lib.mpvae_predictive_scale.restype = C.c_int
+    lib.mpvae_predictive_scale.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]
+    lib.mpvae_predictive_rho.restype = C.c_int
+    lib.mpvae_predictive_rho.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                         C.c_void_p]
+    lib.mpvae_predict_exact.restype = C.c_int
+    lib.mpvae_predict_exact.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p]
+    lib.mpvae_predict_pairs.restype = C.c_int
+    lib.mpvae_predict_pairs.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
+                                        C.c_uint32, C.c_void_p, C.c_void_p]
     for fn in (lib.mpvae_contract_nt, lib.mpvae_contract_tn):
         fn.restype = C.c_int
         fn.argtypes = [C.c_void_p] * 3 + [C.c_int32] * 4 + [C.c_void_p, C.c_uint64, C.c_void_p]

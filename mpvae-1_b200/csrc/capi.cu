@@ -683,6 +683,37 @@ int mpvae_batch_metrics(const float* indiv_prob, const float* input_label, int32
     return launch_batch_metrics(indiv_prob, input_label, B, L, threshold, out, workspace, static_cast<cudaStream_t>(cuda_stream));
 }
 
+int mpvae_predictive_scale(const float* r, int32_t L, int32_t Z, double* scale_out, void* cuda_stream) {
+    if (!r || !scale_out) { set_error("predictive_scale: NULL pointer (r/scale_out)"); return 1; }
+    if (L <= 0 || Z <= 0) { set_error("predictive_scale: bad sizes L=%d Z=%d", L, Z); return 1; }
+    return launch_predictive_scale(r, L, Z, scale_out, static_cast<cudaStream_t>(cuda_stream));
+}
+
+int mpvae_predictive_rho(const float* r, int32_t L, int32_t Z, const double* scale, const int32_t* pairs, int32_t P,
+                         double* rho_out, void* cuda_stream) {
+    if (!r || !scale || !pairs || !rho_out) { set_error("predictive_rho: NULL pointer (r/scale/pairs/rho_out)"); return 1; }
+    if (L <= 0 || Z <= 0 || P < 0) { set_error("predictive_rho: bad sizes L=%d Z=%d P=%d", L, Z, P); return 1; }
+    if (reinterpret_cast<uintptr_t>(pairs) & 7u) { set_error("predictive_rho: pairs must be 8-byte aligned"); return 1; }
+    return launch_predictive_rho(r, L, Z, scale, pairs, P, rho_out, static_cast<cudaStream_t>(cuda_stream));
+}
+
+int mpvae_predict_exact(const float* fx_out, int32_t B, int32_t L, const double* scale, uint32_t flags, float* indiv_prob,
+                        void* cuda_stream) {
+    if (!fx_out || !scale || !indiv_prob) { set_error("predict_exact: NULL pointer (fx_out/scale/indiv_prob)"); return 1; }
+    if (B < 0 || L <= 0) { set_error("predict_exact: bad sizes B=%d L=%d", B, L); return 1; }
+    return launch_predict_exact(fx_out, B, L, scale, (flags & MPVAE_FLAG_STABLE_CDF) != 0, indiv_prob,
+                                static_cast<cudaStream_t>(cuda_stream));
+}
+
+int mpvae_predict_pairs(const float* fx_out, int32_t B, int32_t L, const double* scale, const int32_t* pairs,
+                        const double* rho, int32_t P, uint32_t flags, float* out, void* cuda_stream) {
+    if (!fx_out || !scale || !pairs || !rho || !out) { set_error("predict_pairs: NULL pointer (fx_out/scale/pairs/rho/out)"); return 1; }
+    if (B < 0 || L <= 0 || P < 0) { set_error("predict_pairs: bad sizes B=%d L=%d P=%d", B, L, P); return 1; }
+    if (reinterpret_cast<uintptr_t>(pairs) & 7u) { set_error("predict_pairs: pairs must be 8-byte aligned"); return 1; }
+    return launch_predict_pairs(fx_out, B, L, scale, pairs, rho, P, (flags & MPVAE_FLAG_STABLE_CDF) != 0, out,
+                                static_cast<cudaStream_t>(cuda_stream));
+}
+
 uint64_t mpvae_contract_workspace_bytes(int32_t M, int32_t N, int32_t K, int32_t engine) {
     // covers both orientations: nt (M,N,K) and tn (M = reduction, N1 = N, N2 = K)
     size_t a = contract_tn_fma_workspace(M, N, K);

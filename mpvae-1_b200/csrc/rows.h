@@ -91,6 +91,17 @@ int launch_gxs_bound(RowArgs a, const unsigned int* gp_absmax, unsigned int* out
 int launch_predict_rows(RowArgs a, cudaStream_t stream);                           // after the nt product (a.nr)
 int launch_small_predict(RowArgs a, const SmallNoise& n, cudaStream_t stream);     // small regime, one launch
 
+// Closed-form predictive distribution (predictive.cu), the S -> infinity limit of the above: per-label scales
+// 1 / sqrt(1 + |R_l|^2), pair correlations, exact marginals and pair co-occurrence probabilities.  pairs: P int32 pairs
+// (i, j); an index outside [0, L) gives NaN.
+int launch_predictive_scale(const float* r, int L, int Z, double* scale, cudaStream_t stream);
+int launch_predictive_rho(const float* r, int L, int Z, const double* scale, const int* pairs, int P, double* rho,
+                          cudaStream_t stream);
+int launch_predict_exact(const float* fx_out, int B, int L, const double* scale, bool stable, float* out,
+                         cudaStream_t stream);
+int launch_predict_pairs(const float* fx_out, int B, int L, const double* scale, const int* pairs, const double* rho, int P,
+                         bool stable, float* out, cudaStream_t stream);
+
 // CUDA-core contraction (contract_fma.cu)
 //   nt: C[M,N] = A[M,K] . B[N,K]^T
 //   tn: C[N1,N2] = A[M,N1]^T . B[M,N2]   (split over M, partials reduced in a fixed order)

@@ -25,7 +25,9 @@ import torch.nn.functional as F
 
 from . import _lib
 from .dense import linear
-from .probit import ProbitELBO, philox_normal, probit_predict
+from .probit import ProbitELBO, label_pairs, philox_normal, predictive_rho, predictive_scale, probit_predict
+from .probit import predict_exact_from_r
+from .probit import predict_pairs as probit_predict_pairs
 
 _state = {"seed": 0x5EED_B200, "offset": 0}
 
@@ -190,6 +192,66 @@ def predict(fx_out, r_sqrt_sigma, args, noise=None):
     noise, spec = noise_plan(args, n_sample, n_batch, device, noise)
     flags = int(getattr(args, "mpvae_flags", 0))
     return probit_predict(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags)
+
+
+def _inference_only(name, *tensors):
+    if torch.is_grad_enabled() and any(t.requires_grad for t in tensors):
+        raise RuntimeError(f"mpvae_b200.{name} is inference only and returns no gradient: call it under torch.no_grad() "
+                           "(or detach its inputs); compute_loss is the differentiable path")
+
+
+def _cuda_only(name, t):
+    if t.device.type != "cuda":
+        raise RuntimeError(f"mpvae_b200.{name} needs CUDA tensors: the closed-form prediction is implemented as sm_100a "
+                           "kernels only (no CPU fallback)")
+
+
+def predict_exact(fx_out, r_sqrt_sigma, args):
+    """The exact limit as S -> infinity of `predict`'s indiv_prob (B, L): with n = R eps the noise of mpvae.py:162-170,
+        indiv_prob[b, l] = c + k Phi(fx_out[b, l] / sqrt(1 + |R_l|^2))      (E = c + k Phi: the clamp of mpvae.py:177)
+    without samples, noise or product, so it consumes no noise offset and does not depend on args.n_test_sample.  Each
+    call computes the per-label scale from R first (one read of R, fp64 sums) and then one elementwise pass over fx_out.
+    args.mpvae_flags may carry MPVAE_FLAG_STABLE_CDF; other flags do not apply.  Same arguments as `predict`, so it
+    serves as `infer.predict_proba(..., predict_fn=predict_exact)`.
+    fx_out itself is still random: `VAE.feat_forward` samples the latent through `_reparameterize` (randn_like).  Like
+    predict's Monte Carlo, the closed form integrates out the probit noise only.  Inference only."""
+    _inference_only("predict_exact", fx_out, r_sqrt_sigma)
+    _cuda_only("predict_exact", fx_out)
+    if fx_out.shape[0] == 0:
+        return fx_out.new_empty((0, fx_out.shape[1]))
+    r32 = r_sqrt_sigma.to(fx_out.device).float()
+    return predict_exact_from_r(fx_out, r32, int(getattr(args, "mpvae_flags", 0)))
+
+
+def all_pairs(label_dim):
+    """The (L (L - 1) / 2, 2) int64 label pairs (i, j), i < j, in row-major upper-triangle order."""
+    return torch.triu_indices(label_dim, label_dim, 1).T.contiguous()
+
+
+class PairPredictor:
+    """P(y_i = 1, y_j = 1 | x) for a fixed list of label pairs: the pairwise co-occurrence of the probit predictive
+    distribution in closed form,
+        c^2 + c k (Phi(h_i) + Phi(h_j)) + k^2 Phi2(h_i, h_j; rho_ij),   h = fx_out / sqrt(1 + |R_l|^2),
+        rho_ij = R_i . R_j / sqrt((1 + |R_i|^2)(1 + |R_j|^2))
+    (Phi2: the bivariate normal CDF).  The scale and rho (P * Z fp64 FMAs) are prepared once here, from R as it is now;
+    a call with fx_out (B, L) returns (B, P) in one launch.  A pair (i, i) returns predict_exact's P(y_i = 1) bit for bit.
+    As for predict_exact, only the probit noise is integrated out; fx_out stays random through feat_forward.
+    Inference only; build a new one after R changes."""
+
+    def __init__(self, r_sqrt_sigma, pairs, args):
+        _inference_only("PairPredictor", r_sqrt_sigma)
+        r32 = r_sqrt_sigma.float()
+        self.label_dim = r32.shape[0]
+        self.pairs = label_pairs(pairs, self.label_dim, r32.device)
+        _cuda_only("PairPredictor", r32)
+        self.flags = int(getattr(args, "mpvae_flags", 0))
+        self.scale = predictive_scale(r32)
+        self.rho = predictive_rho(r32, self.scale, self.pairs)
+
+    def __call__(self, fx_out):
+        _inference_only("PairPredictor", fx_out)
+        _cuda_only("PairPredictor", fx_out)
+        return probit_predict_pairs(fx_out, self.scale, self.pairs, self.rho, self.flags)
 
 
 probit_elbo = compute_loss

@@ -230,6 +230,156 @@ def probit_predict(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0):
     return prob
 
 
+# ---- closed-form prediction (csrc/predictive.cu): the S -> infinity limit of probit_predict ----
+
+def _stream(dev):
+    return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+
+
+def _check_f64(name, t, n, dev):
+    if not t.is_cuda or t.device != dev:
+        raise RuntimeError(f"mpvae_b200: {name} is on {t.device}, expected {dev} (CUDA only, no CPU fallback)")
+    if t.dtype != torch.float64 or t.shape != (n,):
+        raise TypeError(f"mpvae_b200: {name} must be a float64 ({n},) tensor, got {t.dtype} {tuple(t.shape)}")
+
+
+def label_pairs(pairs, L, device=None):
+    """(P, 2) label index pairs as the contiguous int32 tensor the kernels read, on `device`.  Indices are checked
+    against [0, L) here on the host (ValueError); the kernels still return NaN for a pair outside it."""
+    p = torch.as_tensor(pairs)
+    if p.dim() != 2 or p.shape[1] != 2:
+        raise ValueError(f"pairs must be (P, 2), got {tuple(p.shape)}")
+    if p.dtype.is_floating_point or p.dtype.is_complex or p.dtype == torch.bool:
+        raise TypeError(f"pairs must be integers, got {p.dtype}")
+    if p.shape[0] > 0:
+        lo, hi = int(p.min()), int(p.max())
+        if lo < 0 or hi >= L:
+            raise ValueError(f"pairs hold label indices in [{lo}, {hi}], outside [0, {L})")
+    if p.shape[0] >= 2 ** 31:
+        raise ValueError(f"{p.shape[0]} pairs do not fit int32")
+    return p.to(device=device if device is not None else p.device, dtype=torch.int32).contiguous()
+
+
+def predictive_scale(r32):
+    """(L,) fp64 scale_l = 1 / sqrt(1 + sum_z R[l, z]^2) of the fp32 R (mpvae_predictive_scale)."""
+    if r32.dim() != 2:
+        raise ValueError(f"r_sqrt_sigma must be (label_dim, z_dim), got {tuple(r32.shape)}")
+    _check_tensors(("r_sqrt_sigma",), (r32,))
+    r32 = r32.contiguous()
+    L, Z = r32.shape
+    dev = r32.device
+    scale = torch.empty(L, dtype=torch.float64, device=dev)
+    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
+        scale.fill_(float("nan"))
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().mpvae_predictive_scale(_ptr(r32), L, Z, _ptr(scale), _stream(dev)), "mpvae_predictive_scale")
+    return scale
+
+
+def predictive_rho(r32, scale, pairs):
+    """(P,) fp64 correlation R_i . R_j * scale_i * scale_j of each (i, j) label pair of the probit predictive
+    distribution (mpvae_predictive_rho): P * Z fp64 FMAs, so compute it once per R and pair list."""
+    if r32.dim() != 2:
+        raise ValueError(f"r_sqrt_sigma must be (label_dim, z_dim), got {tuple(r32.shape)}")
+    L, Z = r32.shape
+    pairs = label_pairs(pairs, L, r32.device)
+    _check_tensors(("r_sqrt_sigma",), (r32,))
+    dev = r32.device
+    _check_f64("scale", scale, L, dev)
+    r32 = r32.contiguous()
+    P = pairs.shape[0]
+    rho = torch.empty(P, dtype=torch.float64, device=dev)
+    if P == 0:
+        return rho
+    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
+        rho.fill_(float("nan"))
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().mpvae_predictive_rho(_ptr(r32), L, Z, _ptr(scale), _ptr(pairs), P, _ptr(rho), _stream(dev)),
+                   "mpvae_predictive_rho")
+    return rho
+
+
+def predict_exact(fx_out, scale, flags=0):
+    """(B, L) fp32 P(y = 1) = E(x'), x' = fp32(fx_out * scale) (mpvae_predict_exact): the S -> infinity limit of
+    probit_predict's indiv_prob for the R that `scale` came from.  Only MPVAE_FLAG_STABLE_CDF in `flags` matters."""
+    if fx_out.dim() != 2:
+        raise ValueError(f"fx_out must be (batch, label_dim), got {tuple(fx_out.shape)}")
+    B, L = fx_out.shape
+    _check_tensors(("fx_out",), (fx_out,))
+    dev = fx_out.device
+    _check_f64("scale", scale, L, dev)
+    fx_out = fx_out.contiguous()
+    prob = torch.empty((B, L), dtype=torch.float32, device=dev)
+    if B == 0:
+        return prob
+    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
+        prob.fill_(float("nan"))
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().mpvae_predict_exact(_ptr(fx_out), B, L, _ptr(scale), int(flags), _ptr(prob), _stream(dev)),
+                   "mpvae_predict_exact")
+    return prob
+
+
+def predict_exact_from_r(fx_out, r32, flags=0):
+    """predictive_scale(r32) then predict_exact(fx_out, scale, flags) in one host pass: one check, one stream lookup and
+    no device switch when fx_out's device is current.  Small batches are bound by the host's time per call, and this is
+    what mpvae.predict_exact runs on every batch."""
+    if fx_out.dim() != 2:
+        raise ValueError(f"fx_out must be (batch, label_dim), got {tuple(fx_out.shape)}")
+    B, L = fx_out.shape
+    if r32.dim() != 2 or r32.shape[0] != L:
+        raise ValueError(f"r_sqrt_sigma has shape {tuple(r32.shape)}, expected ({L}, z_dim)")
+    _check_tensors(("fx_out", "r_sqrt_sigma"), (fx_out, r32))
+    fx_out, r32 = fx_out.contiguous(), r32.contiguous()
+    dev = fx_out.device
+    scale = fx_out.new_empty(L, dtype=torch.float64)
+    prob = fx_out.new_empty((B, L))
+    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
+        scale.fill_(float("nan"))
+        prob.fill_(float("nan"))
+    lib = _lib.lib()
+
+    def launch():
+        # the raw handle of the current stream, without building a torch.cuda.Stream object on every batch
+        stream = C.c_void_p(torch._C._cuda_getCurrentRawStream(dev.index))
+        _lib.check(lib.mpvae_predictive_scale(_ptr(r32), L, r32.shape[1], _ptr(scale), stream), "mpvae_predictive_scale")
+        if B:
+            _lib.check(lib.mpvae_predict_exact(_ptr(fx_out), B, L, _ptr(scale), int(flags), _ptr(prob), stream),
+                       "mpvae_predict_exact")
+
+    if dev.index == torch.cuda.current_device():
+        launch()
+    else:
+        with torch.cuda.device(dev):
+            launch()
+    return prob
+
+
+def predict_pairs(fx_out, scale, pairs, rho, flags=0):
+    """(B, P) fp32 P(y_i = 1, y_j = 1) of each label pair (mpvae_predict_pairs), `rho` from predictive_rho for the same
+    pairs.  A pair (i, i) returns predict_exact's P(y_i = 1) bit for bit under the same flags.  The range check of
+    `pairs` reads them on the host (a device synchronisation when they live on the GPU)."""
+    if fx_out.dim() != 2:
+        raise ValueError(f"fx_out must be (batch, label_dim), got {tuple(fx_out.shape)}")
+    B, L = fx_out.shape
+    pairs = label_pairs(pairs, L, fx_out.device)
+    P = pairs.shape[0]
+    _check_tensors(("fx_out",), (fx_out,))
+    dev = fx_out.device
+    _check_f64("scale", scale, L, dev)
+    _check_f64("rho", rho, P, dev)
+    fx_out = fx_out.contiguous()
+    out = torch.empty((B, P), dtype=torch.float32, device=dev)
+    if B == 0 or P == 0:
+        return out
+    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
+        out.fill_(float("nan"))
+    with torch.cuda.device(dev):
+        _lib.check(_lib.lib().mpvae_predict_pairs(_ptr(fx_out), B, L, _ptr(scale), _ptr(pairs), _ptr(rho), P, int(flags),
+                                                  _ptr(out), _stream(dev)), "mpvae_predict_pairs")
+    return out
+
+
 def philox_normal(S, B, Z, *, seed, offset=0, device="cuda", global_batch=None, row0=0):
     """Standard-normal (S, B, Z) noise from the library's counter-based generator (mpvae.py:162 stand-in).
     Rows [row0, row0+B) of a `global_batch`-row draw: independent of how the batch is sharded."""
