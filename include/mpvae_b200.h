@@ -178,6 +178,24 @@ int mpvae_probit_forward(const mpvae_probit_params *p, void *cuda_stream);
  * the bits of its indiv_prob for the same fx_out, R and noise. */
 int mpvae_probit_predict(const mpvae_probit_params *p, void *cuda_stream);
 
+/* Conditional prediction: P(y_l = 1 | the row's observed labels, x), by importance-weighting the S samples that
+ * mpvae_probit_predict draws.  observed (B, L) int8: 0 or 1 = the label is observed with that value, any other value
+ * (use -1) = unobserved.  With x = noise.R^T + fx_out and E = the clamped probit of mpvae_probit_predict, per row b:
+ *   lp_s = sum over the observed l of the Bernoulli log-likelihood ll(x_{s,l}, y_l)   (fp64, the loss's order)
+ *   m = max_s fp32(lp_s);  u_s = exp(fp32(lp_s) - m);  se = sum_s (double) u_s;  fse = fp32(se)
+ *   indiv_prob[b, l]  = (sum_s u_s E_{s,l}) / fse for an unobserved l, in fp32 with predict's pair order;
+ *                       observed[b, l] (exactly 0.0 or 1.0) for an observed l
+ *   log_evidence[b]   = log(fse / S) + m, the Monte Carlo estimate of log P(y_O | x)
+ *   ess[b]            = se^2 / sum_s (double) u_s^2, the effective sample size of the weights, in [1, S]
+ * With nothing observed indiv_prob is mpvae_probit_predict's bit for bit (log_evidence = 0, ess = S); with every label
+ * observed -log_evidence is the row's nll_loss_x of mpvae_probit_forward on the same fx_out, R and noise (except under
+ * MPVAE_FLAG_FUSED_FORWARD there).  Reads what mpvae_probit_predict reads plus observed; writes indiv_prob, log_evidence
+ * (B) and ess (B), all required.  STABLE_CDF, CONTRACT_FMA, CONTRACT_TENSOR and SEPARATE_NOISE apply as for
+ * mpvae_probit_predict; the other flags are ignored.  Same workspace size as mpvae_probit_predict.  Many observed labels
+ * make the weights degenerate (ess -> 1): the estimate is then carried by few samples. */
+int mpvae_probit_predict_conditional(const mpvae_probit_params *p, const int8_t *observed, float *log_evidence,
+                                     float *ess, void *cuda_stream);
+
 /* Backward: the autograd backward of compute_loss (implicit in the reference, train.py:125),
  * closed form in SURVEY.md 8(a-12).  Must follow a forward on the same workspace. */
 int mpvae_probit_backward(const mpvae_probit_params *p, void *cuda_stream);

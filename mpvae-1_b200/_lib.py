@@ -33,6 +33,7 @@ EXPORTS = (
     "mpvae_abi_version", "mpvae_launch_count", "mpvae_batch_metrics", "mpvae_batch_metrics_workspace",
     "mpvae_peer_error", "mpvae_profile", "mpvae_profile_read", "mpvae_profile_name", "mpvae_test_log_normal",
     "mpvae_predictive_scale", "mpvae_predictive_rho", "mpvae_predict_exact", "mpvae_predict_pairs",
+    "mpvae_probit_predict_conditional",
 )
 
 _f = C.c_void_p  # device pointer
@@ -78,7 +79,7 @@ def _load():
     lib = C.CDLL(LIB_PATH)
     missing = [s for s in EXPORTS if not hasattr(lib, s)]
     if missing:
-        raise LibraryMissing(f"{LIB_PATH} lacks symbols {missing}")
+        raise LibraryMissing(f"{LIB_PATH} lacks symbols {missing}; rebuild")
     lib.mpvae_abi_version.restype = C.c_int
     if lib.mpvae_abi_version() != ABI_VERSION:
         raise LibraryMissing(f"ABI mismatch: library {lib.mpvae_abi_version()} vs binding {ABI_VERSION}; rebuild")
@@ -90,6 +91,8 @@ def _load():
     lib.mpvae_probit_forward.argtypes = [C.POINTER(ProbitParams), C.c_void_p]
     lib.mpvae_probit_predict.restype = C.c_int
     lib.mpvae_probit_predict.argtypes = [C.POINTER(ProbitParams), C.c_void_p]
+    lib.mpvae_probit_predict_conditional.restype = C.c_int
+    lib.mpvae_probit_predict_conditional.argtypes = [C.POINTER(ProbitParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.mpvae_probit_backward.restype = C.c_int
     lib.mpvae_probit_backward.argtypes = [C.POINTER(ProbitParams), C.c_void_p]
     lib.mpvae_philox_normal.restype = C.c_int

@@ -504,6 +504,32 @@ int mpvae_probit_predict(const mpvae_probit_params* p_in, void* cuda_stream) {
     return launch_predict_rows(a, stream);
 }
 
+int mpvae_probit_predict_conditional(const mpvae_probit_params* p_in, const int8_t* observed, float* log_evidence,
+                                     float* ess, void* cuda_stream) {
+    mpvae_probit_params tmp;
+    const mpvae_probit_params* p = normalize(p_in, &tmp);
+    if (!p) return 1;
+    if (int rc = validate_predict(p)) return rc;
+    if (!observed || !log_evidence || !ess) { set_error("NULL pointer (observed/log_evidence/ess)"); return 1; }
+    cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
+    const Workspace w = carve(p->S, p->B, p->L, p->Z, false, p->flags);
+    const RowArgs a = row_args(p, w);
+    FusePart* part = reinterpret_cast<FusePart*>(static_cast<char*>(p->workspace) + w.fuse_part);
+    int rc;
+    // predict's product; the CUDA-core product also where predict takes the one-launch small kernel, which never
+    // materialises nr (its forward outputs equal the CUDA-core path's bit for bit)
+    if (use_tensor(p->flags, p->S, p->B, p->L, p->Z)) {
+        uint32_t* slots = reinterpret_cast<uint32_t*>(static_cast<char*>(p->workspace) + w.slots);
+        const cudaError_t e = cudaMemsetAsync(slots, 0, w.slots_bytes, stream);
+        if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
+        if ((rc = dense_nt_product(p, w, nullptr, stream))) return rc;
+    } else if ((rc = fma_nt_product(p, w, stream))) {
+        return rc;
+    }
+    ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
+    return launch_conditional_rows(a, observed, part, log_evidence, ess, stream);
+}
+
 int mpvae_probit_backward(const mpvae_probit_params* p_in, void* cuda_stream) {
     mpvae_probit_params tmp;
     const mpvae_probit_params* p = normalize(p_in, &tmp);

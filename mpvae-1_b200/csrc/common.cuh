@@ -1,6 +1,7 @@
 // Shared host/device helpers for the mpvae_b200 CUDA library (error slot, launch counter, warp reductions).
 #pragma once
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdarg.h>
@@ -58,6 +59,26 @@ __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
     return v;
+}
+
+// Log-mean-exp over the S per-sample log-likelihoods of one row (mpvae.py:188-190), by one whole warp in a fixed order:
+//   m = max_s fp32(lp_s);  se = sum_s (double) exp(fp32(lp_s) - m)  (lane-strided, then the butterfly);  fse = fp32(se)
+//   nll = -log(fse / S) - m    (the row's negative log-likelihood; -nll is the log of the Monte Carlo mean of exp(lp))
+// lp(s) returns fp32(lp_s).  The per-row tail of the loss and the conditional prediction both call this, so the two
+// share every bit of it.
+struct LogMeanExp { float m; double se; float fse, nll; };
+template <typename LP>
+__device__ __forceinline__ LogMeanExp warp_log_mean_exp(int S, int lane, LP lp) {
+    LogMeanExp r;
+    float m = -INFINITY;
+    for (int s = lane; s < S; s += 32) m = fmaxf(m, lp(s));
+    r.m = warp_max(m);
+    double se = 0.0;
+    for (int s = lane; s < S; s += 32) se += (double)expf(lp(s) - r.m);
+    r.se = warp_sum(se);
+    r.fse = (float)r.se;
+    r.nll = -logf(r.fse / (float)S) - r.m;
+    return r;
 }
 #endif
 

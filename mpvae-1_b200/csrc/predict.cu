@@ -14,17 +14,6 @@ namespace mpv {
 
 namespace {
 
-// the clamped probability of cell_forward, without the rest of the cell
-template <bool STABLE>
-__device__ __forceinline__ float predict_E(float x) {
-    if (STABLE) {
-        float E, om;
-        probit_E_stable(x, E, om);
-        return E;
-    }
-    return probit_E(x);
-}
-
 constexpr int kThreads = 256;
 constexpr int kWarps = kThreads / 32;
 constexpr int kChunk = 128;   // labels per warp and iteration: four per lane, one 16-byte load per sample row

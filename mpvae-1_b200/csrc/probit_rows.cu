@@ -79,7 +79,6 @@ __device__ __forceinline__ void row_tail(const RowArgs& a, int b) {
     __shared__ int s_last;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int S = a.S, B = a.B;
-    const float fS = (float)S;
     const BlockCounts cnt = count_labels<NT>(a.y + (size_t)b * a.L, a.L, s_cnt);   // contains a __syncthreads()
     {
         double kp = 0.0;
@@ -95,14 +94,10 @@ __device__ __forceinline__ void row_tail(const RowArgs& a, int b) {
         double outv[5];
 #pragma unroll
         for (int q = 0; q < 2; ++q) {
-            float m = -INFINITY;
-            for (int s = lane; s < S; s += 32) m = fmaxf(m, (float)a.lp[((size_t)b * S + s) * 2 + q]);
-            m = warp_max(m);
-            double se = 0.0;
-            for (int s = lane; s < S; s += 32) se += (double)expf((float)a.lp[((size_t)b * S + s) * 2 + q] - m);
-            se = warp_sum(se);
-            const float fse = (float)se;
-            outv[q] = (double)(-logf(fse / fS) - m);
+            const LogMeanExp lme =
+                warp_log_mean_exp(S, lane, [&](int s) { return (float)a.lp[((size_t)b * S + s) * 2 + q]; });
+            const float m = lme.m, fse = lme.fse;
+            outv[q] = (double)lme.nll;
             double cs = 0.0;
             for (int s = lane; s < S; s += 32) {
                 const size_t o = (size_t)b * S + s;

@@ -100,3 +100,21 @@ def predict_pairs(model, feats: torch.Tensor, pairs, args, batch_size: Optional[
     width = torch.as_tensor(pairs).shape[0]
     return _score_rows(model, feats, args, batch_size, gather, group, width,
                        lambda a, b, _: predictor(model.feat_forward(feats[a:b])[0]))
+
+
+@torch.no_grad()
+def predict_conditional(model, feats: torch.Tensor, observed: torch.Tensor, args, batch_size: Optional[int] = None,
+                        gather: bool = True, group=None):
+    """(prob (N, L), log_evidence (N,), ess (N,)): `mpvae.predict_conditional` for each row of `feats` given that row's
+    known labels.  `observed` is the int8 (N, L) device tensor of states for ALL N rows (0 / 1 observed, -1 unobserved),
+    sliced per batch as predict_proba slices labels.  Same row sharding, batching, global-row noise keys and gather as
+    predict_proba; with nothing observed, prob is predict_proba(labels=None)'s under the same torch seed."""
+    from . import mpvae
+    L = model.r_sqrt_sigma.shape[0]
+
+    def score(a, b, args):
+        res = mpvae.predict_conditional(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, observed[a:b], args)
+        return torch.cat([res.prob, res.log_evidence[:, None], res.ess[:, None]], 1)
+
+    out = _score_rows(model, feats, args, batch_size, gather, group, L + 2, score)
+    return out[:, :L].contiguous(), out[:, L].contiguous(), out[:, L + 1].contiguous()

@@ -17,6 +17,7 @@ Noise (reference mpvae.py:162) -- `args.noise_mode` (optional attribute, default
 from __future__ import annotations
 
 import math
+from collections import namedtuple
 
 import numpy as np
 import torch
@@ -26,7 +27,7 @@ import torch.nn.functional as F
 from . import _lib
 from .dense import linear
 from .probit import ProbitELBO, label_pairs, philox_normal, predictive_rho, predictive_scale, probit_predict
-from .probit import predict_exact_from_r
+from .probit import predict_exact_from_r, probit_predict_conditional
 from .probit import predict_pairs as probit_predict_pairs
 
 _state = {"seed": 0x5EED_B200, "offset": 0}
@@ -192,6 +193,50 @@ def predict(fx_out, r_sqrt_sigma, args, noise=None):
     noise, spec = noise_plan(args, n_sample, n_batch, device, noise)
     flags = int(getattr(args, "mpvae_flags", 0))
     return probit_predict(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags)
+
+
+ConditionalPrediction = namedtuple("ConditionalPrediction", ["prob", "log_evidence", "ess"])
+
+
+def predict_conditional(fx_out, r_sqrt_sigma, observed, args, noise=None):
+    """P(y_l = 1 | the row's observed labels, x) for the labels a row does not have, given the ones it has.
+
+    The probit model's residual label correlation I + R R^T makes the labels of a row dependent; this conditions on
+    the known ones.  Each of `predict`'s S samples (args.n_test_sample, the same noise: `noise_plan`, so a call without
+    args.noise_offset consumes one offset, and with the same offset it uses predict's noise) is weighted by the
+    likelihood of the observed labels, u_s = prod_o E_o^y_o (1 - E_o)^(1 - y_o), and the unobserved cells take the
+    weighted mean of E instead of the plain mean.  Returns ConditionalPrediction(prob, log_evidence, ess):
+      prob          (B, L) fp32: the conditional probability of each unobserved label; observed cells hold their value
+      log_evidence  (B,): the Monte Carlo estimate of log P(observed labels | x); 0 with nothing observed, and with
+                    everything observed the row's nll_loss_x of compute_loss, negated
+      ess           (B,): the effective sample size of the weights, in [1, S].  It drops towards 1 as more labels are
+                    observed; a small ess means few samples carry the estimate.
+    With nothing observed, prob is predict's indiv_prob bit for bit.
+
+    `observed` is an int8 (B, L) tensor on fx_out's device: 0 or 1 = observed with that value, any other value (use -1)
+    = unobserved.  From labels y and a boolean mask of the known ones:
+        observed = torch.where(mask, y.to(torch.int8), -1)
+    Its values are not checked (no host synchronisation).  Inference only, CUDA only; args.mpvae_flags as for predict."""
+    _inference_only("predict_conditional", fx_out, r_sqrt_sigma)
+    device = fx_out.device
+    if device.type != "cuda":
+        raise RuntimeError("mpvae_b200.predict_conditional needs CUDA tensors: the conditional prediction is implemented "
+                           "as sm_100a kernels only (no CPU fallback)")
+    if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
+        raise TypeError(f"observed must be an int8 tensor, got {getattr(observed, 'dtype', type(observed))}")
+    if observed.shape != fx_out.shape:
+        raise ValueError(f"observed has shape {tuple(observed.shape)}, expected {tuple(fx_out.shape)} (batch, label_dim)")
+    if observed.device != device:
+        raise ValueError(f"observed is on {observed.device}, expected {device}")
+    n_batch = fx_out.shape[0]
+    if n_batch == 0:
+        return ConditionalPrediction(fx_out.new_empty((0, fx_out.shape[1])), fx_out.new_empty(0), fx_out.new_empty(0))
+    n_sample = args.n_test_sample
+    r32 = r_sqrt_sigma.to(device).float()
+    noise, spec = noise_plan(args, n_sample, n_batch, device, noise)
+    flags = int(getattr(args, "mpvae_flags", 0))
+    return ConditionalPrediction(*probit_predict_conditional(fx_out, r32, observed, n_sample, noise=noise, noise_spec=spec,
+                                                             flags=flags))
 
 
 def _inference_only(name, *tensors):

@@ -186,12 +186,10 @@ class ProbitELBO(torch.autograd.Function):
                 None)
 
 
-def probit_predict(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0):
-    """indiv_prob (B, L) = mean over S samples of clamp(Phi(fx_out + noise.R^T)) (mpvae.py:170,180,203): the prediction
-    of the feature branch, without labels and without the loss.  Bit-equal to `ProbitELBO`'s indiv_prob on the same
-    fx_out, R and noise.  `noise` / `noise_spec` as for `ProbitELBO`; inference only (no autograd graph)."""
+def _predict_inputs(name, fx_out, r32, S, noise, noise_spec):
+    """The checks of mpvae_probit_predict's inputs: (fx_out, r32, noise) contiguous, and (S, B, L, Z)."""
     if noise is None and noise_spec is None:
-        raise ValueError("probit_predict needs either a noise tensor or a noise_spec")
+        raise ValueError(f"{name} needs either a noise tensor or a noise_spec")
     if fx_out.dim() != 2:
         raise ValueError(f"fx_out must be (batch, label_dim), got {tuple(fx_out.shape)}")
     B, L = fx_out.shape
@@ -204,10 +202,29 @@ def probit_predict(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0):
     if noise is not None and noise.shape != (S, B, Z):
         raise ValueError(f"noise has shape {tuple(noise.shape)}, expected {(S, B, Z)} (n_sample, batch, z_dim)")
     _check_tensors(("fx_out", "r_sqrt_sigma", "noise"), (fx_out, r32, noise))
+    return fx_out.contiguous(), r32.contiguous(), (noise.contiguous() if noise is not None else None), (S, B, L, Z)
+
+
+def _predict_params(fx_out, r32, noise, noise_spec, flags, dims, prob, ws):
+    S, B, L, Z = dims
+    p = _lib.ProbitParams()
+    p.struct_bytes = C.sizeof(_lib.ProbitParams)
+    p.flags = flags
+    p.S, p.B, p.L, p.Z = S, B, L, Z
+    p.fx_out, p.r, p.noise = _ptr(fx_out), _ptr(r32), _ptr(noise)
+    _set_noise_spec(p, noise_spec, B)
+    p.indiv_prob = _ptr(prob)
+    p.workspace, p.workspace_bytes = _ptr(ws), ws.numel()
+    return p
+
+
+def probit_predict(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0):
+    """indiv_prob (B, L) = mean over S samples of clamp(Phi(fx_out + noise.R^T)) (mpvae.py:170,180,203): the prediction
+    of the feature branch, without labels and without the loss.  Bit-equal to `ProbitELBO`'s indiv_prob on the same
+    fx_out, R and noise.  `noise` / `noise_spec` as for `ProbitELBO`; inference only (no autograd graph)."""
+    fx_out, r32, noise, dims = _predict_inputs("probit_predict", fx_out, r32, S, noise, noise_spec)
+    S, B, L, Z = dims
     lib = _lib.lib()
-    fx_out, r32 = fx_out.contiguous(), r32.contiguous()
-    if noise is not None:
-        noise = noise.contiguous()
     dev = fx_out.device
     with torch.cuda.device(dev):
         ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 0, flags))
@@ -217,17 +234,45 @@ def probit_predict(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0):
             # test hook: see ProbitELBO.forward
             ws.fill_(255)
             prob.fill_(float("nan"))
-        p = _lib.ProbitParams()
-        p.struct_bytes = C.sizeof(_lib.ProbitParams)
-        p.flags = flags
-        p.S, p.B, p.L, p.Z = S, B, L, Z
-        p.fx_out, p.r, p.noise = _ptr(fx_out), _ptr(r32), _ptr(noise)
-        _set_noise_spec(p, noise_spec, B)
-        p.indiv_prob = _ptr(prob)
-        p.workspace, p.workspace_bytes = _ptr(ws), ws_bytes
+        p = _predict_params(fx_out, r32, noise, noise_spec, flags, dims, prob, ws)
         stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         _lib.check(lib.mpvae_probit_predict(C.byref(p), stream), "mpvae_probit_predict")
     return prob
+
+
+def probit_predict_conditional(fx_out, r32, observed, S, *, noise=None, noise_spec=None, flags=0):
+    """(prob (B, L), log_evidence (B,), ess (B,)): P(y_l = 1 | the row's observed labels, x) by importance-weighting
+    probit_predict's S samples with the likelihood of the observed labels (mpvae_probit_predict_conditional).
+    `observed` is an int8 (B, L) tensor on fx_out's device: 0 or 1 = observed with that value, any other value =
+    unobserved; it is not read on the host.  Observed cells return their value; with nothing observed prob is
+    probit_predict's bit for bit.  `noise` / `noise_spec` / `flags` as for probit_predict; inference only."""
+    fx_out, r32, noise, dims = _predict_inputs("probit_predict_conditional", fx_out, r32, S, noise, noise_spec)
+    S, B, L, Z = dims
+    if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
+        raise TypeError(f"observed must be an int8 tensor, got {getattr(observed, 'dtype', type(observed))}")
+    if observed.shape != (B, L):
+        raise ValueError(f"observed has shape {tuple(observed.shape)}, expected {(B, L)} (batch, label_dim)")
+    if observed.device != fx_out.device:
+        raise ValueError(f"observed is on {observed.device}, expected {fx_out.device}")
+    observed = observed.contiguous()
+    lib = _lib.lib()
+    dev = fx_out.device
+    with torch.cuda.device(dev):
+        ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 0, flags))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        prob = torch.empty((B, L), dtype=torch.float32, device=dev)
+        log_evidence = torch.empty(B, dtype=torch.float32, device=dev)
+        ess = torch.empty(B, dtype=torch.float32, device=dev)
+        if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
+            # test hook: see ProbitELBO.forward
+            ws.fill_(255)
+            for t in (prob, log_evidence, ess):
+                t.fill_(float("nan"))
+        p = _predict_params(fx_out, r32, noise, noise_spec, flags, dims, prob, ws)
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(lib.mpvae_probit_predict_conditional(C.byref(p), _ptr(observed), _ptr(log_evidence), _ptr(ess), stream),
+                   "mpvae_probit_predict_conditional")
+    return prob, log_evidence, ess
 
 
 # ---- closed-form prediction (csrc/predictive.cu): the S -> infinity limit of probit_predict ----
