@@ -200,6 +200,23 @@ int mpvae_probit_predict_conditional(const mpvae_probit_params *p, const int8_t 
  * closed form in SURVEY.md 8(a-12).  Must follow a forward on the same workspace. */
 int mpvae_probit_backward(const mpvae_probit_params *p, void *cuda_stream);
 
+/* Partially labelled rows: the forward and backward of the ELBO on the likelihood of the OBSERVED labels only.
+ * label_mask (B, L) bytes on the device, nonzero = the label is observed; y is read only where it is.  Per row b with
+ * observed set O_b:
+ *   lp_{s,b} = sum over l in O_b of ll(x_{s,b,l}, y_{b,l})   (both branches; the log-mean-exp and the batch means are
+ *              unchanged: a row with nothing observed has lp = 0 and adds exactly 0 to nll_loss / nll_loss_x)
+ *   ranking  : pos = observed and y == 1, neg = observed and y == 0; n_pos, n_neg count observed cells only
+ *   KL, indiv_prob and indiv_prob_label (every cell) and the means over all B rows are unchanged
+ * Backward: an unobserved cell's logit gradient carries only the cotangent of indiv_prob / indiv_prob_label.  A row whose
+ * observed labels lack a positive or a negative adds 0 to the forward; its OBSERVED cells get NaN in the backward as an
+ * unmasked degenerate row does (zero ranking gradient under MPVAE_FLAG_SANITIZE_DEGENERATE), never its unobserved cells.
+ * A mask of all ones gives the unmasked results bit for bit; label_mask == NULL is the unmasked entry point.  The backward
+ * must receive the forward's mask.  Under MPVAE_FLAG_FUSED_FORWARD a masked forward runs the separate row kernel.  Same
+ * workspace size as the unmasked calls.  With y = the labels and the same mask, observed = where(mask, y, -1) gives
+ * mpvae_probit_predict_conditional's encoding: -log_evidence of a one-row batch is then nll_loss_x. */
+int mpvae_probit_forward_masked(const mpvae_probit_params *p, const uint8_t *label_mask, void *cuda_stream);
+int mpvae_probit_backward_masked(const mpvae_probit_params *p, const uint8_t *label_mask, void *cuda_stream);
+
 /* Counter-based standard-normal noise, replaces torch.normal(0,1,(S,B,Z)) of mpvae.py:162.
  * Element (s, b_global, z) depends only on (seed, offset, s, b_global, z): a rank holding rows
  * [row0, row0+B) of a B_global-row batch draws the same numbers a single GPU would. */

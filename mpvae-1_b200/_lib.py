@@ -33,7 +33,7 @@ EXPORTS = (
     "mpvae_abi_version", "mpvae_launch_count", "mpvae_batch_metrics", "mpvae_batch_metrics_workspace",
     "mpvae_peer_error", "mpvae_profile", "mpvae_profile_read", "mpvae_profile_name", "mpvae_test_log_normal",
     "mpvae_predictive_scale", "mpvae_predictive_rho", "mpvae_predict_exact", "mpvae_predict_pairs",
-    "mpvae_probit_predict_conditional",
+    "mpvae_probit_predict_conditional", "mpvae_probit_forward_masked", "mpvae_probit_backward_masked",
 )
 
 _f = C.c_void_p  # device pointer
@@ -95,6 +95,9 @@ def _load():
     lib.mpvae_probit_predict_conditional.argtypes = [C.POINTER(ProbitParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.mpvae_probit_backward.restype = C.c_int
     lib.mpvae_probit_backward.argtypes = [C.POINTER(ProbitParams), C.c_void_p]
+    for fn in (lib.mpvae_probit_forward_masked, lib.mpvae_probit_backward_masked):
+        fn.restype = C.c_int
+        fn.argtypes = [C.POINTER(ProbitParams), C.c_void_p, C.c_void_p]
     lib.mpvae_philox_normal.restype = C.c_int
     lib.mpvae_philox_normal.argtypes = [C.c_void_p] + [C.c_int32] * 5 + [C.c_uint64, C.c_uint64, C.c_void_p]
     lib.mpvae_contract_workspace_bytes.restype = C.c_uint64

@@ -407,6 +407,10 @@ uint64_t mpvae_workspace_bytes(int32_t S, int32_t B, int32_t L, int32_t Z, int32
 }
 
 int mpvae_probit_forward(const mpvae_probit_params* p_in, void* cuda_stream) {
+    return mpvae_probit_forward_masked(p_in, nullptr, cuda_stream);
+}
+
+int mpvae_probit_forward_masked(const mpvae_probit_params* p_in, const uint8_t* label_mask, void* cuda_stream) {
     mpvae_probit_params tmp;
     const mpvae_probit_params* p = normalize(p_in, &tmp);
     if (!p) return 1;
@@ -422,6 +426,7 @@ int mpvae_probit_forward(const mpvae_probit_params* p_in, void* cuda_stream) {
     if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
     int rc;
     RowArgs a = row_args(p, w);
+    a.mask = label_mask;
     // a scratch block sized for the backward means a training call: the forward keeps E for it (same placement in
     // both layouts: the backward-only buffers follow everything the forward shares)
     const Workspace wb = carve(p->S, p->B, p->L, p->Z, true, p->flags);
@@ -430,7 +435,8 @@ int mpvae_probit_forward(const mpvae_probit_params* p_in, void* cuda_stream) {
         a.E_x = reinterpret_cast<float*>(base + wb.e_x);
     }
     if (use_tensor(p->flags, p->S, p->B, p->L, p->Z)) {
-        const bool fused = use_fused_forward(p->flags, p->S, p->B, p->L, p->Z);
+        // the fused row forward has no mask: a masked call takes the separate row kernel (tested equal to it unmasked)
+        const bool fused = use_fused_forward(p->flags, p->S, p->B, p->L, p->Z) && !label_mask;
         FuseFwd fz{};
         if (fused) {
             fz.S = p->S; fz.B = p->B; fz.L = p->L; fz.ldn = row_pitch(p->L);
@@ -531,6 +537,10 @@ int mpvae_probit_predict_conditional(const mpvae_probit_params* p_in, const int8
 }
 
 int mpvae_probit_backward(const mpvae_probit_params* p_in, void* cuda_stream) {
+    return mpvae_probit_backward_masked(p_in, nullptr, cuda_stream);
+}
+
+int mpvae_probit_backward_masked(const mpvae_probit_params* p_in, const uint8_t* label_mask, void* cuda_stream) {
     mpvae_probit_params tmp;
     const mpvae_probit_params* p = normalize(p_in, &tmp);
     if (!p) return 1;
@@ -541,6 +551,7 @@ int mpvae_probit_backward(const mpvae_probit_params* p_in, void* cuda_stream) {
     uint32_t* slots = reinterpret_cast<uint32_t*>(base + w.slots);
     const bool tensor = use_tensor(p->flags, p->S, p->B, p->L, p->Z);
     RowArgs a = row_args(p, w);
+    a.mask = label_mask;
     a.E_l = reinterpret_cast<float*>(base + w.e_l);
     a.E_x = reinterpret_cast<float*>(base + w.e_x);
     const int M = p->S * p->B;

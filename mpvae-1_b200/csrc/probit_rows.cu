@@ -31,27 +31,33 @@ constexpr int kST = 2;   // samples per inner tile (unrolled)
 
 struct BlockCounts { int npos, nneg; };
 
-// One lane's inputs for one 32-label chunk and kST samples.
-struct RowChunk { float y, fe, fx, nr[kST]; };
+// One lane's inputs for one 32-label chunk and kST samples.  obs: the label is observed (always, unmasked); an
+// unobserved label's y reads as 0.
+struct RowChunk { float y, fe, fx, nr[kST]; bool obs; };
 
+template <bool MASKED>
 __device__ __forceinline__ void load_chunk(RowChunk& in, const RowArgs& a, const float* __restrict__ yrow,
                                            const float* __restrict__ ferow, const float* __restrict__ fxrow, int c, int lane,
                                            int b, int s0) {
     const int l = (c << 5) + lane;
     if (l < a.L) {
-        in.y = yrow[l]; in.fe = ferow[l]; in.fx = fxrow[l];
+        in.obs = !MASKED || a.mask[(size_t)b * a.L + l] != 0;
+        in.y = in.obs ? yrow[l] : 0.0f; in.fe = ferow[l]; in.fx = fxrow[l];
 #pragma unroll
         for (int i = 0; i < kST; ++i)
             in.nr[i] = (s0 + i < a.S) ? a.nr[row_of(a, s0 + i, b) * a.ldn + l] : 0.0f;
     }
 }
 
-template <int NT = kThreads>
-__device__ __forceinline__ BlockCounts count_labels(const float* __restrict__ yrow, int L, int* s_tmp) {
+// n_pos / n_neg of a row; MASKED: over its observed labels only (mrow: the row's mask bytes)
+template <int NT = kThreads, bool MASKED = false>
+__device__ __forceinline__ BlockCounts count_labels(const float* __restrict__ yrow, const uint8_t* __restrict__ mrow, int L,
+                                                    int* s_tmp) {
     constexpr int kWarps = NT / 32;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     int cp = 0, cn = 0;
     for (int l = tid; l < L; l += NT) {
+        if (MASKED && mrow[l] == 0) continue;
         const float v = yrow[l];
         cp += (v == 1.0f);   // torch.eq(labels, ones)   mpvae.py:107
         cn += (v == 0.0f);   // torch.eq(labels, zeros)  mpvae.py:108
@@ -69,8 +75,9 @@ __device__ __forceinline__ BlockCounts count_labels(const float* __restrict__ yr
 // The per-row tail of the forward, shared by every forward kernel: label counts, KL row term (mpvae.py:147-148), per-row
 // log-mean-exp over samples, softmax weights, ranking sums (mpvae.py:188-190,115-122), and -- in the last CTA to
 // arrive -- the batch means and the total (mpvae.py:190,122,147,207-208) in a fixed summation order.  Expects the
-// row's a.lp / a.stat entries to have been written by threads of this CTA (any of them); blockDim.x == NT.
-template <int NT = kThreads>
+// row's a.lp / a.stat entries to have been written by threads of this CTA (any of them); blockDim.x == NT.  MASKED: the
+// label counts run over the observed labels (a.mask); the rest is unchanged.
+template <int NT = kThreads, bool MASKED = false>
 __device__ __forceinline__ void row_tail(const RowArgs& a, int b) {
     constexpr int kWarps = NT / 32;
     __shared__ int s_cnt[2 * kWarps];
@@ -79,7 +86,8 @@ __device__ __forceinline__ void row_tail(const RowArgs& a, int b) {
     __shared__ int s_last;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int S = a.S, B = a.B;
-    const BlockCounts cnt = count_labels<NT>(a.y + (size_t)b * a.L, a.L, s_cnt);   // contains a __syncthreads()
+    const BlockCounts cnt = count_labels<NT, MASKED>(a.y + (size_t)b * a.L, MASKED ? a.mask + (size_t)b * a.L : nullptr,
+                                                     a.L, s_cnt);   // contains a __syncthreads()
     {
         double kp = 0.0;
         const size_t o = (size_t)b * a.D;
@@ -148,6 +156,7 @@ __device__ __forceinline__ void row_tail(const RowArgs& a, int b) {
 
 // Second half of the tiled forward: adds the per-(sample-row, chunk) partials the cell kernel (or the product kernel's
 // math warps, fused_rows.cuh) left, in a fixed order, and runs the per-row tail.  One CTA per batch row.
+template <bool MASKED>
 __global__ void __launch_bounds__(kThreads, 4)
 probit_row_finalize_kernel(const RowArgs a) {
     const int b = blockIdx.x;
@@ -170,7 +179,7 @@ probit_row_finalize_kernel(const RowArgs a) {
             reinterpret_cast<float4*>(a.stat)[o] = make_float4(q0, q1, q2, q3);
         }
     }
-    row_tail(a, b);
+    row_tail<kThreads, MASKED>(a, b);
 }
 
 // Cell work of the forward, tiled (b, 128-label chunk): a warp owns 128 neighbouring labels of one batch row (a lane:
@@ -182,7 +191,10 @@ probit_row_finalize_kernel(const RowArgs a) {
 constexpr int kChunk = 128;   // labels per warp and iteration
 constexpr int kLL = 4;        // labels per lane
 
-template <bool STABLE, int MINB>
+// MASKED: an unobserved cell (a.mask[b, l] == 0) reads y as 0 and adds nothing to the log-likelihood or the ranking sums;
+// its E still enters the predictions and the saved E_l / E_x.  The mask bytes are byte loads (b * L need not be a
+// multiple of 4).
+template <bool STABLE, int MINB, bool MASKED>
 __global__ void __launch_bounds__(kThreads, MINB)
 probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nchunks) {
     const int b = blockIdx.x;
@@ -193,10 +205,15 @@ probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nc
     for (int c = blockIdx.y * kWarps + warp; c < nchunks; c += gridDim.y * kWarps) {
         const int l0 = c * kChunk + kLL * lane;
         float y[kLL], fe[kLL], fx[kLL], accl[kLL], accx[kLL];
+        bool obs[kLL];
 #pragma unroll
         for (int j = 0; j < kLL; ++j) {
             y[j] = fe[j] = fx[j] = accl[j] = accx[j] = 0.f;
             if (l0 + j < L) { y[j] = a.y[yoff + l0 + j]; fe[j] = a.fe_out[yoff + l0 + j]; fx[j] = a.fx_out[yoff + l0 + j]; }
+            if (MASKED) {
+                obs[j] = l0 + j < L && a.mask[yoff + l0 + j] != 0;
+                if (!obs[j]) y[j] = 0.f;
+            }
         }
         // rows are 16-byte aligned (ldn % 4 == 0) and l0 is a multiple of 4: 16-byte accesses whenever the lane starts
         // inside the row; the pitch padding [L, ldn) is loaded but never used as a label
@@ -228,8 +245,10 @@ probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nc
                     if (l0 + j < L) {
                         const CellFwd cl = cell_forward<STABLE>(nv[j] + fe[j], y[j]);   // mpvae.py:168,177
                         const CellFwd cx = cell_forward<STABLE>(nv[j] + fx[j], y[j]);   // mpvae.py:170,180
-                        lpl[i] += (double)cl.ll; lpx[i] += (double)cx.ll;
-                        pn[i][0] += cl.epos; pn[i][1] += cl.eneg; pn[i][2] += cx.epos; pn[i][3] += cx.eneg;
+                        if (!MASKED || obs[j]) {
+                            lpl[i] += (double)cl.ll; lpx[i] += (double)cx.ll;
+                            pn[i][0] += cl.epos; pn[i][1] += cl.eneg; pn[i][2] += cx.epos; pn[i][3] += cx.eneg;
+                        }
                         pl[j] += cl.E; px[j] += cx.E;
                         el[j] = cl.E; ex[j] = cx.E;
                     }
@@ -301,6 +320,11 @@ __device__ __forceinline__ RowCoeffs row_coeffs(const RowArgs& a, int b) {
 // with phi/E <= 4.3 (the clamp E >= eps/2 caps the inverse Mills ratio near x = -4.2; same by symmetry for 1-E),
 // e^{5E} phi <= 16.1 (x ~ 1) and phi <= 0.4.  Constants rounded up: 5, 17, 0.4.  The bound only has to be an upper
 // bound within a few binades: it sets the power-of-two scale of the fp16 planes (common.cuh).
+// MASKED: an unobserved cell's |dL/dx| is |gp| * phi, a term of the bound already.  One change: a row with no observed
+// positive and no observed negative (e.g. nothing observed) puts no ranking term on any cell, so its ranking part of the
+// bound is 0 -- not the 0/0 NaN of its normaliser, which would leave the whole batch's planes unscaled although the
+// row's gradients are finite.
+template <bool MASKED>
 __global__ void __launch_bounds__(256)
 gxs_bound_kernel(const RowArgs a, const unsigned int* __restrict__ gp_absmax, unsigned int* __restrict__ out_bits) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -311,8 +335,10 @@ gxs_bound_kernel(const RowArgs a, const unsigned int* __restrict__ gp_absmax, un
         const float4 st = reinterpret_cast<const float4*>(a.stat)[i];
         const float2 w = reinterpret_cast<const float2*>(a.wts)[i];
         const float gp = gp_absmax ? (__uint_as_float(gp_absmax[0]) + __uint_as_float(gp_absmax[1])) / (float)a.S : 0.0f;
-        const float bl = 5.0f * fabsf(rc.cnb[0] * w.x) + 17.0f * 5.0f * fabsf(rc.kb[0]) * fmaxf(st.x, st.y);
-        const float bx = 5.0f * fabsf(rc.cnb[1] * w.y) + 17.0f * 5.0f * fabsf(rc.kb[1]) * fmaxf(st.z, st.w);
+        float kl = fabsf(rc.kb[0]), kx = fabsf(rc.kb[1]);
+        if (MASKED && a.rowaux[(size_t)b * 2] == 0.0f && a.rowaux[(size_t)b * 2 + 1] == 0.0f) kl = kx = 0.0f;
+        const float bl = 5.0f * fabsf(rc.cnb[0] * w.x) + 17.0f * 5.0f * kl * fmaxf(st.x, st.y);
+        const float bx = 5.0f * fabsf(rc.cnb[1] * w.y) + 17.0f * 5.0f * kx * fmaxf(st.z, st.w);
         bits = __float_as_uint(bl + bx + 0.4f * gp) & 0x7FFFFFFFu;   // NaN (degenerate row) sorts highest
     }
 #pragma unroll
@@ -323,7 +349,9 @@ gxs_bound_kernel(const RowArgs a, const unsigned int* __restrict__ gp_absmax, un
     if ((threadIdx.x & 31) == 0 && bits != 0u) atomicMax(out_bits, bits);
 }
 
-template <bool STABLE>
+// MASKED: an unobserved cell gets the cotangent of indiv_prob / indiv_prob_label alone (its y reads as 0 and its
+// log-likelihood and ranking coefficients as 0)
+template <bool STABLE, bool MASKED>
 __global__ void __launch_bounds__(kThreads, 4)
 probit_row_bwd_kernel(const RowArgs a) {
     extern __shared__ float s_gacc[];   // [nws][2][L] logit-gradient partial sums
@@ -367,9 +395,9 @@ probit_row_bwd_kernel(const RowArgs a) {
         float* __restrict__ gacc = s_gacc + (size_t)ws * 2 * L;
         RowChunk cur, nxt;
         int c = wl;
-        if (c < nchunks) load_chunk(cur, a, yrow, ferow, fxrow, c, lane, b, s0);
+        if (c < nchunks) load_chunk<MASKED>(cur, a, yrow, ferow, fxrow, c, lane, b, s0);
         for (; c < nchunks; c += nwl) {
-            if (c + nwl < nchunks) load_chunk(nxt, a, yrow, ferow, fxrow, c + nwl, lane, b, s0);
+            if (c + nwl < nchunks) load_chunk<MASKED>(nxt, a, yrow, ferow, fxrow, c + nwl, lane, b, s0);
             const int l = (c << 5) + lane;
             if (l < L) {
                 const float gpl = has_gpl ? a.g_indiv_prob_label[(size_t)b * L + l] / fS : 0.0f;
@@ -378,8 +406,14 @@ probit_row_bwd_kernel(const RowArgs a) {
 #pragma unroll
                 for (int i = 0; i < kST; ++i) {
                     if (s0 + i < S) {
-                        const float dl = cell_backward<STABLE>(cur.nr[i] + cur.fe, cur.y, cn[i][0], cp[i][0], cq[i][0], gpl);
-                        const float dx = cell_backward<STABLE>(cur.nr[i] + cur.fx, cur.y, cn[i][1], cp[i][1], cq[i][1], gpx);
+                        float dl, dx;
+                        if (!MASKED || cur.obs) {
+                            dl = cell_backward<STABLE>(cur.nr[i] + cur.fe, cur.y, cn[i][0], cp[i][0], cq[i][0], gpl);
+                            dx = cell_backward<STABLE>(cur.nr[i] + cur.fx, cur.y, cn[i][1], cp[i][1], cq[i][1], gpx);
+                        } else {
+                            dl = cell_backward<STABLE>(cur.nr[i] + cur.fe, 0.0f, 0.0f, 0.0f, 0.0f, gpl);
+                            dx = cell_backward<STABLE>(cur.nr[i] + cur.fx, 0.0f, 0.0f, 0.0f, 0.0f, gpx);
+                        }
                         gl += dl; gx += dx;
                         if (a.gxs_planes) {
                             // operand planes of gxs^T . noise: hi = fp16(g s), lo = fp16(g s - hi)
@@ -442,6 +476,8 @@ probit_row_bwd_kernel(const RowArgs a) {
 // by instruction issue.  A warp owns 64 neighbouring labels of one batch row (a lane: two of them) and walks the S
 // samples with the logit-gradient sums in registers: no shared-memory accumulators, 8-byte loads, 4-byte plane stores.
 // Grid (B, G): the 64-label chunks of a row are dealt out to G CTAs so that small batches still fill the GPU.
+// MASKED: an unobserved cell gets the cotangent of indiv_prob / indiv_prob_label alone (y, cn, cp, cq read as 0).
+template <bool MASKED>
 __global__ void __launch_bounds__(kThreads, 4)
 probit_row_bwd_saved_kernel(const RowArgs a) {
     extern __shared__ float s_coef[];   // [S][6]: cn_l, cn_x, cp_l, cp_x, cq_l, cq_x
@@ -469,8 +505,10 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
         const int l0 = c * 64 + 2 * lane;
         const bool in0 = l0 < L, in1 = l0 + 1 < L;
         float y0 = 0.f, y1 = 0.f, fe0 = 0.f, fe1 = 0.f, fx0 = 0.f, fx1 = 0.f, gpl0 = 0.f, gpl1 = 0.f, gpx0 = 0.f, gpx1 = 0.f;
-        if (in0) { y0 = a.y[yoff + l0]; fe0 = a.fe_out[yoff + l0]; fx0 = a.fx_out[yoff + l0]; }
-        if (in1) { y1 = a.y[yoff + l0 + 1]; fe1 = a.fe_out[yoff + l0 + 1]; fx1 = a.fx_out[yoff + l0 + 1]; }
+        bool ob0 = true, ob1 = true;
+        if (MASKED) { ob0 = in0 && a.mask[yoff + l0] != 0; ob1 = in1 && a.mask[yoff + l0 + 1] != 0; }
+        if (in0) { if (ob0) y0 = a.y[yoff + l0]; fe0 = a.fe_out[yoff + l0]; fx0 = a.fx_out[yoff + l0]; }
+        if (in1) { if (ob1) y1 = a.y[yoff + l0 + 1]; fe1 = a.fe_out[yoff + l0 + 1]; fx1 = a.fx_out[yoff + l0 + 1]; }
         if (has_gpl) { if (in0) gpl0 = a.g_indiv_prob_label[yoff + l0] / fS; if (in1) gpl1 = a.g_indiv_prob_label[yoff + l0 + 1] / fS; }
         if (has_gp) { if (in0) gpx0 = a.g_indiv_prob[yoff + l0] / fS; if (in1) gpx1 = a.g_indiv_prob[yoff + l0 + 1] / fS; }
         float gl0 = 0.f, gl1 = 0.f, gx0 = 0.f, gx1 = 0.f;
@@ -504,13 +542,25 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
                 const Cell3& v = cur[i];
                 float d0 = 0.f, d1 = 0.f;
                 if (in0) {
-                    const float dl = cell_backward_saved(v.n.x + fe0, v.l.x, y0, cf[0], cf[2], cf[4], gpl0);
-                    const float dx = cell_backward_saved(v.n.x + fx0, v.x.x, y0, cf[1], cf[3], cf[5], gpx0);
+                    float dl, dx;
+                    if (ob0) {
+                        dl = cell_backward_saved(v.n.x + fe0, v.l.x, y0, cf[0], cf[2], cf[4], gpl0);
+                        dx = cell_backward_saved(v.n.x + fx0, v.x.x, y0, cf[1], cf[3], cf[5], gpx0);
+                    } else {
+                        dl = cell_backward_saved(v.n.x + fe0, v.l.x, 0.0f, 0.0f, 0.0f, 0.0f, gpl0);
+                        dx = cell_backward_saved(v.n.x + fx0, v.x.x, 0.0f, 0.0f, 0.0f, 0.0f, gpx0);
+                    }
                     gl0 += dl; gx0 += dx; d0 = dl + dx;
                 }
                 if (in1) {
-                    const float dl = cell_backward_saved(v.n.y + fe1, v.l.y, y1, cf[0], cf[2], cf[4], gpl1);
-                    const float dx = cell_backward_saved(v.n.y + fx1, v.x.y, y1, cf[1], cf[3], cf[5], gpx1);
+                    float dl, dx;
+                    if (ob1) {
+                        dl = cell_backward_saved(v.n.y + fe1, v.l.y, y1, cf[0], cf[2], cf[4], gpl1);
+                        dx = cell_backward_saved(v.n.y + fx1, v.x.y, y1, cf[1], cf[3], cf[5], gpx1);
+                    } else {
+                        dl = cell_backward_saved(v.n.y + fe1, v.l.y, 0.0f, 0.0f, 0.0f, 0.0f, gpl1);
+                        dx = cell_backward_saved(v.n.y + fx1, v.x.y, 0.0f, 0.0f, 0.0f, 0.0f, gpx1);
+                    }
                     gl1 += dl; gx1 += dx; d1 = dl + dx;
                 }
                 if (a.gxs_planes) {
@@ -561,7 +611,8 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
 // The backward is one CTA per row as well (cell_backward_saved from the kept E and nr, logit gradients, KL gradients)
 // and leaves the row's contribution to g_R = gxs^T . noise in a scratch slab; a second, tiny kernel adds the slabs over
 // the batch in row order (deterministic).  R staging, the noise draw and the contraction are small_rows.cuh's.
-template <bool STABLE>
+// MASKED: unobserved cells as in probit_row_fwd_tiled_kernel.
+template <bool STABLE, bool MASKED>
 __global__ void __launch_bounds__(kSmallThreads)
 probit_small_fwd_kernel(const SmallArgs p) {
     extern __shared__ __align__(16) unsigned char s_raw[];
@@ -578,11 +629,16 @@ probit_small_fwd_kernel(const SmallArgs p) {
     // this lane's labels (L <= 128: at most four 32-label chunks)
     const int nch = (L + 31) >> 5;
     float yv[4], fev[4], fxv[4];
+    bool ov[4];
 #pragma unroll
     for (int c = 0; c < 4; ++c) {
         const int l = (c << 5) + lane;
         yv[c] = fev[c] = fxv[c] = 0.f;
         if (c < nch && l < L) { yv[c] = a.y[(size_t)b * L + l]; fev[c] = a.fe_out[(size_t)b * L + l]; fxv[c] = a.fx_out[(size_t)b * L + l]; }
+        if (MASKED) {
+            ov[c] = c < nch && l < L && a.mask[(size_t)b * L + l] != 0;
+            if (!ov[c]) yv[c] = 0.f;
+        }
     }
     small_r_wait(bulk, &s_bar);
     __syncthreads();
@@ -613,8 +669,10 @@ probit_small_fwd_kernel(const SmallArgs p) {
                 const float nr = i == 0 ? acc0 : acc1;
                 const CellFwd cl = cell_forward<STABLE>(nr + fev[c], yv[c]);   // mpvae.py:168,177
                 const CellFwd cx = cell_forward<STABLE>(nr + fxv[c], yv[c]);   // mpvae.py:170,180
-                lpl[i] += (double)cl.ll; lpx[i] += (double)cx.ll;
-                pn[i][0] += cl.epos; pn[i][1] += cl.eneg; pn[i][2] += cx.epos; pn[i][3] += cx.eneg;
+                if (!MASKED || ov[c]) {
+                    lpl[i] += (double)cl.ll; lpx[i] += (double)cx.ll;
+                    pn[i][0] += cl.epos; pn[i][1] += cl.eneg; pn[i][2] += cx.epos; pn[i][3] += cx.eneg;
+                }
                 pl += cl.E; px += cx.E;
                 if (p.nr_out) {   // kept for the backward (training)
                     const size_t o = row_of(a, s0 + i, b) * a.ldn + l;
@@ -647,9 +705,11 @@ probit_small_fwd_kernel(const SmallArgs p) {
         a.indiv_prob_label[(size_t)b * L + l] = sl / fS;
         a.indiv_prob[(size_t)b * L + l] = sx / fS;
     }
-    row_tail<kSmallThreads>(a, b);
+    row_tail<kSmallThreads, MASKED>(a, b);
 }
 
+// MASKED: unobserved cells as in probit_row_bwd_saved_kernel.
+template <bool MASKED>
 __global__ void __launch_bounds__(kThreads)
 probit_small_bwd_kernel(const SmallArgs p) {
     extern __shared__ __align__(16) unsigned char s_raw[];
@@ -683,7 +743,8 @@ probit_small_bwd_kernel(const SmallArgs p) {
         for (int c = 0; c < 4; ++c) {
             const int l = (c << 5) + lane;
             if (c >= nch || l >= L) continue;
-            const float y = a.y[(size_t)b * L + l], fe = a.fe_out[(size_t)b * L + l], fx = a.fx_out[(size_t)b * L + l];
+            const bool ob = !MASKED || a.mask[(size_t)b * L + l] != 0;
+            const float y = ob ? a.y[(size_t)b * L + l] : 0.f, fe = a.fe_out[(size_t)b * L + l], fx = a.fx_out[(size_t)b * L + l];
             const float gpl = a.g_indiv_prob_label ? a.g_indiv_prob_label[(size_t)b * L + l] / fS : 0.f;
             const float gpx = a.g_indiv_prob ? a.g_indiv_prob[(size_t)b * L + l] / fS : 0.f;
             float gl = 0.f, gx = 0.f;
@@ -693,8 +754,14 @@ probit_small_bwd_kernel(const SmallArgs p) {
                 const size_t o = row_of(a, s, b) * a.ldn + l;
                 const float nr = a.nr[o];
                 const float* cf = coef + s * 6;
-                const float dl = cell_backward_saved(nr + fe, a.E_l[o], y, cf[0], cf[2], cf[4], gpl);
-                const float dx = cell_backward_saved(nr + fx, a.E_x[o], y, cf[1], cf[3], cf[5], gpx);
+                float dl, dx;
+                if (ob) {
+                    dl = cell_backward_saved(nr + fe, a.E_l[o], y, cf[0], cf[2], cf[4], gpl);
+                    dx = cell_backward_saved(nr + fx, a.E_x[o], y, cf[1], cf[3], cf[5], gpx);
+                } else {
+                    dl = cell_backward_saved(nr + fe, a.E_l[o], 0.f, 0.f, 0.f, 0.f, gpl);
+                    dx = cell_backward_saved(nr + fx, a.E_x[o], 0.f, 0.f, 0.f, 0.f, gpx);
+                }
                 gl += dl; gx += dx;
                 gxs[(size_t)s * L + l] = dl + dx;
             }
@@ -785,21 +852,30 @@ int launch_small_forward(RowArgs a, const SmallNoise& n, cudaStream_t stream) {
     static bool configured[kMaxDevices] = {};
     const int dev = device_slot();
     if (!configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(probit_small_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
+        cudaError_t e = cudaFuncSetAttribute(probit_small_fwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_fwd_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_fwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_fwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
         if (e != cudaSuccess) { set_error("cudaFuncSetAttribute(small): %s", cudaGetErrorString(e)); return 4; }
         configured[dev] = true;
     }
     const SmallArgs p = small_args(a, n);
-    if (a.stable) probit_small_fwd_kernel<true><<<a.B, kSmallThreads, smem, stream>>>(p);
-    else probit_small_fwd_kernel<false><<<a.B, kSmallThreads, smem, stream>>>(p);
+    if (a.mask) {
+        if (a.stable) probit_small_fwd_kernel<true, true><<<a.B, kSmallThreads, smem, stream>>>(p);
+        else probit_small_fwd_kernel<false, true><<<a.B, kSmallThreads, smem, stream>>>(p);
+    } else {
+        if (a.stable) probit_small_fwd_kernel<true, false><<<a.B, kSmallThreads, smem, stream>>>(p);
+        else probit_small_fwd_kernel<false, false><<<a.B, kSmallThreads, smem, stream>>>(p);
+    }
     return check_launch("probit_small_fwd_kernel");
 }
 
 int launch_small_backward(RowArgs a, const SmallNoise& n, float* g_r, cudaStream_t stream) {
     const SmallArgs p = small_args(a, n);
-    probit_small_bwd_kernel<<<a.B, kThreads, small_bwd_smem(a.S, a.L, n.Z), stream>>>(p);
+    if (a.mask) probit_small_bwd_kernel<true><<<a.B, kThreads, small_bwd_smem(a.S, a.L, n.Z), stream>>>(p);
+    else probit_small_bwd_kernel<false><<<a.B, kThreads, small_bwd_smem(a.S, a.L, n.Z), stream>>>(p);
     if (int rc = check_launch("probit_small_bwd_kernel")) return rc;
     if (g_r == nullptr) return 0;
     const int cnt = a.L * n.Z;
@@ -826,8 +902,14 @@ int launch_row_forward(RowArgs a, cudaStream_t stream) {
     FusePart* part = const_cast<FusePart*>(a.part);
     // two CTAs of 256 threads per SM (<= 128 registers: sixteen cells in flight per lane, no spills); measured equal
     // to or faster than three (80 registers, spills) and four (64) on B200
-    if (a.stable) probit_row_fwd_tiled_kernel<true, 2><<<dim3(a.B, gy), kThreads, 0, stream>>>(a, part, nchunks);
-    else probit_row_fwd_tiled_kernel<false, 2><<<dim3(a.B, gy), kThreads, 0, stream>>>(a, part, nchunks);
+    const dim3 grid(a.B, gy);
+    if (a.mask) {
+        if (a.stable) probit_row_fwd_tiled_kernel<true, 2, true><<<grid, kThreads, 0, stream>>>(a, part, nchunks);
+        else probit_row_fwd_tiled_kernel<false, 2, true><<<grid, kThreads, 0, stream>>>(a, part, nchunks);
+    } else {
+        if (a.stable) probit_row_fwd_tiled_kernel<true, 2, false><<<grid, kThreads, 0, stream>>>(a, part, nchunks);
+        else probit_row_fwd_tiled_kernel<false, 2, false><<<grid, kThreads, 0, stream>>>(a, part, nchunks);
+    }
     if (int rc = check_launch("probit_row_fwd_tiled_kernel")) return rc;
     a.part_tiles = nchunks;
     return launch_row_finalize(a, stream);
@@ -835,12 +917,14 @@ int launch_row_forward(RowArgs a, cudaStream_t stream) {
 
 int launch_row_finalize(RowArgs a, cudaStream_t stream) {
     if (a.part == nullptr || a.part_tiles <= 0) { set_error("row finalize: no partials"); return 1; }
-    probit_row_finalize_kernel<<<a.B, kThreads, 0, stream>>>(a);
+    if (a.mask) probit_row_finalize_kernel<true><<<a.B, kThreads, 0, stream>>>(a);
+    else probit_row_finalize_kernel<false><<<a.B, kThreads, 0, stream>>>(a);
     return check_launch("probit_row_finalize_kernel");
 }
 
 int launch_gxs_bound(RowArgs a, const unsigned int* gp_absmax, unsigned int* out_bits, cudaStream_t stream) {
-    gxs_bound_kernel<<<ceil_div(a.B * a.S, 256), 256, 0, stream>>>(a, gp_absmax, out_bits);
+    if (a.mask) gxs_bound_kernel<true><<<ceil_div(a.B * a.S, 256), 256, 0, stream>>>(a, gp_absmax, out_bits);
+    else gxs_bound_kernel<false><<<ceil_div(a.B * a.S, 256), 256, 0, stream>>>(a, gp_absmax, out_bits);
     return check_launch("gxs_bound_kernel");
 }
 
@@ -853,7 +937,8 @@ int launch_row_backward(RowArgs a, cudaStream_t stream) {
         int gy = ceil_div(2 * 4 * kNumSMs, a.B);
         if (gy > ceil_div(nchunks, kWarps)) gy = ceil_div(nchunks, kWarps);
         if (gy < 1) gy = 1;
-        probit_row_bwd_saved_kernel<<<dim3(a.B, gy), kThreads, smem, stream>>>(a);
+        if (a.mask) probit_row_bwd_saved_kernel<true><<<dim3(a.B, gy), kThreads, smem, stream>>>(a);
+        else probit_row_bwd_saved_kernel<false><<<dim3(a.B, gy), kThreads, smem, stream>>>(a);
         return check_launch("probit_row_bwd_saved_kernel");
     }
     a.nwl = pick_nwl(a.L);
@@ -862,13 +947,20 @@ int launch_row_backward(RowArgs a, cudaStream_t stream) {
     static bool configured[kMaxDevices] = {};
     const int dev = device_slot();
     if (smem > 48 * 1024 && !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(probit_row_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_row_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        cudaError_t e = cudaFuncSetAttribute(probit_row_bwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_row_bwd_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_row_bwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_row_bwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
         if (e != cudaSuccess) { set_error("cudaFuncSetAttribute(bwd): %s", cudaGetErrorString(e)); return 4; }
         configured[dev] = true;
     }
-    if (a.stable) probit_row_bwd_kernel<true><<<a.B, kThreads, smem, stream>>>(a);
-    else probit_row_bwd_kernel<false><<<a.B, kThreads, smem, stream>>>(a);
+    if (a.mask) {
+        if (a.stable) probit_row_bwd_kernel<true, true><<<a.B, kThreads, smem, stream>>>(a);
+        else probit_row_bwd_kernel<false, true><<<a.B, kThreads, smem, stream>>>(a);
+    } else {
+        if (a.stable) probit_row_bwd_kernel<true, false><<<a.B, kThreads, smem, stream>>>(a);
+        else probit_row_bwd_kernel<false, false><<<a.B, kThreads, smem, stream>>>(a);
+    }
     return check_launch("probit_row_bwd_kernel");
 }
 

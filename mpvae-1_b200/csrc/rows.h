@@ -51,6 +51,11 @@ struct RowArgs {
     size_t gxs_plane_elems;     // distance between the hi and the lo plane
     int gxs_pitch;
     const unsigned int* gxs_scale;
+    // partially labelled rows: (B, L) bytes, nonzero = the label is observed; nullptr = every label is observed.  The
+    // launchers pick the kernels' MASKED instantiation from it: an unobserved cell keeps E and the predictions but adds
+    // nothing to the log-likelihood, the ranking sums or the label counts, and its logit gradient is the cotangent of
+    // indiv_prob / indiv_prob_label alone.  Whatever y holds there is never read into the arithmetic.
+    const uint8_t* mask;
 };
 
 size_t row_smem_bytes(int L);

@@ -55,14 +55,15 @@ def _score_rows(model, feats: torch.Tensor, args, batch_size: Optional[int], gat
 
 @torch.no_grad()
 def predict_proba(model, feats: torch.Tensor, labels: Optional[torch.Tensor], args, batch_size: Optional[int] = None,
-                  loss_fn=None, gather: bool = True, group=None, predict_fn=None):
+                  loss_fn=None, gather: bool = True, group=None, predict_fn=None, label_mask=None):
     """Returns (indiv_prob (N, L), summed-loss dict).  `feats` / `labels` are device tensors for ALL N rows.
 
     `labels=None` scores rows that have no labels: each batch runs only the feature branch (`model.feat_forward`) and
     `mpvae.predict` (or `predict_fn`, same signature, e.g. `mpvae.predict_exact`), and the loss dict is None.  With
     labels, `VAE.forward` draws the label branch's reparameterisation noise first, so under the same torch seed the
     feature branch -- and hence the predictions -- differ from the label-free call; on the same fx_out the two give the
-    same bits."""
+    same bits.  `label_mask` (N, L), with labels: the mask of observed labels (`compute_loss`); the summed losses are
+    then those of the observed labels, and the predictions do not change."""
     if labels is None and predict_fn is None:
         from .mpvae import predict as predict_fn
     if labels is not None and loss_fn is None:
@@ -76,7 +77,8 @@ def predict_proba(model, feats: torch.Tensor, labels: Optional[torch.Tensor], ar
             return predict_fn(feat_out, model.r_sqrt_sigma, args)
         y = labels[a:b].float()
         label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar = model(y, x)
-        out = loss_fn(y, label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar, model.r_sqrt_sigma, args)
+        kw = {} if label_mask is None else {"label_mask": label_mask[a:b]}
+        out = loss_fn(y, label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar, model.r_sqrt_sigma, args, **kw)
         sums["total_loss"] = sums["total_loss"] + out[0] * (b - a)                   # test.py:67-70
         sums["nll_loss"] = sums["nll_loss"] + out[1] * (b - a)
         sums["c_loss"] = sums["c_loss"] + out[3] * (b - a)

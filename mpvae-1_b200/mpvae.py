@@ -151,9 +151,24 @@ def draw_noise(args, n_sample, n_batch, device, noise=None):
                          global_batch=b_global, row0=row0)
 
 
-def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r_sqrt_sigma, args, noise=None):
+def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r_sqrt_sigma, args, noise=None,
+                 label_mask=None):
     """Reference signature (mpvae.py:145) -> (total_loss, nll_loss, nll_loss_x, c_loss, c_loss_x, kl_loss,
-    indiv_prob, indiv_prob_label) (mpvae.py:210)."""
+    indiv_prob, indiv_prob_label) (mpvae.py:210).
+
+    `label_mask` (B, L) bool or uint8 on the batch's device, or None (every label known): partially labelled rows.
+    Nonzero = the label is observed.  Per row, with O the observed labels:
+      - both log-likelihoods sum over O only; the log-mean-exp over samples and the mean over all B rows are unchanged,
+        so a row with nothing observed adds exactly 0 to nll_loss / nll_loss_x;
+      - the ranking losses take pos = observed and y == 1, neg = observed and y == 0, and count only observed cells;
+        a row whose observed labels lack a positive or a negative adds 0 (its observed cells get NaN gradients, as an
+        unmasked degenerate row does, unless MPVAE_FLAG_SANITIZE_DEGENERATE; unobserved cells never do);
+      - kl_loss, indiv_prob and indiv_prob_label (every cell) are unchanged;
+      - an unobserved cell's logit gradient is only the cotangent of indiv_prob / indiv_prob_label.
+    Whatever input_label holds in an unobserved cell, NaN included, has no effect here.  (The label encoder still reads
+    input_label as the caller gives it: filling unknown labels with 0 there is the caller's choice.)  A mask of all ones
+    gives the unmasked results bit for bit.  With one row in test mode, -predict_conditional(...,
+    observed=torch.where(mask, y.to(torch.int8), -1)).log_evidence equals nll_loss_x on the same noise."""
     device = input_label.device
     if device.type != "cuda":
         raise RuntimeError("mpvae_b200.compute_loss needs CUDA tensors: the probit ELBO is implemented as sm_100a "
@@ -170,7 +185,8 @@ def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar
     flags = int(getattr(args, "mpvae_flags", 0))
     # args.peer_ring (peer.PeerRing, data-parallel runs): g_R comes back already summed over the ranks
     return ProbitELBO.apply(input_label.float(), fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise,
-                            float(args.nll_coeff), float(args.c_coeff), flags, spec, getattr(args, "peer_ring", None))
+                            float(args.nll_coeff), float(args.c_coeff), flags, spec, getattr(args, "peer_ring", None),
+                            label_mask)
 
 
 def predict(fx_out, r_sqrt_sigma, args, noise=None):

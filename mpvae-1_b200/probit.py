@@ -55,6 +55,18 @@ def _check_inputs(y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, no
     return S, B, L, Z, D
 
 
+def _check_label_mask(label_mask, B, L, device):
+    """The (B, L) label mask as contiguous uint8 (nonzero = observed), refused before any launch when it is not a bool or
+    uint8 tensor of that shape on the batch's device."""
+    if not isinstance(label_mask, torch.Tensor) or label_mask.dtype not in (torch.bool, torch.uint8):
+        raise TypeError(f"label_mask must be a bool or uint8 tensor, got {getattr(label_mask, 'dtype', type(label_mask))}")
+    if label_mask.shape != (B, L):
+        raise ValueError(f"label_mask has shape {tuple(label_mask.shape)}, expected {(B, L)} (batch, label_dim)")
+    if label_mask.device != device:
+        raise ValueError(f"label_mask is on {label_mask.device}, expected {device}")
+    return label_mask.contiguous().view(torch.uint8)
+
+
 def _set_noise_spec(p, spec, B):
     p.noise_offset_dev = None
     if spec is None:
@@ -77,11 +89,15 @@ class ProbitELBO(torch.autograd.Function):
     """(y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, R32, noise) -> the 8-tuple of mpvae.py:210.
 
     `noise` is either the (S, B, Z) tensor or None, in which case `noise_spec` = (S, seed, offset, B_global, row0)
-    and the library draws the Philox normals itself, straight into the contraction engine's operand layout."""
+    and the library draws the Philox normals itself, straight into the contraction engine's operand layout.
+
+    `label_mask` (B, L) bool / uint8 on the batch's device, or None: nonzero = the label is observed.  The
+    log-likelihood and the ranking loss then run over the observed labels only (mpvae_probit_forward_masked); y is not
+    read where the mask is 0.  None runs the unmasked entry points."""
 
     @staticmethod
     def forward(ctx, y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise, nll_coeff, c_coeff, flags,
-                noise_spec=None, peer=None):
+                noise_spec=None, peer=None, label_mask=None):
         lib = _lib.lib()
         y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32 = (
             t.contiguous() for t in (y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32))
@@ -91,6 +107,8 @@ class ProbitELBO(torch.autograd.Function):
             raise ValueError("ProbitELBO needs either a noise tensor or a noise_spec")
         S, B, L, Z, D = _check_inputs(y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise, noise_spec)
         dev = y.device
+        if label_mask is not None:
+            label_mask = _check_label_mask(label_mask, B, L, dev)
         want_bwd = any(ctx.needs_input_grad)
         with torch.cuda.device(dev):
             ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 1 if want_bwd else 0, flags))
@@ -118,14 +136,20 @@ class ProbitELBO(torch.autograd.Function):
             p.indiv_prob, p.indiv_prob_label = _ptr(prob), _ptr(prob_label)
             p.workspace, p.workspace_bytes = _ptr(ws), ws_bytes
             stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            _lib.check(lib.mpvae_probit_forward(C.byref(p), stream), "mpvae_probit_forward")
+            if label_mask is None:
+                _lib.check(lib.mpvae_probit_forward(C.byref(p), stream), "mpvae_probit_forward")
+            else:
+                _lib.check(lib.mpvae_probit_forward_masked(C.byref(p), _ptr(label_mask), stream),
+                           "mpvae_probit_forward_masked")
         if want_bwd:
             ctx.has_noise = noise is not None
             ctx.noise_spec = noise_spec
             # data-parallel g_R over peer memory (peer.py): the backward then returns the SUM over all ranks
             ctx.peer = peer if (peer is not None and peer.applies(S, B, L, Z, flags)) else None
+            ctx.has_mask = label_mask is not None
             ctx.save_for_backward(y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, ws,
-                                  *([noise] if noise is not None else []))
+                                  *([noise] if noise is not None else []),
+                                  *([label_mask] if label_mask is not None else []))
             ctx.dims = (S, B, L, Z, D)
             ctx.coeffs = (float(nll_coeff), float(c_coeff), int(flags))
             ctx.set_materialize_grads(False)
@@ -136,6 +160,7 @@ class ProbitELBO(torch.autograd.Function):
         lib = _lib.lib()
         y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, ws = ctx.saved_tensors[:9]
         noise = ctx.saved_tensors[9] if ctx.has_noise else None
+        label_mask = ctx.saved_tensors[-1] if ctx.has_mask else None
         S, B, L, Z, D = ctx.dims
         nll_coeff, c_coeff, flags = ctx.coeffs
         dev = y.device
@@ -180,10 +205,14 @@ class ProbitELBO(torch.autograd.Function):
             p.g_r = _ptr(g_r)
             p.workspace, p.workspace_bytes = _ptr(ws), ws.numel()
             stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            _lib.check(lib.mpvae_probit_backward(C.byref(p), stream), "mpvae_probit_backward")
+            if label_mask is None:
+                _lib.check(lib.mpvae_probit_backward(C.byref(p), stream), "mpvae_probit_backward")
+            else:
+                _lib.check(lib.mpvae_probit_backward_masked(C.byref(p), _ptr(label_mask), stream),
+                           "mpvae_probit_backward_masked")
         #       y     fe_out    fe_mu      fe_logvar  fx_out    fx_mu      fx_logvar  r32  noise nll_c c_c flags spec
         return (None, g_fe_out, g_mulv[0], g_mulv[1], g_fx_out, g_mulv[2], g_mulv[3], g_r, None, None, None, None, None,
-                None)
+                None, None)
 
 
 def _predict_inputs(name, fx_out, r32, S, noise, noise_spec):

@@ -207,10 +207,12 @@ class DataParallelStep:
 
     # -- the step -------------------------------------------------------------------------------------------
     def step(self, input_label: torch.Tensor, input_feat: torch.Tensor, noise: Optional[torch.Tensor] = None,
-             r_override: Optional[torch.Tensor] = None) -> StepOutput:
+             r_override: Optional[torch.Tensor] = None, label_mask: Optional[torch.Tensor] = None) -> StepOutput:
         """`input_label` (B, L) and `input_feat` (B, F) are the GLOBAL batch (train.py:106-111); every rank slices
         its rows.  `noise`, if given, is the global (S, B, Z) tensor (validation mode).  `r_override` is the
-        fresh non-trainable R of residue_sigma == 'random' (train.py:120-122)."""
+        fresh non-trainable R of residue_sigma == 'random' (train.py:120-122).  `label_mask`, if given, is the global
+        (B, L) mask of observed labels (`compute_loss`): each rank passes its rows' slice to the loss as
+        `label_mask=`; without it the loss is called exactly as before, so custom loss functions keep working."""
         args = self.args
         n_rows = input_label.shape[0]
         lo, hi = shard_rows(n_rows, self.rank, self.world)
@@ -234,6 +236,8 @@ class DataParallelStep:
             r = r_override if r_override is not None else (self.r_shadow if self.r_shadow is not None
                                                             else self.model.r_sqrt_sigma)
             kw = {} if noise is None else {"noise": noise[:, lo:hi]}
+            if label_mask is not None:
+                kw["label_mask"] = label_mask[lo:hi]
             out = self.loss_fn(y, label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar, r, args, **kw)
             total = out[0]
             if self.regulariser is not None:
@@ -290,9 +294,11 @@ class DataParallelStep:
         return StepOutput(*scal, out[6].detach(), out[7].detach(), grad_norm, stepped)
 
 
-def train_one_epoch(step: DataParallelStep, feats, labels, batch_size: int, order=None, skip_empty: bool = True):
+def train_one_epoch(step: DataParallelStep, feats, labels, batch_size: int, order=None, skip_empty: bool = True,
+                    masks=None):
     """Epoch driver with the reference's batching (train.py:98-111): int(N/bs)+1 steps, ragged (possibly empty)
     last batch.  `feats` / `labels` are device tensors (kept resident: SURVEY 8f-N4); returns per-step outputs.
+    `masks`, if given, is the (N, L) mask of observed labels (`compute_loss`), sliced by the same index as `labels`.
     `skip_empty=False` reproduces the reference literally when bs | N: it runs the step on the empty batch, whose
     losses are NaN means (train.py:102; compute_loss returns them) and whose NaN gradients then reach Adam."""
     n = feats.shape[0]
@@ -303,7 +309,10 @@ def train_one_epoch(step: DataParallelStep, feats, labels, batch_size: int, orde
         idx = order[i * batch_size:min(batch_size * (i + 1), n)]
         if idx.numel() == 0 and skip_empty:
             continue          # the reference computes NaN losses on the empty batch and steps on them
-        outs.append(step.step(labels[idx], feats[idx]))
+        if masks is None:
+            outs.append(step.step(labels[idx], feats[idx]))
+        else:
+            outs.append(step.step(labels[idx], feats[idx], label_mask=masks[idx]))
     return outs
 
 
