@@ -196,6 +196,28 @@ int mpvae_probit_predict(const mpvae_probit_params *p, void *cuda_stream);
 int mpvae_probit_predict_conditional(const mpvae_probit_params *p, const int8_t *observed, float *log_evidence,
                                      float *ess, void *cuda_stream);
 
+/* Conditional prediction by a GHK sampler: the same outputs and the same observed encoding as
+ * mpvae_probit_predict_conditional, from a sequential sampler of the probit posterior whose effective sample size stays
+ * usable when hundreds of labels are observed.  In the latent form u = fx_out + R eps + w (w ~ N(0, I)), per row with O
+ * its observed labels in ascending order and C the Cholesky factor of I + G[O, O] (G = R R^T, fp64), each of the S
+ * samples draws u_O = fx_O + C eta label by label: eta_k from its clamped truncated conditional (one uniform per
+ * observed cell), weight factor c + k Phi(+-m_k / C_kk).  The prior sample x_s = noise_s . R^T of mpvae_probit_predict is
+ * then conditioned on u_O by Matheron's rule (one fresh normal zeta per observed cell): x_s += G[:, O] v_s with
+ * v_s = C^-T (eta_s - C^-1 (x_s[O] + zeta_s)).  The weights go through the same log-mean-exp and the unobserved cells
+ * through the same weighted mean of E as mpvae_probit_predict_conditional.
+ *   gram      (L, L) fp32 R R^T prepared by the caller (mpvae_contract_nt with the engine of MPVAE_FLAG_CONTRACT_FMA or
+ *             auto gives the library's own bits), or NULL: computed here
+ *   zeta, uniform  (S, B, L) fp32, read at observed cells only (uniform in the open interval (0, 1)), or NULL: a Philox
+ *             stream keyed by (sample, noise_row0 + row, label) with its own key, disjoint from the noise
+ *   ghk_ws    >= mpvae_ghk_workspace_bytes(S, B, L, Z, max_observed, flags) bytes, 256-byte aligned; max_observed in
+ *             [0, L] bounds every row's observed count (a row with more gets NaN outputs)
+ * With nothing observed indiv_prob is mpvae_probit_predict's bit for bit (log_evidence = 0, ess = S).  p's workspace is
+ * mpvae_probit_predict's. */
+uint64_t mpvae_ghk_workspace_bytes(int32_t S, int32_t B, int32_t L, int32_t Z, int32_t max_observed, uint32_t flags);
+int mpvae_probit_predict_conditional_ghk(const mpvae_probit_params *p, const int8_t *observed, const float *gram,
+                                         const float *zeta, const float *uniform, void *ghk_ws, uint64_t ghk_ws_bytes,
+                                         int32_t max_observed, float *log_evidence, float *ess, void *cuda_stream);
+
 /* Backward: the autograd backward of compute_loss (implicit in the reference, train.py:125),
  * closed form in SURVEY.md 8(a-12).  Must follow a forward on the same workspace. */
 int mpvae_probit_backward(const mpvae_probit_params *p, void *cuda_stream);

@@ -34,6 +34,7 @@ EXPORTS = (
     "mpvae_peer_error", "mpvae_profile", "mpvae_profile_read", "mpvae_profile_name", "mpvae_test_log_normal",
     "mpvae_predictive_scale", "mpvae_predictive_rho", "mpvae_predict_exact", "mpvae_predict_pairs",
     "mpvae_probit_predict_conditional", "mpvae_probit_forward_masked", "mpvae_probit_backward_masked",
+    "mpvae_ghk_workspace_bytes", "mpvae_probit_predict_conditional_ghk",
 )
 
 _f = C.c_void_p  # device pointer
@@ -93,6 +94,11 @@ def _load():
     lib.mpvae_probit_predict.argtypes = [C.POINTER(ProbitParams), C.c_void_p]
     lib.mpvae_probit_predict_conditional.restype = C.c_int
     lib.mpvae_probit_predict_conditional.argtypes = [C.POINTER(ProbitParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.mpvae_ghk_workspace_bytes.restype = C.c_uint64
+    lib.mpvae_ghk_workspace_bytes.argtypes = [C.c_int32] * 5 + [C.c_uint32]
+    lib.mpvae_probit_predict_conditional_ghk.restype = C.c_int
+    lib.mpvae_probit_predict_conditional_ghk.argtypes = [C.POINTER(ProbitParams)] + [C.c_void_p] * 5 + [
+        C.c_uint64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.mpvae_probit_backward.restype = C.c_int
     lib.mpvae_probit_backward.argtypes = [C.POINTER(ProbitParams), C.c_void_p]
     for fn in (lib.mpvae_probit_forward_masked, lib.mpvae_probit_backward_masked):

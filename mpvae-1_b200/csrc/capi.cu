@@ -536,6 +536,78 @@ int mpvae_probit_predict_conditional(const mpvae_probit_params* p_in, const int8
     return launch_conditional_rows(a, observed, part, log_evidence, ess, stream);
 }
 
+// G = R R^T takes the engine its own (L, L, Z) shape selects, as mpvae_contract_nt's auto engine does, unless
+// MPVAE_FLAG_CONTRACT_FMA asks for the CUDA-core product
+static bool gram_uses_tensor(uint32_t flags, int L, int Z) {
+    return !(flags & MPVAE_FLAG_CONTRACT_FMA) && use_tensor(0, 1, L, L, Z);
+}
+
+static GhkLayout ghk_layout_for(int S, int B, int L, int Z, int mo, uint32_t flags) {
+    return ghk_layout(S, B, L, mo, gram_uses_tensor(flags, L, Z) ? tc_workspace_nt(L, L, Z) : 0);
+}
+
+uint64_t mpvae_ghk_workspace_bytes(int32_t S, int32_t B, int32_t L, int32_t Z, int32_t max_observed, uint32_t flags) {
+    if (S <= 0 || B <= 0 || L <= 0 || Z <= 0 || max_observed < 0 || max_observed > L) return 256;
+    return ghk_layout_for(S, B, L, Z, max_observed, flags).total;
+}
+
+int mpvae_probit_predict_conditional_ghk(const mpvae_probit_params* p_in, const int8_t* observed, const float* gram,
+                                         const float* zeta, const float* uniform, void* ghk_ws, uint64_t ghk_ws_bytes,
+                                         int32_t max_observed, float* log_evidence, float* ess, void* cuda_stream) {
+    mpvae_probit_params tmp;
+    const mpvae_probit_params* p = normalize(p_in, &tmp);
+    if (!p) return 1;
+    if (int rc = validate_predict(p)) return rc;
+    if (!observed || !log_evidence || !ess || !ghk_ws) { set_error("NULL pointer (observed/log_evidence/ess/ghk_ws)"); return 1; }
+    if (max_observed < 0 || max_observed > p->L) { set_error("max_observed=%d outside [0, L=%d]", max_observed, p->L); return 1; }
+    const GhkLayout gl = ghk_layout_for(p->S, p->B, p->L, p->Z, max_observed, p->flags);
+    if (ghk_ws_bytes < gl.total) {
+        set_error("ghk workspace too small for max_observed=%d: %llu < %llu bytes", max_observed,
+                  (unsigned long long)ghk_ws_bytes, (unsigned long long)gl.total);
+        return 1;
+    }
+    if ((reinterpret_cast<uintptr_t>(ghk_ws) & 255u) != 0) { set_error("ghk workspace must be 256-byte aligned"); return 1; }
+    if ((!zeta || !uniform) && (p->noise_row0 < 0 || p->noise_b_global < p->noise_row0 + p->B)) {
+        set_error("GHK draws: rows [%d, %d) do not fit a global batch of %d", p->noise_row0, p->noise_row0 + p->B,
+                  p->noise_b_global);
+        return 1;
+    }
+    cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
+    const Workspace w = carve(p->S, p->B, p->L, p->Z, false, p->flags);
+    const RowArgs a = row_args(p, w);
+    char* gbase = static_cast<char*>(ghk_ws);
+    int rc;
+    if (!gram && max_observed > 0) {
+        float* G = reinterpret_cast<float*>(gbase + gl.gram);
+        rc = gram_uses_tensor(p->flags, p->L, p->Z)
+                 ? tc_contract_nt(p->r, p->r, G, p->L, p->L, p->Z, gbase + gl.gram_scratch, tc_workspace_nt(p->L, p->L, p->Z), stream)
+                 : launch_contract_nt_fma(p->r, p->r, G, p->L, p->L, p->Z, stream);
+        if (rc) return rc;
+        gram = G;
+    }
+    // predict's product, as mpvae_probit_predict_conditional runs it
+    if (use_tensor(p->flags, p->S, p->B, p->L, p->Z)) {
+        uint32_t* slots = reinterpret_cast<uint32_t*>(static_cast<char*>(p->workspace) + w.slots);
+        const cudaError_t e = cudaMemsetAsync(slots, 0, w.slots_bytes, stream);
+        if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
+        if ((rc = dense_nt_product(p, w, nullptr, stream))) return rc;
+    } else if ((rc = fma_nt_product(p, w, stream))) {
+        return rc;
+    }
+    GhkInputs in{};
+    in.layout = gl;
+    in.ws = ghk_ws;
+    in.max_observed = max_observed;
+    in.observed = observed;
+    in.gram = gram;
+    in.zeta = zeta; in.uniform = uniform;
+    in.noise_b_global = p->noise_b_global; in.noise_row0 = p->noise_row0;
+    in.noise_seed = p->noise_seed; in.noise_offset = p->noise_offset; in.noise_offset_dev = p->noise_offset_dev;
+    in.log_evidence = log_evidence; in.ess = ess;
+    ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
+    return launch_ghk_rows(a, in, stream);
+}
+
 int mpvae_probit_backward(const mpvae_probit_params* p_in, void* cuda_stream) {
     return mpvae_probit_backward_masked(p_in, nullptr, cuda_stream);
 }

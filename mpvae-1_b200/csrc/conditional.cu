@@ -96,21 +96,23 @@ probit_cond_loglik_kernel(const RowArgs a, const int8_t* __restrict__ observed, 
 
 // Row reduction, one CTA per row: lp_s = the chunk partials added as probit_row_finalize_kernel adds them (a lane per
 // chunk, stride 32, then the butterfly), then warp 0 runs the loss's log-mean-exp and leaves u_s in a.wts (B, S) and fse
-// in a.rowaux[2b].
+// in a.rowaux[2b].  part == nullptr: lp_s is already in a.lp (the GHK sampler's log-weights).
 __global__ void __launch_bounds__(kThreads)
 probit_cond_weights_kernel(const RowArgs a, const FusePart* __restrict__ part, int nchunks, float* __restrict__ log_evidence,
                            float* __restrict__ ess) {
     const int b = blockIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int S = a.S;
-    for (int s = warp; s < S; s += kWarps) {
-        const FusePart* __restrict__ pp = part + ((size_t)b * S + s) * nchunks;
-        double l = 0.0;
-        for (int t = lane; t < nchunks; t += 32) l += pp[t].lp_x;
-        l = warp_sum(l);
-        if (lane == 0) a.lp[(size_t)b * S + s] = l;
+    if (part) {
+        for (int s = warp; s < S; s += kWarps) {
+            const FusePart* __restrict__ pp = part + ((size_t)b * S + s) * nchunks;
+            double l = 0.0;
+            for (int t = lane; t < nchunks; t += 32) l += pp[t].lp_x;
+            l = warp_sum(l);
+            if (lane == 0) a.lp[(size_t)b * S + s] = l;
+        }
+        __syncthreads();
     }
-    __syncthreads();
     if (warp != 0) return;
     const double* __restrict__ lp = a.lp + (size_t)b * S;
     const LogMeanExp lme = warp_log_mean_exp(S, lane, [&](int s) { return (float)lp[s]; });
@@ -178,21 +180,32 @@ probit_cond_predict_kernel(const RowArgs a, const int8_t* __restrict__ observed,
     }
 }
 
+// the grid of launch_predict_rows: ~2 waves of 4 resident CTAs per SM, at most one CTA per 8 chunks (a warp each)
+dim3 rows_grid(const RowArgs& a, int nchunks) {
+    int gy = ceil_div(2 * 4 * kNumSMs, a.B);
+    if (gy > ceil_div(nchunks, kWarps)) gy = ceil_div(nchunks, kWarps);
+    if (gy < 1) gy = 1;
+    return dim3(a.B, gy);
+}
+
 }  // namespace
 
 int launch_conditional_rows(RowArgs a, const int8_t* observed, FusePart* part, float* log_evidence, float* ess,
                             cudaStream_t stream) {
     const int nchunks = (a.L + kChunk - 1) / kChunk;
-    // the grid of launch_predict_rows: ~2 waves of 4 resident CTAs per SM, at most one CTA per 8 chunks (a warp each)
-    int gy = ceil_div(2 * 4 * kNumSMs, a.B);
-    if (gy > ceil_div(nchunks, kWarps)) gy = ceil_div(nchunks, kWarps);
-    if (gy < 1) gy = 1;
-    const dim3 grid(a.B, gy);
+    const dim3 grid = rows_grid(a, nchunks);
     if (a.stable) probit_cond_loglik_kernel<true><<<grid, kThreads, 0, stream>>>(a, observed, part, nchunks);
     else probit_cond_loglik_kernel<false><<<grid, kThreads, 0, stream>>>(a, observed, part, nchunks);
     if (int rc = check_launch("probit_cond_loglik_kernel")) return rc;
-    probit_cond_weights_kernel<<<a.B, kThreads, 0, stream>>>(a, part, nchunks, log_evidence, ess);
+    return launch_conditional_tail(a, observed, part, nchunks, log_evidence, ess, stream);
+}
+
+int launch_conditional_tail(RowArgs a, const int8_t* observed, const FusePart* part, int part_chunks, float* log_evidence,
+                            float* ess, cudaStream_t stream) {
+    probit_cond_weights_kernel<<<a.B, kThreads, 0, stream>>>(a, part, part_chunks, log_evidence, ess);
     if (int rc = check_launch("probit_cond_weights_kernel")) return rc;
+    const int nchunks = (a.L + kChunk - 1) / kChunk;
+    const dim3 grid = rows_grid(a, nchunks);
     if (a.stable) probit_cond_predict_kernel<true><<<grid, kThreads, 0, stream>>>(a, observed, nchunks);
     else probit_cond_predict_kernel<false><<<grid, kThreads, 0, stream>>>(a, observed, nchunks);
     return check_launch("probit_cond_predict_kernel");

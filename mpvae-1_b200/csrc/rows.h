@@ -101,6 +101,29 @@ int launch_small_predict(RowArgs a, const SmallNoise& n, cudaStream_t stream);  
 // other value unobserved); log_evidence (B), ess (B).  Uses part (B * S * row_chunks(L) records), a.lp, a.wts, a.rowaux.
 int launch_conditional_rows(RowArgs a, const int8_t* observed, FusePart* part, float* log_evidence, float* ess,
                             cudaStream_t stream);
+// Its last two passes: the per-row log-mean-exp of lp_s (the sum of part_chunks FusePart records per sample from part,
+// or a.lp itself when part is nullptr), then the weighted mean of E over the samples of a.nr.
+int launch_conditional_tail(RowArgs a, const int8_t* observed, const FusePart* part, int part_chunks, float* log_evidence,
+                            float* ess, cudaStream_t stream);
+
+// Conditional prediction by a GHK sampler (conditional_ghk.cu), after the nt product (a.nr, overwritten with the
+// conditioned samples).  Its own scratch block: G = R R^T (L, L) fp32, the G product's scratch, per row the observed
+// count and index list, the fp64 Cholesky factor (mo x mo) and two fp64 (S, mo) vectors.
+struct GhkLayout { size_t gram, gram_scratch, nobs, idx, fac, eta, wv, total; };
+GhkLayout ghk_layout(int S, int B, int L, int mo, size_t gram_scratch);
+struct GhkInputs {
+    GhkLayout layout;
+    void* ws;
+    int max_observed;
+    const int8_t* observed;
+    const float* gram;                 // (L, L), read at [o_i, o_j] with o_i >= o_j and at rows o
+    const float *zeta, *uniform;       // (S, B, L) or nullptr (the library's Philox draws)
+    int noise_b_global, noise_row0;
+    uint64_t noise_seed, noise_offset;
+    const uint64_t* noise_offset_dev;
+    float *log_evidence, *ess;
+};
+int launch_ghk_rows(RowArgs a, const GhkInputs& in, cudaStream_t stream);
 
 // Closed-form predictive distribution (predictive.cu), the S -> infinity limit of the above: per-label scales
 // 1 / sqrt(1 + |R_l|^2), pair correlations, exact marginals and pair co-occurrence probabilities.  pairs: P int32 pairs

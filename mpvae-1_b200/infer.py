@@ -106,16 +106,18 @@ def predict_pairs(model, feats: torch.Tensor, pairs, args, batch_size: Optional[
 
 @torch.no_grad()
 def predict_conditional(model, feats: torch.Tensor, observed: torch.Tensor, args, batch_size: Optional[int] = None,
-                        gather: bool = True, group=None):
+                        gather: bool = True, group=None, predict_fn=None):
     """(prob (N, L), log_evidence (N,), ess (N,)): `mpvae.predict_conditional` for each row of `feats` given that row's
     known labels.  `observed` is the int8 (N, L) device tensor of states for ALL N rows (0 / 1 observed, -1 unobserved),
     sliced per batch as predict_proba slices labels.  Same row sharding, batching, global-row noise keys and gather as
-    predict_proba; with nothing observed, prob is predict_proba(labels=None)'s under the same torch seed."""
+    predict_proba; with nothing observed, prob is predict_proba(labels=None)'s under the same torch seed.
+    `predict_fn` (same signature and result, e.g. `mpvae.predict_conditional_ghk`) replaces mpvae.predict_conditional."""
     from . import mpvae
     L = model.r_sqrt_sigma.shape[0]
+    fn = predict_fn or mpvae.predict_conditional
 
     def score(a, b, args):
-        res = mpvae.predict_conditional(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, observed[a:b], args)
+        res = fn(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, observed[a:b], args)
         return torch.cat([res.prob, res.log_evidence[:, None], res.ess[:, None]], 1)
 
     out = _score_rows(model, feats, args, batch_size, gather, group, L + 2, score)

@@ -27,7 +27,8 @@ import torch.nn.functional as F
 from . import _lib
 from .dense import linear
 from .probit import ProbitELBO, label_pairs, philox_normal, predictive_rho, predictive_scale, probit_predict
-from .probit import predict_exact_from_r, probit_predict_conditional
+from .probit import contract_nt, ghk_workspace_bytes, predict_exact_from_r, probit_predict_conditional
+from .probit import probit_predict_conditional_ghk
 from .probit import predict_pairs as probit_predict_pairs
 
 _state = {"seed": 0x5EED_B200, "offset": 0}
@@ -253,6 +254,84 @@ def predict_conditional(fx_out, r_sqrt_sigma, observed, args, noise=None):
     flags = int(getattr(args, "mpvae_flags", 0))
     return ConditionalPrediction(*probit_predict_conditional(fx_out, r32, observed, n_sample, noise=noise, noise_spec=spec,
                                                              flags=flags))
+
+
+# The GHK sampler's scratch (its per-row Cholesky factors and per-sample vectors grow as B * max|O|^2 and B * S * max|O|)
+# is kept under this many bytes by splitting the batch into row groups.
+GHK_WORKSPACE_BOUND = 8 << 30
+
+
+def label_gram(r_sqrt_sigma, args=None):
+    """G = R R^T (L, L) fp32, the label covariance of the probit noise, for predict_conditional_ghk(..., gram=G): the
+    product the library runs when no gram is passed (the CUDA-core product under MPVAE_FLAG_CONTRACT_FMA in
+    args.mpvae_flags, else the engine G's own shape selects), so a prepared G gives the same bits.  Prepare it once per R
+    for repeated calls, as PairPredictor prepares rho.  Inference only."""
+    _inference_only("label_gram", r_sqrt_sigma)
+    _cuda_only("label_gram", r_sqrt_sigma)
+    flags = int(getattr(args, "mpvae_flags", 0)) if args is not None else 0
+    r32 = r_sqrt_sigma.float()
+    return contract_nt(r32, r32, engine=1 if flags & FLAG_CONTRACT_FMA else 0)
+
+
+def predict_conditional_ghk(fx_out, r_sqrt_sigma, observed, args, noise=None, gram=None):
+    """predict_conditional's ConditionalPrediction(prob, log_evidence, ess) from a GHK sampler of the probit posterior,
+    whose effective sample size stays usable when many labels are observed (where the importance weights of
+    predict_conditional collapse onto one sample).
+
+    In the model's latent form u = fx + R eps + w, each of predict's S samples (same noise, same offset consumption)
+    draws the observed latents label by label, each from its clamped truncated conditional given the ones before, and
+    takes the product of the observed labels' conditional probabilities as its weight; the sample's R eps is then
+    conditioned on those latents (Matheron's rule) before E is averaged.  prob, log_evidence and ess mean what they mean
+    for predict_conditional; with nothing observed in a row, its prob is predict's bits, log_evidence 0 and ess S.  The
+    two are different estimators of the same quantities: this one costs a Cholesky factor of I + G[O, O] per row and a
+    (S x |O|) . (|O| x L) product per row, and is the one to use when rows carry more than a handful of labels.
+
+    `observed`: int8 (B, L) as for predict_conditional.  `gram`: label_gram(r_sqrt_sigma, args), or None to compute it
+    here.  The call reads max_b |O_b| on the host (one synchronisation) to size its scratch, and runs the batch in row
+    groups that keep that scratch under GHK_WORKSPACE_BOUND bytes; rows are keyed by their global row, so the split
+    changes no bits.  The sampler's own uniforms and normals come from a Philox stream separate from the noise.
+    Inference only, CUDA only; args.mpvae_flags as for predict."""
+    _inference_only("predict_conditional_ghk", fx_out, r_sqrt_sigma)
+    device = fx_out.device
+    if device.type != "cuda":
+        raise RuntimeError("mpvae_b200.predict_conditional_ghk needs CUDA tensors: the GHK sampler is implemented as "
+                           "sm_100a kernels only (no CPU fallback)")
+    if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
+        raise TypeError(f"observed must be an int8 tensor, got {getattr(observed, 'dtype', type(observed))}")
+    if observed.shape != fx_out.shape:
+        raise ValueError(f"observed has shape {tuple(observed.shape)}, expected {tuple(fx_out.shape)} (batch, label_dim)")
+    if observed.device != device:
+        raise ValueError(f"observed is on {observed.device}, expected {device}")
+    n_batch, L = fx_out.shape
+    if n_batch == 0:
+        return ConditionalPrediction(fx_out.new_empty((0, L)), fx_out.new_empty(0), fx_out.new_empty(0))
+    n_sample = args.n_test_sample
+    r32 = r_sqrt_sigma.to(device).float()
+    Z = r32.shape[1]
+    noise, spec = noise_plan(args, n_sample, n_batch, device, noise)
+    flags = int(getattr(args, "mpvae_flags", 0))
+    max_obs = int(((observed == 0) | (observed == 1)).sum(1).max().item())      # the one host synchronisation
+    one = ghk_workspace_bytes(n_sample, 1, L, Z, max_obs, flags)
+    per_row = max(ghk_workspace_bytes(n_sample, 2, L, Z, max_obs, flags) - one, 1)
+    rows = max(1, (GHK_WORKSPACE_BOUND - (one - per_row)) // per_row)
+    n_groups = -(-n_batch // rows)
+    rows = -(-n_batch // n_groups)
+    if gram is None and n_groups > 1 and max_obs > 0:
+        gram = label_gram(r32, args)
+    if spec is not None:
+        b_global = spec[3] if spec[3] is not None else n_batch
+    out = []
+    for a in range(0, n_batch, rows):
+        b = min(n_batch, a + rows)
+        if spec is not None:
+            group_noise, group_spec = None, (spec[0], spec[1], spec[2], b_global, spec[4] + a) + tuple(spec[5:])
+        else:
+            group_noise, group_spec = noise[:, a:b], (n_sample, 0, 0, n_batch, a)
+        out.append(probit_predict_conditional_ghk(fx_out[a:b], r32, observed[a:b], n_sample, max_obs, noise=group_noise,
+                                                  noise_spec=group_spec, flags=flags, gram=gram))
+    if len(out) == 1:
+        return ConditionalPrediction(*out[0])
+    return ConditionalPrediction(*(torch.cat(t, 0) for t in zip(*out)))
 
 
 def _inference_only(name, *tensors):

@@ -304,6 +304,62 @@ def probit_predict_conditional(fx_out, r32, observed, S, *, noise=None, noise_sp
     return prob, log_evidence, ess
 
 
+def ghk_workspace_bytes(S, B, L, Z, max_observed, flags=0):
+    """Bytes of the GHK sampler's own scratch block (G, the per-row factors and index lists, the per-sample vectors)."""
+    return int(_lib.lib().mpvae_ghk_workspace_bytes(S, B, L, Z, max_observed, flags))
+
+
+def probit_predict_conditional_ghk(fx_out, r32, observed, S, max_observed, *, noise=None, noise_spec=None, flags=0,
+                                   gram=None, zeta=None, uniform=None):
+    """(prob (B, L), log_evidence (B,), ess (B,)): probit_predict_conditional's outputs from the GHK sampler
+    (mpvae_probit_predict_conditional_ghk).  `max_observed` bounds every row's observed count (a row with more gets
+    NaN outputs).  `gram`: the (L, L) fp32 R R^T of `contract_nt(r32, r32)` with the engine mpvae.label_gram picks, or
+    None.  `zeta` / `uniform`: optional (S, B, L) fp32 draws for the observed cells (uniform in (0, 1)); None = the
+    library's Philox stream.  `noise` / `noise_spec` / `flags` as for probit_predict; inference only."""
+    if fx_out.dim() != 2:
+        raise ValueError(f"fx_out must be (batch, label_dim), got {tuple(fx_out.shape)}")
+    B, L = fx_out.shape
+    if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
+        raise TypeError(f"observed must be an int8 tensor, got {getattr(observed, 'dtype', type(observed))}")
+    if observed.shape != (B, L):
+        raise ValueError(f"observed has shape {tuple(observed.shape)}, expected {(B, L)} (batch, label_dim)")
+    if observed.device != fx_out.device:
+        raise ValueError(f"observed is on {observed.device}, expected {fx_out.device}")
+    if not 0 <= int(max_observed) <= L:
+        raise ValueError(f"max_observed={max_observed} outside [0, {L}]")
+    for name, t, shape in (("gram", gram, (L, L)), ("zeta", zeta, (S, B, L)), ("uniform", uniform, (S, B, L))):
+        if t is not None and tuple(t.shape) != shape:
+            raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {shape}")
+    fx_out, r32, noise, dims = _predict_inputs("probit_predict_conditional_ghk", fx_out, r32, S, noise, noise_spec)
+    S, B, L, Z = dims
+    _check_tensors(("fx_out", "gram", "zeta", "uniform"), (fx_out, gram, zeta, uniform))
+    observed = observed.contiguous()
+    gram, zeta, uniform = (t.contiguous() if t is not None else None for t in (gram, zeta, uniform))
+    lib = _lib.lib()
+    dev = fx_out.device
+    with torch.cuda.device(dev):
+        ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 0, flags))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        gws_bytes = ghk_workspace_bytes(S, B, L, Z, int(max_observed), flags)
+        gws = torch.empty(gws_bytes, dtype=torch.uint8, device=dev)
+        prob = torch.empty((B, L), dtype=torch.float32, device=dev)
+        log_evidence = torch.empty(B, dtype=torch.float32, device=dev)
+        ess = torch.empty(B, dtype=torch.float32, device=dev)
+        if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
+            # test hook: see ProbitELBO.forward
+            ws.fill_(255)
+            gws.fill_(255)
+            for t in (prob, log_evidence, ess):
+                t.fill_(float("nan"))
+        p = _predict_params(fx_out, r32, noise, noise_spec, flags, dims, prob, ws)
+        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _lib.check(lib.mpvae_probit_predict_conditional_ghk(C.byref(p), _ptr(observed), _ptr(gram), _ptr(zeta),
+                                                            _ptr(uniform), _ptr(gws), gws_bytes, int(max_observed),
+                                                            _ptr(log_evidence), _ptr(ess), stream),
+                   "mpvae_probit_predict_conditional_ghk")
+    return prob, log_evidence, ess
+
+
 # ---- closed-form prediction (csrc/predictive.cu): the S -> infinity limit of probit_predict ----
 
 def _stream(dev):
