@@ -351,6 +351,38 @@ int fma_nt_product(const mpvae_probit_params* p, const Workspace& w, cudaStream_
                                   row_pitch(p->L));
 }
 
+// The start of every sampled-prediction entry point: the params in full layout, checked for prediction, and the
+// inference layout of mpvae_probit_forward, of which only nr, the noise / R operands and the slots are touched.
+// The struct is not copied: p may point at tmp.
+struct PredictCall {
+    mpvae_probit_params tmp;
+    const mpvae_probit_params* p;
+    Workspace w;
+    RowArgs a;
+};
+
+int open_predict(const mpvae_probit_params* p_in, PredictCall& c) {
+    c.p = normalize(p_in, &c.tmp);
+    if (!c.p) return 1;
+    if (int rc = validate_predict(c.p)) return rc;
+    c.w = carve(c.p->S, c.p->B, c.p->L, c.p->Z, false, c.p->flags);
+    c.a = row_args(c.p, c.w);
+    return 0;
+}
+
+// predict's nt product, nr in the workspace: tcgen05 where mpvae_probit_forward takes it for the same
+// (S, B, L, Z, flags), the CUDA-core product otherwise
+int predict_product(const PredictCall& c, cudaStream_t stream) {
+    const mpvae_probit_params* p = c.p;
+    if (!use_tensor(p->flags, p->S, p->B, p->L, p->Z)) return fma_nt_product(p, c.w, stream);
+    // absmax slot of R, per-block counters of the just-in-time noise
+    uint32_t* slots = reinterpret_cast<uint32_t*>(static_cast<char*>(p->workspace) + c.w.slots);
+    const cudaError_t e = cudaMemsetAsync(slots, 0, c.w.slots_bytes, stream);
+    if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
+    // the fused row forward (MPVAE_FLAG_FUSED_FORWARD) is loss work: predictions take the separate row kernels
+    return dense_nt_product(p, c.w, nullptr, stream);
+}
+
 }  // namespace
 }  // namespace mpv
 
@@ -476,26 +508,10 @@ int mpvae_probit_forward_masked(const mpvae_probit_params* p_in, const uint8_t* 
 }
 
 int mpvae_probit_predict(const mpvae_probit_params* p_in, void* cuda_stream) {
-    mpvae_probit_params tmp;
-    const mpvae_probit_params* p = normalize(p_in, &tmp);
-    if (!p) return 1;
-    if (int rc = validate_predict(p)) return rc;
+    PredictCall c;
+    if (int rc = open_predict(p_in, c)) return rc;
+    const mpvae_probit_params* p = c.p;
     cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
-    // the inference layout of mpvae_probit_forward; only nr, the noise / R operands and the slots are touched
-    const Workspace w = carve(p->S, p->B, p->L, p->Z, false, p->flags);
-    const RowArgs a = row_args(p, w);
-    int rc;
-    // the same regime as mpvae_probit_forward for the same (S, B, L, Z, flags)
-    if (use_tensor(p->flags, p->S, p->B, p->L, p->Z)) {
-        // absmax slot of R, per-block counters of the just-in-time noise
-        uint32_t* slots = reinterpret_cast<uint32_t*>(static_cast<char*>(p->workspace) + w.slots);
-        const cudaError_t e = cudaMemsetAsync(slots, 0, w.slots_bytes, stream);
-        if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
-        // the fused row forward (MPVAE_FLAG_FUSED_FORWARD) is loss work: predictions take the separate row kernel
-        if ((rc = dense_nt_product(p, w, nullptr, stream))) return rc;
-        ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
-        return launch_predict_rows(a, stream);
-    }
     if (use_small(p->flags, p->S, p->B, p->L, p->Z)) {
         ProfScope ps(MPVAE_PROF_FUSED_SMALL_FWD, stream);
         SmallNoise sn{};
@@ -503,37 +519,25 @@ int mpvae_probit_predict(const mpvae_probit_params* p_in, void* cuda_stream) {
         sn.noise_ext = p->noise;
         sn.Bg = p->noise_b_global; sn.row0 = p->noise_row0;
         sn.seed = p->noise_seed; sn.offset = p->noise_offset; sn.offset_dev = p->noise_offset_dev;
-        return launch_small_predict(a, sn, stream);
+        return launch_small_predict(c.a, sn, stream);
     }
-    if ((rc = fma_nt_product(p, w, stream))) return rc;
+    if (int rc = predict_product(c, stream)) return rc;
     ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
-    return launch_predict_rows(a, stream);
+    return launch_predict_rows(c.a, stream);
 }
 
 int mpvae_probit_predict_conditional(const mpvae_probit_params* p_in, const int8_t* observed, float* log_evidence,
                                      float* ess, void* cuda_stream) {
-    mpvae_probit_params tmp;
-    const mpvae_probit_params* p = normalize(p_in, &tmp);
-    if (!p) return 1;
-    if (int rc = validate_predict(p)) return rc;
+    PredictCall c;
+    if (int rc = open_predict(p_in, c)) return rc;
     if (!observed || !log_evidence || !ess) { set_error("NULL pointer (observed/log_evidence/ess)"); return 1; }
     cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
-    const Workspace w = carve(p->S, p->B, p->L, p->Z, false, p->flags);
-    const RowArgs a = row_args(p, w);
-    FusePart* part = reinterpret_cast<FusePart*>(static_cast<char*>(p->workspace) + w.fuse_part);
-    int rc;
-    // predict's product; the CUDA-core product also where predict takes the one-launch small kernel, which never
-    // materialises nr (its forward outputs equal the CUDA-core path's bit for bit)
-    if (use_tensor(p->flags, p->S, p->B, p->L, p->Z)) {
-        uint32_t* slots = reinterpret_cast<uint32_t*>(static_cast<char*>(p->workspace) + w.slots);
-        const cudaError_t e = cudaMemsetAsync(slots, 0, w.slots_bytes, stream);
-        if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
-        if ((rc = dense_nt_product(p, w, nullptr, stream))) return rc;
-    } else if ((rc = fma_nt_product(p, w, stream))) {
-        return rc;
-    }
+    FusePart* part = reinterpret_cast<FusePart*>(static_cast<char*>(c.p->workspace) + c.w.fuse_part);
+    // the CUDA-core product also where predict takes the one-launch small kernel, which never materialises nr (its
+    // forward outputs equal the CUDA-core path's bit for bit)
+    if (int rc = predict_product(c, stream)) return rc;
     ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
-    return launch_conditional_rows(a, observed, part, log_evidence, ess, stream);
+    return launch_conditional_rows(c.a, observed, part, log_evidence, ess, stream);
 }
 
 // G = R R^T takes the engine its own (L, L, Z) shape selects, as mpvae_contract_nt's auto engine does, unless
@@ -554,10 +558,9 @@ uint64_t mpvae_ghk_workspace_bytes(int32_t S, int32_t B, int32_t L, int32_t Z, i
 int mpvae_probit_predict_conditional_ghk(const mpvae_probit_params* p_in, const int8_t* observed, const float* gram,
                                          const float* zeta, const float* uniform, void* ghk_ws, uint64_t ghk_ws_bytes,
                                          int32_t max_observed, float* log_evidence, float* ess, void* cuda_stream) {
-    mpvae_probit_params tmp;
-    const mpvae_probit_params* p = normalize(p_in, &tmp);
-    if (!p) return 1;
-    if (int rc = validate_predict(p)) return rc;
+    PredictCall c;
+    if (int rc = open_predict(p_in, c)) return rc;
+    const mpvae_probit_params* p = c.p;
     if (!observed || !log_evidence || !ess || !ghk_ws) { set_error("NULL pointer (observed/log_evidence/ess/ghk_ws)"); return 1; }
     if (max_observed < 0 || max_observed > p->L) { set_error("max_observed=%d outside [0, L=%d]", max_observed, p->L); return 1; }
     const GhkLayout gl = ghk_layout_for(p->S, p->B, p->L, p->Z, max_observed, p->flags);
@@ -573,8 +576,6 @@ int mpvae_probit_predict_conditional_ghk(const mpvae_probit_params* p_in, const 
         return 1;
     }
     cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
-    const Workspace w = carve(p->S, p->B, p->L, p->Z, false, p->flags);
-    const RowArgs a = row_args(p, w);
     char* gbase = static_cast<char*>(ghk_ws);
     int rc;
     if (!gram && max_observed > 0) {
@@ -585,15 +586,7 @@ int mpvae_probit_predict_conditional_ghk(const mpvae_probit_params* p_in, const 
         if (rc) return rc;
         gram = G;
     }
-    // predict's product, as mpvae_probit_predict_conditional runs it
-    if (use_tensor(p->flags, p->S, p->B, p->L, p->Z)) {
-        uint32_t* slots = reinterpret_cast<uint32_t*>(static_cast<char*>(p->workspace) + w.slots);
-        const cudaError_t e = cudaMemsetAsync(slots, 0, w.slots_bytes, stream);
-        if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
-        if ((rc = dense_nt_product(p, w, nullptr, stream))) return rc;
-    } else if ((rc = fma_nt_product(p, w, stream))) {
-        return rc;
-    }
+    if ((rc = predict_product(c, stream))) return rc;
     GhkInputs in{};
     in.layout = gl;
     in.ws = ghk_ws;
@@ -605,7 +598,7 @@ int mpvae_probit_predict_conditional_ghk(const mpvae_probit_params* p_in, const 
     in.noise_seed = p->noise_seed; in.noise_offset = p->noise_offset; in.noise_offset_dev = p->noise_offset_dev;
     in.log_evidence = log_evidence; in.ess = ess;
     ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
-    return launch_ghk_rows(a, in, stream);
+    return launch_ghk_rows(c.a, in, stream);
 }
 
 int mpvae_probit_backward(const mpvae_probit_params* p_in, void* cuda_stream) {

@@ -11,8 +11,8 @@
 //            then v_s = C^-T (eta - w)                                      (backward solve)
 //   update   x_s = n_s + G[:, O] v_s, in place on nr: R eps_s for an exact draw of eps given u_O = fx_O + C eta_s
 //            (Matheron's rule: prior sample n_s = R xi_s of predict, fresh zeta_s for w_O)
-//   rows     conditional.cu's weights and predict kernels with lw_s in the lp slot: the loss's log-mean-exp, then the
-//            weighted mean of E(fx + x_s) over the samples
+//   rows     predict.cu's conditional weights and predict kernels with lw_s in the lp slot: the loss's log-mean-exp,
+//            then the weighted mean of E(fx + x_s) over the samples
 // With O empty: lw = 0 and no update, so prob is predict's bits.  zeta and U are either the caller's (S, B, L) tensors
 // (read at observed cells only) or a Philox stream with its own key, counter = (s, global row, label), so predict's
 // noise xi is untouched.

@@ -96,7 +96,7 @@ int launch_gxs_bound(RowArgs a, const unsigned int* gp_absmax, unsigned int* out
 int launch_predict_rows(RowArgs a, cudaStream_t stream);                           // after the nt product (a.nr)
 int launch_small_predict(RowArgs a, const SmallNoise& n, cudaStream_t stream);     // small regime, one launch
 
-// Conditional prediction (conditional.cu), after the nt product (a.nr): a.indiv_prob = the importance-weighted mean of E
+// Conditional prediction (predict.cu), after the nt product (a.nr): a.indiv_prob = the importance-weighted mean of E
 // over the samples, weighted by the likelihood of the row's observed labels (observed (B, L) int8: 0 / 1 observed, any
 // other value unobserved); log_evidence (B), ess (B).  Uses part (B * S * row_chunks(L) records), a.lp, a.wts, a.rowaux.
 int launch_conditional_rows(RowArgs a, const int8_t* observed, FusePart* part, float* log_evidence, float* ess,

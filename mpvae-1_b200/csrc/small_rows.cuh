@@ -1,6 +1,6 @@
 // Building blocks of the small-regime kernels (L, Z <= 128, L * Z <= 8192: one CTA per batch row), shared by the loss
 // forward (probit_rows.cu::probit_small_fwd_kernel) and the prediction-only kernel (predict.cu), so that both stage R,
-// draw the noise and contract it in exactly the same way.
+// draw the noise and contract it in exactly the same way.  predict.cu's row passes also take row_of from here.
 #pragma once
 #include "philox.cuh"
 #include "rows.h"

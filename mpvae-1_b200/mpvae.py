@@ -28,7 +28,7 @@ from . import _lib
 from .dense import linear
 from .probit import ProbitELBO, label_pairs, philox_normal, predictive_rho, predictive_scale, probit_predict
 from .probit import contract_nt, ghk_workspace_bytes, predict_exact_from_r, probit_predict_conditional
-from .probit import probit_predict_conditional_ghk
+from .probit import _check_observed, probit_predict_conditional_ghk
 from .probit import predict_pairs as probit_predict_pairs
 
 _state = {"seed": 0x5EED_B200, "offset": 0}
@@ -195,21 +195,33 @@ def predict(fx_out, r_sqrt_sigma, args, noise=None):
     alone (`VAE.feat_forward(feature)[0]`): no labels, no label branch, no loss.  Same S (args.n_test_sample), same
     noise (`noise_plan`: a call without args.noise_offset consumes one offset, as compute_loss does), same flags, and
     bit for bit the indiv_prob compute_loss returns for the same fx_out.  Inference only: it builds no autograd graph."""
-    if torch.is_grad_enabled() and (fx_out.requires_grad or r_sqrt_sigma.requires_grad):
-        raise RuntimeError("mpvae_b200.predict is inference only and returns no gradient: call it under torch.no_grad() "
-                           "(or detach its inputs); compute_loss is the differentiable path")
+    plan = _sample_plan("predict", fx_out, r_sqrt_sigma, args, noise)
+    if plan is None:
+        return fx_out.new_empty((0, fx_out.shape[1]))
+    n_sample, r32, noise, spec, flags = plan
+    return probit_predict(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags)
+
+
+_UNCONDITIONAL = object()     # _sample_plan's `observed` for predict, which conditions on none
+
+
+def _sample_plan(name, fx_out, r_sqrt_sigma, args, noise, observed=_UNCONDITIONAL):
+    """The start of predict, predict_conditional and predict_conditional_ghk: the refusals, in this order, then
+    (n_sample, r32, noise, noise_spec, flags) as compute_loss plans them in test mode, or None for an empty batch."""
+    _inference_only(name, fx_out, r_sqrt_sigma)
     device = fx_out.device
     if device.type != "cuda":
-        raise RuntimeError("mpvae_b200.predict needs CUDA tensors: the probit prediction is implemented as sm_100a "
+        raise RuntimeError(f"mpvae_b200.{name} needs CUDA tensors: the probit prediction is implemented as sm_100a "
                            "kernels only (no CPU fallback)")
-    n_sample = args.n_test_sample
+    if observed is not _UNCONDITIONAL:
+        _check_observed(observed, fx_out.shape, device)
     n_batch = fx_out.shape[0]
     if n_batch == 0:
-        return fx_out.new_empty((0, fx_out.shape[1]))
+        return None
+    n_sample = args.n_test_sample
     r32 = r_sqrt_sigma.to(device).float()
     noise, spec = noise_plan(args, n_sample, n_batch, device, noise)
-    flags = int(getattr(args, "mpvae_flags", 0))
-    return probit_predict(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags)
+    return n_sample, r32, noise, spec, int(getattr(args, "mpvae_flags", 0))
 
 
 ConditionalPrediction = namedtuple("ConditionalPrediction", ["prob", "log_evidence", "ess"])
@@ -234,24 +246,10 @@ def predict_conditional(fx_out, r_sqrt_sigma, observed, args, noise=None):
     = unobserved.  From labels y and a boolean mask of the known ones:
         observed = torch.where(mask, y.to(torch.int8), -1)
     Its values are not checked (no host synchronisation).  Inference only, CUDA only; args.mpvae_flags as for predict."""
-    _inference_only("predict_conditional", fx_out, r_sqrt_sigma)
-    device = fx_out.device
-    if device.type != "cuda":
-        raise RuntimeError("mpvae_b200.predict_conditional needs CUDA tensors: the conditional prediction is implemented "
-                           "as sm_100a kernels only (no CPU fallback)")
-    if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
-        raise TypeError(f"observed must be an int8 tensor, got {getattr(observed, 'dtype', type(observed))}")
-    if observed.shape != fx_out.shape:
-        raise ValueError(f"observed has shape {tuple(observed.shape)}, expected {tuple(fx_out.shape)} (batch, label_dim)")
-    if observed.device != device:
-        raise ValueError(f"observed is on {observed.device}, expected {device}")
-    n_batch = fx_out.shape[0]
-    if n_batch == 0:
+    plan = _sample_plan("predict_conditional", fx_out, r_sqrt_sigma, args, noise, observed)
+    if plan is None:
         return ConditionalPrediction(fx_out.new_empty((0, fx_out.shape[1])), fx_out.new_empty(0), fx_out.new_empty(0))
-    n_sample = args.n_test_sample
-    r32 = r_sqrt_sigma.to(device).float()
-    noise, spec = noise_plan(args, n_sample, n_batch, device, noise)
-    flags = int(getattr(args, "mpvae_flags", 0))
+    n_sample, r32, noise, spec, flags = plan
     return ConditionalPrediction(*probit_predict_conditional(fx_out, r32, observed, n_sample, noise=noise, noise_spec=spec,
                                                              flags=flags))
 
@@ -291,25 +289,12 @@ def predict_conditional_ghk(fx_out, r_sqrt_sigma, observed, args, noise=None, gr
     groups that keep that scratch under GHK_WORKSPACE_BOUND bytes; rows are keyed by their global row, so the split
     changes no bits.  The sampler's own uniforms and normals come from a Philox stream separate from the noise.
     Inference only, CUDA only; args.mpvae_flags as for predict."""
-    _inference_only("predict_conditional_ghk", fx_out, r_sqrt_sigma)
-    device = fx_out.device
-    if device.type != "cuda":
-        raise RuntimeError("mpvae_b200.predict_conditional_ghk needs CUDA tensors: the GHK sampler is implemented as "
-                           "sm_100a kernels only (no CPU fallback)")
-    if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
-        raise TypeError(f"observed must be an int8 tensor, got {getattr(observed, 'dtype', type(observed))}")
-    if observed.shape != fx_out.shape:
-        raise ValueError(f"observed has shape {tuple(observed.shape)}, expected {tuple(fx_out.shape)} (batch, label_dim)")
-    if observed.device != device:
-        raise ValueError(f"observed is on {observed.device}, expected {device}")
+    plan = _sample_plan("predict_conditional_ghk", fx_out, r_sqrt_sigma, args, noise, observed)
     n_batch, L = fx_out.shape
-    if n_batch == 0:
+    if plan is None:
         return ConditionalPrediction(fx_out.new_empty((0, L)), fx_out.new_empty(0), fx_out.new_empty(0))
-    n_sample = args.n_test_sample
-    r32 = r_sqrt_sigma.to(device).float()
+    n_sample, r32, noise, spec, flags = plan
     Z = r32.shape[1]
-    noise, spec = noise_plan(args, n_sample, n_batch, device, noise)
-    flags = int(getattr(args, "mpvae_flags", 0))
     max_obs = int(((observed == 0) | (observed == 1)).sum(1).max().item())      # the one host synchronisation
     one = ghk_workspace_bytes(n_sample, 1, L, Z, max_obs, flags)
     per_row = max(ghk_workspace_bytes(n_sample, 2, L, Z, max_obs, flags) - one, 1)

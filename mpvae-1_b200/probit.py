@@ -21,6 +21,12 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
 
 
+def _stream(dev):
+    # the raw handle of the current stream, without building a torch.cuda.Stream object on every call: small batches
+    # are bound by the host's time per call
+    return C.c_void_p(torch._C._cuda_getCurrentRawStream(dev.index))
+
+
 def _check_tensors(names, tensors):
     dev = tensors[0].device
     for name, t in zip(names, tensors):
@@ -65,6 +71,24 @@ def _check_label_mask(label_mask, B, L, device):
     if label_mask.device != device:
         raise ValueError(f"label_mask is on {label_mask.device}, expected {device}")
     return label_mask.contiguous().view(torch.uint8)
+
+
+def _check_observed(observed, shape, device):
+    """Refuses an `observed` argument that is not an int8 tensor of `shape` (batch, label_dim) on `device`."""
+    if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
+        raise TypeError(f"observed must be an int8 tensor, got {getattr(observed, 'dtype', type(observed))}")
+    if observed.shape != shape:
+        raise ValueError(f"observed has shape {tuple(observed.shape)}, expected {tuple(shape)} (batch, label_dim)")
+    if observed.device != device:
+        raise ValueError(f"observed is on {observed.device}, expected {device}")
+
+
+def _poison(*tensors):
+    """Test hook (MPVAE_POISON_WORKSPACE=1): every scratch byte starts as 0xFF (NaN as fp16 / fp32 / fp64, huge as a
+    counter) and every output as NaN, so anything the kernels read before writing, or leave unwritten, shows."""
+    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
+        for t in tensors:
+            t.fill_(255 if t.dtype == torch.uint8 else float("nan"))
 
 
 def _set_noise_spec(p, spec, B):
@@ -116,12 +140,7 @@ class ProbitELBO(torch.autograd.Function):
             scalars = [torch.empty((), dtype=torch.float32, device=dev) for _ in range(6)]
             prob = torch.empty((B, L), dtype=torch.float32, device=dev)
             prob_label = torch.empty((B, L), dtype=torch.float32, device=dev)
-            if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
-                # test hook (compute-sanitizer --tool initcheck is closed on this pool): every scratch / output byte starts
-                # as 0xFF (NaN as fp16 / fp32 / fp64, huge as a counter), so anything the kernels read before writing shows
-                ws.fill_(255)
-                for t in [prob, prob_label] + scalars:
-                    t.fill_(float("nan"))
+            _poison(ws, prob, prob_label, *scalars)
             p = _lib.ProbitParams()
             p.struct_bytes = C.sizeof(_lib.ProbitParams)
             p.flags = flags
@@ -181,9 +200,7 @@ class ProbitELBO(torch.autograd.Function):
             g_fe_out = torch.empty_like(fe_out)
             g_fx_out = torch.empty_like(fx_out)
             g_mulv = [torch.empty_like(fe_mu) for _ in range(4)]
-            if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
-                for t in [g_fe_out, g_fx_out] + g_mulv:
-                    t.fill_(float("nan"))
+            _poison(g_fe_out, g_fx_out, *g_mulv)
             peer = ctx.peer if need_r else None
             g_r = (torch.empty_like(r32) if peer is None else None) if need_r else None
             p = _lib.ProbitParams()
@@ -215,8 +232,8 @@ class ProbitELBO(torch.autograd.Function):
                 None, None)
 
 
-def _predict_inputs(name, fx_out, r32, S, noise, noise_spec):
-    """The checks of mpvae_probit_predict's inputs: (fx_out, r32, noise) contiguous, and (S, B, L, Z)."""
+def _predict_dims(name, fx_out, r32, S, noise, noise_spec):
+    """The shape checks of a sampled prediction's inputs: (S, B, L, Z)."""
     if noise is None and noise_spec is None:
         raise ValueError(f"{name} needs either a noise tensor or a noise_spec")
     if fx_out.dim() != 2:
@@ -230,21 +247,40 @@ def _predict_inputs(name, fx_out, r32, S, noise, noise_spec):
     Z = r32.shape[1]
     if noise is not None and noise.shape != (S, B, Z):
         raise ValueError(f"noise has shape {tuple(noise.shape)}, expected {(S, B, Z)} (n_sample, batch, z_dim)")
+    return S, B, L, Z
+
+
+def _predict_inputs(name, fx_out, r32, S, noise, noise_spec):
+    """The checks of mpvae_probit_predict's inputs: (fx_out, r32, noise) contiguous, and (S, B, L, Z)."""
+    dims = _predict_dims(name, fx_out, r32, S, noise, noise_spec)
     _check_tensors(("fx_out", "r_sqrt_sigma", "noise"), (fx_out, r32, noise))
-    return fx_out.contiguous(), r32.contiguous(), (noise.contiguous() if noise is not None else None), (S, B, L, Z)
+    return fx_out.contiguous(), r32.contiguous(), (noise.contiguous() if noise is not None else None), dims
 
 
-def _predict_params(fx_out, r32, noise, noise_spec, flags, dims, prob, ws):
+def _run_predict(entry, fx_out, r32, noise, noise_spec, flags, dims, *args, row_outputs=0):
+    """Runs the sampled-prediction entry point `entry` of the library: allocates its workspace, prob (B, L) and
+    `row_outputs` fp32 (B,) outputs, and calls it with the params, `args`, the row outputs and the current stream.
+    Returns [prob, *row outputs]."""
     S, B, L, Z = dims
-    p = _lib.ProbitParams()
-    p.struct_bytes = C.sizeof(_lib.ProbitParams)
-    p.flags = flags
-    p.S, p.B, p.L, p.Z = S, B, L, Z
-    p.fx_out, p.r, p.noise = _ptr(fx_out), _ptr(r32), _ptr(noise)
-    _set_noise_spec(p, noise_spec, B)
-    p.indiv_prob = _ptr(prob)
-    p.workspace, p.workspace_bytes = _ptr(ws), ws.numel()
-    return p
+    lib = _lib.lib()
+    dev = fx_out.device
+    with torch.cuda.device(dev):
+        ws = torch.empty(int(lib.mpvae_workspace_bytes(S, B, L, Z, 0, flags)), dtype=torch.uint8, device=dev)
+        out = [torch.empty((B, L), dtype=torch.float32, device=dev)]
+        for _ in range(row_outputs):
+            out.append(torch.empty(B, dtype=torch.float32, device=dev))
+            args += (_ptr(out[-1]),)
+        _poison(ws, *out)
+        p = _lib.ProbitParams()
+        p.struct_bytes = C.sizeof(_lib.ProbitParams)
+        p.flags = flags
+        p.S, p.B, p.L, p.Z = S, B, L, Z
+        p.fx_out, p.r, p.noise = _ptr(fx_out), _ptr(r32), _ptr(noise)
+        _set_noise_spec(p, noise_spec, B)
+        p.indiv_prob = _ptr(out[0])
+        p.workspace, p.workspace_bytes = _ptr(ws), ws.numel()
+        _lib.check(getattr(lib, entry)(C.byref(p), *args, _stream(dev)), entry)
+    return out
 
 
 def probit_predict(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0):
@@ -252,21 +288,7 @@ def probit_predict(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0):
     of the feature branch, without labels and without the loss.  Bit-equal to `ProbitELBO`'s indiv_prob on the same
     fx_out, R and noise.  `noise` / `noise_spec` as for `ProbitELBO`; inference only (no autograd graph)."""
     fx_out, r32, noise, dims = _predict_inputs("probit_predict", fx_out, r32, S, noise, noise_spec)
-    S, B, L, Z = dims
-    lib = _lib.lib()
-    dev = fx_out.device
-    with torch.cuda.device(dev):
-        ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 0, flags))
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        prob = torch.empty((B, L), dtype=torch.float32, device=dev)
-        if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
-            # test hook: see ProbitELBO.forward
-            ws.fill_(255)
-            prob.fill_(float("nan"))
-        p = _predict_params(fx_out, r32, noise, noise_spec, flags, dims, prob, ws)
-        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        _lib.check(lib.mpvae_probit_predict(C.byref(p), stream), "mpvae_probit_predict")
-    return prob
+    return _run_predict("mpvae_probit_predict", fx_out, r32, noise, noise_spec, flags, dims)[0]
 
 
 def probit_predict_conditional(fx_out, r32, observed, S, *, noise=None, noise_spec=None, flags=0):
@@ -276,32 +298,10 @@ def probit_predict_conditional(fx_out, r32, observed, S, *, noise=None, noise_sp
     unobserved; it is not read on the host.  Observed cells return their value; with nothing observed prob is
     probit_predict's bit for bit.  `noise` / `noise_spec` / `flags` as for probit_predict; inference only."""
     fx_out, r32, noise, dims = _predict_inputs("probit_predict_conditional", fx_out, r32, S, noise, noise_spec)
-    S, B, L, Z = dims
-    if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
-        raise TypeError(f"observed must be an int8 tensor, got {getattr(observed, 'dtype', type(observed))}")
-    if observed.shape != (B, L):
-        raise ValueError(f"observed has shape {tuple(observed.shape)}, expected {(B, L)} (batch, label_dim)")
-    if observed.device != fx_out.device:
-        raise ValueError(f"observed is on {observed.device}, expected {fx_out.device}")
+    _check_observed(observed, dims[1:3], fx_out.device)     # (B, L)
     observed = observed.contiguous()
-    lib = _lib.lib()
-    dev = fx_out.device
-    with torch.cuda.device(dev):
-        ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 0, flags))
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        prob = torch.empty((B, L), dtype=torch.float32, device=dev)
-        log_evidence = torch.empty(B, dtype=torch.float32, device=dev)
-        ess = torch.empty(B, dtype=torch.float32, device=dev)
-        if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
-            # test hook: see ProbitELBO.forward
-            ws.fill_(255)
-            for t in (prob, log_evidence, ess):
-                t.fill_(float("nan"))
-        p = _predict_params(fx_out, r32, noise, noise_spec, flags, dims, prob, ws)
-        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        _lib.check(lib.mpvae_probit_predict_conditional(C.byref(p), _ptr(observed), _ptr(log_evidence), _ptr(ess), stream),
-                   "mpvae_probit_predict_conditional")
-    return prob, log_evidence, ess
+    return tuple(_run_predict("mpvae_probit_predict_conditional", fx_out, r32, noise, noise_spec, flags, dims,
+                              _ptr(observed), row_outputs=2))
 
 
 def ghk_workspace_bytes(S, B, L, Z, max_observed, flags=0):
@@ -316,55 +316,27 @@ def probit_predict_conditional_ghk(fx_out, r32, observed, S, max_observed, *, no
     NaN outputs).  `gram`: the (L, L) fp32 R R^T of `contract_nt(r32, r32)` with the engine mpvae.label_gram picks, or
     None.  `zeta` / `uniform`: optional (S, B, L) fp32 draws for the observed cells (uniform in (0, 1)); None = the
     library's Philox stream.  `noise` / `noise_spec` / `flags` as for probit_predict; inference only."""
-    if fx_out.dim() != 2:
-        raise ValueError(f"fx_out must be (batch, label_dim), got {tuple(fx_out.shape)}")
-    B, L = fx_out.shape
-    if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
-        raise TypeError(f"observed must be an int8 tensor, got {getattr(observed, 'dtype', type(observed))}")
-    if observed.shape != (B, L):
-        raise ValueError(f"observed has shape {tuple(observed.shape)}, expected {(B, L)} (batch, label_dim)")
-    if observed.device != fx_out.device:
-        raise ValueError(f"observed is on {observed.device}, expected {fx_out.device}")
+    dims = _predict_dims("probit_predict_conditional_ghk", fx_out, r32, S, noise, noise_spec)
+    S, B, L, Z = dims
+    _check_observed(observed, (B, L), fx_out.device)
     if not 0 <= int(max_observed) <= L:
         raise ValueError(f"max_observed={max_observed} outside [0, {L}]")
     for name, t, shape in (("gram", gram, (L, L)), ("zeta", zeta, (S, B, L)), ("uniform", uniform, (S, B, L))):
         if t is not None and tuple(t.shape) != shape:
             raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {shape}")
-    fx_out, r32, noise, dims = _predict_inputs("probit_predict_conditional_ghk", fx_out, r32, S, noise, noise_spec)
-    S, B, L, Z = dims
-    _check_tensors(("fx_out", "gram", "zeta", "uniform"), (fx_out, gram, zeta, uniform))
+    tensors = (fx_out, r32, noise, gram, zeta, uniform)
+    _check_tensors(("fx_out", "r_sqrt_sigma", "noise", "gram", "zeta", "uniform"), tensors)
+    fx_out, r32, noise, gram, zeta, uniform = (t.contiguous() if t is not None else None for t in tensors)
     observed = observed.contiguous()
-    gram, zeta, uniform = (t.contiguous() if t is not None else None for t in (gram, zeta, uniform))
-    lib = _lib.lib()
-    dev = fx_out.device
-    with torch.cuda.device(dev):
-        ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 0, flags))
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        gws_bytes = ghk_workspace_bytes(S, B, L, Z, int(max_observed), flags)
-        gws = torch.empty(gws_bytes, dtype=torch.uint8, device=dev)
-        prob = torch.empty((B, L), dtype=torch.float32, device=dev)
-        log_evidence = torch.empty(B, dtype=torch.float32, device=dev)
-        ess = torch.empty(B, dtype=torch.float32, device=dev)
-        if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
-            # test hook: see ProbitELBO.forward
-            ws.fill_(255)
-            gws.fill_(255)
-            for t in (prob, log_evidence, ess):
-                t.fill_(float("nan"))
-        p = _predict_params(fx_out, r32, noise, noise_spec, flags, dims, prob, ws)
-        stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        _lib.check(lib.mpvae_probit_predict_conditional_ghk(C.byref(p), _ptr(observed), _ptr(gram), _ptr(zeta),
-                                                            _ptr(uniform), _ptr(gws), gws_bytes, int(max_observed),
-                                                            _ptr(log_evidence), _ptr(ess), stream),
-                   "mpvae_probit_predict_conditional_ghk")
-    return prob, log_evidence, ess
+    gws_bytes = ghk_workspace_bytes(S, B, L, Z, int(max_observed), flags)
+    gws = torch.empty(gws_bytes, dtype=torch.uint8, device=fx_out.device)
+    _poison(gws)
+    return tuple(_run_predict("mpvae_probit_predict_conditional_ghk", fx_out, r32, noise, noise_spec, flags, dims,
+                              _ptr(observed), _ptr(gram), _ptr(zeta), _ptr(uniform), _ptr(gws), gws_bytes,
+                              int(max_observed), row_outputs=2))
 
 
 # ---- closed-form prediction (csrc/predictive.cu): the S -> infinity limit of probit_predict ----
-
-def _stream(dev):
-    return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-
 
 def _check_f64(name, t, n, dev):
     if not t.is_cuda or t.device != dev:
@@ -399,8 +371,7 @@ def predictive_scale(r32):
     L, Z = r32.shape
     dev = r32.device
     scale = torch.empty(L, dtype=torch.float64, device=dev)
-    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
-        scale.fill_(float("nan"))
+    _poison(scale)
     with torch.cuda.device(dev):
         _lib.check(_lib.lib().mpvae_predictive_scale(_ptr(r32), L, Z, _ptr(scale), _stream(dev)), "mpvae_predictive_scale")
     return scale
@@ -421,8 +392,7 @@ def predictive_rho(r32, scale, pairs):
     rho = torch.empty(P, dtype=torch.float64, device=dev)
     if P == 0:
         return rho
-    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
-        rho.fill_(float("nan"))
+    _poison(rho)
     with torch.cuda.device(dev):
         _lib.check(_lib.lib().mpvae_predictive_rho(_ptr(r32), L, Z, _ptr(scale), _ptr(pairs), P, _ptr(rho), _stream(dev)),
                    "mpvae_predictive_rho")
@@ -442,8 +412,7 @@ def predict_exact(fx_out, scale, flags=0):
     prob = torch.empty((B, L), dtype=torch.float32, device=dev)
     if B == 0:
         return prob
-    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
-        prob.fill_(float("nan"))
+    _poison(prob)
     with torch.cuda.device(dev):
         _lib.check(_lib.lib().mpvae_predict_exact(_ptr(fx_out), B, L, _ptr(scale), int(flags), _ptr(prob), _stream(dev)),
                    "mpvae_predict_exact")
@@ -464,14 +433,11 @@ def predict_exact_from_r(fx_out, r32, flags=0):
     dev = fx_out.device
     scale = fx_out.new_empty(L, dtype=torch.float64)
     prob = fx_out.new_empty((B, L))
-    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
-        scale.fill_(float("nan"))
-        prob.fill_(float("nan"))
+    _poison(scale, prob)
     lib = _lib.lib()
 
     def launch():
-        # the raw handle of the current stream, without building a torch.cuda.Stream object on every batch
-        stream = C.c_void_p(torch._C._cuda_getCurrentRawStream(dev.index))
+        stream = _stream(dev)
         _lib.check(lib.mpvae_predictive_scale(_ptr(r32), L, r32.shape[1], _ptr(scale), stream), "mpvae_predictive_scale")
         if B:
             _lib.check(lib.mpvae_predict_exact(_ptr(fx_out), B, L, _ptr(scale), int(flags), _ptr(prob), stream),
@@ -502,8 +468,7 @@ def predict_pairs(fx_out, scale, pairs, rho, flags=0):
     out = torch.empty((B, P), dtype=torch.float32, device=dev)
     if B == 0 or P == 0:
         return out
-    if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
-        out.fill_(float("nan"))
+    _poison(out)
     with torch.cuda.device(dev):
         _lib.check(_lib.lib().mpvae_predict_pairs(_ptr(fx_out), B, L, _ptr(scale), _ptr(pairs), _ptr(rho), P, int(flags),
                                                   _ptr(out), _stream(dev)), "mpvae_predict_pairs")

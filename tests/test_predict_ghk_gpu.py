@@ -1,6 +1,6 @@
 """GPU: the GHK conditional prediction (mpvae_probit_predict_conditional_ghk: the nt product, the G product,
-ghk_gather_kernel, ghk_factor_kernel, ghk_chain_kernel, ghk_update_kernel, then conditional.cu's weights and predict
-kernels) against predict with nothing observed, its exact cases (R = 0, one observed label), the fp64 oracle on the same
+ghk_gather_kernel, ghk_factor_kernel, ghk_chain_kernel, ghk_update_kernel, then predict.cu's conditional weights and
+predict kernels) against predict with nothing observed, its exact cases (R = 0, one observed label), the fp64 oracle on the same
 draws, quadrature, the importance path and PairPredictor; a planted model where it must beat the importance path; and
 batching, row groups, repetition, a poisoned workspace, a prepared G, offsets and launch counts."""
 import math
