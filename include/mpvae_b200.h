@@ -257,16 +257,21 @@ int mpvae_philox_normal(float *noise, int32_t S, int32_t B, int32_t Z, int32_t B
 #define MPVAE_ENGINE_KSPLIT 0x100
 int mpvae_contract_nt(const float *A, const float *Bm, float *C, int32_t M, int32_t N, int32_t K, int32_t engine,
                       void *workspace, uint64_t workspace_bytes, void *cuda_stream);
-/* Same with a row pitch of ldc >= N floats for C.  The loss kernels keep noise.R^T in rows padded to 16 bytes
- * (ldc = N rounded up to 4) so that the GEMM epilogue can use 16-byte stores; this entry times exactly that variant. */
+/* Same with a row pitch of ldc >= N floats for C.  Only columns [0, N) of rows [0, M) are written: the columns
+ * [N, ldc) and everything past the last row are left as they are, for every engine and ldc.  The loss kernels keep
+ * noise.R^T in rows padded to 16 bytes (ldc = N rounded up to 4) so that the GEMM epilogue can use 16-byte stores;
+ * this entry times that variant (the loss path itself may also fill its own row padding, which this entry never does). */
 int mpvae_contract_nt_pitched(const float *A, const float *Bm, float *C, int32_t M, int32_t N, int32_t K, int32_t ldc,
                               int32_t engine, void *workspace, uint64_t workspace_bytes, void *cuda_stream);
 
 /* The tcgen05 engine in stages, for callers that use an operand more than once (mpvae_b200/dense.py: a layer's input
  * planes serve its forward and its weight gradient, the output-gradient planes both backward products):
- *   mpvae_tc_split      fp32 [rows][cols] -> operand planes [hi|lo][rows][pitch] (mpvae_tc_planes_bytes) + the max |x|
- *                       slot (4 bytes, device) that fixes the power-of-two scale of the fp16 pieces
- *   mpvae_tc_gemm_nt    C[M,N] (pitch ldc) = A[M,K] . B[N,K]^T from planes;  ksplit != 0 allows K-sliced partial waves
+ *   mpvae_tc_split      fp32 [rows][cols] (cols >= 8) -> operand planes [hi|lo][rows][pitch] (mpvae_tc_planes_bytes)
+ *                       + the max |x| slot (4 bytes, device) that fixes the power-of-two scale s = 2^(14 - e) of the
+ *                       fp16 pieces: e is the exponent of the largest FINITE |x|, clamped to [-112, 127]; an all-zero
+ *                       or non-finite-only tensor gets s = 1.  An Inf element is the piece pair (+-Inf, 0).
+ *   mpvae_tc_gemm_nt    C[M,N] (pitch ldc >= N, 0 = N) = A[M,K] . B[N,K]^T from planes; writes columns [0, N) of
+ *                       rows [0, M) only;  ksplit != 0 allows K-sliced partial waves
  *   mpvae_tc_gemm_tn    C[N1,N2] = A[M,N1]^T . B[M,N2] from planes
  * tail_scratch: mpvae_tc_tail_scratch_bytes() of device memory (may be NULL: no K-slicing). */
 uint64_t mpvae_tc_planes_bytes(int32_t rows, int32_t cols);

@@ -329,9 +329,10 @@ int dense_nt_product(const mpvae_probit_params* p, const Workspace& w, const Fus
     ProfScope ps(MPVAE_PROF_PRODUCT_NT, stream);
     // library noise sits on the fp16 grid: one plane, two MMA passes.
     // No tail scratch here: K-slicing the last wave would make the summation order of x = noise.R^T depend on
-    // how many rows the call holds, and a row's predictions must not change with the shard it is computed in
+    // how many rows the call holds, and a row's predictions must not change with the shard it is computed in.
+    // nr's rows are padded to 16 bytes inside the workspace: the product may fill the padding with whole-vector stores.
     return tc_gemm_nt(npl, rpl, nr, M, p->L, p->Z, nullptr, slots + SLOT_ABSMAX_R, stream, row_pitch(p->L), p->noise ? 0 : 1,
-                      nullptr, 0, fz, jit_noise ? &fnz : nullptr);
+                      nullptr, 0, fz, jit_noise ? &fnz : nullptr, 1);
 }
 
 // CUDA-core regime, up to and including the product: the Philox normals (unless the caller gives the noise) and

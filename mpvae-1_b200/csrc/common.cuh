@@ -23,20 +23,49 @@ static inline int ceil_div(int a, int b) { return (a + b - 1) / b; }
 // Per-tensor power-of-two scale of the fp16 operand split (contract_tc.cu): s = 2^(14 - e) with e the exponent of
 // `bits` (max |x|, or an upper bound of it, as raw fp32 bits), so that max|x| * s lies in [2^14, 2^15): one binade
 // under the fp16 maximum, which keeps the hi piece normal for elements down to 2^-28 of the maximum and the lo piece
-// normal down to 2^-17 of it.  0, Inf or NaN (e.g. the NaN gradients of degenerate rows) -> s = 1, values pass through.
+// normal down to 2^-17 of it.  e is clamped to [-112, 127], where s and 1 / s are both fp32 normals: every finite
+// maximum from 2^-112 up is scaled into [2^14, 2^15); a smaller one only scales to less.  0, Inf or NaN (e.g. the NaN
+// gradients of degenerate rows) -> s = 1, values pass through.  The function returns log2(s).
 #ifdef __CUDACC__
 __host__ __device__
 #endif
-static inline float scale_from_absmax_bits(uint32_t bits) {
+static inline int scale_exp_from_absmax_bits(uint32_t bits) {
     bits &= 0x7FFFFFFFu;
-    if (bits == 0u || bits >= 0x7F800000u) return 1.0f;
+    if (bits == 0u || bits >= 0x7F800000u) return 0;
     int e = (int)(bits >> 23) - 127;
-    if (e < -100) e = -100;
-    if (e > 100) e = 100;
-    const uint32_t sb = (uint32_t)(127 + 14 - e) << 23;
+    if (e < -112) e = -112;
+    return 14 - e;
+}
+
+// 2^k as fp32 for k in [-126, 127]
+#ifdef __CUDACC__
+__host__ __device__
+#endif
+static inline float pow2f(int k) {
+    const uint32_t b = (uint32_t)(127 + k) << 23;
     float f;
-    memcpy(&f, &sb, 4);
+    memcpy(&f, &b, 4);
     return f;
+}
+
+#ifdef __CUDACC__
+__host__ __device__
+#endif
+static inline float scale_from_absmax_bits(uint32_t bits) { return pow2f(scale_exp_from_absmax_bits(bits)); }
+
+// Undoing both operands' scales: a product accumulated from scaled pieces is multiplied by 2^-(ka + kb), which lies in
+// [2^-252, 2^226] and so is not always one fp32 number.  It is applied as two powers of two: `extra` first, then `main`
+// = 2^clamp(-(ka + kb), -126, 127).  Either order of the two products is exact whenever the descaled value is an fp32
+// normal (the intermediate then lies between the scaled and the descaled value); when the whole factor fits one fp32
+// number, extra = 1 and the result is the single product acc * main.
+struct Descale { float main, extra; };
+#ifdef __CUDACC__
+__host__ __device__
+#endif
+static inline Descale descale_from_absmax_bits(uint32_t a_bits, uint32_t b_bits) {
+    const int k = -(scale_exp_from_absmax_bits(a_bits) + scale_exp_from_absmax_bits(b_bits));
+    const int km = k < -126 ? -126 : (k > 127 ? 127 : k);
+    return {pow2f(km), pow2f(k - km)};
 }
 
 #ifdef __CUDACC__

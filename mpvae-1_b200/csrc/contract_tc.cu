@@ -213,9 +213,11 @@ __device__ __forceinline__ void store_row64(float* __restrict__ dst, const float
 // last, partial wave may be cut into `ksplit` slices of K so that the wave keeps every pair busy for 1/ksplit of a
 // tile time instead of leaving most of them idle for a whole one: slice 0 writes C, slice j > 0 writes a 256 x 256
 // scratch tile that tail_fixup_kernel adds to C afterwards (fixed order -> reproducible).
+// store_cols: the epilogue writes columns [0, store_cols) of a row, Nc unless the caller owns the row padding up to ldc
+// (the loss path's 16-byte rows, capi.cu) and lets the last 64-column block of a row go out as 16-byte stores.
 struct GemmArgs {
     float* C;
-    int Mc, Nc, K, ldc, tiles_m, tiles_n, kc;
+    int Mc, Nc, K, ldc, store_cols, tiles_m, tiles_n, kc;
     const uint32_t *absmax_a, *absmax_b;
     int full_tiles, ksplit;
     float* partials;
@@ -388,9 +390,10 @@ gemm_split_2sm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
     } else {   // --------------------------------------------------- promotion + epilogue (both CTAs, own 128 rows)
         if (FUSE) reg_inc<kRegEpi>();
         const int q = warp & 3, h = (warp - kFirstEpi) >> 2;      // TMEM lane quadrant = warp id mod 4
-        const float sa = g.absmax_a ? scale_from_absmax_bits(*g.absmax_a) : 1.0f;
-        const float sb = g.absmax_b ? scale_from_absmax_bits(*g.absmax_b) : 1.0f;
-        const float inv_scale = 1.0f / (sa * sb);                // powers of two: exact
+        // 1 / (s_a * s_b) as two powers of two (common.cuh): exact for every normal result; extra == 1 unless the two
+        // scales together leave the fp32 exponent range
+        const Descale ds = descale_from_absmax_bits(g.absmax_a ? *g.absmax_a : 0u, g.absmax_b ? *g.absmax_b : 0u);
+        const float inv_scale = ds.main;
         const bool vec_store = (g.ldc & 3) == 0 && (reinterpret_cast<uintptr_t>(g.C) & 15u) == 0;
         float acc[64];
 #pragma unroll
@@ -420,6 +423,10 @@ gemm_split_2sm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
             }
             const int row = (st / g.tiles_n) * 256 + (int)rank * BM + q * 32 + lane;
             const int col0 = (st % g.tiles_n) * BN + h * 64;
+            if (ds.extra != 1.0f) {   // extreme operand scales only (uniform over the CTA)
+#pragma unroll
+                for (int j = 0; j < 64; ++j) acc[j] *= ds.extra;
+            }
             if (it.slice > 0) {
                 // K-slice of a tail tile: the whole 256 x 256 scratch tile is written (rows / columns beyond the
                 // matrix hold sums of zero-filled boxes, i.e. zeros)
@@ -431,8 +438,9 @@ gemm_split_2sm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
                         make_float4(acc[j] * inv_scale, acc[j + 1] * inv_scale, acc[j + 2] * inv_scale, acc[j + 3] * inv_scale);
             } else if (row < g.Mc && col0 < g.Nc) {
                 float* __restrict__ crow = g.C + (size_t)row * g.ldc;
-                if (vec_store && col0 + 64 <= g.ldc) {
-                    // 16-byte stores: rows are 16 B aligned (ldc % 4 == 0); columns in [Nc, ldc) are pitch padding
+                if (vec_store && col0 + 64 <= g.store_cols) {
+                    // 16-byte stores: rows are 16 B aligned (ldc % 4 == 0); columns in [Nc, store_cols) are padding
+                    // the caller owns
 #pragma unroll
                     for (int j = 0; j < 64; j += 4)
                         *reinterpret_cast<float4*>(crow + col0 + j) =
@@ -492,7 +500,14 @@ tail_fixup_kernel(float* __restrict__ C, int Mc, int Nc, int ldc, int tiles_n, i
 }
 
 // ------------------------------------------------------------------------------------------------ pre-passes
-// max |x| as raw fp32 bits (ordering of non-negative floats == ordering of their bit patterns; NaN sorts highest)
+// |x| as raw fp32 bits, 0 for Inf and NaN
+__device__ __forceinline__ uint32_t finite_abs_bits(uint32_t b) {
+    b &= 0x7FFFFFFFu;
+    return b < 0x7F800000u ? b : 0u;
+}
+
+// max |x| over the FINITE elements as raw fp32 bits (ordering of non-negative floats == ordering of their bit
+// patterns): an Inf or NaN element must not cost the finite ones their scale
 __global__ void __launch_bounds__(256)
 absmax_kernel(const float* __restrict__ src, size_t n, uint32_t* __restrict__ out) {
     uint32_t m = 0;
@@ -503,13 +518,13 @@ absmax_kernel(const float* __restrict__ src, size_t n, uint32_t* __restrict__ ou
         const uint4* __restrict__ s4 = reinterpret_cast<const uint4*>(src);
         for (size_t i = tid; i < n4; i += nthr) {
             const uint4 v = s4[i];
-            const uint32_t a = max(max(v.x & 0x7FFFFFFFu, v.y & 0x7FFFFFFFu), max(v.z & 0x7FFFFFFFu, v.w & 0x7FFFFFFFu));
+            const uint32_t a = max(max(finite_abs_bits(v.x), finite_abs_bits(v.y)), max(finite_abs_bits(v.z), finite_abs_bits(v.w)));
             m = a > m ? a : m;
         }
         done = n4 * 4;
     }
     for (size_t i = done + tid; i < n; i += nthr) {
-        const uint32_t b = __float_as_uint(src[i]) & 0x7FFFFFFFu;
+        const uint32_t b = finite_abs_bits(__float_as_uint(src[i]));
         m = b > m ? b : m;
     }
 #pragma unroll
@@ -527,7 +542,8 @@ absmax_kernel(const float* __restrict__ src, size_t n, uint32_t* __restrict__ ou
     }
 }
 
-// hi = fp16(x * s), lo = fp16(x * s - hi) with s from the tensor's absmax; four elements per thread.  dst planes are
+// hi = fp16(x * s), lo = fp16(x * s - hi) with s from the tensor's absmax; lo = 0 where x is infinite (Inf - Inf
+// would make it NaN; x * s of a finite x stays below 2^15); four elements per thread.  dst planes are
 // [rows][dpitch], pad columns zero.  perm_S > 0: the source rows are s-major (r = s * perm_B + b, the (S, B, Z) noise
 // tensor of mpvae.py:162) and are written b-major (b * perm_S + s), the row order of the loss path's products.
 __global__ void __launch_bounds__(256)
@@ -544,7 +560,10 @@ split_f16_kernel(const float* __restrict__ src, __half* __restrict__ dst, int ro
         for (int j = 0; j < 4; ++j) x[j] = (c + j < cols) ? sp[j] * s : 0.0f;
         __half h[4], l[4];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) { h[j] = __float2half_rn(x[j]); l[j] = __float2half_rn(x[j] - __half2float(h[j])); }
+        for (int j = 0; j < 4; ++j) {
+            h[j] = __float2half_rn(x[j]);
+            l[j] = __hisinf(h[j]) ? __float2half_rn(0.0f) : __float2half_rn(x[j] - __half2float(h[j]));
+        }
         const __half2 h01 = __halves2half2(h[0], h[1]), h23 = __halves2half2(h[2], h[3]);
         const __half2 l01 = __halves2half2(l[0], l[1]), l23 = __halves2half2(l[2], l[3]);
         uint2 hv, lv;
@@ -699,9 +718,10 @@ template <bool MN>
 int launch_gemm(const CUtensorMap& a, const CUtensorMap& b, float* C, int Mc, int Nc, int K, int ldc, const uint32_t* ma,
                 const uint32_t* mb, cudaStream_t stream, int ex, float* partials, size_t partials_bytes,
                 const FuseFwd* fuse = nullptr, const FuseNoise* noise = nullptr, const FusePeer* peer = nullptr,
-                int* exchanged_tiles = nullptr, int peer_mode = 3) {
+                int* exchanged_tiles = nullptr, int peer_mode = 3, bool write_pad = false) {
     GemmArgs g{};
     g.C = C; g.Mc = Mc; g.Nc = Nc; g.K = K; g.ldc = ldc;
+    g.store_cols = write_pad ? ldc : Nc;
     g.tiles_m = ceil_div(Mc, 256); g.tiles_n = ceil_div(Nc, BN);
     // k-blocks per TMEM chunk: the same number of truncating MMAs per chunk (48) whether a k-step is 3 or 2 MMAs
     g.kc = chunk_kblocks(ex == 0 ? Geo<MN>::default_kc : (Geo<MN>::default_kc * 3) / 2);
@@ -890,14 +910,14 @@ size_t tc_tail_scratch_bytes() { return (size_t)(kNumSMs / 2 - 1) * 2 * 256 * BN
 
 int tc_gemm_nt(const void* a_planes, const void* b_planes, float* C, int M, int N, int K, const uint32_t* absmax_a,
                const uint32_t* absmax_b, cudaStream_t stream, int ldc, int a_exact, void* tail_scratch, size_t tail_scratch_bytes,
-               const FuseFwd* fuse, const FuseNoise* noise) {
+               const FuseFwd* fuse, const FuseNoise* noise, int write_pad) {
     if (ldc <= 0) ldc = N;
     const int kp = pitch_of(K);
     CUtensorMap ma, mb;
     if (int rc = make_map(&ma, a_planes, K, M, kp, 64, BM, a_exact ? 1 : 2)) return rc;
     if (int rc = make_map(&mb, b_planes, K, N, kp, 64, HB)) return rc;
     return launch_gemm<false>(ma, mb, C, M, N, K, ldc, absmax_a, absmax_b, stream, a_exact ? 1 : 0, static_cast<float*>(tail_scratch),
-                              tail_scratch_bytes, fuse, noise);
+                              tail_scratch_bytes, fuse, noise, nullptr, nullptr, 3, write_pad != 0);
 }
 
 int tc_gemm_tn(const void* a_planes, const void* b_planes, float* C, int M, int N1, int N2, const uint32_t* absmax_a,

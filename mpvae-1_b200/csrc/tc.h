@@ -42,15 +42,18 @@ int tc_philox_planes(void* planes, int S, int B, int Z, int B_global, int row0, 
 // a_exact / b_exact: that operand lies exactly on the 11-bit piece grid and is stored as ONE plane (the library's own
 // Philox noise): two MMA passes instead of three.
 // fuse != nullptr: the kernel also runs the probit row forward on its finished tiles (fused_rows.cuh; no K-slicing).
+// Columns [N, ldc) of C are left alone unless write_pad != 0: then they are padding the caller owns, and the epilogue
+// may fill them (with zeros) to store whole 16-byte vectors.
 int tc_gemm_nt(const void* a_planes, const void* b_planes, float* C, int M, int N, int K, const uint32_t* absmax_a,
                const uint32_t* absmax_b, cudaStream_t stream, int ldc = 0, int a_exact = 0,   // ldc: pitch of C (0 = N)
                void* tail_scratch = nullptr, size_t tail_scratch_bytes = 0, const FuseFwd* fuse = nullptr,
-               const FuseNoise* noise = nullptr);   // noise != nullptr: a_planes is written by the kernel itself (a_exact)
+               const FuseNoise* noise = nullptr,    // noise != nullptr: a_planes is written by the kernel itself (a_exact)
+               int write_pad = 0);
 // tail_scratch (optional, tc_tail_scratch_bytes()): lets the kernel cut the tiles of the last, partial wave of its
 // persistent grid into K-slices so that the wave does not leave most SMs idle.
 size_t tc_tail_scratch_bytes();
 int tc_pitch(int cols);                                      // plane row pitch (elements) for `cols` columns
-int tc_absmax(const float* src, size_t n, uint32_t* out_bits, cudaStream_t stream);   // atomicMax of |x| bits into *out
+int tc_absmax(const float* src, size_t n, uint32_t* out_bits, cudaStream_t stream);   // atomicMax of finite |x| bits into *out
 int tc_gemm_tn(const void* a_planes, const void* b_planes, float* C, int M, int N1, int N2, const uint32_t* absmax_a,
                const uint32_t* absmax_b, cudaStream_t stream, int b_exact = 0, void* tail_scratch = nullptr,
                size_t tail_scratch_bytes = 0, int a_pitch = 0,

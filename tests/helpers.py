@@ -105,3 +105,42 @@ def rel_err_l2_trimmed(a, b, drop=0.02):
     den = float(np.sqrt(np.sum(b[keep] ** 2)))
     num = float(np.sqrt(np.sum(err[keep])))
     return 0.0 if num == 0 else num / max(den, 1e-300)
+
+
+# ----------------------------------------------------------------------------- element-wise bound of the tcgen05 product
+def contract_c_rel(K, ksplit=False):
+    """c_rel(K) of the split-precision product's element-wise error model (derivation: tests/test_contract_bound_gpu.py).
+    K is the reduction length (M for the tn product)."""
+    k_blocks = -(-K // 64)
+    chunks = -(-k_blocks // 4)                 # TMEM chunks of kc k-blocks: kc = 4 (three-pass), 6 (two-pass)
+    rounds = chunks + (14 if ksplit else 0)    # a K-sliced tail tile: up to 8 slices, each a chunk more and a fix-up add
+    return 3 * 2.0 ** -22 + 8e-7 + 12 * 2.0 ** -23 + rounds * 2.0 ** -24
+
+
+def contract_bound(a, b, ksplit=False):
+    """For C = a . b^T (a: M x K, b: N x K, any float dtype, on the device), in fp64:
+        ref   = a . b^T
+        bound = c_rel(K) |a| . |b|^T + 2^-38 (max|a| ||b_j||_1 + max|b| ||a_i||_1)
+    The second term is the floor of the per-tensor scale: pieces of entries below ~2^-17 of their tensor's maximum carry
+    fewer than 22 bits."""
+    a, b = a.double(), b.double()
+    ref = a @ b.T
+    aa, ab = a.abs(), b.abs()
+    floor = 2.0 ** -38 * (aa.max() * ab.sum(1)[None, :] + ab.max() * aa.sum(1)[:, None])
+    return ref, contract_c_rel(a.shape[1], ksplit) * (aa @ ab.T) + floor
+
+
+def assert_within_contract_bound(got, a, b, ksplit=False, what="", extra=None):
+    """Every element of `got` (= a . b^T computed by the engine) within contract_bound; `extra` is added to the bound
+    (a caller's own rounding after the product).  Returns the worst error / bound ratio."""
+    ref, bound = contract_bound(a, b, ksplit)
+    if extra is not None:
+        bound = bound + extra
+    err = (got.double() - ref).abs()
+    bad = ~(err <= bound)                      # NaN counts as a violation
+    if bool(bad.any()):
+        i, j = [int(v) for v in bad.nonzero()[0]]
+        raise AssertionError(f"{what}: {int(bad.sum())} of {err.numel()} elements outside the bound; first ({i}, {j}): "
+                             f"got {float(got[i, j])!r} want {float(ref[i, j])!r} err {float(err[i, j]):.3e} "
+                             f"bound {float(bound[i, j]):.3e}")
+    return float((err / bound.clamp_min(1e-300)).max())

@@ -254,6 +254,14 @@ def test_tensor_linear_matches_fp64_linear(B, n_in, n_out, x_grad):
         err = H.rel_err(got[k].cpu().numpy(), truth[k].cpu().numpy())
         err32 = H.rel_err(ref32[k].cpu().numpy(), truth[k].cpu().numpy())
         assert err <= max(3e-6, 2 * err32), (k, err, err32)
+    # element by element, the split-precision product's error bound (tests/test_contract_bound_gpu.py): y less its bias
+    # (plus the bias add's own rounding), gx = gy . W and gW = gy^T . x, K-sliced partial waves allowed
+    xd32, wd32 = x.detach(), layer.weight.detach()
+    H.assert_within_contract_bound(got["y"].double() - bd, xd32, wd32, ksplit=True, what="y",
+                                   extra=2.0 ** -24 * ((xd.abs() @ wd.abs().T) + bd.abs()))
+    H.assert_within_contract_bound(got["gw"], gy.T, xd32.T, ksplit=True, what="gW")
+    if x_grad:
+        H.assert_within_contract_bound(got["gx"], gy, wd32.T, ksplit=True, what="gx")
 
 
 def test_fused_adam_state_dict_round_trip():
