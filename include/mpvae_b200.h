@@ -218,6 +218,33 @@ int mpvae_probit_predict_conditional_ghk(const mpvae_probit_params *p, const int
                                          const float *zeta, const float *uniform, void *ghk_ws, uint64_t ghk_ws_bytes,
                                          int32_t max_observed, float *log_evidence, float *ess, void *cuda_stream);
 
+/* Joint label samples of the probit predictive distribution: for each of the S samples mpvae_probit_predict draws, the
+ * whole label vector y_s ~ P(y | x), y_{s,b,l} = (U_{s,b,l} < E_{s,b,l}) with E the clamped probit that
+ * mpvae_probit_predict averages (the same noise, offset and regime, so mean_s y is an unbiased estimate of its output).
+ *   uniform   (S, B, L) fp32 in the open interval (0, 1), or NULL: a Philox stream with its own key (the seed xor-ed with
+ *             a constant of its own), one call per (sample, noise_row0 + row, four labels), U = (k + 1/2) 2^-24 from 24
+ *             bits k; the comparison is exact.  Keyed by global row, so a row's draws do not depend on batching.
+ *   bits      (B, S, W) int32 words, W = ceil(L / 32): label l of sample s is bit l % 32 of word l / 32; bits at and above
+ *             L are zero.  Viewed as bytes on a little-endian host, a sample row has train.pack_labels' bit order.
+ * Reads what mpvae_probit_predict reads (indiv_prob is not written and may be NULL).  STABLE_CDF, CONTRACT_FMA,
+ * CONTRACT_TENSOR and SEPARATE_NOISE apply as for mpvae_probit_predict; the other flags are ignored.  Same workspace. */
+int mpvae_probit_sample_labels(const mpvae_probit_params *p, const float *uniform, int32_t *bits, void *cuda_stream);
+
+/* The set of labels that maximises the expected F_beta over the empirical distribution of S label samples per row (the
+ * GFM algorithm of Dembczynski et al., NIPS 2011), on bits in mpvae_probit_sample_labels' layout.  Per row, with
+ * s_i = |y_i|, U_b the labels set in any sample and P0 the share of empty samples:
+ *   Delta_{l,k} = (1/S) sum_i y_{i,l} (1 + beta^2) / (beta^2 s_i + k)      (fp64, samples added in order)
+ *   EF(k) = the sum of the k largest Delta_{., k}, k = 1 .. min(|U_b|, max_size);  EF(0) = P0  (F(empty, empty) = 1)
+ *   set_size[b] = k*, the smallest k with the largest EF;  expected_f[b] = EF(k*)
+ *   sets[b, l] = 1 for the top k* labels of Delta_{., k*} (ties to the lower label index), 0 elsewhere
+ * The result is the exact optimum over all sets of at most max_size labels (>= 0; L for no bound): sizes above |U_b| only
+ * score less.  Bits at and above L in a sample's last word are ignored, whatever they hold.  The cost grows as
+ * min(|U_b|, max_size) * |U_b| * S per row.  beta > 0 with beta^2 finite (beta < ~1.3e154).
+ * ws >= mpvae_f1_sets_workspace_bytes(B, S, L) bytes, 256-byte aligned.  One launch; deterministic bits. */
+uint64_t mpvae_f1_sets_workspace_bytes(int32_t B, int32_t S, int32_t L);
+int mpvae_f1_sets(const int32_t *bits, int32_t B, int32_t S, int32_t L, double beta, int32_t max_size, uint8_t *sets,
+                  double *expected_f, int32_t *set_size, void *ws, uint64_t ws_bytes, void *cuda_stream);
+
 /* Backward: the autograd backward of compute_loss (implicit in the reference, train.py:125),
  * closed form in SURVEY.md 8(a-12).  Must follow a forward on the same workspace. */
 int mpvae_probit_backward(const mpvae_probit_params *p, void *cuda_stream);

@@ -35,6 +35,7 @@ EXPORTS = (
     "mpvae_predictive_scale", "mpvae_predictive_rho", "mpvae_predict_exact", "mpvae_predict_pairs",
     "mpvae_probit_predict_conditional", "mpvae_probit_forward_masked", "mpvae_probit_backward_masked",
     "mpvae_ghk_workspace_bytes", "mpvae_probit_predict_conditional_ghk",
+    "mpvae_probit_sample_labels", "mpvae_f1_sets_workspace_bytes", "mpvae_f1_sets",
 )
 
 _f = C.c_void_p  # device pointer
@@ -99,6 +100,13 @@ def _load():
     lib.mpvae_probit_predict_conditional_ghk.restype = C.c_int
     lib.mpvae_probit_predict_conditional_ghk.argtypes = [C.POINTER(ProbitParams)] + [C.c_void_p] * 5 + [
         C.c_uint64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.mpvae_probit_sample_labels.restype = C.c_int
+    lib.mpvae_probit_sample_labels.argtypes = [C.POINTER(ProbitParams), C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.mpvae_f1_sets_workspace_bytes.restype = C.c_uint64
+    lib.mpvae_f1_sets_workspace_bytes.argtypes = [C.c_int32] * 3
+    lib.mpvae_f1_sets.restype = C.c_int
+    lib.mpvae_f1_sets.argtypes = [C.c_void_p] + [C.c_int32] * 3 + [C.c_double, C.c_int32] + [C.c_void_p] * 4 + [
+        C.c_uint64, C.c_void_p]
     lib.mpvae_probit_backward.restype = C.c_int
     lib.mpvae_probit_backward.argtypes = [C.POINTER(ProbitParams), C.c_void_p]
     for fn in (lib.mpvae_probit_forward_masked, lib.mpvae_probit_backward_masked):

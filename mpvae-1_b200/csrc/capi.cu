@@ -209,8 +209,8 @@ int validate(const mpvae_probit_params* p, bool backward) {
     return check_workspace(p, backward);
 }
 
-// mpvae_probit_predict reads fx_out, r, the noise fields and indiv_prob only
-int validate_predict(const mpvae_probit_params* p) {
+// mpvae_probit_predict reads fx_out, r, the noise fields and indiv_prob only (mpvae_probit_sample_labels: no indiv_prob)
+int validate_predict(const mpvae_probit_params* p, bool writes_prob) {
     if (p->S <= 0 || p->B <= 0 || p->L <= 0 || p->Z <= 0) {
         set_error("bad sizes S=%d B=%d L=%d Z=%d (empty batches are handled by the host wrapper)", p->S, p->B, p->L, p->Z);
         return 1;
@@ -218,7 +218,7 @@ int validate_predict(const mpvae_probit_params* p) {
     if ((long long)p->S * p->B > 0x7fffffffLL) { set_error("S*B overflows int32"); return 1; }
     if (!p->fx_out || !p->r || !p->workspace) { set_error("NULL input pointer (fx_out/r/workspace)"); return 1; }
     if (int rc = check_noise_rows(p)) return rc;
-    if (!p->indiv_prob) { set_error("NULL forward output pointer (indiv_prob)"); return 1; }
+    if (writes_prob && !p->indiv_prob) { set_error("NULL forward output pointer (indiv_prob)"); return 1; }
     return check_workspace(p, false);
 }
 
@@ -362,10 +362,10 @@ struct PredictCall {
     RowArgs a;
 };
 
-int open_predict(const mpvae_probit_params* p_in, PredictCall& c) {
+int open_predict(const mpvae_probit_params* p_in, PredictCall& c, bool writes_prob = true) {
     c.p = normalize(p_in, &c.tmp);
     if (!c.p) return 1;
-    if (int rc = validate_predict(c.p)) return rc;
+    if (int rc = validate_predict(c.p, writes_prob)) return rc;
     c.w = carve(c.p->S, c.p->B, c.p->L, c.p->Z, false, c.p->flags);
     c.a = row_args(c.p, c.w);
     return 0;
@@ -539,6 +539,57 @@ int mpvae_probit_predict_conditional(const mpvae_probit_params* p_in, const int8
     if (int rc = predict_product(c, stream)) return rc;
     ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
     return launch_conditional_rows(c.a, observed, part, log_evidence, ess, stream);
+}
+
+int mpvae_probit_sample_labels(const mpvae_probit_params* p_in, const float* uniform, int32_t* bits, void* cuda_stream) {
+    PredictCall c;
+    if (int rc = open_predict(p_in, c, false)) return rc;
+    const mpvae_probit_params* p = c.p;
+    if (!bits) { set_error("NULL pointer (bits)"); return 1; }
+    if (!uniform && (p->noise_row0 < 0 || p->noise_b_global < p->noise_row0 + p->B)) {
+        set_error("label draws: rows [%d, %d) do not fit a global batch of %d", p->noise_row0, p->noise_row0 + p->B,
+                  p->noise_b_global);
+        return 1;
+    }
+    cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
+    // the CUDA-core product also where predict takes the one-launch small kernel, which never materialises nr
+    if (int rc = predict_product(c, stream)) return rc;
+    SampleInputs in{};
+    in.uniform = uniform;
+    in.bits = bits;
+    in.noise_b_global = p->noise_b_global; in.noise_row0 = p->noise_row0;
+    in.noise_seed = p->noise_seed; in.noise_offset = p->noise_offset; in.noise_offset_dev = p->noise_offset_dev;
+    ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
+    return launch_sample_labels(c.a, in, stream);
+}
+
+uint64_t mpvae_f1_sets_workspace_bytes(int32_t B, int32_t S, int32_t L) {
+    if (B <= 0 || S <= 0 || L <= 0) return 256;
+    return f1_layout(B, S, L).total;
+}
+
+int mpvae_f1_sets(const int32_t* bits, int32_t B, int32_t S, int32_t L, double beta, int32_t max_size, uint8_t* sets,
+                  double* expected_f, int32_t* set_size, void* ws, uint64_t ws_bytes, void* cuda_stream) {
+    if (B <= 0 || S <= 0 || L <= 0) {
+        set_error("bad sizes B=%d S=%d L=%d (empty batches are handled by the host wrapper)", B, S, L);
+        return 1;
+    }
+    if (!(beta > 0.0) || !isfinite(beta * beta)) {   // beta^2 enters every weight: it must be finite too
+        set_error("beta=%g must be positive with a finite square", beta);
+        return 1;
+    }
+    if (max_size < 0) { set_error("max_size=%d must be >= 0", max_size); return 1; }
+    if (!bits || !sets || !expected_f || !set_size || !ws) {
+        set_error("NULL pointer (bits/sets/expected_f/set_size/ws)");
+        return 1;
+    }
+    const uint64_t need = mpvae_f1_sets_workspace_bytes(B, S, L);
+    if (ws_bytes < need) {
+        set_error("f1 sets workspace too small: %llu < %llu bytes", (unsigned long long)ws_bytes, (unsigned long long)need);
+        return 1;
+    }
+    if ((reinterpret_cast<uintptr_t>(ws) & 255u) != 0) { set_error("f1 sets workspace must be 256-byte aligned"); return 1; }
+    return launch_f1_sets(bits, B, S, L, beta, max_size, sets, expected_f, set_size, ws, static_cast<cudaStream_t>(cuda_stream));
 }
 
 // G = R R^T takes the engine its own (L, L, Z) shape selects, as mpvae_contract_nt's auto engine does, unless

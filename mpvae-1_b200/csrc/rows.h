@@ -125,6 +125,23 @@ struct GhkInputs {
 };
 int launch_ghk_rows(RowArgs a, const GhkInputs& in, cudaStream_t stream);
 
+// Set prediction (sets.cu).  The sampler, after the nt product (a.nr): bits (B, S, ceil(L / 32)) words of y = (U < E),
+// E = predict_E(nr + fx_out), U the caller's (S, B, L) uniforms or the library's Philox stream with its own key.
+struct SampleInputs {
+    const float* uniform;              // (S, B, L) in (0, 1), or nullptr
+    int32_t* bits;
+    int noise_b_global, noise_row0;
+    uint64_t noise_seed, noise_offset;
+    const uint64_t* noise_offset_dev;
+};
+int launch_sample_labels(RowArgs a, const SampleInputs& in, cudaStream_t stream);
+// The F-measure-optimal decoder, one CTA per row, and its scratch: per row the sample cardinalities and weights (S each)
+// and the labels set in any sample with their Delta (L each).
+struct F1Layout { size_t card, wsmp, ulist, delta, total; };
+F1Layout f1_layout(int B, int S, int L);
+int launch_f1_sets(const int32_t* bits, int B, int S, int L, double beta, int max_size, uint8_t* sets, double* expected_f,
+                   int32_t* set_size, void* ws, cudaStream_t stream);
+
 // Closed-form predictive distribution (predictive.cu), the S -> infinity limit of the above: per-label scales
 // 1 / sqrt(1 + |R_l|^2), pair correlations, exact marginals and pair co-occurrence probabilities.  pairs: P int32 pairs
 // (i, j); an index outside [0, L) gives NaN.

@@ -122,3 +122,20 @@ def predict_conditional(model, feats: torch.Tensor, observed: torch.Tensor, args
 
     out = _score_rows(model, feats, args, batch_size, gather, group, L + 2, score)
     return out[:, :L].contiguous(), out[:, L].contiguous(), out[:, L + 1].contiguous()
+
+
+@torch.no_grad()
+def predict_sets(model, feats: torch.Tensor, args, beta: float = 1.0, max_size: Optional[int] = None,
+                 batch_size: Optional[int] = None, gather: bool = True, group=None):
+    """SetPrediction(sets (N, L) bool, expected_f (N,) float64, size (N,) int32): `mpvae.predict_sets` for each row of
+    `feats` (device tensor, ALL N rows), the F_beta-optimal label set under the model's joint label distribution.  Same
+    row sharding, batching, global-row noise keys and gather as predict_proba, so a row's set does not depend on either."""
+    from . import mpvae
+    L = model.r_sqrt_sigma.shape[0]
+
+    def score(a, b, args):
+        res = mpvae.predict_sets(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, args, beta, max_size)
+        return torch.cat([res.sets.double(), res.expected_f[:, None], res.size[:, None].double()], 1)
+
+    out = _score_rows(model, feats, args, batch_size, gather, group, L + 2, score)
+    return mpvae.SetPrediction(out[:, :L] > 0.5, out[:, L].double().contiguous(), out[:, L + 1].to(torch.int32))

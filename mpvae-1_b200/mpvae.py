@@ -29,6 +29,7 @@ from .dense import linear
 from .probit import ProbitELBO, label_pairs, philox_normal, predictive_rho, predictive_scale, probit_predict
 from .probit import contract_nt, ghk_workspace_bytes, predict_exact_from_r, probit_predict_conditional
 from .probit import _check_observed, probit_predict_conditional_ghk
+from .probit import check_set_args, f1_sets, probit_sample_labels
 from .probit import predict_pairs as probit_predict_pairs
 
 _state = {"seed": 0x5EED_B200, "offset": 0}
@@ -317,6 +318,65 @@ def predict_conditional_ghk(fx_out, r_sqrt_sigma, observed, args, noise=None, gr
     if len(out) == 1:
         return ConditionalPrediction(*out[0])
     return ConditionalPrediction(*(torch.cat(t, 0) for t in zip(*out)))
+
+
+def sample_labels(fx_out, r_sqrt_sigma, args, noise=None, uniform=None):
+    """Joint label samples of the probit predictive distribution: (B, S, ceil(L / 32)) int32 bits, S =
+    args.n_test_sample, label l of sample s of row b at bit l % 32 of word [b, s, l // 32] (unpack_label_samples gives
+    the (B, S, L) bool tensor).  Sample s is the whole label vector y = (U < E_s), E_s the clamped probit of predict's
+    sample s: same noise (`noise_plan`: a call without args.noise_offset consumes one offset, and with the same offset it
+    uses predict's noise), so the mean of the samples over s estimates predict's indiv_prob without bias, and the
+    samples keep the joint structure of I + R R^T that the marginals lose.  `uniform`: optional (S, B, L) fp32 draws in
+    (0, 1); None = the library's own Philox stream, keyed by global row (args.dp_row0), so a row's samples do not depend
+    on batching.  Inference only, CUDA only; args.mpvae_flags as for predict."""
+    plan = _sample_plan("sample_labels", fx_out, r_sqrt_sigma, args, noise)
+    if plan is None:
+        return torch.empty((0, args.n_test_sample, (fx_out.shape[1] + 31) // 32), dtype=torch.int32, device=fx_out.device)
+    n_sample, r32, noise, spec, flags = plan
+    return probit_sample_labels(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags, uniform=uniform)
+
+
+def unpack_label_samples(bits, label_dim):
+    """(B, S, L) bool from sample_labels' (B, S, ceil(L / 32)) int32 bits, on the tensor's device."""
+    shifts = torch.arange(32, dtype=torch.int32, device=bits.device)
+    y = torch.bitwise_and(torch.bitwise_right_shift(bits.unsqueeze(-1), shifts), 1)
+    return y.reshape(bits.shape[0], bits.shape[1], -1)[:, :, :label_dim].bool()
+
+
+SetPrediction = namedtuple("SetPrediction", ["sets", "expected_f", "size"])
+
+
+def f1_optimal_sets(bits, label_dim, beta=1.0, max_size=None):
+    """The F_beta-optimal label set of each row for the empirical distribution of its label samples (sample_labels'
+    bits, or any bits in that layout), by the GFM algorithm (Dembczynski et al., NIPS 2011).  Per row, with s_i the size
+    of sample i, Delta_{l,k} = mean_i y_{i,l} (1 + beta^2) / (beta^2 s_i + k): the best set of size k is the top k labels
+    of Delta_{., k}, its expected F is their sum, and the empty set scores the share of empty samples.  The result is
+    the exact optimum over every set of at most `max_size` labels (None: no bound); ties go to the smaller set and the
+    lower label index.  Returns SetPrediction(sets (B, L) bool, expected_f (B,) float64, size (B,) int32).  The cost
+    per row grows as min(|U|, max_size) * |U| * S, |U| the number of labels set in any sample: bound max_size when rows
+    are dense.  CUDA only; no host synchronisation."""
+    if isinstance(bits, torch.Tensor) and not bits.is_cuda:
+        raise RuntimeError("mpvae_b200.f1_optimal_sets needs CUDA tensors: the F-measure decoder is implemented as sm_100a "
+                           "kernels only (no CPU fallback)")
+    return SetPrediction(*f1_sets(bits, label_dim, beta, max_size))
+
+
+def predict_sets(fx_out, r_sqrt_sigma, args, beta=1.0, max_size=None, noise=None):
+    """Per row, the label set with the largest expected F_beta under the model: sample_labels' S joint draws, then
+    f1_optimal_sets on them.  Thresholding predict's marginals is the best decision for the Hamming loss, not for the
+    example-based F1; this uses the joint distribution of the row's labels.  Returns SetPrediction(sets (B, L) bool,
+    expected_f (B,) float64: the expected F_beta of the set on the samples, size (B,) int32).  Same noise and offset
+    consumption as predict.  Inference only, CUDA only."""
+    label_dim = fx_out.shape[1]
+    check_set_args(beta, max_size)          # before the plan: a refused call consumes no noise offset
+    plan = _sample_plan("predict_sets", fx_out, r_sqrt_sigma, args, noise)
+    if plan is None:
+        return SetPrediction(torch.zeros((0, label_dim), dtype=torch.bool, device=fx_out.device),
+                             torch.empty(0, dtype=torch.float64, device=fx_out.device),
+                             torch.empty(0, dtype=torch.int32, device=fx_out.device))
+    n_sample, r32, noise, spec, flags = plan
+    bits = probit_sample_labels(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags)
+    return SetPrediction(*f1_sets(bits, label_dim, beta, max_size))
 
 
 def _inference_only(name, *tensors):

@@ -8,6 +8,7 @@ regulariser, fairsoft_train.py:76-140).  PyTorch is used for device memory and t
 from __future__ import annotations
 
 import ctypes as C
+import math
 import os
 
 import torch
@@ -88,7 +89,7 @@ def _poison(*tensors):
     counter) and every output as NaN, so anything the kernels read before writing, or leave unwritten, shows."""
     if os.environ.get("MPVAE_POISON_WORKSPACE") == "1":
         for t in tensors:
-            t.fill_(255 if t.dtype == torch.uint8 else float("nan"))
+            t.fill_(255 if t.dtype == torch.uint8 else float("nan") if t.is_floating_point() else -1)
 
 
 def _set_noise_spec(p, spec, B):
@@ -257,16 +258,18 @@ def _predict_inputs(name, fx_out, r32, S, noise, noise_spec):
     return fx_out.contiguous(), r32.contiguous(), (noise.contiguous() if noise is not None else None), dims
 
 
-def _run_predict(entry, fx_out, r32, noise, noise_spec, flags, dims, *args, row_outputs=0):
+def _run_predict(entry, fx_out, r32, noise, noise_spec, flags, dims, *args, row_outputs=0, out=None):
     """Runs the sampled-prediction entry point `entry` of the library: allocates its workspace, prob (B, L) and
     `row_outputs` fp32 (B,) outputs, and calls it with the params, `args`, the row outputs and the current stream.
-    Returns [prob, *row outputs]."""
+    Returns [prob, *row outputs].  `out`: the entry point's own output tensor instead of prob (it is poisoned here and
+    passed in `args` by the caller; indiv_prob stays NULL)."""
     S, B, L, Z = dims
     lib = _lib.lib()
     dev = fx_out.device
     with torch.cuda.device(dev):
         ws = torch.empty(int(lib.mpvae_workspace_bytes(S, B, L, Z, 0, flags)), dtype=torch.uint8, device=dev)
-        out = [torch.empty((B, L), dtype=torch.float32, device=dev)]
+        writes_prob = out is None
+        out = [torch.empty((B, L), dtype=torch.float32, device=dev) if writes_prob else out]
         for _ in range(row_outputs):
             out.append(torch.empty(B, dtype=torch.float32, device=dev))
             args += (_ptr(out[-1]),)
@@ -277,7 +280,7 @@ def _run_predict(entry, fx_out, r32, noise, noise_spec, flags, dims, *args, row_
         p.S, p.B, p.L, p.Z = S, B, L, Z
         p.fx_out, p.r, p.noise = _ptr(fx_out), _ptr(r32), _ptr(noise)
         _set_noise_spec(p, noise_spec, B)
-        p.indiv_prob = _ptr(out[0])
+        p.indiv_prob = _ptr(out[0]) if writes_prob else None
         p.workspace, p.workspace_bytes = _ptr(ws), ws.numel()
         _lib.check(getattr(lib, entry)(C.byref(p), *args, _stream(dev)), entry)
     return out
@@ -334,6 +337,70 @@ def probit_predict_conditional_ghk(fx_out, r32, observed, S, max_observed, *, no
     return tuple(_run_predict("mpvae_probit_predict_conditional_ghk", fx_out, r32, noise, noise_spec, flags, dims,
                               _ptr(observed), _ptr(gram), _ptr(zeta), _ptr(uniform), _ptr(gws), gws_bytes,
                               int(max_observed), row_outputs=2))
+
+
+def probit_sample_labels(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0, uniform=None):
+    """(B, S, ceil(L / 32)) int32 bits of S joint label samples per row, y = (U < E) with E the clamped probit that
+    probit_predict averages, on its noise (mpvae_probit_sample_labels): label l of sample s is bit l % 32 of word l / 32.
+    `uniform`: optional (S, B, L) fp32 U in (0, 1); None = the library's own Philox stream, keyed by global row.
+    `noise` / `noise_spec` / `flags` as for probit_predict; inference only."""
+    dims = _predict_dims("probit_sample_labels", fx_out, r32, S, noise, noise_spec)
+    S, B, L, Z = dims
+    if uniform is not None and tuple(uniform.shape) != (S, B, L):
+        raise ValueError(f"uniform has shape {tuple(uniform.shape)}, expected {(S, B, L)}")
+    tensors = (fx_out, r32, noise, uniform)
+    _check_tensors(("fx_out", "r_sqrt_sigma", "noise", "uniform"), tensors)
+    fx_out, r32, noise, uniform = (t.contiguous() if t is not None else None for t in tensors)
+    bits = torch.empty((B, S, (L + 31) // 32), dtype=torch.int32, device=fx_out.device)
+    return _run_predict("mpvae_probit_sample_labels", fx_out, r32, noise, noise_spec, flags, dims, _ptr(uniform),
+                        _ptr(bits), out=bits)[0]
+
+
+def check_set_args(beta, max_size):
+    """beta as a float, refused unless it is positive with a finite square (beta^2 enters every weight of the F-measure
+    decoder); max_size refused below 0 (None: no bound)."""
+    beta = float(beta)
+    if not (beta > 0.0 and math.isfinite(beta * beta)):
+        raise ValueError(f"beta must be positive with a finite square, got {beta}")
+    if max_size is not None and int(max_size) < 0:
+        raise ValueError(f"max_size must be >= 0 (None for no bound), got {max_size}")
+    return beta
+
+
+def f1_sets(bits, L, beta=1.0, max_size=None):
+    """(sets (B, L) bool, expected_f (B,) fp64, size (B,) int32): per row, the set of at most `max_size` labels (None:
+    no bound) that maximises the expected F_beta over the row's S label samples in `bits` ((B, S, ceil(L / 32)) int32,
+    probit_sample_labels' layout), by the GFM algorithm (mpvae_f1_sets).  One launch; no host synchronisation."""
+    if not isinstance(bits, torch.Tensor) or bits.dtype != torch.int32:
+        raise TypeError(f"bits must be an int32 tensor, got {getattr(bits, 'dtype', type(bits))}")
+    L = int(L)
+    if L < 1:
+        raise ValueError(f"label_dim must be positive, got {L}")
+    W = (L + 31) // 32
+    if bits.dim() != 3 or bits.shape[2] != W or bits.shape[1] < 1:
+        raise ValueError(f"bits has shape {tuple(bits.shape)}, expected (batch, n_sample >= 1, {W}) for {L} labels")
+    beta = check_set_args(beta, max_size)
+    max_size = L if max_size is None else int(max_size)
+    max_size = min(max_size, L)
+    if not bits.is_cuda:
+        raise RuntimeError(f"mpvae_b200: bits is on {bits.device}; the F-measure decoder runs on CUDA only "
+                           "(there is no CPU fallback)")
+    B, S = bits.shape[0], bits.shape[1]
+    dev = bits.device
+    sets = torch.empty((B, L), dtype=torch.uint8, device=dev)
+    expected_f = torch.empty(B, dtype=torch.float64, device=dev)
+    size = torch.empty(B, dtype=torch.int32, device=dev)
+    if B == 0:
+        return sets.view(torch.bool), expected_f, size
+    bits = bits.contiguous()
+    lib = _lib.lib()
+    with torch.cuda.device(dev):
+        ws_bytes = int(lib.mpvae_f1_sets_workspace_bytes(B, S, L))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        _poison(ws, sets, expected_f, size)
+        _lib.check(lib.mpvae_f1_sets(_ptr(bits), B, S, L, beta, max_size, _ptr(sets), _ptr(expected_f), _ptr(size),
+                                     _ptr(ws), ws_bytes, _stream(dev)), "mpvae_f1_sets")
+    return sets.view(torch.bool), expected_f, size
 
 
 # ---- closed-form prediction (csrc/predictive.cu): the S -> infinity limit of probit_predict ----
