@@ -245,6 +245,32 @@ uint64_t mpvae_f1_sets_workspace_bytes(int32_t B, int32_t S, int32_t L);
 int mpvae_f1_sets(const int32_t *bits, int32_t B, int32_t S, int32_t L, double beta, int32_t max_size, uint8_t *sets,
                   double *expected_f, int32_t *set_size, void *ws, uint64_t ws_bytes, void *cuda_stream);
 
+/* The model's probability of whole label sets, on the S samples mpvae_probit_predict draws (the same noise, offset and
+ * regime).  Given sample s the labels are independent Bernoulli(E_s), so with ll+ = log E and ll- = log(1 - E), the fp32
+ * cell logs of the loss (either CDF mode):
+ *   lp_s(y) = sum_l (y_l ? ll+_sl : ll-_sl)                             (fp64)
+ *   log_prob(y) = M + log((1/S) sum_s exp(lp_s - M)),  M = max_s lp_s    (fp64, a fixed order)
+ *   ess(y) = (sum_s w_s)^2 / sum_s w_s^2,  w_s = exp(lp_s - M)
+ * exp(log_prob) is the model's expected exact-match accuracy of y; ess (in [1, S]) is how many samples carry the
+ * estimate, and falls towards 1 as L grows.
+ * mpvae_probit_score_sets: bits (B, C, W) int32, W = ceil(L / 32), C >= 1 sets per row in mpvae_probit_sample_labels'
+ * layout (bits at and above L are ignored, whatever they hold); log_prob and ess (B, C) fp64.
+ * mpvae_probit_predict_mode: per row the set that maximises log_prob.  Candidates, in order: 1[indiv_prob >= 1/2] (the
+ * bits mpvae_probit_predict returns), the empty set, and each sample's mode 1[ll+_s > ll-_s]; from the best (ties to the
+ * earliest), the label whose flip raises log_prob most (ties to the lower index) is flipped while the gain is positive
+ * and fewer than max_flips (>= 0) flips were taken.  sets (B, L) 0 / 1, log_prob and ess (B) fp64 -- bit for bit
+ * mpvae_probit_score_sets of the result --, size and flips (B) int32.  With flips < max_flips the set is a single-flip
+ * local maximum.  One flip costs S * L exp per row.
+ * Both read what mpvae_probit_predict reads (indiv_prob is not written and may be NULL) and apply its flags; same
+ * workspace, plus mode_ws >= mpvae_mode_workspace_bytes(S, B, L) bytes, 256-byte aligned: about 8 S L bytes per row.
+ * Four launches after the product (mode), two (score); no host synchronisation; deterministic bits. */
+uint64_t mpvae_mode_workspace_bytes(int32_t S, int32_t B, int32_t L);
+int mpvae_probit_score_sets(const mpvae_probit_params *p, const int32_t *bits, int32_t C, double *log_prob, double *ess,
+                            void *mode_ws, uint64_t mode_ws_bytes, void *cuda_stream);
+int mpvae_probit_predict_mode(const mpvae_probit_params *p, int32_t max_flips, uint8_t *sets, double *log_prob,
+                              double *ess, int32_t *size, int32_t *flips, void *mode_ws, uint64_t mode_ws_bytes,
+                              void *cuda_stream);
+
 /* Backward: the autograd backward of compute_loss (implicit in the reference, train.py:125),
  * closed form in SURVEY.md 8(a-12).  Must follow a forward on the same workspace. */
 int mpvae_probit_backward(const mpvae_probit_params *p, void *cuda_stream);

@@ -36,6 +36,7 @@ EXPORTS = (
     "mpvae_probit_predict_conditional", "mpvae_probit_forward_masked", "mpvae_probit_backward_masked",
     "mpvae_ghk_workspace_bytes", "mpvae_probit_predict_conditional_ghk",
     "mpvae_probit_sample_labels", "mpvae_f1_sets_workspace_bytes", "mpvae_f1_sets",
+    "mpvae_mode_workspace_bytes", "mpvae_probit_score_sets", "mpvae_probit_predict_mode",
 )
 
 _f = C.c_void_p  # device pointer
@@ -106,6 +107,14 @@ def _load():
     lib.mpvae_f1_sets_workspace_bytes.argtypes = [C.c_int32] * 3
     lib.mpvae_f1_sets.restype = C.c_int
     lib.mpvae_f1_sets.argtypes = [C.c_void_p] + [C.c_int32] * 3 + [C.c_double, C.c_int32] + [C.c_void_p] * 4 + [
+        C.c_uint64, C.c_void_p]
+    lib.mpvae_mode_workspace_bytes.restype = C.c_uint64
+    lib.mpvae_mode_workspace_bytes.argtypes = [C.c_int32] * 3
+    lib.mpvae_probit_score_sets.restype = C.c_int
+    lib.mpvae_probit_score_sets.argtypes = [C.POINTER(ProbitParams), C.c_void_p, C.c_int32] + [C.c_void_p] * 3 + [
+        C.c_uint64, C.c_void_p]
+    lib.mpvae_probit_predict_mode.restype = C.c_int
+    lib.mpvae_probit_predict_mode.argtypes = [C.POINTER(ProbitParams), C.c_int32] + [C.c_void_p] * 6 + [
         C.c_uint64, C.c_void_p]
     lib.mpvae_probit_backward.restype = C.c_int
     lib.mpvae_probit_backward.argtypes = [C.POINTER(ProbitParams), C.c_void_p]

@@ -592,6 +592,52 @@ int mpvae_f1_sets(const int32_t* bits, int32_t B, int32_t S, int32_t L, double b
     return launch_f1_sets(bits, B, S, L, beta, max_size, sets, expected_f, set_size, ws, static_cast<cudaStream_t>(cuda_stream));
 }
 
+uint64_t mpvae_mode_workspace_bytes(int32_t S, int32_t B, int32_t L) {
+    if (S <= 0 || B <= 0 || L <= 0) return 256;
+    return mode_layout(S, B, L).total;
+}
+
+// the mode entry points' own checks, after open_predict's
+static int check_mode_ws(const PredictCall& c, void* ws, uint64_t ws_bytes) {
+    if (!ws) { set_error("NULL pointer (mode_ws)"); return 1; }
+    const uint64_t need = mpvae_mode_workspace_bytes(c.p->S, c.p->B, c.p->L);
+    if (ws_bytes < need) {
+        set_error("mode workspace too small: %llu < %llu bytes", (unsigned long long)ws_bytes, (unsigned long long)need);
+        return 1;
+    }
+    if ((reinterpret_cast<uintptr_t>(ws) & 255u) != 0) { set_error("mode workspace must be 256-byte aligned"); return 1; }
+    return 0;
+}
+
+int mpvae_probit_score_sets(const mpvae_probit_params* p_in, const int32_t* bits, int32_t C, double* log_prob,
+                            double* ess, void* mode_ws, uint64_t mode_ws_bytes, void* cuda_stream) {
+    PredictCall c;
+    if (int rc = open_predict(p_in, c, false)) return rc;
+    if (!bits || !log_prob || !ess) { set_error("NULL pointer (bits/log_prob/ess)"); return 1; }
+    if (C <= 0) { set_error("bad set count C=%d", C); return 1; }
+    if ((long long)c.p->B * C > 0x7fffffffLL) { set_error("B*C overflows int32"); return 1; }
+    if (int rc = check_mode_ws(c, mode_ws, mode_ws_bytes)) return rc;
+    cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
+    // the CUDA-core product also where predict takes the one-launch small kernel, which never materialises nr
+    if (int rc = predict_product(c, stream)) return rc;
+    ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
+    return launch_score_sets(c.a, bits, C, log_prob, ess, mode_ws, stream);
+}
+
+int mpvae_probit_predict_mode(const mpvae_probit_params* p_in, int32_t max_flips, uint8_t* sets, double* log_prob,
+                              double* ess, int32_t* size, int32_t* flips, void* mode_ws, uint64_t mode_ws_bytes,
+                              void* cuda_stream) {
+    PredictCall c;
+    if (int rc = open_predict(p_in, c, false)) return rc;
+    if (!sets || !log_prob || !ess || !size || !flips) { set_error("NULL pointer (sets/log_prob/ess/size/flips)"); return 1; }
+    if (max_flips < 0) { set_error("max_flips=%d must be >= 0", max_flips); return 1; }
+    if (int rc = check_mode_ws(c, mode_ws, mode_ws_bytes)) return rc;
+    cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
+    if (int rc = predict_product(c, stream)) return rc;
+    ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
+    return launch_predict_mode(c.a, max_flips, sets, log_prob, ess, size, flips, mode_ws, stream);
+}
+
 // G = R R^T takes the engine its own (L, L, Z) shape selects, as mpvae_contract_nt's auto engine does, unless
 // MPVAE_FLAG_CONTRACT_FMA asks for the CUDA-core product
 static bool gram_uses_tensor(uint32_t flags, int L, int Z) {

@@ -142,6 +142,18 @@ F1Layout f1_layout(int B, int S, int L);
 int launch_f1_sets(const int32_t* bits, int B, int S, int L, double beta, int max_size, uint8_t* sets, double* expected_f,
                    int32_t* set_size, void* ws, cudaStream_t stream);
 
+// Mode prediction (mode.cu), after the nt product (a.nr).  Its own scratch block: per row the fp64 chunk partials of
+// A_s = sum_l log(1 - E_sl) (S * ceil(L / 128)), A_s, lp_s and the weights (S each), d_sl = log E_sl - log(1 - E_sl)
+// (S * L), the candidate sets and their scores (S + 2 each) and the mode's bits.
+struct ModeLayout { size_t part, a, d, lp, wts, cand, cand_lp, cand_ess, yhat, total; };
+ModeLayout mode_layout(int S, int B, int L);
+// log P and ess of the caller's C sets per row (bits (B, C, ceil(L / 32)) words, sample_labels' layout)
+int launch_score_sets(RowArgs a, const int32_t* bits, int C, double* log_prob, double* ess, void* ws, cudaStream_t stream);
+// per row the set that maximises P: the best candidate, then at most max_flips steepest single flips; log P and ess
+// of the result by the scoring kernel of launch_score_sets
+int launch_predict_mode(RowArgs a, int max_flips, uint8_t* sets, double* log_prob, double* ess, int32_t* size,
+                        int32_t* flips, void* ws, cudaStream_t stream);
+
 // Closed-form predictive distribution (predictive.cu), the S -> infinity limit of the above: per-label scales
 // 1 / sqrt(1 + |R_l|^2), pair correlations, exact marginals and pair co-occurrence probabilities.  pairs: P int32 pairs
 // (i, j); an index outside [0, L) gives NaN.

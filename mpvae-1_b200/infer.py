@@ -139,3 +139,24 @@ def predict_sets(model, feats: torch.Tensor, args, beta: float = 1.0, max_size: 
 
     out = _score_rows(model, feats, args, batch_size, gather, group, L + 2, score)
     return mpvae.SetPrediction(out[:, :L] > 0.5, out[:, L].double().contiguous(), out[:, L + 1].to(torch.int32))
+
+
+@torch.no_grad()
+def predict_mode(model, feats: torch.Tensor, args, max_flips: Optional[int] = None, batch_size: Optional[int] = None,
+                 gather: bool = True, group=None):
+    """ModePrediction(sets (N, L) bool, log_prob (N,) float64, ess (N,) float64, size (N,) int32, flips (N,) int32):
+    `mpvae.predict_mode` for each row of `feats` (device tensor, ALL N rows), the label set the model finds most
+    probable.  Same row sharding, batching, global-row noise keys and gather as predict_proba, so a row's set does not
+    depend on either."""
+    from . import mpvae
+    mpvae.check_max_flips(max_flips)
+    L = model.r_sqrt_sigma.shape[0]
+
+    def score(a, b, args):
+        res = mpvae.predict_mode(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, args, max_flips)
+        return torch.cat([res.sets.double(), res.log_prob[:, None], res.ess[:, None], res.size[:, None].double(),
+                          res.flips[:, None].double()], 1)
+
+    out = _score_rows(model, feats, args, batch_size, gather, group, L + 4, score)
+    return mpvae.ModePrediction(out[:, :L] > 0.5, out[:, L].contiguous(), out[:, L + 1].contiguous(),
+                                out[:, L + 2].to(torch.int32), out[:, L + 3].to(torch.int32))

@@ -30,6 +30,7 @@ from .probit import ProbitELBO, label_pairs, philox_normal, predictive_rho, pred
 from .probit import contract_nt, ghk_workspace_bytes, predict_exact_from_r, probit_predict_conditional
 from .probit import _check_observed, probit_predict_conditional_ghk
 from .probit import check_set_args, f1_sets, probit_sample_labels
+from .probit import check_max_flips, check_set_bits, probit_predict_mode, probit_score_sets
 from .probit import predict_pairs as probit_predict_pairs
 
 _state = {"seed": 0x5EED_B200, "offset": 0}
@@ -377,6 +378,58 @@ def predict_sets(fx_out, r_sqrt_sigma, args, beta=1.0, max_size=None, noise=None
     n_sample, r32, noise, spec, flags = plan
     bits = probit_sample_labels(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags)
     return SetPrediction(*f1_sets(bits, label_dim, beta, max_size))
+
+
+SetScores = namedtuple("SetScores", ["log_prob", "ess"])
+
+
+def score_sets(fx_out, r_sqrt_sigma, bits, args, noise=None):
+    """The model's log-probability of given label sets: C sets per row in `bits`, an int32 (B, C, ceil(L / 32)) tensor
+    in sample_labels' layout (label l of set c of row b at bit l % 32 of word [b, c, l // 32]; bits at and above L are
+    ignored).  On predict's S samples (same noise, same offset consumption: a call without args.noise_offset consumes
+    one offset, and with the same offset it uses predict's noise), sample s gives every label its own Bernoulli(E_s),
+    and the set's probability is the mean over s of the product, in logs:
+        lp_s = sum_l log(y_l ? E_sl : 1 - E_sl)      (the loss's fp32 cell logs, summed in fp64)
+        log_prob = log mean_s exp(lp_s),   ess = (sum_s w_s)^2 / sum_s w_s^2,  w_s = exp(lp_s - max lp)
+    exp(log_prob) is the model's expected exact-match accuracy of the set; ess says how many samples carry the estimate
+    (it falls towards 1 when L is large).  With the row's true labels, log_prob is the row's -nll_loss_x of
+    compute_loss up to that path's fp32 rounding.  Returns SetScores(log_prob (B, C) float64, ess (B, C) float64).
+    Inference only, CUDA only; args.mpvae_flags as for predict."""
+    n_batch, label_dim = fx_out.shape
+    check_set_bits(bits, n_batch, label_dim, fx_out.device)
+    plan = _sample_plan("score_sets", fx_out, r_sqrt_sigma, args, noise)
+    if plan is None:
+        empty = torch.empty((0, bits.shape[1]), dtype=torch.float64, device=fx_out.device)
+        return SetScores(empty, empty.clone())
+    n_sample, r32, noise, spec, flags = plan
+    return SetScores(*probit_score_sets(fx_out, r32, bits, n_sample, noise=noise, noise_spec=spec, flags=flags))
+
+
+ModePrediction = namedtuple("ModePrediction", ["sets", "log_prob", "ess", "size", "flips"])
+
+
+def predict_mode(fx_out, r_sqrt_sigma, args, max_flips=None, noise=None):
+    """Per row, the label set the model finds most probable: the decision that maximises the expected exact-match
+    (subset) accuracy, where thresholding predict's marginals maximises the Hamming accuracy and predict_sets the F1.
+    The search is deterministic: the best of the candidates 1[predict >= 0.5], the empty set and each sample's own mode
+    (ties to the earliest), then steepest single-label flips while one raises score_sets' log_prob, at most `max_flips`
+    of them (None: no bound; one flip costs S * L per row).  With flips < max_flips the set is a local maximum: no
+    single flip scores higher.  Returns ModePrediction(sets (B, L) bool, log_prob (B,) float64, ess (B,) float64 --
+    score_sets of the set, bit for bit --, size (B,) int32, flips (B,) int32).  Same noise and offset consumption as
+    predict.  Inference only, CUDA only; args.mpvae_flags as for predict."""
+    label_dim = fx_out.shape[1]
+    check_max_flips(max_flips)              # before the plan: a refused call consumes no noise offset
+    plan = _sample_plan("predict_mode", fx_out, r_sqrt_sigma, args, noise)
+    if plan is None:
+        dev = fx_out.device
+        return ModePrediction(torch.zeros((0, label_dim), dtype=torch.bool, device=dev),
+                              torch.empty(0, dtype=torch.float64, device=dev),
+                              torch.empty(0, dtype=torch.float64, device=dev),
+                              torch.empty(0, dtype=torch.int32, device=dev),
+                              torch.empty(0, dtype=torch.int32, device=dev))
+    n_sample, r32, noise, spec, flags = plan
+    return ModePrediction(*probit_predict_mode(fx_out, r32, n_sample, max_flips, noise=noise, noise_spec=spec,
+                                               flags=flags))
 
 
 def _inference_only(name, *tensors):

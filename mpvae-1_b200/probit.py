@@ -403,6 +403,79 @@ def f1_sets(bits, L, beta=1.0, max_size=None):
     return sets.view(torch.bool), expected_f, size
 
 
+def check_set_bits(bits, B, L, device):
+    """Refuses `bits` that are not an int32 (B, C >= 1, ceil(L / 32)) tensor on `device` (sets in sample_labels'
+    layout)."""
+    if not isinstance(bits, torch.Tensor) or bits.dtype != torch.int32:
+        raise TypeError(f"bits must be an int32 tensor, got {getattr(bits, 'dtype', type(bits))}")
+    W = (L + 31) // 32
+    if bits.dim() != 3 or bits.shape[0] != B or bits.shape[1] < 1 or bits.shape[2] != W:
+        raise ValueError(f"bits has shape {tuple(bits.shape)}, expected ({B}, n_sets >= 1, {W}) for {L} labels")
+    if bits.device != device:
+        raise RuntimeError(f"mpvae_b200: bits is on {bits.device}, expected {device}")
+
+
+def check_max_flips(max_flips):
+    """max_flips as an int (None: no bound, 2^31 - 1), refused below 0."""
+    if max_flips is None:
+        return 2 ** 31 - 1
+    if int(max_flips) < 0:
+        raise ValueError(f"max_flips must be >= 0 (None for no bound), got {max_flips}")
+    return min(int(max_flips), 2 ** 31 - 1)
+
+
+def mode_workspace_bytes(S, B, L):
+    """Bytes of the mode entry points' own scratch block (about 8 S L bytes per row)."""
+    return int(_lib.lib().mpvae_mode_workspace_bytes(S, B, L))
+
+
+def _mode_ws(dims, dev):
+    S, B, L, _ = dims
+    n = mode_workspace_bytes(S, B, L)
+    return torch.empty(n, dtype=torch.uint8, device=dev), n
+
+
+def probit_score_sets(fx_out, r32, bits, S, *, noise=None, noise_spec=None, flags=0):
+    """(log_prob (B, C) fp64, ess (B, C) fp64) of the C label sets per row in `bits` ((B, C, ceil(L / 32)) int32,
+    sample_labels' layout) under the S-sample mixture probit_predict averages, on its noise
+    (mpvae_probit_score_sets).  `noise` / `noise_spec` / `flags` as for probit_predict; inference only."""
+    fx_out, r32, noise, dims = _predict_inputs("probit_score_sets", fx_out, r32, S, noise, noise_spec)
+    S, B, L, Z = dims
+    check_set_bits(bits, B, L, fx_out.device)
+    bits = bits.contiguous()
+    C_ = bits.shape[1]
+    dev = fx_out.device
+    with torch.cuda.device(dev):
+        ws, n = _mode_ws(dims, dev)
+        log_prob = torch.empty((B, C_), dtype=torch.float64, device=dev)
+        ess = torch.empty((B, C_), dtype=torch.float64, device=dev)
+        _poison(ws, ess)
+    _run_predict("mpvae_probit_score_sets", fx_out, r32, noise, noise_spec, flags, dims, _ptr(bits), C_,
+                 _ptr(log_prob), _ptr(ess), _ptr(ws), n, out=log_prob)
+    return log_prob, ess
+
+
+def probit_predict_mode(fx_out, r32, S, max_flips=None, *, noise=None, noise_spec=None, flags=0):
+    """(sets (B, L) bool, log_prob (B,) fp64, ess (B,) fp64, size (B,) int32, flips (B,) int32): per row the label set
+    that maximises the S-sample mixture's probability, by candidates and steepest single-flip ascent
+    (mpvae_probit_predict_mode).  `noise` / `noise_spec` / `flags` as for probit_predict; inference only."""
+    max_flips = check_max_flips(max_flips)
+    fx_out, r32, noise, dims = _predict_inputs("probit_predict_mode", fx_out, r32, S, noise, noise_spec)
+    S, B, L, Z = dims
+    dev = fx_out.device
+    with torch.cuda.device(dev):
+        ws, n = _mode_ws(dims, dev)
+        sets = torch.empty((B, L), dtype=torch.uint8, device=dev)
+        log_prob = torch.empty(B, dtype=torch.float64, device=dev)
+        ess = torch.empty(B, dtype=torch.float64, device=dev)
+        size = torch.empty(B, dtype=torch.int32, device=dev)
+        flips = torch.empty(B, dtype=torch.int32, device=dev)
+        _poison(ws, log_prob, ess, size, flips)
+    _run_predict("mpvae_probit_predict_mode", fx_out, r32, noise, noise_spec, flags, dims, max_flips, _ptr(sets),
+                 _ptr(log_prob), _ptr(ess), _ptr(size), _ptr(flips), _ptr(ws), n, out=sets)
+    return sets.view(torch.bool), log_prob, ess, size, flips
+
+
 # ---- closed-form prediction (csrc/predictive.cu): the S -> infinity limit of probit_predict ----
 
 def _check_f64(name, t, n, dev):
