@@ -168,13 +168,32 @@ const mpvae_probit_params* normalize(const mpvae_probit_params* p, mpvae_probit_
     return nullptr;
 }
 
-int check_noise_rows(const mpvae_probit_params* p) {
-    if (!p->noise && (p->noise_row0 < 0 || p->noise_b_global < p->noise_row0 + p->B)) {
-        set_error("library-side noise: rows [%d, %d) do not fit a global batch of %d", p->noise_row0, p->noise_row0 + p->B,
+// Rows [row0, row0 + B) must lie in the global batch that keys a Philox stream the library draws (library_draws);
+// `what` names that stream in the message.
+int check_rows_fit(const mpvae_probit_params* p, bool library_draws, const char* what) {
+    if (library_draws && (p->noise_row0 < 0 || p->noise_b_global < p->noise_row0 + p->B)) {
+        set_error("%s: rows [%d, %d) do not fit a global batch of %d", what, p->noise_row0, p->noise_row0 + p->B,
                   p->noise_b_global);
         return 1;
     }
     return 0;
+}
+
+// A scratch block an entry point takes besides the params' workspace: present, at least `need` bytes, 256-byte aligned.
+// `what` names the block in the messages; `sized_for`, when not NULL, says what its size was computed for.
+int check_scratch(const char* what, const void* ptr, uint64_t have, uint64_t need, const char* sized_for = nullptr) {
+    if (!ptr) { set_error("NULL pointer (%s)", what); return 1; }
+    if (have < need) {
+        set_error("%s too small%s%s: %llu < %llu bytes", what, sized_for ? " for " : "", sized_for ? sized_for : "",
+                  (unsigned long long)have, (unsigned long long)need);
+        return 1;
+    }
+    if ((reinterpret_cast<uintptr_t>(ptr) & 255u) != 0) { set_error("%s must be 256-byte aligned", what); return 1; }
+    return 0;
+}
+
+PhiloxRows philox_rows(const mpvae_probit_params* p) {
+    return PhiloxRows{p->noise_b_global, p->noise_row0, p->noise_seed, p->noise_offset, p->noise_offset_dev};
 }
 
 int check_workspace(const mpvae_probit_params* p, bool backward) {
@@ -198,7 +217,7 @@ int validate(const mpvae_probit_params* p, bool backward) {
         set_error("NULL input pointer (y/fe_out/fx_out/r/workspace)");
         return 1;
     }
-    if (int rc = check_noise_rows(p)) return rc;
+    if (int rc = check_rows_fit(p, !p->noise, "library-side noise")) return rc;
     if (p->D > 0 && (!p->fe_mu || !p->fe_logvar || !p->fx_mu || !p->fx_logvar)) { set_error("NULL mu/logvar pointer"); return 1; }
     if (!backward && (!p->scalars[0] || !p->scalars[1] || !p->scalars[2] || !p->scalars[3] || !p->scalars[4] ||
                       !p->scalars[5] || !p->indiv_prob || !p->indiv_prob_label)) { set_error("NULL forward output pointer"); return 1; }
@@ -217,7 +236,7 @@ int validate_predict(const mpvae_probit_params* p, bool writes_prob) {
     }
     if ((long long)p->S * p->B > 0x7fffffffLL) { set_error("S*B overflows int32"); return 1; }
     if (!p->fx_out || !p->r || !p->workspace) { set_error("NULL input pointer (fx_out/r/workspace)"); return 1; }
-    if (int rc = check_noise_rows(p)) return rc;
+    if (int rc = check_rows_fit(p, !p->noise, "library-side noise")) return rc;
     if (writes_prob && !p->indiv_prob) { set_error("NULL forward output pointer (indiv_prob)"); return 1; }
     return check_workspace(p, false);
 }
@@ -546,19 +565,11 @@ int mpvae_probit_sample_labels(const mpvae_probit_params* p_in, const float* uni
     if (int rc = open_predict(p_in, c, false)) return rc;
     const mpvae_probit_params* p = c.p;
     if (!bits) { set_error("NULL pointer (bits)"); return 1; }
-    if (!uniform && (p->noise_row0 < 0 || p->noise_b_global < p->noise_row0 + p->B)) {
-        set_error("label draws: rows [%d, %d) do not fit a global batch of %d", p->noise_row0, p->noise_row0 + p->B,
-                  p->noise_b_global);
-        return 1;
-    }
+    if (int rc = check_rows_fit(p, !uniform, "label draws")) return rc;
     cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
     // the CUDA-core product also where predict takes the one-launch small kernel, which never materialises nr
     if (int rc = predict_product(c, stream)) return rc;
-    SampleInputs in{};
-    in.uniform = uniform;
-    in.bits = bits;
-    in.noise_b_global = p->noise_b_global; in.noise_row0 = p->noise_row0;
-    in.noise_seed = p->noise_seed; in.noise_offset = p->noise_offset; in.noise_offset_dev = p->noise_offset_dev;
+    const SampleInputs in{uniform, bits, philox_rows(p)};
     ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
     return launch_sample_labels(c.a, in, stream);
 }
@@ -583,30 +594,13 @@ int mpvae_f1_sets(const int32_t* bits, int32_t B, int32_t S, int32_t L, double b
         set_error("NULL pointer (bits/sets/expected_f/set_size/ws)");
         return 1;
     }
-    const uint64_t need = mpvae_f1_sets_workspace_bytes(B, S, L);
-    if (ws_bytes < need) {
-        set_error("f1 sets workspace too small: %llu < %llu bytes", (unsigned long long)ws_bytes, (unsigned long long)need);
-        return 1;
-    }
-    if ((reinterpret_cast<uintptr_t>(ws) & 255u) != 0) { set_error("f1 sets workspace must be 256-byte aligned"); return 1; }
+    if (int rc = check_scratch("f1 sets workspace", ws, ws_bytes, mpvae_f1_sets_workspace_bytes(B, S, L))) return rc;
     return launch_f1_sets(bits, B, S, L, beta, max_size, sets, expected_f, set_size, ws, static_cast<cudaStream_t>(cuda_stream));
 }
 
 uint64_t mpvae_mode_workspace_bytes(int32_t S, int32_t B, int32_t L) {
     if (S <= 0 || B <= 0 || L <= 0) return 256;
     return mode_layout(S, B, L).total;
-}
-
-// the mode entry points' own checks, after open_predict's
-static int check_mode_ws(const PredictCall& c, void* ws, uint64_t ws_bytes) {
-    if (!ws) { set_error("NULL pointer (mode_ws)"); return 1; }
-    const uint64_t need = mpvae_mode_workspace_bytes(c.p->S, c.p->B, c.p->L);
-    if (ws_bytes < need) {
-        set_error("mode workspace too small: %llu < %llu bytes", (unsigned long long)ws_bytes, (unsigned long long)need);
-        return 1;
-    }
-    if ((reinterpret_cast<uintptr_t>(ws) & 255u) != 0) { set_error("mode workspace must be 256-byte aligned"); return 1; }
-    return 0;
 }
 
 int mpvae_probit_score_sets(const mpvae_probit_params* p_in, const int32_t* bits, int32_t C, double* log_prob,
@@ -616,7 +610,7 @@ int mpvae_probit_score_sets(const mpvae_probit_params* p_in, const int32_t* bits
     if (!bits || !log_prob || !ess) { set_error("NULL pointer (bits/log_prob/ess)"); return 1; }
     if (C <= 0) { set_error("bad set count C=%d", C); return 1; }
     if ((long long)c.p->B * C > 0x7fffffffLL) { set_error("B*C overflows int32"); return 1; }
-    if (int rc = check_mode_ws(c, mode_ws, mode_ws_bytes)) return rc;
+    if (int rc = check_scratch("mode_ws", mode_ws, mode_ws_bytes, mpvae_mode_workspace_bytes(c.p->S, c.p->B, c.p->L))) return rc;
     cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
     // the CUDA-core product also where predict takes the one-launch small kernel, which never materialises nr
     if (int rc = predict_product(c, stream)) return rc;
@@ -631,7 +625,7 @@ int mpvae_probit_predict_mode(const mpvae_probit_params* p_in, int32_t max_flips
     if (int rc = open_predict(p_in, c, false)) return rc;
     if (!sets || !log_prob || !ess || !size || !flips) { set_error("NULL pointer (sets/log_prob/ess/size/flips)"); return 1; }
     if (max_flips < 0) { set_error("max_flips=%d must be >= 0", max_flips); return 1; }
-    if (int rc = check_mode_ws(c, mode_ws, mode_ws_bytes)) return rc;
+    if (int rc = check_scratch("mode_ws", mode_ws, mode_ws_bytes, mpvae_mode_workspace_bytes(c.p->S, c.p->B, c.p->L))) return rc;
     cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
     if (int rc = predict_product(c, stream)) return rc;
     ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
@@ -662,17 +656,10 @@ int mpvae_probit_predict_conditional_ghk(const mpvae_probit_params* p_in, const 
     if (!observed || !log_evidence || !ess || !ghk_ws) { set_error("NULL pointer (observed/log_evidence/ess/ghk_ws)"); return 1; }
     if (max_observed < 0 || max_observed > p->L) { set_error("max_observed=%d outside [0, L=%d]", max_observed, p->L); return 1; }
     const GhkLayout gl = ghk_layout_for(p->S, p->B, p->L, p->Z, max_observed, p->flags);
-    if (ghk_ws_bytes < gl.total) {
-        set_error("ghk workspace too small for max_observed=%d: %llu < %llu bytes", max_observed,
-                  (unsigned long long)ghk_ws_bytes, (unsigned long long)gl.total);
-        return 1;
-    }
-    if ((reinterpret_cast<uintptr_t>(ghk_ws) & 255u) != 0) { set_error("ghk workspace must be 256-byte aligned"); return 1; }
-    if ((!zeta || !uniform) && (p->noise_row0 < 0 || p->noise_b_global < p->noise_row0 + p->B)) {
-        set_error("GHK draws: rows [%d, %d) do not fit a global batch of %d", p->noise_row0, p->noise_row0 + p->B,
-                  p->noise_b_global);
-        return 1;
-    }
+    char sized_for[32];
+    snprintf(sized_for, sizeof(sized_for), "max_observed=%d", max_observed);
+    if (int rc = check_scratch("ghk workspace", ghk_ws, ghk_ws_bytes, gl.total, sized_for)) return rc;
+    if (int rc = check_rows_fit(p, !zeta || !uniform, "GHK draws")) return rc;
     cudaStream_t stream = static_cast<cudaStream_t>(cuda_stream);
     char* gbase = static_cast<char*>(ghk_ws);
     int rc;
@@ -685,16 +672,7 @@ int mpvae_probit_predict_conditional_ghk(const mpvae_probit_params* p_in, const 
         gram = G;
     }
     if ((rc = predict_product(c, stream))) return rc;
-    GhkInputs in{};
-    in.layout = gl;
-    in.ws = ghk_ws;
-    in.max_observed = max_observed;
-    in.observed = observed;
-    in.gram = gram;
-    in.zeta = zeta; in.uniform = uniform;
-    in.noise_b_global = p->noise_b_global; in.noise_row0 = p->noise_row0;
-    in.noise_seed = p->noise_seed; in.noise_offset = p->noise_offset; in.noise_offset_dev = p->noise_offset_dev;
-    in.log_evidence = log_evidence; in.ess = ess;
+    const GhkInputs in{gl, ghk_ws, max_observed, observed, gram, zeta, uniform, philox_rows(p), log_evidence, ess};
     ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
     return launch_ghk_rows(c.a, in, stream);
 }

@@ -332,10 +332,10 @@ int launch_ghk_rows(RowArgs a, const GhkInputs& in, cudaStream_t stream) {
     g.wv = reinterpret_cast<double*>(base + w.wv);
     g.observed = in.observed;
     g.zeta = in.zeta; g.uniform = in.uniform;
-    g.Bg = in.noise_b_global; g.row0 = in.noise_row0;
-    g.key = make_uint2((uint32_t)in.noise_seed ^ kGhkKey, (uint32_t)(in.noise_seed >> 32));
-    g.off = make_uint2((uint32_t)in.noise_offset, (uint32_t)(in.noise_offset >> 32));
-    g.off_dev = reinterpret_cast<const unsigned long long*>(in.noise_offset_dev);
+    g.Bg = in.rows.b_global; g.row0 = in.rows.row0;
+    g.key = make_uint2((uint32_t)in.rows.seed ^ kGhkKey, (uint32_t)(in.rows.seed >> 32));
+    g.off = make_uint2((uint32_t)in.rows.offset, (uint32_t)(in.rows.offset >> 32));
+    g.off_dev = reinterpret_cast<const unsigned long long*>(in.rows.offset_dev);
     const size_t smem = (size_t)g.kb * (mo > 0 ? mo : 1) * sizeof(double);
     if (smem > kChainSmem) {
         const cudaError_t e = cudaFuncSetAttribute(ghk_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -109,6 +109,14 @@ int launch_conditional_tail(RowArgs a, const int8_t* observed, const FusePart* p
 // Conditional prediction by a GHK sampler (conditional_ghk.cu), after the nt product (a.nr, overwritten with the
 // conditioned samples).  Its own scratch block: G = R R^T (L, L) fp32, the G product's scratch, per row the observed
 // count and index list, the fp64 Cholesky factor (mo x mo) and two fp64 (S, mo) vectors.
+// The params' Philox key of a batch: rows [row0, row0 + B) of a b_global-row draw, seed, offset and the optional device
+// counter added to the offset.  The GHK sampler and the label sampler key their own streams by it.
+struct PhiloxRows {
+    int b_global, row0;
+    uint64_t seed, offset;
+    const uint64_t* offset_dev;
+};
+
 struct GhkLayout { size_t gram, gram_scratch, nobs, idx, fac, eta, wv, total; };
 GhkLayout ghk_layout(int S, int B, int L, int mo, size_t gram_scratch);
 struct GhkInputs {
@@ -118,9 +126,7 @@ struct GhkInputs {
     const int8_t* observed;
     const float* gram;                 // (L, L), read at [o_i, o_j] with o_i >= o_j and at rows o
     const float *zeta, *uniform;       // (S, B, L) or nullptr (the library's Philox draws)
-    int noise_b_global, noise_row0;
-    uint64_t noise_seed, noise_offset;
-    const uint64_t* noise_offset_dev;
+    PhiloxRows rows;
     float *log_evidence, *ess;
 };
 int launch_ghk_rows(RowArgs a, const GhkInputs& in, cudaStream_t stream);
@@ -130,9 +136,7 @@ int launch_ghk_rows(RowArgs a, const GhkInputs& in, cudaStream_t stream);
 struct SampleInputs {
     const float* uniform;              // (S, B, L) in (0, 1), or nullptr
     int32_t* bits;
-    int noise_b_global, noise_row0;
-    uint64_t noise_seed, noise_offset;
-    const uint64_t* noise_offset_dev;
+    PhiloxRows rows;
 };
 int launch_sample_labels(RowArgs a, const SampleInputs& in, cudaStream_t stream);
 // The F-measure-optimal decoder, one CTA per row, and its scratch: per row the sample cardinalities and weights (S each)

@@ -307,10 +307,10 @@ int launch_sample_labels(RowArgs a, const SampleInputs& in, cudaStream_t stream)
     g.bits = reinterpret_cast<uint32_t*>(in.bits);
     g.W = (a.L + 31) / 32;
     g.quads = (a.L + 3) / 4;
-    g.Bg = in.noise_b_global; g.row0 = in.noise_row0;
-    g.key = make_uint2((uint32_t)in.noise_seed ^ kSetKey, (uint32_t)(in.noise_seed >> 32));
-    g.off = make_uint2((uint32_t)in.noise_offset, (uint32_t)(in.noise_offset >> 32));
-    g.off_dev = reinterpret_cast<const unsigned long long*>(in.noise_offset_dev);
+    g.Bg = in.rows.b_global; g.row0 = in.rows.row0;
+    g.key = make_uint2((uint32_t)in.rows.seed ^ kSetKey, (uint32_t)(in.rows.seed >> 32));
+    g.off = make_uint2((uint32_t)in.rows.offset, (uint32_t)(in.rows.offset >> 32));
+    g.off_dev = reinterpret_cast<const unsigned long long*>(in.rows.offset_dev);
     if (a.stable) probit_sample_labels_kernel<true><<<grid, kThreads, 0, stream>>>(a, g, nchunks);
     else probit_sample_labels_kernel<false><<<grid, kThreads, 0, stream>>>(a, g, nchunks);
     return check_launch("probit_sample_labels_kernel");

@@ -7,6 +7,7 @@ and the predictions are gathered (no exchange inside the path, SURVEY 8e)."""
 from __future__ import annotations
 
 import copy
+import math
 from typing import Optional
 
 import torch
@@ -15,11 +16,24 @@ import torch.distributed as dist
 from .train import shard_rows
 
 
-def _score_rows(model, feats: torch.Tensor, args, batch_size: Optional[int], gather: bool, group, width: int, score):
+def _fields(res):
+    return (res,) if isinstance(res, torch.Tensor) else tuple(res)
+
+
+def _like(res, fields):
+    """`fields` in the type of the result `res`: a tensor, a tuple or a namedtuple."""
+    if isinstance(res, torch.Tensor):
+        return fields[0]
+    return type(res)(*fields) if hasattr(res, "_fields") else tuple(fields)
+
+
+def _score_rows(model, feats: torch.Tensor, args, batch_size: Optional[int], gather: bool, group, score):
     """The test-time row loop: `model.eval()`, `args.mode = 'test'`, this rank's contiguous slice of the N rows in
     batches of `batch_size` (default args.batch_size, test.py:41-43), then the gather of the slices.  score(a, b, args)
-    returns the (b - a, width) result of rows [a, b); it sees args.dp_global_batch = N, args.dp_row0 = a and the
-    pass's one noise offset."""
+    returns the result of rows [a, b): a tensor, or a tuple / namedtuple of tensors, each with b - a leading rows; it
+    sees args.dp_global_batch = N, args.dp_row0 = a and the pass's one noise offset.  The result has the same type,
+    with N rows.  A rank that owns no rows scores the empty slice [lo, lo), which gives each field's trailing shape and
+    dtype."""
     args = copy.copy(args)
     args.mode = "test"
     was_training = model.training
@@ -30,7 +44,7 @@ def _score_rows(model, feats: torch.Tensor, args, batch_size: Optional[int], gat
     lo, hi = shard_rows(n, rank, world)
     bs = min(batch_size or getattr(args, "batch_size", 128), max(hi - lo, 1))       # test.py:41
     out = []
-    n_batches = (hi - lo - 1) // bs + 1 if hi > lo else 0                            # test.py:43
+    n_batches = max((hi - lo - 1) // bs + 1, 1)                                      # test.py:43
     for i in range(n_batches):
         a, b = lo + bs * i, min(lo + bs * (i + 1), hi)
         args.dp_global_batch, args.dp_row0 = n, a
@@ -38,19 +52,28 @@ def _score_rows(model, feats: torch.Tensor, args, batch_size: Optional[int], gat
         # predictions do not depend on the world size or on how the rows are batched
         args.noise_offset = getattr(args, "noise_offset_base", 0)
         out.append(score(a, b, args))
-    local = torch.cat(out, 0) if out else feats.new_empty((0, width))
+    local = [torch.cat(f, 0) for f in zip(*map(_fields, out))]
     if was_training:
         model.train()
     if world == 1 or not gather:
-        return local
-    # gather the row slices (padded to the largest shard so one all_gather serves unequal shards)
+        return _like(out[0], local)
+    # gather the row slices as bytes, every field side by side (exact for every dtype), padded to the largest shard so
+    # one all_gather serves unequal shards
     sizes = [h - l for l, h in (shard_rows(n, r, world) for r in range(world))]
-    width = local.shape[1]
-    padded = local.new_zeros((max(sizes), width))
-    padded[:local.shape[0]] = local
+    rows = hi - lo
+    blob = torch.cat([f.reshape(rows, math.prod(f.shape[1:])).view(torch.uint8) for f in local], 1)
+    padded = blob.new_zeros((max(sizes), blob.shape[1]))
+    padded[:rows] = blob
     parts = [torch.empty_like(padded) for _ in range(world)]
     dist.all_gather(parts, padded, group=group)
-    return torch.cat([p[:k] for p, k in zip(parts, sizes)], 0)
+    blob = torch.cat([p[:k] for p, k in zip(parts, sizes)], 0)
+    fields, col = [], 0
+    for f in local:
+        nbytes = math.prod(f.shape[1:]) * f.element_size()
+        field = blob[:, col:col + nbytes].clone(memory_format=torch.contiguous_format)
+        fields.append(field.view(f.dtype).reshape(n, *f.shape[1:]))
+        col += nbytes
+    return _like(out[0], fields)
 
 
 @torch.no_grad()
@@ -79,13 +102,13 @@ def predict_proba(model, feats: torch.Tensor, labels: Optional[torch.Tensor], ar
         label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar = model(y, x)
         kw = {} if label_mask is None else {"label_mask": label_mask[a:b]}
         out = loss_fn(y, label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar, model.r_sqrt_sigma, args, **kw)
-        sums["total_loss"] = sums["total_loss"] + out[0] * (b - a)                   # test.py:67-70
-        sums["nll_loss"] = sums["nll_loss"] + out[1] * (b - a)
-        sums["c_loss"] = sums["c_loss"] + out[3] * (b - a)
+        if b > a:           # the empty slice of a rank without rows has NaN losses, means over nothing
+            sums["total_loss"] = sums["total_loss"] + out[0] * (b - a)               # test.py:67-70
+            sums["nll_loss"] = sums["nll_loss"] + out[1] * (b - a)
+            sums["c_loss"] = sums["c_loss"] + out[3] * (b - a)
         return out[6]
 
-    width = labels.shape[1] if labels is not None else model.r_sqrt_sigma.shape[0]
-    probs = _score_rows(model, feats, args, batch_size, gather, group, width, score)
+    probs = _score_rows(model, feats, args, batch_size, gather, group, score)
     return probs, (sums if labels is not None else None)
 
 
@@ -99,29 +122,22 @@ def predict_pairs(model, feats: torch.Tensor, pairs, args, batch_size: Optional[
     `model.feat_forward` (its latent sample); the probit noise is integrated out."""
     from .mpvae import PairPredictor
     predictor = PairPredictor(model.r_sqrt_sigma, pairs, args)
-    width = torch.as_tensor(pairs).shape[0]
-    return _score_rows(model, feats, args, batch_size, gather, group, width,
+    return _score_rows(model, feats, args, batch_size, gather, group,
                        lambda a, b, _: predictor(model.feat_forward(feats[a:b])[0]))
 
 
 @torch.no_grad()
 def predict_conditional(model, feats: torch.Tensor, observed: torch.Tensor, args, batch_size: Optional[int] = None,
                         gather: bool = True, group=None, predict_fn=None):
-    """(prob (N, L), log_evidence (N,), ess (N,)): `mpvae.predict_conditional` for each row of `feats` given that row's
-    known labels.  `observed` is the int8 (N, L) device tensor of states for ALL N rows (0 / 1 observed, -1 unobserved),
-    sliced per batch as predict_proba slices labels.  Same row sharding, batching, global-row noise keys and gather as
+    """ConditionalPrediction(prob (N, L), log_evidence (N,), ess (N,)): `mpvae.predict_conditional` for each row of
+    `feats` given that row's known labels.  `observed` is the int8 (N, L) device tensor of states for ALL N rows (0 / 1
+    observed, -1 unobserved), sliced per batch as predict_proba slices labels.  Same row sharding, batching, global-row noise keys and gather as
     predict_proba; with nothing observed, prob is predict_proba(labels=None)'s under the same torch seed.
     `predict_fn` (same signature and result, e.g. `mpvae.predict_conditional_ghk`) replaces mpvae.predict_conditional."""
     from . import mpvae
-    L = model.r_sqrt_sigma.shape[0]
     fn = predict_fn or mpvae.predict_conditional
-
-    def score(a, b, args):
-        res = fn(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, observed[a:b], args)
-        return torch.cat([res.prob, res.log_evidence[:, None], res.ess[:, None]], 1)
-
-    out = _score_rows(model, feats, args, batch_size, gather, group, L + 2, score)
-    return out[:, :L].contiguous(), out[:, L].contiguous(), out[:, L + 1].contiguous()
+    return _score_rows(model, feats, args, batch_size, gather, group,
+                       lambda a, b, args: fn(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, observed[a:b], args))
 
 
 @torch.no_grad()
@@ -131,14 +147,9 @@ def predict_sets(model, feats: torch.Tensor, args, beta: float = 1.0, max_size: 
     `feats` (device tensor, ALL N rows), the F_beta-optimal label set under the model's joint label distribution.  Same
     row sharding, batching, global-row noise keys and gather as predict_proba, so a row's set does not depend on either."""
     from . import mpvae
-    L = model.r_sqrt_sigma.shape[0]
-
-    def score(a, b, args):
-        res = mpvae.predict_sets(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, args, beta, max_size)
-        return torch.cat([res.sets.double(), res.expected_f[:, None], res.size[:, None].double()], 1)
-
-    out = _score_rows(model, feats, args, batch_size, gather, group, L + 2, score)
-    return mpvae.SetPrediction(out[:, :L] > 0.5, out[:, L].double().contiguous(), out[:, L + 1].to(torch.int32))
+    return _score_rows(model, feats, args, batch_size, gather, group,
+                       lambda a, b, args: mpvae.predict_sets(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, args,
+                                                             beta, max_size))
 
 
 @torch.no_grad()
@@ -149,14 +160,7 @@ def predict_mode(model, feats: torch.Tensor, args, max_flips: Optional[int] = No
     probable.  Same row sharding, batching, global-row noise keys and gather as predict_proba, so a row's set does not
     depend on either."""
     from . import mpvae
-    mpvae.check_max_flips(max_flips)
-    L = model.r_sqrt_sigma.shape[0]
-
-    def score(a, b, args):
-        res = mpvae.predict_mode(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, args, max_flips)
-        return torch.cat([res.sets.double(), res.log_prob[:, None], res.ess[:, None], res.size[:, None].double(),
-                          res.flips[:, None].double()], 1)
-
-    out = _score_rows(model, feats, args, batch_size, gather, group, L + 4, score)
-    return mpvae.ModePrediction(out[:, :L] > 0.5, out[:, L].contiguous(), out[:, L + 1].contiguous(),
-                                out[:, L + 2].to(torch.int32), out[:, L + 3].to(torch.int32))
+    mpvae.check_max_flips(max_flips)        # before any work
+    return _score_rows(model, feats, args, batch_size, gather, group,
+                       lambda a, b, args: mpvae.predict_mode(model.feat_forward(feats[a:b])[0], model.r_sqrt_sigma, args,
+                                                             max_flips))

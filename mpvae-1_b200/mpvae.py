@@ -197,10 +197,7 @@ def predict(fx_out, r_sqrt_sigma, args, noise=None):
     alone (`VAE.feat_forward(feature)[0]`): no labels, no label branch, no loss.  Same S (args.n_test_sample), same
     noise (`noise_plan`: a call without args.noise_offset consumes one offset, as compute_loss does), same flags, and
     bit for bit the indiv_prob compute_loss returns for the same fx_out.  Inference only: it builds no autograd graph."""
-    plan = _sample_plan("predict", fx_out, r_sqrt_sigma, args, noise)
-    if plan is None:
-        return fx_out.new_empty((0, fx_out.shape[1]))
-    n_sample, r32, noise, spec, flags = plan
+    n_sample, r32, noise, spec, flags = _sample_plan("predict", fx_out, r_sqrt_sigma, args, noise)
     return probit_predict(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags)
 
 
@@ -208,8 +205,9 @@ _UNCONDITIONAL = object()     # _sample_plan's `observed` for predict, which con
 
 
 def _sample_plan(name, fx_out, r_sqrt_sigma, args, noise, observed=_UNCONDITIONAL):
-    """The start of predict, predict_conditional and predict_conditional_ghk: the refusals, in this order, then
-    (n_sample, r32, noise, noise_spec, flags) as compute_loss plans them in test mode, or None for an empty batch."""
+    """The start of every sampled predictor: the refusals, in this order, then (n_sample, r32, noise, noise_spec, flags)
+    as compute_loss plans them in test mode.  An empty batch gets an (S, 0, Z) noise tensor and consumes no noise
+    offset; the probit wrappers return its empty outputs without calling the library."""
     _inference_only(name, fx_out, r_sqrt_sigma)
     device = fx_out.device
     if device.type != "cuda":
@@ -217,12 +215,12 @@ def _sample_plan(name, fx_out, r_sqrt_sigma, args, noise, observed=_UNCONDITIONA
                            "kernels only (no CPU fallback)")
     if observed is not _UNCONDITIONAL:
         _check_observed(observed, fx_out.shape, device)
-    n_batch = fx_out.shape[0]
-    if n_batch == 0:
-        return None
     n_sample = args.n_test_sample
     r32 = r_sqrt_sigma.to(device).float()
-    noise, spec = noise_plan(args, n_sample, n_batch, device, noise)
+    if fx_out.shape[0] == 0:
+        noise, spec = torch.empty((n_sample, 0, r32.shape[1]), dtype=torch.float32, device=device), None
+    else:
+        noise, spec = noise_plan(args, n_sample, fx_out.shape[0], device, noise)
     return n_sample, r32, noise, spec, int(getattr(args, "mpvae_flags", 0))
 
 
@@ -248,10 +246,7 @@ def predict_conditional(fx_out, r_sqrt_sigma, observed, args, noise=None):
     = unobserved.  From labels y and a boolean mask of the known ones:
         observed = torch.where(mask, y.to(torch.int8), -1)
     Its values are not checked (no host synchronisation).  Inference only, CUDA only; args.mpvae_flags as for predict."""
-    plan = _sample_plan("predict_conditional", fx_out, r_sqrt_sigma, args, noise, observed)
-    if plan is None:
-        return ConditionalPrediction(fx_out.new_empty((0, fx_out.shape[1])), fx_out.new_empty(0), fx_out.new_empty(0))
-    n_sample, r32, noise, spec, flags = plan
+    n_sample, r32, noise, spec, flags = _sample_plan("predict_conditional", fx_out, r_sqrt_sigma, args, noise, observed)
     return ConditionalPrediction(*probit_predict_conditional(fx_out, r32, observed, n_sample, noise=noise, noise_spec=spec,
                                                              flags=flags))
 
@@ -291,24 +286,23 @@ def predict_conditional_ghk(fx_out, r_sqrt_sigma, observed, args, noise=None, gr
     groups that keep that scratch under GHK_WORKSPACE_BOUND bytes; rows are keyed by their global row, so the split
     changes no bits.  The sampler's own uniforms and normals come from a Philox stream separate from the noise.
     Inference only, CUDA only; args.mpvae_flags as for predict."""
-    plan = _sample_plan("predict_conditional_ghk", fx_out, r_sqrt_sigma, args, noise, observed)
+    n_sample, r32, noise, spec, flags = _sample_plan("predict_conditional_ghk", fx_out, r_sqrt_sigma, args, noise,
+                                                     observed)
     n_batch, L = fx_out.shape
-    if plan is None:
-        return ConditionalPrediction(fx_out.new_empty((0, L)), fx_out.new_empty(0), fx_out.new_empty(0))
-    n_sample, r32, noise, spec, flags = plan
     Z = r32.shape[1]
-    max_obs = int(((observed == 0) | (observed == 1)).sum(1).max().item())      # the one host synchronisation
+    # the one host synchronisation (none for an empty batch, which runs as one empty group)
+    max_obs = int(((observed == 0) | (observed == 1)).sum(1).max().item()) if n_batch else 0
     one = ghk_workspace_bytes(n_sample, 1, L, Z, max_obs, flags)
     per_row = max(ghk_workspace_bytes(n_sample, 2, L, Z, max_obs, flags) - one, 1)
     rows = max(1, (GHK_WORKSPACE_BOUND - (one - per_row)) // per_row)
-    n_groups = -(-n_batch // rows)
-    rows = -(-n_batch // n_groups)
+    n_groups = max(-(-n_batch // rows), 1)
+    rows = max(-(-n_batch // n_groups), 1)
     if gram is None and n_groups > 1 and max_obs > 0:
         gram = label_gram(r32, args)
     if spec is not None:
         b_global = spec[3] if spec[3] is not None else n_batch
     out = []
-    for a in range(0, n_batch, rows):
+    for a in range(0, max(n_batch, 1), rows):
         b = min(n_batch, a + rows)
         if spec is not None:
             group_noise, group_spec = None, (spec[0], spec[1], spec[2], b_global, spec[4] + a) + tuple(spec[5:])
@@ -330,10 +324,7 @@ def sample_labels(fx_out, r_sqrt_sigma, args, noise=None, uniform=None):
     samples keep the joint structure of I + R R^T that the marginals lose.  `uniform`: optional (S, B, L) fp32 draws in
     (0, 1); None = the library's own Philox stream, keyed by global row (args.dp_row0), so a row's samples do not depend
     on batching.  Inference only, CUDA only; args.mpvae_flags as for predict."""
-    plan = _sample_plan("sample_labels", fx_out, r_sqrt_sigma, args, noise)
-    if plan is None:
-        return torch.empty((0, args.n_test_sample, (fx_out.shape[1] + 31) // 32), dtype=torch.int32, device=fx_out.device)
-    n_sample, r32, noise, spec, flags = plan
+    n_sample, r32, noise, spec, flags = _sample_plan("sample_labels", fx_out, r_sqrt_sigma, args, noise)
     return probit_sample_labels(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags, uniform=uniform)
 
 
@@ -368,16 +359,10 @@ def predict_sets(fx_out, r_sqrt_sigma, args, beta=1.0, max_size=None, noise=None
     example-based F1; this uses the joint distribution of the row's labels.  Returns SetPrediction(sets (B, L) bool,
     expected_f (B,) float64: the expected F_beta of the set on the samples, size (B,) int32).  Same noise and offset
     consumption as predict.  Inference only, CUDA only."""
-    label_dim = fx_out.shape[1]
     check_set_args(beta, max_size)          # before the plan: a refused call consumes no noise offset
-    plan = _sample_plan("predict_sets", fx_out, r_sqrt_sigma, args, noise)
-    if plan is None:
-        return SetPrediction(torch.zeros((0, label_dim), dtype=torch.bool, device=fx_out.device),
-                             torch.empty(0, dtype=torch.float64, device=fx_out.device),
-                             torch.empty(0, dtype=torch.int32, device=fx_out.device))
-    n_sample, r32, noise, spec, flags = plan
+    n_sample, r32, noise, spec, flags = _sample_plan("predict_sets", fx_out, r_sqrt_sigma, args, noise)
     bits = probit_sample_labels(fx_out, r32, n_sample, noise=noise, noise_spec=spec, flags=flags)
-    return SetPrediction(*f1_sets(bits, label_dim, beta, max_size))
+    return SetPrediction(*f1_sets(bits, fx_out.shape[1], beta, max_size))
 
 
 SetScores = namedtuple("SetScores", ["log_prob", "ess"])
@@ -397,11 +382,7 @@ def score_sets(fx_out, r_sqrt_sigma, bits, args, noise=None):
     Inference only, CUDA only; args.mpvae_flags as for predict."""
     n_batch, label_dim = fx_out.shape
     check_set_bits(bits, n_batch, label_dim, fx_out.device)
-    plan = _sample_plan("score_sets", fx_out, r_sqrt_sigma, args, noise)
-    if plan is None:
-        empty = torch.empty((0, bits.shape[1]), dtype=torch.float64, device=fx_out.device)
-        return SetScores(empty, empty.clone())
-    n_sample, r32, noise, spec, flags = plan
+    n_sample, r32, noise, spec, flags = _sample_plan("score_sets", fx_out, r_sqrt_sigma, args, noise)
     return SetScores(*probit_score_sets(fx_out, r32, bits, n_sample, noise=noise, noise_spec=spec, flags=flags))
 
 
@@ -417,17 +398,8 @@ def predict_mode(fx_out, r_sqrt_sigma, args, max_flips=None, noise=None):
     single flip scores higher.  Returns ModePrediction(sets (B, L) bool, log_prob (B,) float64, ess (B,) float64 --
     score_sets of the set, bit for bit --, size (B,) int32, flips (B,) int32).  Same noise and offset consumption as
     predict.  Inference only, CUDA only; args.mpvae_flags as for predict."""
-    label_dim = fx_out.shape[1]
     check_max_flips(max_flips)              # before the plan: a refused call consumes no noise offset
-    plan = _sample_plan("predict_mode", fx_out, r_sqrt_sigma, args, noise)
-    if plan is None:
-        dev = fx_out.device
-        return ModePrediction(torch.zeros((0, label_dim), dtype=torch.bool, device=dev),
-                              torch.empty(0, dtype=torch.float64, device=dev),
-                              torch.empty(0, dtype=torch.float64, device=dev),
-                              torch.empty(0, dtype=torch.int32, device=dev),
-                              torch.empty(0, dtype=torch.int32, device=dev))
-    n_sample, r32, noise, spec, flags = plan
+    n_sample, r32, noise, spec, flags = _sample_plan("predict_mode", fx_out, r_sqrt_sigma, args, noise)
     return ModePrediction(*probit_predict_mode(fx_out, r32, n_sample, max_flips, noise=noise, noise_spec=spec,
                                                flags=flags))
 

@@ -10,6 +10,7 @@ from __future__ import annotations
 import ctypes as C
 import math
 import os
+from collections import namedtuple
 
 import torch
 
@@ -251,39 +252,65 @@ def _predict_dims(name, fx_out, r32, S, noise, noise_spec):
     return S, B, L, Z
 
 
+def _predict_tensors(fx_out, r32, noise, *optional):
+    """The device and dtype checks of a sampled prediction's tensors, after the shape of each optional input:
+    `optional` holds (name, tensor or None, expected shape) triples.  Returns fx_out, r32, noise and the optional
+    tensors, contiguous (None stays None)."""
+    names, tensors = ["fx_out", "r_sqrt_sigma", "noise"], [fx_out, r32, noise]
+    for name, t, shape in optional:
+        if t is not None and tuple(t.shape) != shape:
+            raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {shape}")
+        names.append(name)
+        tensors.append(t)
+    _check_tensors(names, tensors)
+    return [t.contiguous() if t is not None else None for t in tensors]
+
+
 def _predict_inputs(name, fx_out, r32, S, noise, noise_spec):
     """The checks of mpvae_probit_predict's inputs: (fx_out, r32, noise) contiguous, and (S, B, L, Z)."""
     dims = _predict_dims(name, fx_out, r32, S, noise, noise_spec)
-    _check_tensors(("fx_out", "r_sqrt_sigma", "noise"), (fx_out, r32, noise))
-    return fx_out.contiguous(), r32.contiguous(), (noise.contiguous() if noise is not None else None), dims
+    return (*_predict_tensors(fx_out, r32, noise), dims)
 
 
-def _run_predict(entry, fx_out, r32, noise, noise_spec, flags, dims, *args, row_outputs=0, out=None):
-    """Runs the sampled-prediction entry point `entry` of the library: allocates its workspace, prob (B, L) and
-    `row_outputs` fp32 (B,) outputs, and calls it with the params, `args`, the row outputs and the current stream.
-    Returns [prob, *row outputs].  `out`: the entry point's own output tensor instead of prob (it is poisoned here and
-    passed in `args` by the caller; indiv_prob stays NULL)."""
+Out = namedtuple("Out", ["shape", "dtype"])     # an output of a sampled-prediction entry point, for _run_predict
+Scratch = namedtuple("Scratch", ["nbytes"])     # a scratch block of one, besides the params' workspace
+
+
+def _run_predict(entry, fx_out, r32, noise, noise_spec, flags, dims, *args, prob=True):
+    """Runs the sampled-prediction entry point `entry` of the library: `args` are its C arguments between the params and
+    the stream, in order.  Each Out(shape, dtype) is allocated on fx_out's device and passed as its pointer, each
+    Scratch(nbytes) as its pointer and byte count; anything else is passed as is.  Outputs and scratch are poisoned under
+    MPVAE_POISON_WORKSPACE=1.  `prob`: the entry point writes params.indiv_prob, a (B, L) fp32 output that comes first.
+    Returns the outputs, in order.  With B == 0 they are returned with zero rows, and the library is not called."""
     S, B, L, Z = dims
-    lib = _lib.lib()
     dev = fx_out.device
     with torch.cuda.device(dev):
+        outs = [torch.empty((B, L), dtype=torch.float32, device=dev)] if prob else []
+        blocks, c_args = [], []
+        for a in args:
+            if isinstance(a, Out):
+                outs.append(torch.empty(a.shape, dtype=a.dtype, device=dev))
+                c_args.append(_ptr(outs[-1]))
+            elif isinstance(a, Scratch):
+                blocks.append(torch.empty(a.nbytes, dtype=torch.uint8, device=dev))
+                c_args += (_ptr(blocks[-1]), a.nbytes)
+            else:
+                c_args.append(a)
+        if B == 0:
+            return outs
+        lib = _lib.lib()
         ws = torch.empty(int(lib.mpvae_workspace_bytes(S, B, L, Z, 0, flags)), dtype=torch.uint8, device=dev)
-        writes_prob = out is None
-        out = [torch.empty((B, L), dtype=torch.float32, device=dev) if writes_prob else out]
-        for _ in range(row_outputs):
-            out.append(torch.empty(B, dtype=torch.float32, device=dev))
-            args += (_ptr(out[-1]),)
-        _poison(ws, *out)
+        _poison(ws, *blocks, *outs)
         p = _lib.ProbitParams()
         p.struct_bytes = C.sizeof(_lib.ProbitParams)
         p.flags = flags
         p.S, p.B, p.L, p.Z = S, B, L, Z
         p.fx_out, p.r, p.noise = _ptr(fx_out), _ptr(r32), _ptr(noise)
         _set_noise_spec(p, noise_spec, B)
-        p.indiv_prob = _ptr(out[0]) if writes_prob else None
+        p.indiv_prob = _ptr(outs[0]) if prob else None
         p.workspace, p.workspace_bytes = _ptr(ws), ws.numel()
-        _lib.check(getattr(lib, entry)(C.byref(p), *args, _stream(dev)), entry)
-    return out
+        _lib.check(getattr(lib, entry)(C.byref(p), *c_args, _stream(dev)), entry)
+    return outs
 
 
 def probit_predict(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0):
@@ -301,10 +328,11 @@ def probit_predict_conditional(fx_out, r32, observed, S, *, noise=None, noise_sp
     unobserved; it is not read on the host.  Observed cells return their value; with nothing observed prob is
     probit_predict's bit for bit.  `noise` / `noise_spec` / `flags` as for probit_predict; inference only."""
     fx_out, r32, noise, dims = _predict_inputs("probit_predict_conditional", fx_out, r32, S, noise, noise_spec)
-    _check_observed(observed, dims[1:3], fx_out.device)     # (B, L)
+    S, B, L, Z = dims
+    _check_observed(observed, (B, L), fx_out.device)
     observed = observed.contiguous()
     return tuple(_run_predict("mpvae_probit_predict_conditional", fx_out, r32, noise, noise_spec, flags, dims,
-                              _ptr(observed), row_outputs=2))
+                              _ptr(observed), Out((B,), torch.float32), Out((B,), torch.float32)))
 
 
 def ghk_workspace_bytes(S, B, L, Z, max_observed, flags=0):
@@ -322,21 +350,16 @@ def probit_predict_conditional_ghk(fx_out, r32, observed, S, max_observed, *, no
     dims = _predict_dims("probit_predict_conditional_ghk", fx_out, r32, S, noise, noise_spec)
     S, B, L, Z = dims
     _check_observed(observed, (B, L), fx_out.device)
-    if not 0 <= int(max_observed) <= L:
+    max_observed = int(max_observed)
+    if not 0 <= max_observed <= L:
         raise ValueError(f"max_observed={max_observed} outside [0, {L}]")
-    for name, t, shape in (("gram", gram, (L, L)), ("zeta", zeta, (S, B, L)), ("uniform", uniform, (S, B, L))):
-        if t is not None and tuple(t.shape) != shape:
-            raise ValueError(f"{name} has shape {tuple(t.shape)}, expected {shape}")
-    tensors = (fx_out, r32, noise, gram, zeta, uniform)
-    _check_tensors(("fx_out", "r_sqrt_sigma", "noise", "gram", "zeta", "uniform"), tensors)
-    fx_out, r32, noise, gram, zeta, uniform = (t.contiguous() if t is not None else None for t in tensors)
+    fx_out, r32, noise, gram, zeta, uniform = _predict_tensors(
+        fx_out, r32, noise, ("gram", gram, (L, L)), ("zeta", zeta, (S, B, L)), ("uniform", uniform, (S, B, L)))
     observed = observed.contiguous()
-    gws_bytes = ghk_workspace_bytes(S, B, L, Z, int(max_observed), flags)
-    gws = torch.empty(gws_bytes, dtype=torch.uint8, device=fx_out.device)
-    _poison(gws)
     return tuple(_run_predict("mpvae_probit_predict_conditional_ghk", fx_out, r32, noise, noise_spec, flags, dims,
-                              _ptr(observed), _ptr(gram), _ptr(zeta), _ptr(uniform), _ptr(gws), gws_bytes,
-                              int(max_observed), row_outputs=2))
+                              _ptr(observed), _ptr(gram), _ptr(zeta), _ptr(uniform),
+                              Scratch(ghk_workspace_bytes(S, B, L, Z, max_observed, flags)), max_observed,
+                              Out((B,), torch.float32), Out((B,), torch.float32)))
 
 
 def probit_sample_labels(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0, uniform=None):
@@ -346,14 +369,9 @@ def probit_sample_labels(fx_out, r32, S, *, noise=None, noise_spec=None, flags=0
     `noise` / `noise_spec` / `flags` as for probit_predict; inference only."""
     dims = _predict_dims("probit_sample_labels", fx_out, r32, S, noise, noise_spec)
     S, B, L, Z = dims
-    if uniform is not None and tuple(uniform.shape) != (S, B, L):
-        raise ValueError(f"uniform has shape {tuple(uniform.shape)}, expected {(S, B, L)}")
-    tensors = (fx_out, r32, noise, uniform)
-    _check_tensors(("fx_out", "r_sqrt_sigma", "noise", "uniform"), tensors)
-    fx_out, r32, noise, uniform = (t.contiguous() if t is not None else None for t in tensors)
-    bits = torch.empty((B, S, (L + 31) // 32), dtype=torch.int32, device=fx_out.device)
+    fx_out, r32, noise, uniform = _predict_tensors(fx_out, r32, noise, ("uniform", uniform, (S, B, L)))
     return _run_predict("mpvae_probit_sample_labels", fx_out, r32, noise, noise_spec, flags, dims, _ptr(uniform),
-                        _ptr(bits), out=bits)[0]
+                        Out((B, S, (L + 31) // 32), torch.int32), prob=False)[0]
 
 
 def check_set_args(beta, max_size):
@@ -429,12 +447,6 @@ def mode_workspace_bytes(S, B, L):
     return int(_lib.lib().mpvae_mode_workspace_bytes(S, B, L))
 
 
-def _mode_ws(dims, dev):
-    S, B, L, _ = dims
-    n = mode_workspace_bytes(S, B, L)
-    return torch.empty(n, dtype=torch.uint8, device=dev), n
-
-
 def probit_score_sets(fx_out, r32, bits, S, *, noise=None, noise_spec=None, flags=0):
     """(log_prob (B, C) fp64, ess (B, C) fp64) of the C label sets per row in `bits` ((B, C, ceil(L / 32)) int32,
     sample_labels' layout) under the S-sample mixture probit_predict averages, on its noise
@@ -444,15 +456,9 @@ def probit_score_sets(fx_out, r32, bits, S, *, noise=None, noise_spec=None, flag
     check_set_bits(bits, B, L, fx_out.device)
     bits = bits.contiguous()
     C_ = bits.shape[1]
-    dev = fx_out.device
-    with torch.cuda.device(dev):
-        ws, n = _mode_ws(dims, dev)
-        log_prob = torch.empty((B, C_), dtype=torch.float64, device=dev)
-        ess = torch.empty((B, C_), dtype=torch.float64, device=dev)
-        _poison(ws, ess)
-    _run_predict("mpvae_probit_score_sets", fx_out, r32, noise, noise_spec, flags, dims, _ptr(bits), C_,
-                 _ptr(log_prob), _ptr(ess), _ptr(ws), n, out=log_prob)
-    return log_prob, ess
+    return tuple(_run_predict("mpvae_probit_score_sets", fx_out, r32, noise, noise_spec, flags, dims, _ptr(bits), C_,
+                              Out((B, C_), torch.float64), Out((B, C_), torch.float64),
+                              Scratch(mode_workspace_bytes(S, B, L)), prob=False))
 
 
 def probit_predict_mode(fx_out, r32, S, max_flips=None, *, noise=None, noise_spec=None, flags=0):
@@ -462,17 +468,10 @@ def probit_predict_mode(fx_out, r32, S, max_flips=None, *, noise=None, noise_spe
     max_flips = check_max_flips(max_flips)
     fx_out, r32, noise, dims = _predict_inputs("probit_predict_mode", fx_out, r32, S, noise, noise_spec)
     S, B, L, Z = dims
-    dev = fx_out.device
-    with torch.cuda.device(dev):
-        ws, n = _mode_ws(dims, dev)
-        sets = torch.empty((B, L), dtype=torch.uint8, device=dev)
-        log_prob = torch.empty(B, dtype=torch.float64, device=dev)
-        ess = torch.empty(B, dtype=torch.float64, device=dev)
-        size = torch.empty(B, dtype=torch.int32, device=dev)
-        flips = torch.empty(B, dtype=torch.int32, device=dev)
-        _poison(ws, log_prob, ess, size, flips)
-    _run_predict("mpvae_probit_predict_mode", fx_out, r32, noise, noise_spec, flags, dims, max_flips, _ptr(sets),
-                 _ptr(log_prob), _ptr(ess), _ptr(size), _ptr(flips), _ptr(ws), n, out=sets)
+    sets, log_prob, ess, size, flips = _run_predict(
+        "mpvae_probit_predict_mode", fx_out, r32, noise, noise_spec, flags, dims, max_flips,
+        Out((B, L), torch.uint8), Out((B,), torch.float64), Out((B,), torch.float64), Out((B,), torch.int32),
+        Out((B,), torch.int32), Scratch(mode_workspace_bytes(S, B, L)), prob=False)
     return sets.view(torch.bool), log_prob, ess, size, flips
 
 
