@@ -413,6 +413,13 @@ const char *mpvae_profile_name(int32_t slot);
  * main path without its special-case blocks) and ref[i] = logf(in[i]), n device floats each; tests assert bit equality
  * over the whole domain the loss uses, [4.7e-7, 1]. */
 int mpvae_test_log_normal(const float *in, float *out, float *ref, uint64_t n, void *cuda_stream);
+/* Test hook: out[i] = the erf of probit_E on the device (csrc/probit_math.cuh::erf_dual, used by the faithful cells) and
+ * ref[i] = libdevice erff(in[i]), n device floats each; tests assert bit equality over every fp32 input. */
+int mpvae_test_erf(const float *in, float *out, float *ref, uint64_t n, void *cuda_stream);
+/* Test hook: the multi-value warp reduction of the tiled row forward (common.cuh::warp_sum_transposed) against the plain
+ * butterfly, on `groups` warps' worth of input: fp64 != 0: 32 x 4 doubles per group, else 32 x 8 floats (value k of lane
+ * l at in[(g * 32 + l) * N + k]).  out and ref get N totals per group; tests assert bit equality. */
+int mpvae_test_warp_sum(const void *in, void *out, void *ref, int32_t groups, int32_t fp64, void *cuda_stream);
 
 const char *mpvae_last_error(void);
 int mpvae_abi_version(void);

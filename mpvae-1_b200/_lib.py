@@ -31,7 +31,7 @@ EXPORTS = (
     "mpvae_tc_gemm_nt", "mpvae_tc_gemm_tn", "mpvae_peer_flag_bytes", "mpvae_peer_allreduce", "mpvae_peer_allreduce_dev", "mpvae_peer_allreduce_nvls", "mpvae_label_curves",
     "mpvae_peer_alloc", "mpvae_peer_open", "mpvae_peer_close", "mpvae_peer_free", "mpvae_contract_workspace_bytes", "mpvae_last_error",
     "mpvae_abi_version", "mpvae_launch_count", "mpvae_batch_metrics", "mpvae_batch_metrics_workspace",
-    "mpvae_peer_error", "mpvae_profile", "mpvae_profile_read", "mpvae_profile_name", "mpvae_test_log_normal",
+    "mpvae_peer_error", "mpvae_profile", "mpvae_profile_read", "mpvae_profile_name", "mpvae_test_log_normal", "mpvae_test_erf", "mpvae_test_warp_sum",
     "mpvae_predictive_scale", "mpvae_predictive_rho", "mpvae_predict_exact", "mpvae_predict_pairs",
     "mpvae_probit_predict_conditional", "mpvae_probit_forward_masked", "mpvae_probit_backward_masked",
     "mpvae_ghk_workspace_bytes", "mpvae_probit_predict_conditional_ghk",
@@ -190,6 +190,10 @@ def _load():
     lib.mpvae_peer_error.argtypes = [C.c_void_p, C.POINTER(C.c_uint32), C.c_void_p]
     lib.mpvae_test_log_normal.restype = C.c_int
     lib.mpvae_test_log_normal.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]
+    lib.mpvae_test_erf.restype = C.c_int
+    lib.mpvae_test_erf.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]
+    lib.mpvae_test_warp_sum.restype = C.c_int
+    lib.mpvae_test_warp_sum.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]
     lib.mpvae_profile.restype = C.c_int
     lib.mpvae_profile.argtypes = [C.c_int32]
     lib.mpvae_profile_read.restype = C.c_int

@@ -839,6 +839,16 @@ int mpvae_test_log_normal(const float* in, float* out, float* ref, uint64_t n, v
     return launch_log_normal_probe(in, out, ref, (size_t)n, static_cast<cudaStream_t>(cuda_stream));
 }
 
+int mpvae_test_erf(const float* in, float* out, float* ref, uint64_t n, void* cuda_stream) {
+    if (!in || !out || !ref || n == 0) { set_error("test_erf: bad arguments"); return 1; }
+    return launch_erf_probe(in, out, ref, (size_t)n, static_cast<cudaStream_t>(cuda_stream));
+}
+
+int mpvae_test_warp_sum(const void* in, void* out, void* ref, int32_t groups, int32_t fp64, void* cuda_stream) {
+    if (!in || !out || !ref || groups <= 0) { set_error("test_warp_sum: bad arguments"); return 1; }
+    return launch_warp_sum_probe(in, out, ref, groups, fp64 != 0, static_cast<cudaStream_t>(cuda_stream));
+}
+
 int mpvae_philox_normal(float* noise, int32_t S, int32_t B, int32_t Z, int32_t B_global, int32_t row0, uint64_t seed,
                         uint64_t offset, void* cuda_stream) {
     if (!noise) { set_error("philox: NULL output"); return 1; }

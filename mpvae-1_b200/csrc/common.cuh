@@ -84,6 +84,30 @@ __device__ __forceinline__ int warp_sum(int v) {
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
+// warp_sum of N values at once (N a power of two, <= 32) with fewer shuffles: at each of the first log2(N) xor levels a
+// lane keeps half of its values (the upper half where the level's bit of the lane is set) and trades the other half
+// with its partner; the remaining levels reduce the one value left as warp_sum does.  Every partial is added to the
+// same partner's partial at the same level as in warp_sum, with the lower lane's partial as the first operand: the
+// order lane 0 of warp_sum adds in at every level.  So each total has the bits of warp_sum's result in lane 0, NaN
+// payloads included (an fp64 add keeps its first NaN operand's payload; fp32 adds return the canonical NaN).  On return
+// v[0] holds the total of value lane >> (5 - log2 N); the other entries of v are clobbered.
+template <int N, typename T>
+__device__ __forceinline__ void warp_sum_transposed(T (&v)[N], int lane) {
+    static_assert(N >= 1 && N <= 32 && (N & (N - 1)) == 0, "N must be a power of two <= 32");
+    int o = 16;
+#pragma unroll
+    for (int n = N; n > 1; n >>= 1, o >>= 1) {
+        const bool upper = (lane & o) != 0;
+#pragma unroll
+        for (int k = 0; k < n / 2; ++k) {
+            const T recv = __shfl_xor_sync(0xffffffffu, upper ? v[k] : v[k + n / 2], o);
+            v[k] = (upper ? recv : v[k]) + (upper ? v[k + n / 2] : recv);
+        }
+    }
+#pragma unroll
+    for (; o > 0; o >>= 1) v[0] += __shfl_xor_sync(0xffffffffu, v[0], o);
+}
+
 __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));

@@ -12,7 +12,10 @@
 // rows (L = 14..81) still keep every warp busy.  Reductions over labels are warp shuffles (+ one smem
 // hop when nwl > 1); log-likelihood sums are carried in fp64 so the result is independent of the
 // summation order to ~1e-13 (the fp32 reference itself carries ~ulp(lp) of order noise, see DESIGN.md).
+#include <stddef.h>
 #include <stdlib.h>
+
+#include <type_traits>
 
 #include "common.cuh"
 #include "fused_rows.cuh"
@@ -190,6 +193,8 @@ probit_row_finalize_kernel(const RowArgs a) {
 // whatever B is.
 constexpr int kChunk = 128;   // labels per warp and iteration
 constexpr int kLL = 4;        // labels per lane
+static_assert(offsetof(FusePart, lp_x) == offsetof(FusePart, lp_l) + 8 && offsetof(FusePart, neg_x) == offsetof(FusePart, pos_l) + 12,
+              "the tiled forward stores FusePart's two double and four float sums as arrays");
 
 // MASKED: an unobserved cell (a.mask[b, l] == 0) reads y as 0 and adds nothing to the log-likelihood or the ranking sums;
 // its E still enters the predictions and the saved E_l / E_x.  The mask bytes are byte loads (b * L need not be a
@@ -227,18 +232,21 @@ probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nc
         for (int s0 = 0; s0 < S; s0 += kST) {
             const float4 m0 = load(s0 + 2), m1 = load(s0 + 3);        // next pair in flight
             float pl[kLL] = {0.f, 0.f, 0.f, 0.f}, px[kLL] = {0.f, 0.f, 0.f, 0.f};   // same pairwise order as before
-            double lpl[kST], lpx[kST];
-            float pn[kST][4];
+            // the pair's six label sums, laid out for warp_sum_transposed: {lp_l, lp_x} and {pos_l, neg_l, pos_x, neg_x}
+            // per sample; a sample >= S (odd S) keeps zeros, so the reductions below run on every lane unconditionally
+            double lp[2 * kST];
+            float pn[4 * kST];
+#pragma unroll
+            for (int k = 0; k < 2 * kST; ++k) lp[k] = 0.0;
+#pragma unroll
+            for (int k = 0; k < 4 * kST; ++k) pn[k] = 0.f;
 #pragma unroll
             for (int i = 0; i < kST; ++i) {
-                lpl[i] = lpx[i] = 0.0;
-                pn[i][0] = pn[i][1] = pn[i][2] = pn[i][3] = 0.f;
                 const int s = s0 + i;
                 if (s >= S) continue;
                 const float4 n4 = i == 0 ? n0 : n1;
                 const float nv[kLL] = {n4.x, n4.y, n4.z, n4.w};
                 float el[kLL], ex[kLL];
-                float ll_l = 0.f, ll_x = 0.f;
 #pragma unroll
                 for (int j = 0; j < kLL; ++j) {
                     el[j] = ex[j] = 0.f;
@@ -246,14 +254,13 @@ probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nc
                         const CellFwd cl = cell_forward<STABLE>(nv[j] + fe[j], y[j]);   // mpvae.py:168,177
                         const CellFwd cx = cell_forward<STABLE>(nv[j] + fx[j], y[j]);   // mpvae.py:170,180
                         if (!MASKED || obs[j]) {
-                            lpl[i] += (double)cl.ll; lpx[i] += (double)cx.ll;
-                            pn[i][0] += cl.epos; pn[i][1] += cl.eneg; pn[i][2] += cx.epos; pn[i][3] += cx.eneg;
+                            lp[2 * i] += (double)cl.ll; lp[2 * i + 1] += (double)cx.ll;
+                            pn[4 * i] += cl.epos; pn[4 * i + 1] += cl.eneg; pn[4 * i + 2] += cx.epos; pn[4 * i + 3] += cx.eneg;
                         }
                         pl[j] += cl.E; px[j] += cx.E;
                         el[j] = cl.E; ex[j] = cx.E;
                     }
                 }
-                (void)ll_l; (void)ll_x;
                 if (a.E_l && any) {   // kept for the backward (training)
                     const size_t o = row_of(a, s, b) * a.ldn + l0;
                     *reinterpret_cast<float4*>(a.E_l + o) = make_float4(el[0], el[1], el[2], el[3]);
@@ -262,18 +269,14 @@ probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nc
             }
 #pragma unroll
             for (int j = 0; j < kLL; ++j) { accl[j] += pl[j]; accx[j] += px[j]; }
-#pragma unroll
-            for (int i = 0; i < kST; ++i) {
-                if (s0 + i >= S) continue;
-                lpl[i] = warp_sum(lpl[i]); lpx[i] = warp_sum(lpx[i]);
-#pragma unroll
-                for (int q = 0; q < 4; ++q) pn[i][q] = warp_sum(pn[i][q]);
-                if (lane == 0) {
-                    FusePart p;
-                    p.lp_l = lpl[i]; p.lp_x = lpx[i];
-                    p.pos_l = pn[i][0]; p.neg_l = pn[i][1]; p.pos_x = pn[i][2]; p.neg_x = pn[i][3];
-                    part[((size_t)b * S + s0 + i) * nchunks + c] = p;
-                }
+            // warp_sum's bits for each of the six sums; lane 8k holds lp[k], lane 4k holds pn[k]
+            warp_sum_transposed(lp, lane);
+            warp_sum_transposed(pn, lane);
+            FusePart* __restrict__ dst = part + ((size_t)b * S + s0) * nchunks + c;
+            if (s0 + (lane >> 4) < S) {
+                char* rec = reinterpret_cast<char*>(dst + (size_t)(lane >> 4) * nchunks);
+                if ((lane & 7) == 0) reinterpret_cast<double*>(rec + offsetof(FusePart, lp_l))[(lane >> 3) & 1] = lp[0];
+                if ((lane & 3) == 0) reinterpret_cast<float*>(rec + offsetof(FusePart, pos_l))[(lane >> 2) & 3] = pn[0];
             }
             n0 = m0; n1 = m1;
         }
@@ -501,9 +504,11 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
     // chunks of 64 labels; with operand planes the chunks run to the plane pitch (a multiple of 64): pad columns get zeros
     const int nchunks = a.gxs_planes ? a.gxs_pitch / 64 : (L + 63) / 64;
     const size_t yoff = (size_t)b * L;
-    for (int c = blockIdx.y * kWarps + warp; c < nchunks; c += gridDim.y * kWarps) {
+    // FULL: all 64 labels of the chunk lie inside the row (every chunk but a row's last and the plane pitch's padding)
+    auto chunk = [&](int c, auto full) {
+        constexpr bool FULL = decltype(full)::value;
         const int l0 = c * 64 + 2 * lane;
-        const bool in0 = l0 < L, in1 = l0 + 1 < L;
+        const bool in0 = FULL || l0 < L, in1 = FULL || l0 + 1 < L;
         float y0 = 0.f, y1 = 0.f, fe0 = 0.f, fe1 = 0.f, fx0 = 0.f, fx1 = 0.f, gpl0 = 0.f, gpl1 = 0.f, gpx0 = 0.f, gpx1 = 0.f;
         bool ob0 = true, ob1 = true;
         if (MASKED) { ob0 = in0 && a.mask[yoff + l0] != 0; ob1 = in1 && a.mask[yoff + l0 + 1] != 0; }
@@ -514,7 +519,7 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
         float gl0 = 0.f, gl1 = 0.f, gx0 = 0.f, gx1 = 0.f;
         // rows are 16-byte aligned (ldn % 4 == 0) and l0 is even: 8-byte loads; columns [L, ldn) of the cubes are pitch
         // padding that is never read as a label (in0 / in1)
-        const bool pair = l0 + 1 < a.ldn;
+        const bool pair = FULL || l0 + 1 < a.ldn;
         struct Cell3 { float2 n, l, x; };
         auto load = [&](int s) {
             Cell3 v;
@@ -542,25 +547,17 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
                 const Cell3& v = cur[i];
                 float d0 = 0.f, d1 = 0.f;
                 if (in0) {
-                    float dl, dx;
-                    if (ob0) {
-                        dl = cell_backward_saved(v.n.x + fe0, v.l.x, y0, cf[0], cf[2], cf[4], gpl0);
-                        dx = cell_backward_saved(v.n.x + fx0, v.x.x, y0, cf[1], cf[3], cf[5], gpx0);
-                    } else {
-                        dl = cell_backward_saved(v.n.x + fe0, v.l.x, 0.0f, 0.0f, 0.0f, 0.0f, gpl0);
-                        dx = cell_backward_saved(v.n.x + fx0, v.x.x, 0.0f, 0.0f, 0.0f, 0.0f, gpx0);
-                    }
+                    const float dl = cell_backward_saved(v.n.x + fe0, v.l.x, y0, ob0 ? cf[0] : 0.0f, ob0 ? cf[2] : 0.0f,
+                                                         ob0 ? cf[4] : 0.0f, gpl0);
+                    const float dx = cell_backward_saved(v.n.x + fx0, v.x.x, y0, ob0 ? cf[1] : 0.0f, ob0 ? cf[3] : 0.0f,
+                                                         ob0 ? cf[5] : 0.0f, gpx0);
                     gl0 += dl; gx0 += dx; d0 = dl + dx;
                 }
                 if (in1) {
-                    float dl, dx;
-                    if (ob1) {
-                        dl = cell_backward_saved(v.n.y + fe1, v.l.y, y1, cf[0], cf[2], cf[4], gpl1);
-                        dx = cell_backward_saved(v.n.y + fx1, v.x.y, y1, cf[1], cf[3], cf[5], gpx1);
-                    } else {
-                        dl = cell_backward_saved(v.n.y + fe1, v.l.y, 0.0f, 0.0f, 0.0f, 0.0f, gpl1);
-                        dx = cell_backward_saved(v.n.y + fx1, v.x.y, 0.0f, 0.0f, 0.0f, 0.0f, gpx1);
-                    }
+                    const float dl = cell_backward_saved(v.n.y + fe1, v.l.y, y1, ob1 ? cf[0] : 0.0f, ob1 ? cf[2] : 0.0f,
+                                                         ob1 ? cf[4] : 0.0f, gpl1);
+                    const float dx = cell_backward_saved(v.n.y + fx1, v.x.y, y1, ob1 ? cf[1] : 0.0f, ob1 ? cf[3] : 0.0f,
+                                                         ob1 ? cf[5] : 0.0f, gpx1);
                     gl1 += dl; gx1 += dx; d1 = dl + dx;
                 }
                 if (a.gxs_planes) {
@@ -582,6 +579,10 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
         }
         if (in0) { a.g_fe_out[yoff + l0] = gl0; a.g_fx_out[yoff + l0] = gx0; }
         if (in1) { a.g_fe_out[yoff + l0 + 1] = gl1; a.g_fx_out[yoff + l0 + 1] = gx1; }
+    };
+    for (int c = blockIdx.y * kWarps + warp; c < nchunks; c += gridDim.y * kWarps) {
+        if ((c + 1) * 64 <= L) chunk(c, std::true_type{});
+        else chunk(c, std::false_type{});
     }
     if (blockIdx.y == 0) {   // KL gradients (SURVEY 8a-12): c = a_kl * 0.5 / B
         const float kc = rc.a_kl * 0.5f / fB;
@@ -814,6 +815,32 @@ __global__ void log_normal_probe_kernel(const float* __restrict__ in, float* __r
     }
 }
 
+__global__ void erf_probe_kernel(const float* __restrict__ in, float* __restrict__ out, float* __restrict__ ref, size_t n) {
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
+        out[i] = MPV_ERF(in[i]);
+        ref[i] = erff(in[i]);
+    }
+}
+
+// in: groups of 32 lanes x N values (value k of lane l at in[(g * 32 + l) * N + k]); out[g * N + k]: the total of value k
+// from warp_sum_transposed (written by the lane that holds it), ref[g * N + k]: warp_sum's total from lane 0
+template <int N, typename T>
+__global__ void warp_sum_probe_kernel(const T* __restrict__ in, T* __restrict__ out, T* __restrict__ ref, int groups) {
+    const int lane = threadIdx.x & 31;
+    for (int g = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); g < groups; g += gridDim.x * (blockDim.x >> 5)) {
+        T v[N];
+#pragma unroll
+        for (int k = 0; k < N; ++k) {
+            v[k] = in[((size_t)g * 32 + lane) * N + k];
+            const T r = warp_sum(v[k]);
+            if (lane == 0) ref[(size_t)g * N + k] = r;
+        }
+        warp_sum_transposed(v, lane);
+        constexpr int shift = N == 1 ? 5 : N == 2 ? 4 : N == 4 ? 3 : N == 8 ? 2 : N == 16 ? 1 : 0;
+        if ((lane & ((1 << shift) - 1)) == 0) out[(size_t)g * N + (lane >> shift)] = v[0];
+    }
+}
+
 int pick_nwl(int L) {
     const int nchunks = (L + 31) / 32;
     int nwl = 1;
@@ -886,6 +913,23 @@ int launch_small_backward(RowArgs a, const SmallNoise& n, float* g_r, cudaStream
 int launch_log_normal_probe(const float* in, float* out, float* ref, size_t n, cudaStream_t stream) {
     log_normal_probe_kernel<<<4 * kNumSMs, 256, 0, stream>>>(in, out, ref, n);
     return check_launch("log_normal_probe_kernel");
+}
+
+int launch_erf_probe(const float* in, float* out, float* ref, size_t n, cudaStream_t stream) {
+    erf_probe_kernel<<<4 * kNumSMs, 256, 0, stream>>>(in, out, ref, n);
+    return check_launch("erf_probe_kernel");
+}
+
+// the two shapes the tiled forward reduces: eight float sums and four double sums per (sample pair, chunk)
+int launch_warp_sum_probe(const void* in, void* out, void* ref, int groups, bool fp64, cudaStream_t stream) {
+    const int grid = ceil_div(groups, kWarps) < 4 * kNumSMs ? ceil_div(groups, kWarps) : 4 * kNumSMs;
+    if (fp64)
+        warp_sum_probe_kernel<4, double><<<grid, kThreads, 0, stream>>>(static_cast<const double*>(in), static_cast<double*>(out),
+                                                                        static_cast<double*>(ref), groups);
+    else
+        warp_sum_probe_kernel<8, float><<<grid, kThreads, 0, stream>>>(static_cast<const float*>(in), static_cast<float*>(out),
+                                                                       static_cast<float*>(ref), groups);
+    return check_launch("warp_sum_probe_kernel");
 }
 
 int row_chunks(int L) { return (L + kChunk - 1) / kChunk; }

@@ -81,6 +81,8 @@ int launch_small_forward(RowArgs a, const SmallNoise& n, cudaStream_t stream);
 // g_r may be nullptr (R frozen); needs the forward's kept nr / E / noise
 int launch_small_backward(RowArgs a, const SmallNoise& n, float* g_r, cudaStream_t stream);
 int launch_log_normal_probe(const float* in, float* out, float* ref, size_t n, cudaStream_t stream);   // test hook
+int launch_erf_probe(const float* in, float* out, float* ref, size_t n, cudaStream_t stream);          // test hook
+int launch_warp_sum_probe(const void* in, void* out, void* ref, int groups, bool fp64, cudaStream_t stream);   // test hook
 int row_chunks(int L);   // 64-label chunks of a row: launch_row_forward needs B * S * row_chunks(L) FusePart records in a.part
 int launch_row_forward(RowArgs a, cudaStream_t stream);
 // the tail of the forward when the product kernel has already done the cell work (a.part != nullptr)
