@@ -292,6 +292,24 @@ int mpvae_probit_backward(const mpvae_probit_params *p, void *cuda_stream);
 int mpvae_probit_forward_masked(const mpvae_probit_params *p, const uint8_t *label_mask, void *cuda_stream);
 int mpvae_probit_backward_masked(const mpvae_probit_params *p, const uint8_t *label_mask, void *cuda_stream);
 
+/* Weighted rows: the forward and backward of the ELBO with a weight per batch row.  row_weight (B) fp32 on the device;
+ * label_mask as above; either may be NULL (NULL, NULL = mpvae_probit_forward / _backward).  Per row b the terms
+ *   t_b = nll_b (the label branch's -log mean_s exp lp_{s,b}), nll_x_b (the feature branch's), c_b and c_x_b (the row's
+ *         ranking sum over samples / S), kl_b (the row's KL term)
+ * give the five loss scalars sum_b w_b t_b / B -- the divisor is B, not sum w, so a weight of 1 on every row gives the
+ * unweighted bits and data-parallel shards add with no extra reduction -- and total_loss from them as before.
+ * indiv_prob and indiv_prob_label do not depend on the weights.  A row with w_b == 0 is skipped in the batch sums (its
+ * inf / NaN terms do not enter) and gets all-zero loss coefficients in the backward: no NaN from a degenerate row, even
+ * without MPVAE_FLAG_SANITIZE_DEGENERATE; with finite inputs its logit gradient is the cotangent of the predictions
+ * alone and its KL gradients are 0.  Other weights are used as given (negatives included; NaN propagates) and are not
+ * checked.  The weights enter before the bound that scales the fp16 operands of the g_R product, so any weights keep
+ * that product's accuracy.  The backward must receive the forward's weights and mask.  Same workspace size as the
+ * unweighted calls. */
+int mpvae_probit_forward_weighted(const mpvae_probit_params *p, const uint8_t *label_mask, const float *row_weight,
+                                  void *cuda_stream);
+int mpvae_probit_backward_weighted(const mpvae_probit_params *p, const uint8_t *label_mask, const float *row_weight,
+                                   void *cuda_stream);
+
 /* Counter-based standard-normal noise, replaces torch.normal(0,1,(S,B,Z)) of mpvae.py:162.
  * Element (s, b_global, z) depends only on (seed, offset, s, b_global, z): a rank holding rows
  * [row0, row0+B) of a B_global-row batch draws the same numbers a single GPU would. */

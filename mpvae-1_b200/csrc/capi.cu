@@ -459,10 +459,15 @@ uint64_t mpvae_workspace_bytes(int32_t S, int32_t B, int32_t L, int32_t Z, int32
 }
 
 int mpvae_probit_forward(const mpvae_probit_params* p_in, void* cuda_stream) {
-    return mpvae_probit_forward_masked(p_in, nullptr, cuda_stream);
+    return mpvae_probit_forward_weighted(p_in, nullptr, nullptr, cuda_stream);
 }
 
 int mpvae_probit_forward_masked(const mpvae_probit_params* p_in, const uint8_t* label_mask, void* cuda_stream) {
+    return mpvae_probit_forward_weighted(p_in, label_mask, nullptr, cuda_stream);
+}
+
+int mpvae_probit_forward_weighted(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
+                                  void* cuda_stream) {
     mpvae_probit_params tmp;
     const mpvae_probit_params* p = normalize(p_in, &tmp);
     if (!p) return 1;
@@ -479,6 +484,7 @@ int mpvae_probit_forward_masked(const mpvae_probit_params* p_in, const uint8_t* 
     int rc;
     RowArgs a = row_args(p, w);
     a.mask = label_mask;
+    a.row_weight = row_weight;   // read by row_tail only: the fused forward's finalize kernel takes it as well
     // a scratch block sized for the backward means a training call: the forward keeps E for it (same placement in
     // both layouts: the backward-only buffers follow everything the forward shares)
     const Workspace wb = carve(p->S, p->B, p->L, p->Z, true, p->flags);
@@ -678,10 +684,15 @@ int mpvae_probit_predict_conditional_ghk(const mpvae_probit_params* p_in, const 
 }
 
 int mpvae_probit_backward(const mpvae_probit_params* p_in, void* cuda_stream) {
-    return mpvae_probit_backward_masked(p_in, nullptr, cuda_stream);
+    return mpvae_probit_backward_weighted(p_in, nullptr, nullptr, cuda_stream);
 }
 
 int mpvae_probit_backward_masked(const mpvae_probit_params* p_in, const uint8_t* label_mask, void* cuda_stream) {
+    return mpvae_probit_backward_weighted(p_in, label_mask, nullptr, cuda_stream);
+}
+
+int mpvae_probit_backward_weighted(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
+                                   void* cuda_stream) {
     mpvae_probit_params tmp;
     const mpvae_probit_params* p = normalize(p_in, &tmp);
     if (!p) return 1;
@@ -693,6 +704,7 @@ int mpvae_probit_backward_masked(const mpvae_probit_params* p_in, const uint8_t*
     const bool tensor = use_tensor(p->flags, p->S, p->B, p->L, p->Z);
     RowArgs a = row_args(p, w);
     a.mask = label_mask;
+    a.row_weight = row_weight;   // scales the per-row coefficients, and with them the gxs bound of the fp16 planes
     a.E_l = reinterpret_cast<float*>(base + w.e_l);
     a.E_x = reinterpret_cast<float*>(base + w.e_x);
     const int M = p->S * p->B;

@@ -139,7 +139,15 @@ __device__ __forceinline__ void row_tail(const RowArgs& a, int b) {
     __threadfence();
     if (warp < 5) {
         double acc = 0.0;
-        for (int r = lane; r < B; r += 32) acc += __ldcg(&a.rowout[(size_t)r * 8 + warp]);
+        if (a.row_weight == nullptr) {
+            for (int r = lane; r < B; r += 32) acc += __ldcg(&a.rowout[(size_t)r * 8 + warp]);
+        } else {
+            // sum_r w_r t_r in the same order; a zero-weight row is skipped, so its inf / NaN terms stay out of the sum
+            for (int r = lane; r < B; r += 32) {
+                const float w = a.row_weight[r];
+                if (w != 0.0f) acc += (double)w * __ldcg(&a.rowout[(size_t)r * 8 + warp]);
+            }
+        }
         acc = warp_sum(acc);
         if (lane == 0) s_fin[warp] = acc;
     }
@@ -292,16 +300,25 @@ probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nc
 
 // Per-row coefficients of the backward (see cell_backward): effective weights of the loss terms = d objective / d term
 // (mpvae.py:207-208 + upstream cotangents), the ranking normaliser k_b and the log-likelihood factor -(a_nll / B).
+// Weighted rows: a_nll, a_c and a_kl are multiplied by w_b before the divisions (a weight of 1 keeps the unweighted
+// bits); a zero-weight row gets all-zero coefficients, returned before the 0/0 of a degenerate row.
 struct RowCoeffs { float kb[2], cnb[2], a_kl; };
 
 __device__ __forceinline__ RowCoeffs row_coeffs(const RowArgs& a, int b) {
     const float gt = a.g_scalars[0] ? *a.g_scalars[0] : 0.0f, g1 = a.g_scalars[1] ? *a.g_scalars[1] : 0.0f,
                 g2 = a.g_scalars[2] ? *a.g_scalars[2] : 0.0f, g3 = a.g_scalars[3] ? *a.g_scalars[3] : 0.0f,
                 g4 = a.g_scalars[4] ? *a.g_scalars[4] : 0.0f, g5 = a.g_scalars[5] ? *a.g_scalars[5] : 0.0f;
-    const float a_nll[2] = {gt * a.nll_coeff + g1, gt * a.nll_coeff + g2};
-    const float a_c[2] = {gt * a.c_coeff + g3, gt * a.c_coeff + g4};
+    float a_nll[2] = {gt * a.nll_coeff + g1, gt * a.nll_coeff + g2};
+    float a_c[2] = {gt * a.c_coeff + g3, gt * a.c_coeff + g4};
     RowCoeffs rc;
     rc.a_kl = gt * 1.1f + g5;
+    if (a.row_weight != nullptr) {
+        const float w = a.row_weight[b];
+        if (w == 0.0f) return RowCoeffs{{0.0f, 0.0f}, {0.0f, 0.0f}, 0.0f};
+        a_nll[0] = MPV_MUL(a_nll[0], w); a_nll[1] = MPV_MUL(a_nll[1], w);
+        a_c[0] = MPV_MUL(a_c[0], w); a_c[1] = MPV_MUL(a_c[1], w);
+        rc.a_kl = MPV_MUL(rc.a_kl, w);
+    }
     const float npos = a.rowaux[(size_t)b * 2], nneg = a.rowaux[(size_t)b * 2 + 1];
     const float norm5 = 5.0f * (npos * nneg);
     const float fS = (float)a.S, fB = (float)a.B;

@@ -56,6 +56,10 @@ struct RowArgs {
     // nothing to the log-likelihood, the ranking sums or the label counts, and its logit gradient is the cotangent of
     // indiv_prob / indiv_prob_label alone.  Whatever y holds there is never read into the arithmetic.
     const uint8_t* mask;
+    // weighted rows: (B) fp32, the weight of each row's loss terms; nullptr = every row weighs 1.  Enters only the last
+    // CTA's batch sums of row_tail (sum_b w_b t_b, a zero-weight row skipped) and row_coeffs (a_nll, a_c, a_kl scaled
+    // by w_b; all zero when w_b == 0).  No kernel is instantiated for it: the code branches on the pointer.
+    const float* row_weight;
 };
 
 size_t row_smem_bytes(int L);

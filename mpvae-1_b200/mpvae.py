@@ -28,7 +28,7 @@ from . import _lib
 from .dense import linear
 from .probit import ProbitELBO, label_pairs, philox_normal, predictive_rho, predictive_scale, probit_predict
 from .probit import contract_nt, ghk_workspace_bytes, predict_exact_from_r, probit_predict_conditional
-from .probit import _check_observed, probit_predict_conditional_ghk
+from .probit import _check_observed, _check_row_weight, probit_predict_conditional_ghk
 from .probit import check_set_args, f1_sets, probit_sample_labels
 from .probit import check_max_flips, check_set_bits, probit_predict_mode, probit_score_sets
 from .probit import predict_pairs as probit_predict_pairs
@@ -155,7 +155,7 @@ def draw_noise(args, n_sample, n_batch, device, noise=None):
 
 
 def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r_sqrt_sigma, args, noise=None,
-                 label_mask=None):
+                 label_mask=None, row_weight=None):
     """Reference signature (mpvae.py:145) -> (total_loss, nll_loss, nll_loss_x, c_loss, c_loss_x, kl_loss,
     indiv_prob, indiv_prob_label) (mpvae.py:210).
 
@@ -171,8 +171,25 @@ def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar
     Whatever input_label holds in an unobserved cell, NaN included, has no effect here.  (The label encoder still reads
     input_label as the caller gives it: filling unknown labels with 0 there is the caller's choice.)  A mask of all ones
     gives the unmasked results bit for bit.  With one row in test mode, -predict_conditional(...,
-    observed=torch.where(mask, y.to(torch.int8), -1)).log_evidence equals nll_loss_x on the same noise."""
+    observed=torch.where(mask, y.to(torch.int8), -1)).log_evidence equals nll_loss_x on the same noise.
+
+    `row_weight` (B,) floating tensor on the batch's device, or None (every row weighs 1): weighted rows, e.g. importance
+    weights, down-weighted noisy rows, or one weighted row for several duplicates.  It can be combined with label_mask.
+    With t_b the row's terms -- its negative log-mean-exp over samples of each branch, its ranking sum over samples / S
+    in each branch, its KL term -- the five loss scalars become sum_b w_b t_b / B, and total_loss is formed from them as
+    before:
+      - the divisor is B, not sum(w): a weight of 1 on every row gives the bits of row_weight=None on all 8 outputs and
+        every gradient, and data-parallel shards combine as before (for sum(w) normalisation pass w * B / w.sum());
+      - indiv_prob and indiv_prob_label do not depend on the weights;
+      - a row with weight 0 is removed from the loss: its terms (inf / NaN included) are skipped, and its loss gradients
+        are exactly 0 -- a degenerate row gets no NaN, even without MPVAE_FLAG_SANITIZE_DEGENERATE; with finite inputs
+        its logit gradient is the cotangent of the predictions alone;
+      - other values are used as given (negatives included; NaN propagates); they are not checked on the host.
+    The weights are converted to contiguous fp32 and receive no gradient: a weight that requires grad is refused, as are
+    a wrong shape, device or a non-floating dtype, before any noise offset is consumed."""
     device = input_label.device
+    if row_weight is not None:
+        row_weight = _check_row_weight(row_weight, fe_out.shape[0], device)
     if device.type != "cuda":
         raise RuntimeError("mpvae_b200.compute_loss needs CUDA tensors: the probit ELBO is implemented as sm_100a "
                            "kernels only (no CPU fallback)")
@@ -189,7 +206,7 @@ def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar
     # args.peer_ring (peer.PeerRing, data-parallel runs): g_R comes back already summed over the ranks
     return ProbitELBO.apply(input_label.float(), fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise,
                             float(args.nll_coeff), float(args.c_coeff), flags, spec, getattr(args, "peer_ring", None),
-                            label_mask)
+                            label_mask, row_weight)
 
 
 def predict(fx_out, r_sqrt_sigma, args, noise=None):

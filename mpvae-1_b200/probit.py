@@ -75,6 +75,21 @@ def _check_label_mask(label_mask, B, L, device):
     return label_mask.contiguous().view(torch.uint8)
 
 
+def _check_row_weight(row_weight, B, device):
+    """The (B,) row weights as a contiguous fp32 tensor, refused before any launch when they are not a floating tensor of
+    that shape on the batch's device, or when they require grad: the loss returns no gradient for them, and a silent
+    zero would mislead.  The values are not checked (that would synchronise with the host)."""
+    if not isinstance(row_weight, torch.Tensor) or not row_weight.is_floating_point():
+        raise TypeError(f"row_weight must be a floating tensor, got {getattr(row_weight, 'dtype', type(row_weight))}")
+    if row_weight.requires_grad:
+        raise ValueError("row_weight requires grad, but the loss returns no gradient for it: pass row_weight.detach()")
+    if row_weight.shape != (B,):
+        raise ValueError(f"row_weight has shape {tuple(row_weight.shape)}, expected {(B,)} (batch,)")
+    if row_weight.device != device:
+        raise ValueError(f"row_weight is on {row_weight.device}, expected {device}")
+    return row_weight.to(torch.float32).contiguous()
+
+
 def _check_observed(observed, shape, device):
     """Refuses an `observed` argument that is not an int8 tensor of `shape` (batch, label_dim) on `device`."""
     if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
@@ -119,11 +134,14 @@ class ProbitELBO(torch.autograd.Function):
 
     `label_mask` (B, L) bool / uint8 on the batch's device, or None: nonzero = the label is observed.  The
     log-likelihood and the ranking loss then run over the observed labels only (mpvae_probit_forward_masked); y is not
-    read where the mask is 0.  None runs the unmasked entry points."""
+    read where the mask is 0.  None runs the unmasked entry points.
+
+    `row_weight` (B,) floating on the batch's device, or None: the weight of each row's loss terms
+    (mpvae_probit_forward_weighted, semantics in mpvae.compute_loss).  It receives no gradient."""
 
     @staticmethod
     def forward(ctx, y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise, nll_coeff, c_coeff, flags,
-                noise_spec=None, peer=None, label_mask=None):
+                noise_spec=None, peer=None, label_mask=None, row_weight=None):
         lib = _lib.lib()
         y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32 = (
             t.contiguous() for t in (y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32))
@@ -135,6 +153,8 @@ class ProbitELBO(torch.autograd.Function):
         dev = y.device
         if label_mask is not None:
             label_mask = _check_label_mask(label_mask, B, L, dev)
+        if row_weight is not None:
+            row_weight = _check_row_weight(row_weight, B, dev)
         want_bwd = any(ctx.needs_input_grad)
         with torch.cuda.device(dev):
             ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 1 if want_bwd else 0, flags))
@@ -157,7 +177,10 @@ class ProbitELBO(torch.autograd.Function):
             p.indiv_prob, p.indiv_prob_label = _ptr(prob), _ptr(prob_label)
             p.workspace, p.workspace_bytes = _ptr(ws), ws_bytes
             stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            if label_mask is None:
+            if row_weight is not None:
+                _lib.check(lib.mpvae_probit_forward_weighted(C.byref(p), _ptr(label_mask), _ptr(row_weight), stream),
+                           "mpvae_probit_forward_weighted")
+            elif label_mask is None:
                 _lib.check(lib.mpvae_probit_forward(C.byref(p), stream), "mpvae_probit_forward")
             else:
                 _lib.check(lib.mpvae_probit_forward_masked(C.byref(p), _ptr(label_mask), stream),
@@ -168,9 +191,11 @@ class ProbitELBO(torch.autograd.Function):
             # data-parallel g_R over peer memory (peer.py): the backward then returns the SUM over all ranks
             ctx.peer = peer if (peer is not None and peer.applies(S, B, L, Z, flags)) else None
             ctx.has_mask = label_mask is not None
+            ctx.has_weight = row_weight is not None
             ctx.save_for_backward(y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, ws,
                                   *([noise] if noise is not None else []),
-                                  *([label_mask] if label_mask is not None else []))
+                                  *([label_mask] if label_mask is not None else []),
+                                  *([row_weight] if row_weight is not None else []))
             ctx.dims = (S, B, L, Z, D)
             ctx.coeffs = (float(nll_coeff), float(c_coeff), int(flags))
             ctx.set_materialize_grads(False)
@@ -180,8 +205,10 @@ class ProbitELBO(torch.autograd.Function):
     def backward(ctx, g_total, g_nll, g_nll_x, g_c, g_c_x, g_kl, g_prob, g_prob_label):
         lib = _lib.lib()
         y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, ws = ctx.saved_tensors[:9]
-        noise = ctx.saved_tensors[9] if ctx.has_noise else None
-        label_mask = ctx.saved_tensors[-1] if ctx.has_mask else None
+        rest = list(ctx.saved_tensors[9:])
+        noise = rest.pop(0) if ctx.has_noise else None
+        label_mask = rest.pop(0) if ctx.has_mask else None
+        row_weight = rest.pop(0) if ctx.has_weight else None
         S, B, L, Z, D = ctx.dims
         nll_coeff, c_coeff, flags = ctx.coeffs
         dev = y.device
@@ -224,14 +251,17 @@ class ProbitELBO(torch.autograd.Function):
             p.g_r = _ptr(g_r)
             p.workspace, p.workspace_bytes = _ptr(ws), ws.numel()
             stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            if label_mask is None:
+            if row_weight is not None:
+                _lib.check(lib.mpvae_probit_backward_weighted(C.byref(p), _ptr(label_mask), _ptr(row_weight), stream),
+                           "mpvae_probit_backward_weighted")
+            elif label_mask is None:
                 _lib.check(lib.mpvae_probit_backward(C.byref(p), stream), "mpvae_probit_backward")
             else:
                 _lib.check(lib.mpvae_probit_backward_masked(C.byref(p), _ptr(label_mask), stream),
                            "mpvae_probit_backward_masked")
         #       y     fe_out    fe_mu      fe_logvar  fx_out    fx_mu      fx_logvar  r32  noise nll_c c_c flags spec
         return (None, g_fe_out, g_mulv[0], g_mulv[1], g_fx_out, g_mulv[2], g_mulv[3], g_r, None, None, None, None, None,
-                None, None)
+                None, None, None)   # peer, label_mask, row_weight
 
 
 def _predict_dims(name, fx_out, r32, S, noise, noise_spec):

@@ -207,12 +207,16 @@ class DataParallelStep:
 
     # -- the step -------------------------------------------------------------------------------------------
     def step(self, input_label: torch.Tensor, input_feat: torch.Tensor, noise: Optional[torch.Tensor] = None,
-             r_override: Optional[torch.Tensor] = None, label_mask: Optional[torch.Tensor] = None) -> StepOutput:
+             r_override: Optional[torch.Tensor] = None, label_mask: Optional[torch.Tensor] = None,
+             row_weight: Optional[torch.Tensor] = None) -> StepOutput:
         """`input_label` (B, L) and `input_feat` (B, F) are the GLOBAL batch (train.py:106-111); every rank slices
         its rows.  `noise`, if given, is the global (S, B, Z) tensor (validation mode).  `r_override` is the
         fresh non-trainable R of residue_sigma == 'random' (train.py:120-122).  `label_mask`, if given, is the global
         (B, L) mask of observed labels (`compute_loss`): each rank passes its rows' slice to the loss as
-        `label_mask=`; without it the loss is called exactly as before, so custom loss functions keep working."""
+        `label_mask=`; without it the loss is called exactly as before, so custom loss functions keep working.
+        `row_weight`, if given, is the global (B,) row weight (`compute_loss`), sliced and passed as `row_weight=` in the
+        same way.  Each rank's terms are sum_b w_b t_b / (its rows) and the shard weighting below makes the global loss
+        sum over all rows of w_b t_b / B, as in one process."""
         args = self.args
         n_rows = input_label.shape[0]
         lo, hi = shard_rows(n_rows, self.rank, self.world)
@@ -238,6 +242,8 @@ class DataParallelStep:
             kw = {} if noise is None else {"noise": noise[:, lo:hi]}
             if label_mask is not None:
                 kw["label_mask"] = label_mask[lo:hi]
+            if row_weight is not None:
+                kw["row_weight"] = row_weight[lo:hi]
             out = self.loss_fn(y, label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar, r, args, **kw)
             total = out[0]
             if self.regulariser is not None:
@@ -295,10 +301,11 @@ class DataParallelStep:
 
 
 def train_one_epoch(step: DataParallelStep, feats, labels, batch_size: int, order=None, skip_empty: bool = True,
-                    masks=None):
+                    masks=None, weights=None):
     """Epoch driver with the reference's batching (train.py:98-111): int(N/bs)+1 steps, ragged (possibly empty)
     last batch.  `feats` / `labels` are device tensors (kept resident: SURVEY 8f-N4); returns per-step outputs.
-    `masks`, if given, is the (N, L) mask of observed labels (`compute_loss`), sliced by the same index as `labels`.
+    `masks`, if given, is the (N, L) mask of observed labels (`compute_loss`), sliced by the same index as `labels`;
+    `weights`, if given, the (N,) row weights (`compute_loss(..., row_weight=)`), sliced the same way.
     `skip_empty=False` reproduces the reference literally when bs | N: it runs the step on the empty batch, whose
     losses are NaN means (train.py:102; compute_loss returns them) and whose NaN gradients then reach Adam."""
     n = feats.shape[0]
@@ -309,10 +316,12 @@ def train_one_epoch(step: DataParallelStep, feats, labels, batch_size: int, orde
         idx = order[i * batch_size:min(batch_size * (i + 1), n)]
         if idx.numel() == 0 and skip_empty:
             continue          # the reference computes NaN losses on the empty batch and steps on them
-        if masks is None:
-            outs.append(step.step(labels[idx], feats[idx]))
-        else:
-            outs.append(step.step(labels[idx], feats[idx], label_mask=masks[idx]))
+        kw = {}
+        if masks is not None:
+            kw["label_mask"] = masks[idx]
+        if weights is not None:
+            kw["row_weight"] = weights[idx]
+        outs.append(step.step(labels[idx], feats[idx], **kw))
     return outs
 
 
@@ -329,7 +338,8 @@ class GraphedTrainStep:
         replays and writes the new rate into that tensor;
       * gradients are views into the flat bucket (no per-step allocation).
     Not supported in graph mode: world_size > 1 (see __init__), `skip_nonfinite` (needs a host decision) and Python-side
-    regularisers that branch on data.  Outputs are static tensors that the next replay overwrites."""
+    regularisers that branch on data.  Outputs are static tensors that the next replay overwrites.  Row weights
+    (`step(..., row_weight=)`) go into a static buffer as well; a weighted step is a capture of its own."""
 
     def __init__(self, stepper: DataParallelStep, warmup: int = 3):
         if stepper.skip_nonfinite:
@@ -403,8 +413,9 @@ class GraphedTrainStep:
                         else:
                             v.zero_()                                     # state born during the warm-up: back to "fresh"
 
-    def _capture(self, y, x):
+    def _capture(self, y, x, w):
         static_y, static_x = y.clone(), x.clone()
+        static_w = None if w is None else w.clone()
         st = self.stepper
         if st.world > 1:
             st.pbucket.enable_graph_replay()
@@ -417,31 +428,37 @@ class GraphedTrainStep:
         side.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(side):
             for _ in range(self.warmup):                                  # also initialises optimizer state
-                self._body(static_y, static_x)
+                self._body(static_y, static_x, static_w)
         torch.cuda.current_stream(self.device).wait_stream(side)
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
-            out = self._body(static_y, static_x)
+            out = self._body(static_y, static_x, static_w)
         self._restore(snap)                                               # parameters, moments, counters, RNG: as before
-        return {"graph": graph, "y": static_y, "x": static_x, "out": out}
+        return {"graph": graph, "y": static_y, "x": static_x, "w": static_w, "out": out}
 
-    def _body(self, y, x):
+    def _body(self, y, x, w):
         st = self.stepper
         sched, st.scheduler = st.scheduler, None                          # the scheduler is stepped on the host
         try:
-            out = st.step(y, x)
+            out = st.step(y, x) if w is None else st.step(y, x, row_weight=w)
         finally:
             st.scheduler = sched
         self.counter.add_(1)
         return out
 
-    def step(self, input_label: torch.Tensor, input_feat: torch.Tensor) -> StepOutput:
-        key = (tuple(input_label.shape), tuple(input_feat.shape))
+    def step(self, input_label: torch.Tensor, input_feat: torch.Tensor,
+             row_weight: Optional[torch.Tensor] = None) -> StepOutput:
+        if row_weight is not None:
+            from .probit import _check_row_weight
+            row_weight = _check_row_weight(row_weight, input_label.shape[0], self.device)
+        key = (tuple(input_label.shape), tuple(input_feat.shape), row_weight is not None)
         entry = self.graphs.get(key)
         if entry is None:
-            entry = self.graphs[key] = self._capture(input_label, input_feat)   # warm-up ran on a snapshot: no update yet
+            entry = self.graphs[key] = self._capture(input_label, input_feat, row_weight)   # warm-up on a snapshot
         entry["y"].copy_(input_label)
         entry["x"].copy_(input_feat)
+        if row_weight is not None:
+            entry["w"].copy_(row_weight)
         entry["graph"].replay()
         if self.stepper.scheduler is not None:
             self.stepper.scheduler.step()
