@@ -310,6 +310,23 @@ int mpvae_probit_forward_weighted(const mpvae_probit_params *p, const uint8_t *l
 int mpvae_probit_backward_weighted(const mpvae_probit_params *p, const uint8_t *label_mask, const float *row_weight,
                                    void *cuda_stream);
 
+/* Label-weighted rows: the ELBO with a weight per label and label value inside each row's log-likelihood.
+ * label_weight (2 * L) fp32 on the device, laid out [w0 (L) | w1 (L)]: w0_l weighs label l's y == 0 cells, w1_l its
+ * y == 1 cells.  label_mask and row_weight as above; any of the three may be NULL (label_weight == NULL =
+ * mpvae_probit_forward_weighted / _backward_weighted).  Per cell of both branches
+ *   ll = w1_l log E (y = 1),  w0_l log(1 - E) (y = 0),  w1_l y log E + w0_l (1 - y) log(1 - E) (a soft label)
+ * and t_b = -log mean_s exp(sum over observed l of ll_{s,b,l}); the softmax sample weights, the row weights and the batch
+ * means are otherwise unchanged.  The ranking losses, KL, indiv_prob and indiv_prob_label do not depend on the label
+ * weights.  Weights of 1 give the bits of label_weight == NULL on every output and gradient.  A zero weight drops the
+ * cell's term (0, not 0 * ll) and its log-likelihood gradient is exactly 0.  Other values are used as given (negatives
+ * included) and are not checked.  max |w| enters the bound that scales the fp16 operands of the g_R product.  Under
+ * MPVAE_FLAG_FUSED_FORWARD a label-weighted forward runs the separate row kernel.  The backward must receive the
+ * forward's weights and mask.  Same workspace size as the unweighted calls. */
+int mpvae_probit_forward_label_weighted(const mpvae_probit_params *p, const uint8_t *label_mask, const float *row_weight,
+                                        const float *label_weight, void *cuda_stream);
+int mpvae_probit_backward_label_weighted(const mpvae_probit_params *p, const uint8_t *label_mask, const float *row_weight,
+                                         const float *label_weight, void *cuda_stream);
+
 /* Counter-based standard-normal noise, replaces torch.normal(0,1,(S,B,Z)) of mpvae.py:162.
  * Element (s, b_global, z) depends only on (seed, offset, s, b_global, z): a rank holding rows
  * [row0, row0+B) of a B_global-row batch draws the same numbers a single GPU would. */

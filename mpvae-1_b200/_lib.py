@@ -35,6 +35,7 @@ EXPORTS = (
     "mpvae_predictive_scale", "mpvae_predictive_rho", "mpvae_predict_exact", "mpvae_predict_pairs",
     "mpvae_probit_predict_conditional", "mpvae_probit_forward_masked", "mpvae_probit_backward_masked",
     "mpvae_probit_forward_weighted", "mpvae_probit_backward_weighted",
+    "mpvae_probit_forward_label_weighted", "mpvae_probit_backward_label_weighted",
     "mpvae_ghk_workspace_bytes", "mpvae_probit_predict_conditional_ghk",
     "mpvae_probit_sample_labels", "mpvae_f1_sets_workspace_bytes", "mpvae_f1_sets",
     "mpvae_mode_workspace_bytes", "mpvae_probit_score_sets", "mpvae_probit_predict_mode",
@@ -125,6 +126,9 @@ def _load():
     for fn in (lib.mpvae_probit_forward_weighted, lib.mpvae_probit_backward_weighted):
         fn.restype = C.c_int
         fn.argtypes = [C.POINTER(ProbitParams), C.c_void_p, C.c_void_p, C.c_void_p]
+    for fn in (lib.mpvae_probit_forward_label_weighted, lib.mpvae_probit_backward_label_weighted):
+        fn.restype = C.c_int
+        fn.argtypes = [C.POINTER(ProbitParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.mpvae_philox_normal.restype = C.c_int
     lib.mpvae_philox_normal.argtypes = [C.c_void_p] + [C.c_int32] * 5 + [C.c_uint64, C.c_uint64, C.c_void_p]
     lib.mpvae_contract_workspace_bytes.restype = C.c_uint64

@@ -82,7 +82,7 @@ struct Workspace {
     size_t total;
 };
 // 32-bit slots of the first 256 bytes of the `slots` block; the per-tile counters of the fused forward follow
-enum { SLOT_COUNTER = 0, SLOT_ABSMAX_R = 1, SLOT_ABSMAX_GXS = 2, SLOT_ABSMAX_GP = 3 /* and 4 */ };
+enum { SLOT_COUNTER = 0, SLOT_ABSMAX_R = 1, SLOT_ABSMAX_GXS = 2, SLOT_ABSMAX_GP = 3 /* and 4 */, SLOT_ABSMAX_LW = 5 };
 
 // row pitch (floats) of the (S*B, L) scratch matrices nr and gxs: 16-byte aligned rows for vector loads / stores
 int row_pitch(int L) { return (L + 3) & ~3; }
@@ -468,6 +468,11 @@ int mpvae_probit_forward_masked(const mpvae_probit_params* p_in, const uint8_t* 
 
 int mpvae_probit_forward_weighted(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
                                   void* cuda_stream) {
+    return mpvae_probit_forward_label_weighted(p_in, label_mask, row_weight, nullptr, cuda_stream);
+}
+
+int mpvae_probit_forward_label_weighted(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
+                                        const float* label_weight, void* cuda_stream) {
     mpvae_probit_params tmp;
     const mpvae_probit_params* p = normalize(p_in, &tmp);
     if (!p) return 1;
@@ -485,6 +490,7 @@ int mpvae_probit_forward_weighted(const mpvae_probit_params* p_in, const uint8_t
     RowArgs a = row_args(p, w);
     a.mask = label_mask;
     a.row_weight = row_weight;   // read by row_tail only: the fused forward's finalize kernel takes it as well
+    a.label_weight = label_weight;
     // a scratch block sized for the backward means a training call: the forward keeps E for it (same placement in
     // both layouts: the backward-only buffers follow everything the forward shares)
     const Workspace wb = carve(p->S, p->B, p->L, p->Z, true, p->flags);
@@ -493,8 +499,9 @@ int mpvae_probit_forward_weighted(const mpvae_probit_params* p_in, const uint8_t
         a.E_x = reinterpret_cast<float*>(base + wb.e_x);
     }
     if (use_tensor(p->flags, p->S, p->B, p->L, p->Z)) {
-        // the fused row forward has no mask: a masked call takes the separate row kernel (tested equal to it unmasked)
-        const bool fused = use_fused_forward(p->flags, p->S, p->B, p->L, p->Z) && !label_mask;
+        // the fused row forward has no mask and no label weights: such a call takes the separate row kernel (tested equal
+        // to it without them)
+        const bool fused = use_fused_forward(p->flags, p->S, p->B, p->L, p->Z) && !label_mask && !label_weight;
         FuseFwd fz{};
         if (fused) {
             fz.S = p->S; fz.B = p->B; fz.L = p->L; fz.ldn = row_pitch(p->L);
@@ -693,6 +700,11 @@ int mpvae_probit_backward_masked(const mpvae_probit_params* p_in, const uint8_t*
 
 int mpvae_probit_backward_weighted(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
                                    void* cuda_stream) {
+    return mpvae_probit_backward_label_weighted(p_in, label_mask, row_weight, nullptr, cuda_stream);
+}
+
+int mpvae_probit_backward_label_weighted(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
+                                         const float* label_weight, void* cuda_stream) {
     mpvae_probit_params tmp;
     const mpvae_probit_params* p = normalize(p_in, &tmp);
     if (!p) return 1;
@@ -705,18 +717,20 @@ int mpvae_probit_backward_weighted(const mpvae_probit_params* p_in, const uint8_
     RowArgs a = row_args(p, w);
     a.mask = label_mask;
     a.row_weight = row_weight;   // scales the per-row coefficients, and with them the gxs bound of the fp16 planes
+    a.label_weight = label_weight;
     a.E_l = reinterpret_cast<float*>(base + w.e_l);
     a.E_x = reinterpret_cast<float*>(base + w.e_x);
     const int M = p->S * p->B;
     if (p->g_r && tensor) {
-        // slots 2..4: scale source of the gxs planes, max |g_indiv_prob|, max |g_indiv_prob_label|
-        if (cudaMemsetAsync(slots + SLOT_ABSMAX_GXS, 0, 3 * sizeof(uint32_t), stream) != cudaSuccess) { set_error("cudaMemsetAsync failed"); return 2; }
+        // slots 2..5: scale source of the gxs planes, max |g_indiv_prob|, max |g_indiv_prob_label|, max |label weight|
+        if (cudaMemsetAsync(slots + SLOT_ABSMAX_GXS, 0, 4 * sizeof(uint32_t), stream) != cudaSuccess) { set_error("cudaMemsetAsync failed"); return 2; }
         // the plane scale comes from an upper bound of |gxs| computed from the saved row statistics, so the row
         // kernel can write the operand planes itself
         ProfScope ps(MPVAE_PROF_GXS_BOUND, stream);
         if (p->g_indiv_prob) { if (int rc = tc_absmax(p->g_indiv_prob, (size_t)p->B * p->L, slots + SLOT_ABSMAX_GP, stream)) return rc; }
         if (p->g_indiv_prob_label) { if (int rc = tc_absmax(p->g_indiv_prob_label, (size_t)p->B * p->L, slots + SLOT_ABSMAX_GP + 1, stream)) return rc; }
-        if (int rc = launch_gxs_bound(a, slots + SLOT_ABSMAX_GP, slots + SLOT_ABSMAX_GXS, stream)) return rc;
+        if (label_weight) { if (int rc = tc_absmax(label_weight, (size_t)2 * p->L, slots + SLOT_ABSMAX_LW, stream)) return rc; }
+        if (int rc = launch_gxs_bound(a, slots + SLOT_ABSMAX_GP, slots + SLOT_ABSMAX_GXS, slots + SLOT_ABSMAX_LW, stream)) return rc;
         a.gxs_planes = reinterpret_cast<__half*>(base + w.gxs_planes);
         a.gxs_pitch = tc_pitch(p->L);
         a.gxs_plane_elems = (size_t)M * a.gxs_pitch;

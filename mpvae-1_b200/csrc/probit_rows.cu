@@ -35,10 +35,10 @@ constexpr int kST = 2;   // samples per inner tile (unrolled)
 struct BlockCounts { int npos, nneg; };
 
 // One lane's inputs for one 32-label chunk and kST samples.  obs: the label is observed (always, unmasked); an
-// unobserved label's y reads as 0.
-struct RowChunk { float y, fe, fx, nr[kST]; bool obs; };
+// unobserved label's y reads as 0.  w0 / w1: the label's weights (LW only).
+struct RowChunk { float y, fe, fx, nr[kST], w0, w1; bool obs; };
 
-template <bool MASKED>
+template <bool MASKED, bool LW>
 __device__ __forceinline__ void load_chunk(RowChunk& in, const RowArgs& a, const float* __restrict__ yrow,
                                            const float* __restrict__ ferow, const float* __restrict__ fxrow, int c, int lane,
                                            int b, int s0) {
@@ -46,6 +46,7 @@ __device__ __forceinline__ void load_chunk(RowChunk& in, const RowArgs& a, const
     if (l < a.L) {
         in.obs = !MASKED || a.mask[(size_t)b * a.L + l] != 0;
         in.y = in.obs ? yrow[l] : 0.0f; in.fe = ferow[l]; in.fx = fxrow[l];
+        if (LW) { in.w0 = a.label_weight[l]; in.w1 = a.label_weight[a.L + l]; }
 #pragma unroll
         for (int i = 0; i < kST; ++i)
             in.nr[i] = (s0 + i < a.S) ? a.nr[row_of(a, s0 + i, b) * a.ldn + l] : 0.0f;
@@ -206,8 +207,9 @@ static_assert(offsetof(FusePart, lp_x) == offsetof(FusePart, lp_l) + 8 && offset
 
 // MASKED: an unobserved cell (a.mask[b, l] == 0) reads y as 0 and adds nothing to the log-likelihood or the ranking sums;
 // its E still enters the predictions and the saved E_l / E_x.  The mask bytes are byte loads (b * L need not be a
-// multiple of 4).
-template <bool STABLE, int MINB, bool MASKED>
+// multiple of 4).  LW: each lane loads its four labels' weights once per chunk, and cell_forward weighs the cell
+// log-likelihoods before they enter the sums.
+template <bool STABLE, int MINB, bool MASKED, bool LW>
 __global__ void __launch_bounds__(kThreads, MINB)
 probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nchunks) {
     const int b = blockIdx.x;
@@ -217,12 +219,16 @@ probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nc
     const float fS = (float)S;
     for (int c = blockIdx.y * kWarps + warp; c < nchunks; c += gridDim.y * kWarps) {
         const int l0 = c * kChunk + kLL * lane;
-        float y[kLL], fe[kLL], fx[kLL], accl[kLL], accx[kLL];
+        float y[kLL], fe[kLL], fx[kLL], accl[kLL], accx[kLL], w0[kLL], w1[kLL];
         bool obs[kLL];
 #pragma unroll
         for (int j = 0; j < kLL; ++j) {
             y[j] = fe[j] = fx[j] = accl[j] = accx[j] = 0.f;
             if (l0 + j < L) { y[j] = a.y[yoff + l0 + j]; fe[j] = a.fe_out[yoff + l0 + j]; fx[j] = a.fx_out[yoff + l0 + j]; }
+            if (LW) {
+                w0[j] = w1[j] = 0.f;
+                if (l0 + j < L) { w0[j] = a.label_weight[l0 + j]; w1[j] = a.label_weight[L + l0 + j]; }
+            }
             if (MASKED) {
                 obs[j] = l0 + j < L && a.mask[yoff + l0 + j] != 0;
                 if (!obs[j]) y[j] = 0.f;
@@ -259,8 +265,8 @@ probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nc
                 for (int j = 0; j < kLL; ++j) {
                     el[j] = ex[j] = 0.f;
                     if (l0 + j < L) {
-                        const CellFwd cl = cell_forward<STABLE>(nv[j] + fe[j], y[j]);   // mpvae.py:168,177
-                        const CellFwd cx = cell_forward<STABLE>(nv[j] + fx[j], y[j]);   // mpvae.py:170,180
+                        const CellFwd cl = cell_forward<STABLE, LW>(nv[j] + fe[j], y[j], LW ? w0[j] : 1.f, LW ? w1[j] : 1.f);   // mpvae.py:168,177
+                        const CellFwd cx = cell_forward<STABLE, LW>(nv[j] + fx[j], y[j], LW ? w0[j] : 1.f, LW ? w1[j] : 1.f);   // mpvae.py:170,180
                         if (!MASKED || obs[j]) {
                             lp[2 * i] += (double)cl.ll; lp[2 * i + 1] += (double)cx.ll;
                             pn[4 * i] += cl.epos; pn[4 * i + 1] += cl.eneg; pn[4 * i + 2] += cx.epos; pn[4 * i + 3] += cx.eneg;
@@ -344,9 +350,12 @@ __device__ __forceinline__ RowCoeffs row_coeffs(const RowArgs& a, int b) {
 // positive and no observed negative (e.g. nothing observed) puts no ranking term on any cell, so its ranking part of the
 // bound is 0 -- not the 0/0 NaN of its normaliser, which would leave the whole batch's planes unscaled although the
 // row's gradients are finite.
-template <bool MASKED>
+// LW: every cell's log-likelihood coefficient is cn * w0_l or cn * w1_l, so the log-likelihood part scales by
+// W = max_l max(|w0_l|, |w1_l|), which the caller left as fp32 bits in *lw_absmax (tc_absmax over the 2L weights).
+template <bool MASKED, bool LW>
 __global__ void __launch_bounds__(256)
-gxs_bound_kernel(const RowArgs a, const unsigned int* __restrict__ gp_absmax, unsigned int* __restrict__ out_bits) {
+gxs_bound_kernel(const RowArgs a, const unsigned int* __restrict__ gp_absmax, unsigned int* __restrict__ out_bits,
+                 const unsigned int* __restrict__ lw_absmax) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     unsigned int bits = 0u;
     if (i < a.B * a.S) {
@@ -357,8 +366,13 @@ gxs_bound_kernel(const RowArgs a, const unsigned int* __restrict__ gp_absmax, un
         const float gp = gp_absmax ? (__uint_as_float(gp_absmax[0]) + __uint_as_float(gp_absmax[1])) / (float)a.S : 0.0f;
         float kl = fabsf(rc.kb[0]), kx = fabsf(rc.kb[1]);
         if (MASKED && a.rowaux[(size_t)b * 2] == 0.0f && a.rowaux[(size_t)b * 2 + 1] == 0.0f) kl = kx = 0.0f;
-        const float bl = 5.0f * fabsf(rc.cnb[0] * w.x) + 17.0f * 5.0f * kl * fmaxf(st.x, st.y);
-        const float bx = 5.0f * fabsf(rc.cnb[1] * w.y) + 17.0f * 5.0f * kx * fmaxf(st.z, st.w);
+        float nl = fabsf(rc.cnb[0] * w.x), nx = fabsf(rc.cnb[1] * w.y);
+        if (LW) {
+            const float W = __uint_as_float(*lw_absmax);
+            nl *= W; nx *= W;
+        }
+        const float bl = 5.0f * nl + 17.0f * 5.0f * kl * fmaxf(st.x, st.y);
+        const float bx = 5.0f * nx + 17.0f * 5.0f * kx * fmaxf(st.z, st.w);
         bits = __float_as_uint(bl + bx + 0.4f * gp) & 0x7FFFFFFFu;   // NaN (degenerate row) sorts highest
     }
 #pragma unroll
@@ -370,8 +384,9 @@ gxs_bound_kernel(const RowArgs a, const unsigned int* __restrict__ gp_absmax, un
 }
 
 // MASKED: an unobserved cell gets the cotangent of indiv_prob / indiv_prob_label alone (its y reads as 0 and its
-// log-likelihood and ranking coefficients as 0)
-template <bool STABLE, bool MASKED>
+// log-likelihood and ranking coefficients as 0).  LW: cell_backward weighs each observed cell's log-likelihood
+// coefficient by its label's weight.
+template <bool STABLE, bool MASKED, bool LW>
 __global__ void __launch_bounds__(kThreads, 4)
 probit_row_bwd_kernel(const RowArgs a) {
     extern __shared__ float s_gacc[];   // [nws][2][L] logit-gradient partial sums
@@ -415,9 +430,9 @@ probit_row_bwd_kernel(const RowArgs a) {
         float* __restrict__ gacc = s_gacc + (size_t)ws * 2 * L;
         RowChunk cur, nxt;
         int c = wl;
-        if (c < nchunks) load_chunk<MASKED>(cur, a, yrow, ferow, fxrow, c, lane, b, s0);
+        if (c < nchunks) load_chunk<MASKED, LW>(cur, a, yrow, ferow, fxrow, c, lane, b, s0);
         for (; c < nchunks; c += nwl) {
-            if (c + nwl < nchunks) load_chunk<MASKED>(nxt, a, yrow, ferow, fxrow, c + nwl, lane, b, s0);
+            if (c + nwl < nchunks) load_chunk<MASKED, LW>(nxt, a, yrow, ferow, fxrow, c + nwl, lane, b, s0);
             const int l = (c << 5) + lane;
             if (l < L) {
                 const float gpl = has_gpl ? a.g_indiv_prob_label[(size_t)b * L + l] / fS : 0.0f;
@@ -428,8 +443,10 @@ probit_row_bwd_kernel(const RowArgs a) {
                     if (s0 + i < S) {
                         float dl, dx;
                         if (!MASKED || cur.obs) {
-                            dl = cell_backward<STABLE>(cur.nr[i] + cur.fe, cur.y, cn[i][0], cp[i][0], cq[i][0], gpl);
-                            dx = cell_backward<STABLE>(cur.nr[i] + cur.fx, cur.y, cn[i][1], cp[i][1], cq[i][1], gpx);
+                            dl = cell_backward<STABLE, LW>(cur.nr[i] + cur.fe, cur.y, cn[i][0], cp[i][0], cq[i][0], gpl,
+                                                           LW ? cur.w0 : 1.f, LW ? cur.w1 : 1.f);
+                            dx = cell_backward<STABLE, LW>(cur.nr[i] + cur.fx, cur.y, cn[i][1], cp[i][1], cq[i][1], gpx,
+                                                           LW ? cur.w0 : 1.f, LW ? cur.w1 : 1.f);
                         } else {
                             dl = cell_backward<STABLE>(cur.nr[i] + cur.fe, 0.0f, 0.0f, 0.0f, 0.0f, gpl);
                             dx = cell_backward<STABLE>(cur.nr[i] + cur.fx, 0.0f, 0.0f, 0.0f, 0.0f, gpx);
@@ -497,7 +514,8 @@ probit_row_bwd_kernel(const RowArgs a) {
 // samples with the logit-gradient sums in registers: no shared-memory accumulators, 8-byte loads, 4-byte plane stores.
 // Grid (B, G): the 64-label chunks of a row are dealt out to G CTAs so that small batches still fill the GPU.
 // MASKED: an unobserved cell gets the cotangent of indiv_prob / indiv_prob_label alone (y, cn, cp, cq read as 0).
-template <bool MASKED>
+// LW: a lane loads its two labels' weights once per chunk; cell_backward_saved weighs the log-likelihood coefficient.
+template <bool MASKED, bool LW>
 __global__ void __launch_bounds__(kThreads, 4)
 probit_row_bwd_saved_kernel(const RowArgs a) {
     extern __shared__ float s_coef[];   // [S][6]: cn_l, cn_x, cp_l, cp_x, cq_l, cq_x
@@ -533,6 +551,11 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
         if (in1) { if (ob1) y1 = a.y[yoff + l0 + 1]; fe1 = a.fe_out[yoff + l0 + 1]; fx1 = a.fx_out[yoff + l0 + 1]; }
         if (has_gpl) { if (in0) gpl0 = a.g_indiv_prob_label[yoff + l0] / fS; if (in1) gpl1 = a.g_indiv_prob_label[yoff + l0 + 1] / fS; }
         if (has_gp) { if (in0) gpx0 = a.g_indiv_prob[yoff + l0] / fS; if (in1) gpx1 = a.g_indiv_prob[yoff + l0 + 1] / fS; }
+        float w00 = 1.f, w01 = 1.f, w10 = 1.f, w11 = 1.f;   // w<y><label>
+        if (LW) {
+            if (in0) { w00 = a.label_weight[l0]; w10 = a.label_weight[L + l0]; }
+            if (in1) { w01 = a.label_weight[l0 + 1]; w11 = a.label_weight[L + l0 + 1]; }
+        }
         float gl0 = 0.f, gl1 = 0.f, gx0 = 0.f, gx1 = 0.f;
         // rows are 16-byte aligned (ldn % 4 == 0) and l0 is even: 8-byte loads; columns [L, ldn) of the cubes are pitch
         // padding that is never read as a label (in0 / in1)
@@ -564,17 +587,17 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
                 const Cell3& v = cur[i];
                 float d0 = 0.f, d1 = 0.f;
                 if (in0) {
-                    const float dl = cell_backward_saved(v.n.x + fe0, v.l.x, y0, ob0 ? cf[0] : 0.0f, ob0 ? cf[2] : 0.0f,
-                                                         ob0 ? cf[4] : 0.0f, gpl0);
-                    const float dx = cell_backward_saved(v.n.x + fx0, v.x.x, y0, ob0 ? cf[1] : 0.0f, ob0 ? cf[3] : 0.0f,
-                                                         ob0 ? cf[5] : 0.0f, gpx0);
+                    const float dl = cell_backward_saved<LW>(v.n.x + fe0, v.l.x, y0, ob0 ? cf[0] : 0.0f, ob0 ? cf[2] : 0.0f,
+                                                             ob0 ? cf[4] : 0.0f, gpl0, w00, w10);
+                    const float dx = cell_backward_saved<LW>(v.n.x + fx0, v.x.x, y0, ob0 ? cf[1] : 0.0f, ob0 ? cf[3] : 0.0f,
+                                                             ob0 ? cf[5] : 0.0f, gpx0, w00, w10);
                     gl0 += dl; gx0 += dx; d0 = dl + dx;
                 }
                 if (in1) {
-                    const float dl = cell_backward_saved(v.n.y + fe1, v.l.y, y1, ob1 ? cf[0] : 0.0f, ob1 ? cf[2] : 0.0f,
-                                                         ob1 ? cf[4] : 0.0f, gpl1);
-                    const float dx = cell_backward_saved(v.n.y + fx1, v.x.y, y1, ob1 ? cf[1] : 0.0f, ob1 ? cf[3] : 0.0f,
-                                                         ob1 ? cf[5] : 0.0f, gpx1);
+                    const float dl = cell_backward_saved<LW>(v.n.y + fe1, v.l.y, y1, ob1 ? cf[0] : 0.0f, ob1 ? cf[2] : 0.0f,
+                                                             ob1 ? cf[4] : 0.0f, gpl1, w01, w11);
+                    const float dx = cell_backward_saved<LW>(v.n.y + fx1, v.x.y, y1, ob1 ? cf[1] : 0.0f, ob1 ? cf[3] : 0.0f,
+                                                             ob1 ? cf[5] : 0.0f, gpx1, w01, w11);
                     gl1 += dl; gx1 += dx; d1 = dl + dx;
                 }
                 if (a.gxs_planes) {
@@ -629,8 +652,8 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
 // The backward is one CTA per row as well (cell_backward_saved from the kept E and nr, logit gradients, KL gradients)
 // and leaves the row's contribution to g_R = gxs^T . noise in a scratch slab; a second, tiny kernel adds the slabs over
 // the batch in row order (deterministic).  R staging, the noise draw and the contraction are small_rows.cuh's.
-// MASKED: unobserved cells as in probit_row_fwd_tiled_kernel.
-template <bool STABLE, bool MASKED>
+// MASKED, LW: unobserved cells and label weights as in probit_row_fwd_tiled_kernel.
+template <bool STABLE, bool MASKED, bool LW>
 __global__ void __launch_bounds__(kSmallThreads)
 probit_small_fwd_kernel(const SmallArgs p) {
     extern __shared__ __align__(16) unsigned char s_raw[];
@@ -646,13 +669,17 @@ probit_small_fwd_kernel(const SmallArgs p) {
     const bool bulk = small_r_stage<kSmallThreads>(Rs, p.r, L, Z, &s_bar);
     // this lane's labels (L <= 128: at most four 32-label chunks)
     const int nch = (L + 31) >> 5;
-    float yv[4], fev[4], fxv[4];
+    float yv[4], fev[4], fxv[4], w0v[4], w1v[4];
     bool ov[4];
 #pragma unroll
     for (int c = 0; c < 4; ++c) {
         const int l = (c << 5) + lane;
         yv[c] = fev[c] = fxv[c] = 0.f;
         if (c < nch && l < L) { yv[c] = a.y[(size_t)b * L + l]; fev[c] = a.fe_out[(size_t)b * L + l]; fxv[c] = a.fx_out[(size_t)b * L + l]; }
+        if (LW) {
+            w0v[c] = w1v[c] = 0.f;
+            if (c < nch && l < L) { w0v[c] = a.label_weight[l]; w1v[c] = a.label_weight[L + l]; }
+        }
         if (MASKED) {
             ov[c] = c < nch && l < L && a.mask[(size_t)b * L + l] != 0;
             if (!ov[c]) yv[c] = 0.f;
@@ -685,8 +712,8 @@ probit_small_fwd_kernel(const SmallArgs p) {
             for (int i = 0; i < 2; ++i) {
                 if (s0 + i >= S) continue;
                 const float nr = i == 0 ? acc0 : acc1;
-                const CellFwd cl = cell_forward<STABLE>(nr + fev[c], yv[c]);   // mpvae.py:168,177
-                const CellFwd cx = cell_forward<STABLE>(nr + fxv[c], yv[c]);   // mpvae.py:170,180
+                const CellFwd cl = cell_forward<STABLE, LW>(nr + fev[c], yv[c], LW ? w0v[c] : 1.f, LW ? w1v[c] : 1.f);   // mpvae.py:168,177
+                const CellFwd cx = cell_forward<STABLE, LW>(nr + fxv[c], yv[c], LW ? w0v[c] : 1.f, LW ? w1v[c] : 1.f);   // mpvae.py:170,180
                 if (!MASKED || ov[c]) {
                     lpl[i] += (double)cl.ll; lpx[i] += (double)cx.ll;
                     pn[i][0] += cl.epos; pn[i][1] += cl.eneg; pn[i][2] += cx.epos; pn[i][3] += cx.eneg;
@@ -726,8 +753,8 @@ probit_small_fwd_kernel(const SmallArgs p) {
     row_tail<kSmallThreads, MASKED>(a, b);
 }
 
-// MASKED: unobserved cells as in probit_row_bwd_saved_kernel.
-template <bool MASKED>
+// MASKED, LW: unobserved cells and label weights as in probit_row_bwd_saved_kernel.
+template <bool MASKED, bool LW>
 __global__ void __launch_bounds__(kThreads)
 probit_small_bwd_kernel(const SmallArgs p) {
     extern __shared__ __align__(16) unsigned char s_raw[];
@@ -765,6 +792,7 @@ probit_small_bwd_kernel(const SmallArgs p) {
             const float y = ob ? a.y[(size_t)b * L + l] : 0.f, fe = a.fe_out[(size_t)b * L + l], fx = a.fx_out[(size_t)b * L + l];
             const float gpl = a.g_indiv_prob_label ? a.g_indiv_prob_label[(size_t)b * L + l] / fS : 0.f;
             const float gpx = a.g_indiv_prob ? a.g_indiv_prob[(size_t)b * L + l] / fS : 0.f;
+            const float w0 = LW ? a.label_weight[l] : 1.f, w1 = LW ? a.label_weight[L + l] : 1.f;
             float gl = 0.f, gx = 0.f;
             for (int i = 0; i < 2; ++i) {
                 const int s = (pair << 1) + i;
@@ -774,8 +802,8 @@ probit_small_bwd_kernel(const SmallArgs p) {
                 const float* cf = coef + s * 6;
                 float dl, dx;
                 if (ob) {
-                    dl = cell_backward_saved(nr + fe, a.E_l[o], y, cf[0], cf[2], cf[4], gpl);
-                    dx = cell_backward_saved(nr + fx, a.E_x[o], y, cf[1], cf[3], cf[5], gpx);
+                    dl = cell_backward_saved<LW>(nr + fe, a.E_l[o], y, cf[0], cf[2], cf[4], gpl, w0, w1);
+                    dx = cell_backward_saved<LW>(nr + fx, a.E_x[o], y, cf[1], cf[3], cf[5], gpx, w0, w1);
                 } else {
                     dl = cell_backward_saved(nr + fe, a.E_l[o], 0.f, 0.f, 0.f, 0.f, gpl);
                     dx = cell_backward_saved(nr + fx, a.E_x[o], 0.f, 0.f, 0.f, 0.f, gpx);
@@ -858,6 +886,18 @@ __global__ void warp_sum_probe_kernel(const T* __restrict__ in, T* __restrict__ 
     }
 }
 
+// f(std::true_type / std::false_type): a run-time choice as a kernel's template flag (decltype(flag)::value)
+template <typename F>
+void with_flag(bool v, F&& f) {
+    if (v) f(std::true_type{});
+    else f(std::false_type{});
+}
+template <typename F>
+void for_both(F&& f) {
+    f(std::false_type{});
+    f(std::true_type{});
+}
+
 int pick_nwl(int L) {
     const int nchunks = (L + 31) / 32;
     int nwl = 1;
@@ -896,30 +936,41 @@ int launch_small_forward(RowArgs a, const SmallNoise& n, cudaStream_t stream) {
     static bool configured[kMaxDevices] = {};
     const int dev = device_slot();
     if (!configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(probit_small_fwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_fwd_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_fwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_fwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_small_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
+        cudaError_t e = cudaSuccess;
+        auto allow = [&](const void* k) {
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
+        };
+        for_both([&](auto m) {
+            for_both([&](auto lw) {
+                constexpr bool M = decltype(m)::value, LW = decltype(lw)::value;
+                allow((const void*)probit_small_fwd_kernel<false, M, LW>);
+                allow((const void*)probit_small_fwd_kernel<true, M, LW>);
+                allow((const void*)probit_small_bwd_kernel<M, LW>);
+            });
+        });
         if (e != cudaSuccess) { set_error("cudaFuncSetAttribute(small): %s", cudaGetErrorString(e)); return 4; }
         configured[dev] = true;
     }
     const SmallArgs p = small_args(a, n);
-    if (a.mask) {
-        if (a.stable) probit_small_fwd_kernel<true, true><<<a.B, kSmallThreads, smem, stream>>>(p);
-        else probit_small_fwd_kernel<false, true><<<a.B, kSmallThreads, smem, stream>>>(p);
-    } else {
-        if (a.stable) probit_small_fwd_kernel<true, false><<<a.B, kSmallThreads, smem, stream>>>(p);
-        else probit_small_fwd_kernel<false, false><<<a.B, kSmallThreads, smem, stream>>>(p);
-    }
+    with_flag(a.stable, [&](auto st) {
+        with_flag(a.mask != nullptr, [&](auto m) {
+            with_flag(a.label_weight != nullptr, [&](auto lw) {
+                probit_small_fwd_kernel<decltype(st)::value, decltype(m)::value, decltype(lw)::value>
+                    <<<a.B, kSmallThreads, smem, stream>>>(p);
+            });
+        });
+    });
     return check_launch("probit_small_fwd_kernel");
 }
 
 int launch_small_backward(RowArgs a, const SmallNoise& n, float* g_r, cudaStream_t stream) {
     const SmallArgs p = small_args(a, n);
-    if (a.mask) probit_small_bwd_kernel<true><<<a.B, kThreads, small_bwd_smem(a.S, a.L, n.Z), stream>>>(p);
-    else probit_small_bwd_kernel<false><<<a.B, kThreads, small_bwd_smem(a.S, a.L, n.Z), stream>>>(p);
+    with_flag(a.mask != nullptr, [&](auto m) {
+        with_flag(a.label_weight != nullptr, [&](auto lw) {
+            probit_small_bwd_kernel<decltype(m)::value, decltype(lw)::value>
+                <<<a.B, kThreads, small_bwd_smem(a.S, a.L, n.Z), stream>>>(p);
+        });
+    });
     if (int rc = check_launch("probit_small_bwd_kernel")) return rc;
     if (g_r == nullptr) return 0;
     const int cnt = a.L * n.Z;
@@ -964,13 +1015,14 @@ int launch_row_forward(RowArgs a, cudaStream_t stream) {
     // two CTAs of 256 threads per SM (<= 128 registers: sixteen cells in flight per lane, no spills); measured equal
     // to or faster than three (80 registers, spills) and four (64) on B200
     const dim3 grid(a.B, gy);
-    if (a.mask) {
-        if (a.stable) probit_row_fwd_tiled_kernel<true, 2, true><<<grid, kThreads, 0, stream>>>(a, part, nchunks);
-        else probit_row_fwd_tiled_kernel<false, 2, true><<<grid, kThreads, 0, stream>>>(a, part, nchunks);
-    } else {
-        if (a.stable) probit_row_fwd_tiled_kernel<true, 2, false><<<grid, kThreads, 0, stream>>>(a, part, nchunks);
-        else probit_row_fwd_tiled_kernel<false, 2, false><<<grid, kThreads, 0, stream>>>(a, part, nchunks);
-    }
+    with_flag(a.stable, [&](auto st) {
+        with_flag(a.mask != nullptr, [&](auto m) {
+            with_flag(a.label_weight != nullptr, [&](auto lw) {
+                probit_row_fwd_tiled_kernel<decltype(st)::value, 2, decltype(m)::value, decltype(lw)::value>
+                    <<<grid, kThreads, 0, stream>>>(a, part, nchunks);
+            });
+        });
+    });
     if (int rc = check_launch("probit_row_fwd_tiled_kernel")) return rc;
     a.part_tiles = nchunks;
     return launch_row_finalize(a, stream);
@@ -983,9 +1035,14 @@ int launch_row_finalize(RowArgs a, cudaStream_t stream) {
     return check_launch("probit_row_finalize_kernel");
 }
 
-int launch_gxs_bound(RowArgs a, const unsigned int* gp_absmax, unsigned int* out_bits, cudaStream_t stream) {
-    if (a.mask) gxs_bound_kernel<true><<<ceil_div(a.B * a.S, 256), 256, 0, stream>>>(a, gp_absmax, out_bits);
-    else gxs_bound_kernel<false><<<ceil_div(a.B * a.S, 256), 256, 0, stream>>>(a, gp_absmax, out_bits);
+int launch_gxs_bound(RowArgs a, const unsigned int* gp_absmax, unsigned int* out_bits, const unsigned int* lw_absmax,
+                     cudaStream_t stream) {
+    with_flag(a.mask != nullptr, [&](auto m) {
+        with_flag(a.label_weight != nullptr, [&](auto lw) {
+            gxs_bound_kernel<decltype(m)::value, decltype(lw)::value>
+                <<<ceil_div(a.B * a.S, 256), 256, 0, stream>>>(a, gp_absmax, out_bits, lw_absmax);
+        });
+    });
     return check_launch("gxs_bound_kernel");
 }
 
@@ -998,8 +1055,11 @@ int launch_row_backward(RowArgs a, cudaStream_t stream) {
         int gy = ceil_div(2 * 4 * kNumSMs, a.B);
         if (gy > ceil_div(nchunks, kWarps)) gy = ceil_div(nchunks, kWarps);
         if (gy < 1) gy = 1;
-        if (a.mask) probit_row_bwd_saved_kernel<true><<<dim3(a.B, gy), kThreads, smem, stream>>>(a);
-        else probit_row_bwd_saved_kernel<false><<<dim3(a.B, gy), kThreads, smem, stream>>>(a);
+        with_flag(a.mask != nullptr, [&](auto m) {
+            with_flag(a.label_weight != nullptr, [&](auto lw) {
+                probit_row_bwd_saved_kernel<decltype(m)::value, decltype(lw)::value><<<dim3(a.B, gy), kThreads, smem, stream>>>(a);
+            });
+        });
         return check_launch("probit_row_bwd_saved_kernel");
     }
     a.nwl = pick_nwl(a.L);
@@ -1008,20 +1068,25 @@ int launch_row_backward(RowArgs a, cudaStream_t stream) {
     static bool configured[kMaxDevices] = {};
     const int dev = device_slot();
     if (smem > 48 * 1024 && !configured[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(probit_row_bwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_row_bwd_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_row_bwd_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(probit_row_bwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+        cudaError_t e = cudaSuccess;
+        for_both([&](auto st) {
+            for_both([&](auto m) {
+                for_both([&](auto lw) {
+                    const void* k = (const void*)probit_row_bwd_kernel<decltype(st)::value, decltype(m)::value, decltype(lw)::value>;
+                    if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+                });
+            });
+        });
         if (e != cudaSuccess) { set_error("cudaFuncSetAttribute(bwd): %s", cudaGetErrorString(e)); return 4; }
         configured[dev] = true;
     }
-    if (a.mask) {
-        if (a.stable) probit_row_bwd_kernel<true, true><<<a.B, kThreads, smem, stream>>>(a);
-        else probit_row_bwd_kernel<false, true><<<a.B, kThreads, smem, stream>>>(a);
-    } else {
-        if (a.stable) probit_row_bwd_kernel<true, false><<<a.B, kThreads, smem, stream>>>(a);
-        else probit_row_bwd_kernel<false, false><<<a.B, kThreads, smem, stream>>>(a);
-    }
+    with_flag(a.stable, [&](auto st) {
+        with_flag(a.mask != nullptr, [&](auto m) {
+            with_flag(a.label_weight != nullptr, [&](auto lw) {
+                probit_row_bwd_kernel<decltype(st)::value, decltype(m)::value, decltype(lw)::value><<<a.B, kThreads, smem, stream>>>(a);
+            });
+        });
+    });
     return check_launch("probit_row_bwd_kernel");
 }
 

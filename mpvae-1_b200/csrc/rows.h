@@ -60,6 +60,11 @@ struct RowArgs {
     // CTA's batch sums of row_tail (sum_b w_b t_b, a zero-weight row skipped) and row_coeffs (a_nll, a_c, a_kl scaled
     // by w_b; all zero when w_b == 0).  No kernel is instantiated for it: the code branches on the pointer.
     const float* row_weight;
+    // label-weighted rows: (2, L) fp32, [w0 (L) | w1 (L)] -- the weight of a label's y == 0 cells, then of its y == 1
+    // cells; nullptr = every label weighs 1.  The launchers pick the kernels' LW instantiation from it: a cell's
+    // log-likelihood is multiplied by its weight (a zero weight drops it) before the log-mean-exp, and in the backward
+    // its log-likelihood coefficient likewise.  The ranking terms, KL and predictions do not read it.
+    const float* label_weight;
 };
 
 size_t row_smem_bytes(int L);
@@ -94,8 +99,10 @@ int launch_row_finalize(RowArgs a, cudaStream_t stream);
 int launch_row_backward(RowArgs a, cudaStream_t stream);
 // *out_bits = fp32 bits of an upper bound of max |gxs| over the whole batch (NaN for non-sanitised degenerate rows),
 // from the saved per-(row, sample) statistics and the upstream cotangents; gp_absmax: two slots holding max |g_indiv_prob|
-// and max |g_indiv_prob_label| as fp32 bits (zero when absent)
-int launch_gxs_bound(RowArgs a, const unsigned int* gp_absmax, unsigned int* out_bits, cudaStream_t stream);
+// and max |g_indiv_prob_label| as fp32 bits (zero when absent); lw_absmax (read when a.label_weight is set): max |w| over
+// the 2L label weights as fp32 bits
+int launch_gxs_bound(RowArgs a, const unsigned int* gp_absmax, unsigned int* out_bits, const unsigned int* lw_absmax,
+                     cudaStream_t stream);
 
 // Prediction only (predict.cu): a.indiv_prob = mean_s E(nr + fx_out), the feature branch alone -- no labels, no
 // log-likelihoods, no ranking factors, no per-row tail.  Same E and the same sample order as the forward kernels.

@@ -78,7 +78,8 @@ def _score_rows(model, feats: torch.Tensor, args, batch_size: Optional[int], gat
 
 @torch.no_grad()
 def predict_proba(model, feats: torch.Tensor, labels: Optional[torch.Tensor], args, batch_size: Optional[int] = None,
-                  loss_fn=None, gather: bool = True, group=None, predict_fn=None, label_mask=None, row_weight=None):
+                  loss_fn=None, gather: bool = True, group=None, predict_fn=None, label_mask=None, row_weight=None,
+                  pos_weight=None, neg_weight=None):
     """Returns (indiv_prob (N, L), summed-loss dict).  `feats` / `labels` are device tensors for ALL N rows.
 
     `labels=None` scores rows that have no labels: each batch runs only the feature branch (`model.feat_forward`) and
@@ -88,7 +89,8 @@ def predict_proba(model, feats: torch.Tensor, labels: Optional[torch.Tensor], ar
     same bits.  `label_mask` (N, L), with labels: the mask of observed labels (`compute_loss`); the summed losses are
     then those of the observed labels, and the predictions do not change.  `row_weight` (N,), with labels: the row
     weights (`compute_loss`); the summed losses are then the weighted sums sum_n w_n t_n (importance-weighted
-    validation), and the predictions do not change."""
+    validation), and the predictions do not change.  `pos_weight` / `neg_weight` (L,), with labels: the label weights
+    (`compute_loss`); the summed losses are then the label-weighted ones, and the predictions do not change."""
     if labels is None and predict_fn is None:
         from .mpvae import predict as predict_fn
     if labels is not None and loss_fn is None:
@@ -105,6 +107,10 @@ def predict_proba(model, feats: torch.Tensor, labels: Optional[torch.Tensor], ar
         kw = {} if label_mask is None else {"label_mask": label_mask[a:b]}
         if row_weight is not None:
             kw["row_weight"] = row_weight[a:b]
+        if pos_weight is not None:
+            kw["pos_weight"] = pos_weight
+        if neg_weight is not None:
+            kw["neg_weight"] = neg_weight
         out = loss_fn(y, label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar, model.r_sqrt_sigma, args, **kw)
         if b > a:           # the empty slice of a rank without rows has NaN losses, means over nothing
             sums["total_loss"] = sums["total_loss"] + out[0] * (b - a)               # test.py:67-70

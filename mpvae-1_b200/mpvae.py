@@ -28,7 +28,7 @@ from . import _lib
 from .dense import linear
 from .probit import ProbitELBO, label_pairs, philox_normal, predictive_rho, predictive_scale, probit_predict
 from .probit import contract_nt, ghk_workspace_bytes, predict_exact_from_r, probit_predict_conditional
-from .probit import _check_observed, _check_row_weight, probit_predict_conditional_ghk
+from .probit import _check_label_weight, _check_observed, _check_row_weight, probit_predict_conditional_ghk
 from .probit import check_set_args, f1_sets, probit_sample_labels
 from .probit import check_max_flips, check_set_bits, probit_predict_mode, probit_score_sets
 from .probit import predict_pairs as probit_predict_pairs
@@ -155,7 +155,7 @@ def draw_noise(args, n_sample, n_batch, device, noise=None):
 
 
 def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r_sqrt_sigma, args, noise=None,
-                 label_mask=None, row_weight=None):
+                 label_mask=None, row_weight=None, pos_weight=None, neg_weight=None):
     """Reference signature (mpvae.py:145) -> (total_loss, nll_loss, nll_loss_x, c_loss, c_loss_x, kl_loss,
     indiv_prob, indiv_prob_label) (mpvae.py:210).
 
@@ -186,10 +186,26 @@ def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar
         its logit gradient is the cotangent of the predictions alone;
       - other values are used as given (negatives included; NaN propagates); they are not checked on the host.
     The weights are converted to contiguous fp32 and receive no gradient: a weight that requires grad is refused, as are
-    a wrong shape, device or a non-floating dtype, before any noise offset is consumed."""
+    a wrong shape, device or a non-floating dtype, before any noise offset is consumed.
+
+    `pos_weight`, `neg_weight` (L,) floating tensors on the batch's device, or None (all ones): label weights inside each
+    row's log-likelihood, e.g. pos_weight = n_neg / n_pos (clamped) so that rare labels are predicted, or propensity or
+    inverse-frequency weights.  Per cell of both branches the log-likelihood becomes pos_weight[l] * log E (y = 1),
+    neg_weight[l] * log(1 - E) (y = 0), or pos_weight[l] * y * log E + neg_weight[l] * (1 - y) * log(1 - E) for a soft
+    label, before the log-mean-exp over samples: t_b = -log mean_s exp(sum over the observed l of the weighted ll).  So
+    the weights also shift which samples dominate a row.  They can be combined with label_mask and row_weight (the row
+    weight multiplies the row term formed from the label-weighted likelihood):
+      - weights of 1 give the bits of pos_weight=neg_weight=None on all 8 outputs and every gradient;
+      - the ranking losses (c_loss, c_loss_x, normalised per row by n_pos * n_neg already), kl_loss, indiv_prob and
+        indiv_prob_label do not depend on them;
+      - a zero weight drops the cell's term (it is not multiplied by 0) and its log-likelihood gradient is exactly 0;
+      - other values are used as given (negatives included); they are not checked on the host.
+    The weights receive no gradient: a weight that requires grad is refused, as are a wrong shape, device or a
+    non-floating dtype, before any noise offset is consumed."""
     device = input_label.device
     if row_weight is not None:
         row_weight = _check_row_weight(row_weight, fe_out.shape[0], device)
+    label_weight = _check_label_weight(pos_weight, neg_weight, fe_out.shape[1], device)
     if device.type != "cuda":
         raise RuntimeError("mpvae_b200.compute_loss needs CUDA tensors: the probit ELBO is implemented as sm_100a "
                            "kernels only (no CPU fallback)")
@@ -206,7 +222,7 @@ def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar
     # args.peer_ring (peer.PeerRing, data-parallel runs): g_R comes back already summed over the ranks
     return ProbitELBO.apply(input_label.float(), fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise,
                             float(args.nll_coeff), float(args.c_coeff), flags, spec, getattr(args, "peer_ring", None),
-                            label_mask, row_weight)
+                            label_mask, row_weight, label_weight)
 
 
 def predict(fx_out, r_sqrt_sigma, args, noise=None):

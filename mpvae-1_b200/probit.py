@@ -90,6 +90,28 @@ def _check_row_weight(row_weight, B, device):
     return row_weight.to(torch.float32).contiguous()
 
 
+def _check_label_weight(pos_weight, neg_weight, L, device):
+    """The (L,) weights of the y == 1 and y == 0 cells packed as one contiguous (2, L) fp32 tensor [neg_weight;
+    pos_weight] (None for either = all ones), or None when both are None.  Refused before any launch, like row_weight,
+    when a weight is not a floating tensor of that shape on the batch's device or requires grad.  The values are not
+    checked (that would synchronise with the host)."""
+    if pos_weight is None and neg_weight is None:
+        return None
+    for name, w in (("neg_weight", neg_weight), ("pos_weight", pos_weight)):
+        if w is None:
+            continue
+        if not isinstance(w, torch.Tensor) or not w.is_floating_point():
+            raise TypeError(f"{name} must be a floating tensor, got {getattr(w, 'dtype', type(w))}")
+        if w.requires_grad:
+            raise ValueError(f"{name} requires grad, but the loss returns no gradient for it: pass {name}.detach()")
+        if w.shape != (L,):
+            raise ValueError(f"{name} has shape {tuple(w.shape)}, expected {(L,)} (label_dim,)")
+        if w.device != device:
+            raise ValueError(f"{name} is on {w.device}, expected {device}")
+    return torch.stack([torch.ones(L, dtype=torch.float32, device=device) if w is None else w.to(torch.float32)
+                        for w in (neg_weight, pos_weight)]).contiguous()
+
+
 def _check_observed(observed, shape, device):
     """Refuses an `observed` argument that is not an int8 tensor of `shape` (batch, label_dim) on `device`."""
     if not isinstance(observed, torch.Tensor) or observed.dtype != torch.int8:
@@ -137,11 +159,15 @@ class ProbitELBO(torch.autograd.Function):
     read where the mask is 0.  None runs the unmasked entry points.
 
     `row_weight` (B,) floating on the batch's device, or None: the weight of each row's loss terms
-    (mpvae_probit_forward_weighted, semantics in mpvae.compute_loss).  It receives no gradient."""
+    (mpvae_probit_forward_weighted, semantics in mpvae.compute_loss).  It receives no gradient.
+
+    `label_weight` (2, L) fp32 on the batch's device (`_check_label_weight`: row 0 weighs the y == 0 cells, row 1 the
+    y == 1 cells), or None: the label weights of the cell log-likelihoods (mpvae_probit_forward_label_weighted,
+    semantics in mpvae.compute_loss).  It receives no gradient."""
 
     @staticmethod
     def forward(ctx, y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise, nll_coeff, c_coeff, flags,
-                noise_spec=None, peer=None, label_mask=None, row_weight=None):
+                noise_spec=None, peer=None, label_mask=None, row_weight=None, label_weight=None):
         lib = _lib.lib()
         y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32 = (
             t.contiguous() for t in (y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32))
@@ -155,6 +181,12 @@ class ProbitELBO(torch.autograd.Function):
             label_mask = _check_label_mask(label_mask, B, L, dev)
         if row_weight is not None:
             row_weight = _check_row_weight(row_weight, B, dev)
+        if label_weight is not None and (not isinstance(label_weight, torch.Tensor) or label_weight.shape != (2, L) or
+                                         label_weight.dtype != torch.float32 or label_weight.device != dev or
+                                         label_weight.requires_grad):
+            raise ValueError(f"label_weight must be a (2, {L}) fp32 tensor on {dev} without grad (_check_label_weight)")
+        if label_weight is not None:
+            label_weight = label_weight.contiguous()
         want_bwd = any(ctx.needs_input_grad)
         with torch.cuda.device(dev):
             ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 1 if want_bwd else 0, flags))
@@ -177,7 +209,11 @@ class ProbitELBO(torch.autograd.Function):
             p.indiv_prob, p.indiv_prob_label = _ptr(prob), _ptr(prob_label)
             p.workspace, p.workspace_bytes = _ptr(ws), ws_bytes
             stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            if row_weight is not None:
+            if label_weight is not None:
+                _lib.check(lib.mpvae_probit_forward_label_weighted(C.byref(p), _ptr(label_mask), _ptr(row_weight),
+                                                                   _ptr(label_weight), stream),
+                           "mpvae_probit_forward_label_weighted")
+            elif row_weight is not None:
                 _lib.check(lib.mpvae_probit_forward_weighted(C.byref(p), _ptr(label_mask), _ptr(row_weight), stream),
                            "mpvae_probit_forward_weighted")
             elif label_mask is None:
@@ -192,10 +228,12 @@ class ProbitELBO(torch.autograd.Function):
             ctx.peer = peer if (peer is not None and peer.applies(S, B, L, Z, flags)) else None
             ctx.has_mask = label_mask is not None
             ctx.has_weight = row_weight is not None
+            ctx.has_label_weight = label_weight is not None
             ctx.save_for_backward(y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, ws,
                                   *([noise] if noise is not None else []),
                                   *([label_mask] if label_mask is not None else []),
-                                  *([row_weight] if row_weight is not None else []))
+                                  *([row_weight] if row_weight is not None else []),
+                                  *([label_weight] if label_weight is not None else []))
             ctx.dims = (S, B, L, Z, D)
             ctx.coeffs = (float(nll_coeff), float(c_coeff), int(flags))
             ctx.set_materialize_grads(False)
@@ -209,6 +247,7 @@ class ProbitELBO(torch.autograd.Function):
         noise = rest.pop(0) if ctx.has_noise else None
         label_mask = rest.pop(0) if ctx.has_mask else None
         row_weight = rest.pop(0) if ctx.has_weight else None
+        label_weight = rest.pop(0) if ctx.has_label_weight else None
         S, B, L, Z, D = ctx.dims
         nll_coeff, c_coeff, flags = ctx.coeffs
         dev = y.device
@@ -251,7 +290,11 @@ class ProbitELBO(torch.autograd.Function):
             p.g_r = _ptr(g_r)
             p.workspace, p.workspace_bytes = _ptr(ws), ws.numel()
             stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            if row_weight is not None:
+            if label_weight is not None:
+                _lib.check(lib.mpvae_probit_backward_label_weighted(C.byref(p), _ptr(label_mask), _ptr(row_weight),
+                                                                    _ptr(label_weight), stream),
+                           "mpvae_probit_backward_label_weighted")
+            elif row_weight is not None:
                 _lib.check(lib.mpvae_probit_backward_weighted(C.byref(p), _ptr(label_mask), _ptr(row_weight), stream),
                            "mpvae_probit_backward_weighted")
             elif label_mask is None:
@@ -261,7 +304,7 @@ class ProbitELBO(torch.autograd.Function):
                            "mpvae_probit_backward_masked")
         #       y     fe_out    fe_mu      fe_logvar  fx_out    fx_mu      fx_logvar  r32  noise nll_c c_c flags spec
         return (None, g_fe_out, g_mulv[0], g_mulv[1], g_fx_out, g_mulv[2], g_mulv[3], g_r, None, None, None, None, None,
-                None, None, None)   # peer, label_mask, row_weight
+                None, None, None, None)   # peer, label_mask, row_weight, label_weight
 
 
 def _predict_dims(name, fx_out, r32, S, noise, noise_spec):

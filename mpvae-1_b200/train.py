@@ -208,7 +208,8 @@ class DataParallelStep:
     # -- the step -------------------------------------------------------------------------------------------
     def step(self, input_label: torch.Tensor, input_feat: torch.Tensor, noise: Optional[torch.Tensor] = None,
              r_override: Optional[torch.Tensor] = None, label_mask: Optional[torch.Tensor] = None,
-             row_weight: Optional[torch.Tensor] = None) -> StepOutput:
+             row_weight: Optional[torch.Tensor] = None, pos_weight: Optional[torch.Tensor] = None,
+             neg_weight: Optional[torch.Tensor] = None) -> StepOutput:
         """`input_label` (B, L) and `input_feat` (B, F) are the GLOBAL batch (train.py:106-111); every rank slices
         its rows.  `noise`, if given, is the global (S, B, Z) tensor (validation mode).  `r_override` is the
         fresh non-trainable R of residue_sigma == 'random' (train.py:120-122).  `label_mask`, if given, is the global
@@ -216,7 +217,8 @@ class DataParallelStep:
         `label_mask=`; without it the loss is called exactly as before, so custom loss functions keep working.
         `row_weight`, if given, is the global (B,) row weight (`compute_loss`), sliced and passed as `row_weight=` in the
         same way.  Each rank's terms are sum_b w_b t_b / (its rows) and the shard weighting below makes the global loss
-        sum over all rows of w_b t_b / B, as in one process."""
+        sum over all rows of w_b t_b / B, as in one process.  `pos_weight` / `neg_weight`, if given, are the (L,) label
+        weights (`compute_loss`): they weigh labels, not rows, so every rank passes them whole, again only when given."""
         args = self.args
         n_rows = input_label.shape[0]
         lo, hi = shard_rows(n_rows, self.rank, self.world)
@@ -244,6 +246,10 @@ class DataParallelStep:
                 kw["label_mask"] = label_mask[lo:hi]
             if row_weight is not None:
                 kw["row_weight"] = row_weight[lo:hi]
+            if pos_weight is not None:
+                kw["pos_weight"] = pos_weight
+            if neg_weight is not None:
+                kw["neg_weight"] = neg_weight
             out = self.loss_fn(y, label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar, r, args, **kw)
             total = out[0]
             if self.regulariser is not None:
@@ -301,11 +307,12 @@ class DataParallelStep:
 
 
 def train_one_epoch(step: DataParallelStep, feats, labels, batch_size: int, order=None, skip_empty: bool = True,
-                    masks=None, weights=None):
+                    masks=None, weights=None, pos_weight=None, neg_weight=None):
     """Epoch driver with the reference's batching (train.py:98-111): int(N/bs)+1 steps, ragged (possibly empty)
     last batch.  `feats` / `labels` are device tensors (kept resident: SURVEY 8f-N4); returns per-step outputs.
     `masks`, if given, is the (N, L) mask of observed labels (`compute_loss`), sliced by the same index as `labels`;
-    `weights`, if given, the (N,) row weights (`compute_loss(..., row_weight=)`), sliced the same way.
+    `weights`, if given, the (N,) row weights (`compute_loss(..., row_weight=)`), sliced the same way;
+    `pos_weight` / `neg_weight`, if given, the (L,) label weights (`compute_loss`), passed to every step as they are.
     `skip_empty=False` reproduces the reference literally when bs | N: it runs the step on the empty batch, whose
     losses are NaN means (train.py:102; compute_loss returns them) and whose NaN gradients then reach Adam."""
     n = feats.shape[0]
@@ -321,6 +328,10 @@ def train_one_epoch(step: DataParallelStep, feats, labels, batch_size: int, orde
             kw["label_mask"] = masks[idx]
         if weights is not None:
             kw["row_weight"] = weights[idx]
+        if pos_weight is not None:
+            kw["pos_weight"] = pos_weight
+        if neg_weight is not None:
+            kw["neg_weight"] = neg_weight
         outs.append(step.step(labels[idx], feats[idx], **kw))
     return outs
 
@@ -338,8 +349,9 @@ class GraphedTrainStep:
         replays and writes the new rate into that tensor;
       * gradients are views into the flat bucket (no per-step allocation).
     Not supported in graph mode: world_size > 1 (see __init__), `skip_nonfinite` (needs a host decision) and Python-side
-    regularisers that branch on data.  Outputs are static tensors that the next replay overwrites.  Row weights
-    (`step(..., row_weight=)`) go into a static buffer as well; a weighted step is a capture of its own."""
+    regularisers that branch on data.  Outputs are static tensors that the next replay overwrites.  A label mask, row
+    weights and label weights (`step(..., label_mask=, row_weight=, pos_weight=, neg_weight=)`) go into static buffers
+    as well; each combination of the ones given is a capture of its own."""
 
     def __init__(self, stepper: DataParallelStep, warmup: int = 3):
         if stepper.skip_nonfinite:
@@ -413,9 +425,9 @@ class GraphedTrainStep:
                         else:
                             v.zero_()                                     # state born during the warm-up: back to "fresh"
 
-    def _capture(self, y, x, w):
+    def _capture(self, y, x, extra):
         static_y, static_x = y.clone(), x.clone()
-        static_w = None if w is None else w.clone()
+        static_extra = {k: v.clone() for k, v in extra.items()}
         st = self.stepper
         if st.world > 1:
             st.pbucket.enable_graph_replay()
@@ -428,37 +440,46 @@ class GraphedTrainStep:
         side.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(side):
             for _ in range(self.warmup):                                  # also initialises optimizer state
-                self._body(static_y, static_x, static_w)
+                self._body(static_y, static_x, static_extra)
         torch.cuda.current_stream(self.device).wait_stream(side)
         graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(graph):
-            out = self._body(static_y, static_x, static_w)
+            out = self._body(static_y, static_x, static_extra)
         self._restore(snap)                                               # parameters, moments, counters, RNG: as before
-        return {"graph": graph, "y": static_y, "x": static_x, "w": static_w, "out": out}
+        return {"graph": graph, "y": static_y, "x": static_x, "extra": static_extra, "out": out}
 
-    def _body(self, y, x, w):
+    def _body(self, y, x, extra):
         st = self.stepper
         sched, st.scheduler = st.scheduler, None                          # the scheduler is stepped on the host
         try:
-            out = st.step(y, x) if w is None else st.step(y, x, row_weight=w)
+            out = st.step(y, x, **extra)
         finally:
             st.scheduler = sched
         self.counter.add_(1)
         return out
 
-    def step(self, input_label: torch.Tensor, input_feat: torch.Tensor,
-             row_weight: Optional[torch.Tensor] = None) -> StepOutput:
+    def step(self, input_label: torch.Tensor, input_feat: torch.Tensor, row_weight: Optional[torch.Tensor] = None,
+             label_mask: Optional[torch.Tensor] = None, pos_weight: Optional[torch.Tensor] = None,
+             neg_weight: Optional[torch.Tensor] = None) -> StepOutput:
+        from .probit import _check_label_mask, _check_label_weight, _check_row_weight
+        B, L = input_label.shape
+        extra = {}
+        if label_mask is not None:
+            extra["label_mask"] = _check_label_mask(label_mask, B, L, self.device)
         if row_weight is not None:
-            from .probit import _check_row_weight
-            row_weight = _check_row_weight(row_weight, input_label.shape[0], self.device)
-        key = (tuple(input_label.shape), tuple(input_feat.shape), row_weight is not None)
+            extra["row_weight"] = _check_row_weight(row_weight, B, self.device)
+        _check_label_weight(pos_weight, neg_weight, L, self.device)
+        for name, w in (("pos_weight", pos_weight), ("neg_weight", neg_weight)):
+            if w is not None:
+                extra[name] = w.to(torch.float32)
+        key = (tuple(input_label.shape), tuple(input_feat.shape), tuple(sorted(extra)))
         entry = self.graphs.get(key)
         if entry is None:
-            entry = self.graphs[key] = self._capture(input_label, input_feat, row_weight)   # warm-up on a snapshot
+            entry = self.graphs[key] = self._capture(input_label, input_feat, extra)   # warm-up on a snapshot
         entry["y"].copy_(input_label)
         entry["x"].copy_(input_feat)
-        if row_weight is not None:
-            entry["w"].copy_(row_weight)
+        for k, v in extra.items():
+            entry["extra"][k].copy_(v)
         entry["graph"].replay()
         if self.stepper.scheduler is not None:
             self.stepper.scheduler.step()
