@@ -36,11 +36,9 @@ extern "C" {
 #define MPVAE_FLAG_STABLE_CDF          0x8u /* opt-in: Phi and 1 - Phi from erfc(|x| / sqrt 2) (no cancellation in the tails)
                                                instead of the reference's 0.5 (1 + erf) and 1 - E.  More accurate than the
                                                reference, hence NOT within 1e-5 of it in saturated cells. */
-#define MPVAE_FLAG_FUSED_FORWARD        0x10u /* dense regime, opt-in: run the row forward on extra "math" warps INSIDE the tcgen05
-                                               product kernel (csrc/fused_rows.cuh) instead of as its own kernel after it.
-                                               Same results bit for bit; measured slower on B200 (the product's register
-                                               accumulators leave room for 8 math warps per SM, a quarter of what the row
-                                               math needs to hide its latencies: profiles/r02_fused_forward.md) */
+#define MPVAE_FLAG_FUSED_FORWARD        0x10u /* accepted and ignored: the result is that of the default path.  It selected a
+                                               row forward inside the tcgen05 product kernel, measured slower on B200 and
+                                               removed (DESIGN.md section 4a) */
 
 #define MPVAE_FLAG_SEPARATE_NOISE       0x20u /* dense regime, library-side noise: draw the Philox normals with a kernel of their own
                                                before the product instead of on the product kernel's math warps, just
@@ -49,9 +47,9 @@ extern "C" {
 #define MPVAE_FLAG_SERIAL_EXCHANGE      0x80u /* data-parallel dense regime: sum g_R over the ranks only AFTER the g_R product (the
                                                stand-alone reduce kernel) instead of slab by slab on a few reserved SMs beside
                                                it (A/B measurements; same sums) */
-#define MPVAE_FLAG_FUSED_EXCHANGE       0x40u /* data-parallel dense regime, opt-in: sum g_R over the ranks tile by tile INSIDE the
-                                               g_R product kernel (peer_tile_done must be given) instead of with the
-                                               stand-alone reduce kernel after it; same sums */
+#define MPVAE_FLAG_FUSED_EXCHANGE       0x40u /* accepted and ignored: the result is that of the default path.  It selected a
+                                               g_R exchange inside the g_R product kernel, measured slower on B200 and
+                                               removed (DESIGN.md section 4a) */
 
 /* order of the six scalar outputs (first six entries of the 8-tuple at mpvae.py:210) */
 enum { MPVAE_TOTAL = 0, MPVAE_NLL = 1, MPVAE_NLL_X = 2, MPVAE_C = 3, MPVAE_C_X = 4, MPVAE_KL = 5 };
@@ -130,9 +128,8 @@ typedef struct mpvae_probit_params {
        replay correctly).  With them the g_R product of the dense regime publishes every finished
        256 x 256 tile there and leaves a few SMs idle; an exchange kernel on those SMs (csrc/peer_reduce.cu, a side
        stream forked from and joined to the caller's) sums finished 256-row slabs of g_R over the ranks through NVLink
-       while the tensor pipe computes later tiles.  MPVAE_FLAG_FUSED_EXCHANGE moves the sums onto the product kernel's
-       own math warps instead (csrc/fused_rows.cuh; slower), MPVAE_FLAG_SERIAL_EXCHANGE or NULL = the stand-alone
-       reduce kernel after the product.  Products of fewer than 8192 rows (S * B) always take the latter. */
+       while the tensor pipe computes later tiles.  MPVAE_FLAG_SERIAL_EXCHANGE or NULL = the stand-alone reduce kernel
+       after the product.  Products of fewer than 8192 rows (S * B) always take the latter. */
     void *peer_tile_done[8];
 } mpvae_probit_params;
 #define MPVAE_PEER_TILE_BYTES 65536u
@@ -188,10 +185,9 @@ int mpvae_probit_predict(const mpvae_probit_params *p, void *cuda_stream);
  *   log_evidence[b]   = log(fse / S) + m, the Monte Carlo estimate of log P(y_O | x)
  *   ess[b]            = se^2 / sum_s (double) u_s^2, the effective sample size of the weights, in [1, S]
  * With nothing observed indiv_prob is mpvae_probit_predict's bit for bit (log_evidence = 0, ess = S); with every label
- * observed -log_evidence is the row's nll_loss_x of mpvae_probit_forward on the same fx_out, R and noise (except under
- * MPVAE_FLAG_FUSED_FORWARD there).  Reads what mpvae_probit_predict reads plus observed; writes indiv_prob, log_evidence
- * (B) and ess (B), all required.  STABLE_CDF, CONTRACT_FMA, CONTRACT_TENSOR and SEPARATE_NOISE apply as for
- * mpvae_probit_predict; the other flags are ignored.  Same workspace size as mpvae_probit_predict.  Many observed labels
+ * observed -log_evidence is the row's nll_loss_x of mpvae_probit_forward on the same fx_out, R and noise.  Reads what
+ * mpvae_probit_predict reads plus observed; writes indiv_prob, log_evidence (B) and ess (B), all required.  STABLE_CDF,
+ * CONTRACT_FMA, CONTRACT_TENSOR and SEPARATE_NOISE apply as for mpvae_probit_predict; the other flags are ignored.  Same workspace size as mpvae_probit_predict.  Many observed labels
  * make the weights degenerate (ess -> 1): the estimate is then carried by few samples. */
 int mpvae_probit_predict_conditional(const mpvae_probit_params *p, const int8_t *observed, float *log_evidence,
                                      float *ess, void *cuda_stream);
@@ -286,9 +282,9 @@ int mpvae_probit_backward(const mpvae_probit_params *p, void *cuda_stream);
  * observed labels lack a positive or a negative adds 0 to the forward; its OBSERVED cells get NaN in the backward as an
  * unmasked degenerate row does (zero ranking gradient under MPVAE_FLAG_SANITIZE_DEGENERATE), never its unobserved cells.
  * A mask of all ones gives the unmasked results bit for bit; label_mask == NULL is the unmasked entry point.  The backward
- * must receive the forward's mask.  Under MPVAE_FLAG_FUSED_FORWARD a masked forward runs the separate row kernel.  Same
- * workspace size as the unmasked calls.  With y = the labels and the same mask, observed = where(mask, y, -1) gives
- * mpvae_probit_predict_conditional's encoding: -log_evidence of a one-row batch is then nll_loss_x. */
+ * must receive the forward's mask.  Same workspace size as the unmasked calls.  With y = the labels and the same mask,
+ * observed = where(mask, y, -1) gives mpvae_probit_predict_conditional's encoding: -log_evidence of a one-row batch is
+ * then nll_loss_x. */
 int mpvae_probit_forward_masked(const mpvae_probit_params *p, const uint8_t *label_mask, void *cuda_stream);
 int mpvae_probit_backward_masked(const mpvae_probit_params *p, const uint8_t *label_mask, void *cuda_stream);
 
@@ -319,9 +315,8 @@ int mpvae_probit_backward_weighted(const mpvae_probit_params *p, const uint8_t *
  * means are otherwise unchanged.  The ranking losses, KL, indiv_prob and indiv_prob_label do not depend on the label
  * weights.  Weights of 1 give the bits of label_weight == NULL on every output and gradient.  A zero weight drops the
  * cell's term (0, not 0 * ll) and its log-likelihood gradient is exactly 0.  Other values are used as given (negatives
- * included) and are not checked.  max |w| enters the bound that scales the fp16 operands of the g_R product.  Under
- * MPVAE_FLAG_FUSED_FORWARD a label-weighted forward runs the separate row kernel.  The backward must receive the
- * forward's weights and mask.  Same workspace size as the unweighted calls. */
+ * included) and are not checked.  max |w| enters the bound that scales the fp16 operands of the g_R product.  The
+ * backward must receive the forward's weights and mask.  Same workspace size as the unweighted calls. */
 int mpvae_probit_forward_label_weighted(const mpvae_probit_params *p, const uint8_t *label_mask, const float *row_weight,
                                         const float *label_weight, void *cuda_stream);
 int mpvae_probit_backward_label_weighted(const mpvae_probit_params *p, const uint8_t *label_mask, const float *row_weight,

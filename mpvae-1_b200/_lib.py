@@ -17,9 +17,9 @@ FLAG_SANITIZE_DEGENERATE = 0x1
 FLAG_CONTRACT_TENSOR = 0x2
 FLAG_CONTRACT_FMA = 0x4
 FLAG_STABLE_CDF = 0x8
-FLAG_FUSED_FORWARD = 0x10
+FLAG_FUSED_FORWARD = 0x10        # accepted and ignored (the removed in-product row forward)
 FLAG_SEPARATE_NOISE = 0x20
-FLAG_FUSED_EXCHANGE = 0x40
+FLAG_FUSED_EXCHANGE = 0x40       # accepted and ignored (the removed in-product g_R exchange)
 FLAG_SERIAL_EXCHANGE = 0x80
 PEER_TILE_BYTES = 65536
 

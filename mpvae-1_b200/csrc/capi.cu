@@ -10,9 +10,9 @@
 
 #include "../../include/mpvae_b200.h"
 #include "common.cuh"
-#include "fused_rows.cuh"
 #include "rows.h"
 #include "tc.h"
+#include "tc_warps.cuh"
 
 namespace mpv {
 
@@ -78,10 +78,10 @@ struct Workspace {
     size_t small_partials;                        // small regime: per-row contributions to g_R
     size_t tn_tail;                               // tensor engine: K-slices of the g_R product's last wave
     size_t slots_bytes;                           // slots + the counters below (zeroed together at the start of a forward)
-    size_t tile_counters, noise_counters;         // byte offsets inside the slots block
+    size_t noise_counters;                        // byte offset inside the slots block
     size_t total;
 };
-// 32-bit slots of the first 256 bytes of the `slots` block; the per-tile counters of the fused forward follow
+// 32-bit slots of the first 256 bytes of the `slots` block; the counters of the just-in-time noise follow
 enum { SLOT_COUNTER = 0, SLOT_ABSMAX_R = 1, SLOT_ABSMAX_GXS = 2, SLOT_ABSMAX_GP = 3 /* and 4 */, SLOT_ABSMAX_LW = 5 };
 
 // row pitch (floats) of the (S*B, L) scratch matrices nr and gxs: 16-byte aligned rows for vector loads / stores
@@ -102,12 +102,6 @@ bool use_small(uint32_t flags, int S, int B, int L, int Z) {
     return !use_tensor(flags, S, B, L, Z) && small_regime_fits(S, B, L, Z);
 }
 
-// the product kernel carries the row forward on its math warps (fused_rows.cuh); a group of S sample-rows may reach
-// back one tile at most
-bool use_fused_forward(uint32_t flags, int S, int B, int L, int Z) {
-    return use_tensor(flags, S, B, L, Z) && (flags & MPVAE_FLAG_FUSED_FORWARD) && S <= kFuseMaxS;
-}
-
 Workspace carve(int S, int B, int L, int Z, bool want_backward, uint32_t flags) {
     Workspace w{};
     size_t off = 0;
@@ -115,16 +109,14 @@ Workspace carve(int S, int B, int L, int Z, bool want_backward, uint32_t flags) 
     const size_t cube = (size_t)S * B * row_pitch(L);
     const bool tensor = use_tensor(flags, S, B, L, Z);
     const int M = S * B;
-    const size_t tiles = (size_t)ceil_div(M, 256) * ceil_div(L, 256);
     w.nr = take(cube * sizeof(float));
     w.lp = take((size_t)B * S * 2 * sizeof(double));
     w.stat = take((size_t)B * S * 4 * sizeof(float));
     w.wts = take((size_t)B * S * 2 * sizeof(float));
     w.rowaux = take((size_t)B * 2 * sizeof(float));
     w.rowout = take((size_t)B * 8 * sizeof(double));
-    // [256 B of slots][per-tile counters of the fused forward][per-128-row-block counters of the just-in-time noise]
-    w.tile_counters = 256;
-    w.noise_counters = w.tile_counters + (tensor ? align_up(tiles * sizeof(uint32_t), 256) : 0);
+    // [256 B of slots][per-128-row-block counters of the just-in-time noise]
+    w.noise_counters = 256;
     w.slots_bytes = w.noise_counters + (tensor ? align_up((size_t)ceil_div(M, 128) * sizeof(uint32_t), 256) : 0);
     w.slots = take(w.slots_bytes);
     // everything the forward writes and the backward reads sits before the backward-only buffers, so a forward
@@ -309,18 +301,17 @@ RowArgs row_args(const mpvae_probit_params* p, const Workspace& w) {
 }
 
 // Dense regime, up to and including the product: the noise operand (unless the product kernel draws it), the R split and
-// nr = noise . R^T on tcgen05.  fz: the fused row forward to run on the product kernel's math warps, or nullptr.  The
-// caller has zeroed the slots block.
-int dense_nt_product(const mpvae_probit_params* p, const Workspace& w, const FuseFwd* fz, cudaStream_t stream) {
+// nr = noise . R^T on tcgen05.  The caller has zeroed the slots block.
+int dense_nt_product(const mpvae_probit_params* p, const Workspace& w, cudaStream_t stream) {
     char* base = static_cast<char*>(p->workspace);
     float* nr = reinterpret_cast<float*>(base + w.nr);
     uint32_t* slots = reinterpret_cast<uint32_t*>(base + w.slots);
     const int M = p->S * p->B;
     void* npl = base + w.noise_planes;
     void* rpl = base + w.r_planes;
-    // library noise: drawn by the product kernel's own math warps just ahead of the tiles (unless those warps carry
-    // the fused row forward, or the caller asks for the separate kernel)
-    const bool jit_noise = !p->noise && !fz && !(p->flags & MPVAE_FLAG_SEPARATE_NOISE);
+    // library noise: drawn by the product kernel's own math warps just ahead of the tiles (unless the caller asks for
+    // the separate kernel)
+    const bool jit_noise = !p->noise && !(p->flags & MPVAE_FLAG_SEPARATE_NOISE);
     int rc = 0;
     if (!jit_noise) {
         ProfScope ps(MPVAE_PROF_NOISE, stream);
@@ -351,7 +342,7 @@ int dense_nt_product(const mpvae_probit_params* p, const Workspace& w, const Fus
     // how many rows the call holds, and a row's predictions must not change with the shard it is computed in.
     // nr's rows are padded to 16 bytes inside the workspace: the product may fill the padding with whole-vector stores.
     return tc_gemm_nt(npl, rpl, nr, M, p->L, p->Z, nullptr, slots + SLOT_ABSMAX_R, stream, row_pitch(p->L), p->noise ? 0 : 1,
-                      nullptr, 0, fz, jit_noise ? &fnz : nullptr, 1);
+                      nullptr, 0, jit_noise ? &fnz : nullptr, 1);
 }
 
 // CUDA-core regime, up to and including the product: the Philox normals (unless the caller gives the noise) and
@@ -399,8 +390,7 @@ int predict_product(const PredictCall& c, cudaStream_t stream) {
     uint32_t* slots = reinterpret_cast<uint32_t*>(static_cast<char*>(p->workspace) + c.w.slots);
     const cudaError_t e = cudaMemsetAsync(slots, 0, c.w.slots_bytes, stream);
     if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
-    // the fused row forward (MPVAE_FLAG_FUSED_FORWARD) is loss work: predictions take the separate row kernels
-    return dense_nt_product(p, c.w, nullptr, stream);
+    return dense_nt_product(p, c.w, stream);
 }
 
 }  // namespace
@@ -442,7 +432,7 @@ int mpvae_profile_read(int32_t slot, double* total_ms, int32_t* count) {
 const char* mpvae_profile_name(int32_t slot) {
     static const char* names[MPVAE_PROF_SLOTS] = {"noise (philox planes / philox normal / split of an external tensor)",
                                                   "R absmax + split",
-                                                  "product nt (noise.R^T; with the fused row forward in the dense regime)",
+                                                  "product nt (noise.R^T)",
                                                   "row forward / finalize",
                                                   "gxs bound",
                                                   "row backward",
@@ -484,12 +474,12 @@ int mpvae_probit_forward_label_weighted(const mpvae_probit_params* p_in, const u
     char* base = static_cast<char*>(p->workspace);
     float* nr = reinterpret_cast<float*>(base + w.nr);
     uint32_t* slots = reinterpret_cast<uint32_t*>(base + w.slots);
-    cudaError_t e = cudaMemsetAsync(slots, 0, w.slots_bytes, stream);   // last-CTA counter, absmax slots, tile counters
+    cudaError_t e = cudaMemsetAsync(slots, 0, w.slots_bytes, stream);   // last-CTA counter, absmax slots, noise counters
     if (e != cudaSuccess) { set_error("cudaMemsetAsync: %s", cudaGetErrorString(e)); return 2; }
     int rc;
     RowArgs a = row_args(p, w);
     a.mask = label_mask;
-    a.row_weight = row_weight;   // read by row_tail only: the fused forward's finalize kernel takes it as well
+    a.row_weight = row_weight;   // read by row_tail only
     a.label_weight = label_weight;
     // a scratch block sized for the backward means a training call: the forward keeps E for it (same placement in
     // both layouts: the backward-only buffers follow everything the forward shares)
@@ -499,27 +489,8 @@ int mpvae_probit_forward_label_weighted(const mpvae_probit_params* p_in, const u
         a.E_x = reinterpret_cast<float*>(base + wb.e_x);
     }
     if (use_tensor(p->flags, p->S, p->B, p->L, p->Z)) {
-        // the fused row forward has no mask and no label weights: such a call takes the separate row kernel (tested equal
-        // to it without them)
-        const bool fused = use_fused_forward(p->flags, p->S, p->B, p->L, p->Z) && !label_mask && !label_weight;
-        FuseFwd fz{};
-        if (fused) {
-            fz.S = p->S; fz.B = p->B; fz.L = p->L; fz.ldn = row_pitch(p->L);
-            fz.stable = a.stable;
-            fz.y = p->y; fz.fe_out = p->fe_out; fz.fx_out = p->fx_out;
-            fz.nr = nr;
-            fz.indiv_prob = p->indiv_prob; fz.indiv_prob_label = p->indiv_prob_label;
-            fz.E_l = a.E_l; fz.E_x = a.E_x;
-            fz.part = reinterpret_cast<FusePart*>(base + w.fuse_part);
-            fz.done = slots + w.tile_counters / sizeof(uint32_t);
-        }
-        if ((rc = dense_nt_product(p, w, fused ? &fz : nullptr, stream))) return rc;
+        if ((rc = dense_nt_product(p, w, stream))) return rc;
         ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
-        if (fused) {
-            a.part = fz.part;
-            a.part_tiles = ceil_div(p->L, 256);
-            return launch_row_finalize(a, stream);
-        }
         return launch_row_forward(a, stream);
     }
     if (use_small(p->flags, p->S, p->B, p->L, p->Z)) {
@@ -781,66 +752,51 @@ int mpvae_probit_backward_label_weighted(const mpvae_probit_params* p_in, const 
         ProfScope ps(MPVAE_PROF_PRODUCT_TN, stream);
         int rc;
         if (tensor) {
-            // data-parallel: the finished tiles are summed over the ranks inside the product kernel (fused_rows.cuh)
+            // data-parallel: the product publishes its finished tiles in per-tile counters (tc_warps.cuh), and the exchange
+            // sums them over the ranks slab by slab on a few reserved SMs beside the product -- unless the product is too
+            // short to hide it (measured) or the caller asks for the exchange after the product
             FusePeer fp{};
             const bool tiles_ok = peer && p->peer_tile_done[p->peer_rank] != nullptr && !(p->peer_mc_part && p->peer_mc_g_r) &&
                                   (size_t)ceil_div(p->L, 256) * ceil_div(p->Z, 256) < kTileEpochWord;
-            // 3: on the product kernel's own math warps (opt-in); 4: slab by slab on a few reserved SMs beside the product
-            // (default); 0: after the product
-            int xmode = 0;
-            if (tiles_ok && (p->flags & MPVAE_FLAG_FUSED_EXCHANGE)) xmode = 3;
-            else if (tiles_ok && !(p->flags & MPVAE_FLAG_SERIAL_EXCHANGE) && ceil_div(p->Z, 256) <= 32 && p->L >= 512 &&
-                     (long long)p->S * p->B >= 8192) xmode = 4;   // shorter products cannot hide the exchange (measured)
-            const bool fused_x = xmode != 0;
+            const bool beside = tiles_ok && !(p->flags & MPVAE_FLAG_SERIAL_EXCHANGE) && ceil_div(p->Z, 256) <= 32 &&
+                                p->L >= 512 && (long long)p->S * p->B >= 8192;
             SideStream* side = nullptr;
-            if (xmode == 4) {
+            PeerCtx sctx = pctx;                                 // the slab exchange: flag value = the tile epoch
+            if (beside) {
+                for (int i = 0; i < pctx.world; ++i)
+                    if (!p->peer_tile_done[i]) { set_error("peer tables: NULL tile counters for rank %d", i); return 1; }
                 side = side_stream();
                 if (!side) return 2;
                 if (cudaEventRecord(side->fork, stream) != cudaSuccess || cudaStreamWaitEvent(side->stream, side->fork, 0) != cudaSuccess) {
                     set_error("peer: fork failed");
                     return 2;
                 }
-            }
-            PeerCtx sctx = pctx;                                 // the slab exchange: flag value = the tile epoch
-            if (fused_x) {
                 uint32_t* epoch_word = static_cast<uint32_t*>(p->peer_tile_done[p->peer_rank]) + kTileEpochWord;
                 sctx.step = 1; sctx.step_dev = epoch_word; sctx.step_stride = 0;
                 pctx.epoch_dev = epoch_word;                     // advanced by the closing flag phase below
-                fp.world = pctx.world; fp.rank = pctx.rank; fp.step = 1; fp.step_dev = epoch_word;
-                fp.timeout_cycles = pctx.timeout_cycles;
-                fp.err = pctx.flags[pctx.rank] + peer_error_word();
-                for (int i = 0; i < pctx.world; ++i) {
-                    fp.part[i] = pctx.part[i]; fp.g_r[i] = pctx.g_r[i];
-                    fp.done[i] = static_cast<unsigned int*>(p->peer_tile_done[i]);
-                    if (!fp.done[i]) { set_error("peer tables: NULL tile counters for rank %d", i); return 1; }
-                }
-                fp.Mc = p->L; fp.Nc = p->Z; fp.ldc = p->Z;
+                fp.world = pctx.world;
+                fp.done = static_cast<unsigned int*>(p->peer_tile_done[p->peer_rank]);
             }
             int exchanged = 0;
             // the noise planes the forward left in the workspace are the MN-major B operand as they are
             rc = tc_gemm_tn(base + w.gxs_planes, base + w.noise_planes, g_r_out, M, p->L, p->Z, slots + SLOT_ABSMAX_GXS, nullptr, stream,
-                            p->noise ? 0 : 1, base + w.tn_tail, tc_tail_scratch_bytes(), 0, fused_x ? &fp : nullptr, &exchanged,
-                            xmode == 4 ? 4 : 3);
+                            p->noise ? 0 : 1, base + w.tn_tail, tc_tail_scratch_bytes(), 0, beside ? &fp : nullptr, &exchanged);
             if (rc) return rc;
-            if (xmode == 4) {
+            if (beside) {
                 // the complete 256-row slabs among the exchanged tiles go over NVLink beside the product, on the SMs it left free
                 // (only slabs of a full 256 rows: a partial last slab goes with the tail rows)
-                const int tiles_n4 = ceil_div(p->Z, 256);
-                int n_slabs = exchanged / tiles_n4;
+                const int tiles_n = ceil_div(p->Z, 256);
+                int n_slabs = exchanged / tiles_n;
                 if (n_slabs > p->L / 256) n_slabs = p->L / 256;
-                exchanged = n_slabs * tiles_n4;
-                if (int rc2 = launch_peer_reduce_slabs(sctx, p->peer_tile_done, tiles_n4, n_slabs, (size_t)256 * p->Z,
+                if (int rc2 = launch_peer_reduce_slabs(sctx, p->peer_tile_done, tiles_n, n_slabs, (size_t)256 * p->Z,
                                                        exchange_sms(p->peer_world), side->stream)) return rc2;
                 if (cudaEventRecord(side->join, side->stream) != cudaSuccess || cudaStreamWaitEvent(stream, side->join, 0) != cudaSuccess) {
                     set_error("peer: join failed");
                     return 2;
                 }
-            }
-            if (fused_x) {
                 // what is left: the rows of the K-sliced tail tiles (complete only now, after the fix-up kernel), and the
                 // two flag phases that tell every rank that all deliveries of this step have landed
-                const int tiles_n = ceil_div(p->Z, 256);
-                const size_t first_row = (size_t)(exchanged / tiles_n) * 256;
+                const size_t first_row = (size_t)n_slabs * 256;
                 const size_t first = first_row < (size_t)p->L ? first_row * p->Z : (size_t)p->L * p->Z;
                 ProfScope px(MPVAE_PROF_EXCHANGE, stream);
                 return launch_peer_reduce(pctx, (size_t)p->L * p->Z - first, stream, first);

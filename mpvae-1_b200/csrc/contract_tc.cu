@@ -19,7 +19,7 @@
 //   warp 0      : TMA producer  -- cp.async.bulk.tensor (128B-swizzled boxes) into a 3- or 4-stage smem ring
 //   warp 1      : MMA issuer    -- one lane of the pair's leader issues tcgen05.mma.cta_group::2 (M256 N256 K16)
 //   warp 2      : TMEM allocator (512 columns = two 128 x 256 fp32 chunk accumulators per CTA, ping-pong)
-//   [FUSE only] warps 4-11: row math of the probit forward on finished tiles (fused_rows.cuh)
+//   [MATH == 2] warps 4-11: the Philox noise of the A operand, drawn just ahead of the tiles (tc_warps.cuh)
 //   last 16     : promotion + epilogue -- tcgen05.ld a chunk (32 rows x 64 columns per warp), add into registers,
 //                 store the finished tile
 // Pipelines: smem full/empty mbarriers (TMA <-> MMA), tmem full/empty mbarriers (MMA <-> promotion).
@@ -32,9 +32,9 @@
 #include <string.h>
 
 #include "common.cuh"
-#include "fused_rows.cuh"
 #include "philox.cuh"
 #include "tc.h"
+#include "tc_warps.cuh"
 
 namespace mpv {
 namespace {
@@ -47,8 +47,8 @@ constexpr int kCtrlWarps = 4;
 constexpr int kEpiWarps = 16;                            // 4 TMEM lane quadrants x 4 column quarters
 constexpr int HB = BN / 2;                               // B-tile columns staged by each CTA of a pair
 
-// MATH 1..3 add eight math warps; MATH 4 only publishes tile completions (no extra warps)
-constexpr bool has_math_warps(int math) { return math >= 1 && math <= 3; }
+// MATH 2 adds eight math warps; MATH 4 only publishes tile completions (no extra warps)
+__host__ __device__ constexpr bool has_math_warps(int math) { return math == 2; }
 constexpr int threads_of(int math) { return 32 * (kCtrlWarps + (has_math_warps(math) ? kFuseMathWarps : 0) + kEpiWarps); }
 
 // One k-block is one 128-byte swizzle row of K (K-major) or one TMA box of k-rows (MN-major); fp16 pieces.
@@ -87,9 +87,8 @@ struct Ring {
     // measured truncation bias per k-block relative to the 3-pass constant: 1.30e-7 / 1.85e-7
     static constexpr float BIAS_SCALE = (EX == 0) ? 1.0f : 0.70f;
 };
-constexpr int kFusePaccBytes = kFuseMathWarps * 2 * 256 * (int)sizeof(float);   // 16 KiB: per math warp [2][256]
 template <int EX>
-constexpr int smem_bytes_of(int math) { return 1024 + Ring<EX>::RING_BYTES + BAR_BYTES + (math == 1 ? kFusePaccBytes : 0); }
+constexpr int smem_bytes_of() { return 1024 + Ring<EX>::RING_BYTES + BAR_BYTES; }
 
 // ------------------------------------------------------------------------------------------------ PTX
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -172,12 +171,12 @@ __device__ __forceinline__ void tc_mma_2sm(uint32_t d_tmem, uint64_t adesc, uint
         ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc)
         : "memory");
 }
-// Register re-partitioning between the warpgroups of a FUSE kernel (a warpgroup = 4 consecutive warps)
+// Register re-partitioning between the warpgroups of a kernel with math warps (a warpgroup = 4 consecutive warps)
 template <int N> __device__ __forceinline__ void reg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(N)); }
 template <int N> __device__ __forceinline__ void reg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
 // 896 threads x 72 registers at launch = 64512, re-dealt as 128 x 40 + 256 x 56 + 512 x 88 = 64512
 constexpr int kRegCtrl = 40, kRegMath = 56, kRegEpi = 88;
-static_assert(128 * kRegCtrl + 32 * kFuseMathWarps * kRegMath + 512 * kRegEpi <= 896 * 72, "register budget of the fused kernel");
+static_assert(128 * kRegCtrl + 32 * kFuseMathWarps * kRegMath + 512 * kRegEpi <= 896 * 72, "register budget of the kernel with math warps");
 
 // One thread's 64 consecutive output columns.  Rows whose start is not 16-byte aligned (odd ldc: g_R, the 512 -> L
 // heads) get LEAD scalar stores up to the next 16-byte boundary, 15 vector stores, and the rest as scalars; every
@@ -223,20 +222,19 @@ struct GemmArgs {
     float* partials;
 };
 
-// MATH: what the eight extra "math" warps of the CTA do (fused_rows.cuh): 0 = there are none, 1 = the probit row
-// forward on finished tiles (opt-in), 2 = draw the Philox noise of the A operand just ahead of the tiles that read it,
-// 3 = sum the finished tiles over the ranks of a data-parallel run through NVLink peer memory, 4 = no math warps, but
-// finished tiles are published in peer memory for the exchange kernel that runs BESIDE this one on a few reserved SMs.
-template <bool MN, int EX, int MATH, bool STABLE>
+// MATH: the roles beyond the pipeline (tc_warps.cuh).  0 = none; 2 = eight extra "math" warps draw the Philox noise of
+// the A operand just ahead of the tiles that read it; 4 = no math warps, but finished tiles are published in peer memory
+// for the exchange kernel that runs BESIDE this one on a few reserved SMs.
+template <bool MN, int EX, int MATH>
 __global__ void __launch_bounds__(threads_of(MATH), 1)
 gemm_split_2sm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmArgs g,
-                      const FuseFwd fz, const FuseNoise fnz, const FusePeer fpz) {
-    constexpr bool FUSE = MATH >= 1 && MATH <= 3;
-    constexpr bool PUBLISH = MATH == 3 || MATH == 4;
+                      const FuseNoise fnz, const FusePeer fpz) {
+    constexpr bool WARPS = has_math_warps(MATH);
+    constexpr bool PUBLISH = MATH == 4;
     using G = Geo<MN>;
     using R2 = Ring<EX>;
     constexpr int STAGES2 = R2::STAGES, STAGE2_BYTES = R2::STAGE_BYTES;
-    constexpr int kFirstEpi = kCtrlWarps + (FUSE ? kFuseMathWarps : 0);
+    constexpr int kFirstEpi = kCtrlWarps + (WARPS ? kFuseMathWarps : 0);
     extern __shared__ uint8_t smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
     const uint32_t base = (raw + 1023u) & ~1023u;             // 128B-swizzled tiles need 1024 B alignment
@@ -267,10 +265,8 @@ gemm_split_2sm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
         return it;
     };
     if (threadIdx.x == 0) {
-        if (PUBLISH) {   // the peer exchange's watermark and the promotion warps' arrival count
-            *reinterpret_cast<volatile int*>(gen + R2::RING_BYTES + 192) = 0;
+        if (PUBLISH)     // the promotion warps' arrival count
             *reinterpret_cast<volatile int*>(gen + R2::RING_BYTES + 196) = 0;
-        }
         for (int s = 0; s < STAGES2; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
         for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), 2 * kEpiWarps); }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -289,7 +285,7 @@ gemm_split_2sm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
     const int num_kb = (g.K + G::BK - 1) / G::BK;
 
     if (warp < kCtrlWarps) {
-        if (FUSE) reg_dec<kRegCtrl>();
+        if (WARPS) reg_dec<kRegCtrl>();
         if (warp == 0 && lane == 0) {   // ------------------------------------------------ TMA producer (every CTA)
             int stage = 0, noise_block = -1;
             uint32_t phase = 0;
@@ -376,19 +372,11 @@ gemm_split_2sm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
                     peer_publish_tile(fpz, reinterpret_cast<volatile int*>(gen + R2::RING_BYTES + 196), n++, it.st);
             }
         }
-    } else if (FUSE && warp < kFirstEpi) {   // ------------------- math warps
+    } else if (WARPS && warp < kFirstEpi) {   // ------------------ math warps: the A operand's Philox noise, ahead of the tiles
         reg_dec<kRegMath>();
-        const int mw = warp - kCtrlWarps;
-        if (MATH == 1) {         // row math of the probit forward on finished tiles
-            float* pacc = reinterpret_cast<float*>(gen + R2::RING_BYTES + BAR_BYTES) + mw * 512;
-            fuse_math_loop<STABLE>(fz, cluster, num_clusters, num_tiles, g.tiles_n, (int)rank * kFuseMathWarps + mw, pacc, lane);
-        } else if (MATH == 2) {  // the A operand's Philox noise, just ahead of the tiles
-            noise_math_loop(fnz, (int)blockIdx.x * kFuseMathWarps + mw, (int)gridDim.x * kFuseMathWarps, lane);
-        } else {                 // this rank's tiles of the sum over the ranks
-            peer_math_loop(fpz, (int)blockIdx.x, (int)gridDim.x, mw, lane, reinterpret_cast<volatile int*>(gen + R2::RING_BYTES + 192));
-        }
+        noise_math_loop(fnz, (int)blockIdx.x * kFuseMathWarps + (warp - kCtrlWarps), (int)gridDim.x * kFuseMathWarps, lane);
     } else {   // --------------------------------------------------- promotion + epilogue (both CTAs, own 128 rows)
-        if (FUSE) reg_inc<kRegEpi>();
+        if (WARPS) reg_inc<kRegEpi>();
         const int q = warp & 3, h = (warp - kFirstEpi) >> 2;      // TMEM lane quadrant = warp id mod 4
         // 1 / (s_a * s_b) as two powers of two (common.cuh): exact for every normal result; extra == 1 unless the two
         // scales together leave the fp32 exponent range
@@ -460,7 +448,6 @@ gemm_split_2sm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
                         if (col0 + j < g.Nc) crow[col0 + j] = acc[j] * inv_scale;
                 }
             }
-            if (MATH == 1) fuse_signal_tile(fz.done, st, lane);   // this warp's part of the tile is in memory
             if (PUBLISH && it.slice == 0 && st < fpz.full_tiles)
                 peer_arrive_tile(reinterpret_cast<volatile int*>(gen + R2::RING_BYTES + 196), lane);
 #pragma unroll
@@ -643,12 +630,12 @@ int current_device() {
     return (d >= 0 && d < kMaxDevices) ? d : 0;
 }
 
-template <bool MN, int EX, int MATH, bool STABLE>
-int launch_gemm_2sm(const CUtensorMap& a, const CUtensorMap& b, GemmArgs g, const FuseFwd& fz, const FuseNoise& fnz,
-                    cudaStream_t stream, size_t partials_bytes, FusePeer fpz = FusePeer{}, int* exchanged_tiles = nullptr) {
-    auto kernel = gemm_split_2sm_kernel<MN, EX, MATH, STABLE>;
+template <bool MN, int EX, int MATH>
+int launch_gemm_2sm(const CUtensorMap& a, const CUtensorMap& b, GemmArgs g, const FuseNoise& fnz, cudaStream_t stream,
+                    size_t partials_bytes, FusePeer fpz = FusePeer{}, int* exchanged_tiles = nullptr) {
+    auto kernel = gemm_split_2sm_kernel<MN, EX, MATH>;
     static int max_clusters[kMaxDevices] = {};     // co-resident clusters (a cluster must fit inside one GPC)
-    constexpr int smem = smem_bytes_of<EX>(MATH);
+    constexpr int smem = smem_bytes_of<EX>();
     cudaLaunchConfig_t cfg = {};
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -676,7 +663,7 @@ int launch_gemm_2sm(const CUtensorMap& a, const CUtensorMap& b, GemmArgs g, cons
     g.full_tiles = tiles;
     g.ksplit = 1;
     static const bool no_split = getenv("MPVAE_TC_NO_KSPLIT") != nullptr;
-    if (MATH != 1 && g.partials != nullptr && !no_split) {
+    if (g.partials != nullptr && !no_split) {
         const int tail = tiles % mc, num_kb = ceil_div(g.K, Geo<MN>::BK);
         if (tail > 0) {
             // f slices per tail tile: the tail then takes ceil(tail * f / mc) / f of a tile time instead of a whole one;
@@ -695,13 +682,12 @@ int launch_gemm_2sm(const CUtensorMap& a, const CUtensorMap& b, GemmArgs g, cons
     const int items = g.full_tiles + (tiles - g.full_tiles) * g.ksplit;
     const int clusters = items < mc ? items : mc;
     cfg.gridDim = dim3(2 * clusters);
-    if (MATH == 3 || MATH == 4) {
+    if (MATH == 4) {
         // the K-sliced tail tiles are complete only after tail_fixup_kernel: they are exchanged after this kernel
         fpz.full_tiles = g.full_tiles;
-        fpz.tiles_n = g.tiles_n;
         if (exchanged_tiles) *exchanged_tiles = g.full_tiles;
     }
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, a, b, g, fz, fnz, fpz);
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, a, b, g, fnz, fpz);
     if (e != cudaSuccess) { set_error("gemm_split_2sm_kernel launch: %s", cudaGetErrorString(e)); return 3; }
     if (int rc = check_launch("gemm_split_2sm_kernel")) return rc;
     if (g.ksplit > 1) {
@@ -717,8 +703,8 @@ int launch_gemm_2sm(const CUtensorMap& a, const CUtensorMap& b, GemmArgs g, cons
 template <bool MN>
 int launch_gemm(const CUtensorMap& a, const CUtensorMap& b, float* C, int Mc, int Nc, int K, int ldc, const uint32_t* ma,
                 const uint32_t* mb, cudaStream_t stream, int ex, float* partials, size_t partials_bytes,
-                const FuseFwd* fuse = nullptr, const FuseNoise* noise = nullptr, const FusePeer* peer = nullptr,
-                int* exchanged_tiles = nullptr, int peer_mode = 3, bool write_pad = false) {
+                const FuseNoise* noise = nullptr, const FusePeer* peer = nullptr, int* exchanged_tiles = nullptr,
+                bool write_pad = false) {
     GemmArgs g{};
     g.C = C; g.Mc = Mc; g.Nc = Nc; g.K = K; g.ldc = ldc;
     g.store_cols = write_pad ? ldc : Nc;
@@ -727,33 +713,19 @@ int launch_gemm(const CUtensorMap& a, const CUtensorMap& b, float* C, int Mc, in
     g.kc = chunk_kblocks(ex == 0 ? Geo<MN>::default_kc : (Geo<MN>::default_kc * 3) / 2);
     g.absmax_a = ma; g.absmax_b = mb;
     g.partials = partials;
-    const FuseFwd none{};
     const FuseNoise nonoise{};
     if (peer != nullptr) {
-        if (!MN || ex == 1 || fuse != nullptr || noise != nullptr) { set_error("fused exchange: tn products only"); return 7; }
-        if (peer_mode == 4) {
-            if (ex == 2) return launch_gemm_2sm<true, 2, 4, false>(a, b, g, none, nonoise, stream, partials_bytes, *peer, exchanged_tiles);
-            return launch_gemm_2sm<true, 0, 4, false>(a, b, g, none, nonoise, stream, partials_bytes, *peer, exchanged_tiles);
-        }
-        if (ex == 2) return launch_gemm_2sm<true, 2, 3, false>(a, b, g, none, nonoise, stream, partials_bytes, *peer, exchanged_tiles);
-        return launch_gemm_2sm<true, 0, 3, false>(a, b, g, none, nonoise, stream, partials_bytes, *peer, exchanged_tiles);
+        if (!MN || ex == 1 || noise != nullptr) { set_error("tile publishing: tn products only"); return 7; }
+        if (ex == 2) return launch_gemm_2sm<true, 2, 4>(a, b, g, nonoise, stream, partials_bytes, *peer, exchanged_tiles);
+        return launch_gemm_2sm<true, 0, 4>(a, b, g, nonoise, stream, partials_bytes, *peer, exchanged_tiles);
     }
     if (noise != nullptr) {
-        if (MN || ex != 1 || fuse != nullptr) { set_error("just-in-time noise: nt products with an exact A operand only"); return 7; }
-        return launch_gemm_2sm<false, 1, 2, false>(a, b, g, none, *noise, stream, 0);
+        if (MN || ex != 1) { set_error("just-in-time noise: nt products with an exact A operand only"); return 7; }
+        return launch_gemm_2sm<false, 1, 2>(a, b, g, *noise, stream, 0);
     }
-    if (fuse != nullptr) {
-        if (MN || ex == 2) { set_error("fused forward: nt products only"); return 7; }
-        if (fuse->stable) {
-            if (ex == 1) return launch_gemm_2sm<false, 1, 1, true>(a, b, g, *fuse, nonoise, stream, 0);
-            return launch_gemm_2sm<false, 0, 1, true>(a, b, g, *fuse, nonoise, stream, 0);
-        }
-        if (ex == 1) return launch_gemm_2sm<false, 1, 1, false>(a, b, g, *fuse, nonoise, stream, 0);
-        return launch_gemm_2sm<false, 0, 1, false>(a, b, g, *fuse, nonoise, stream, 0);
-    }
-    if (ex == 1) return launch_gemm_2sm<MN, 1, 0, false>(a, b, g, none, nonoise, stream, partials_bytes);
-    if (ex == 2) return launch_gemm_2sm<MN, 2, 0, false>(a, b, g, none, nonoise, stream, partials_bytes);
-    return launch_gemm_2sm<MN, 0, 0, false>(a, b, g, none, nonoise, stream, partials_bytes);
+    if (ex == 1) return launch_gemm_2sm<MN, 1, 0>(a, b, g, nonoise, stream, partials_bytes);
+    if (ex == 2) return launch_gemm_2sm<MN, 2, 0>(a, b, g, nonoise, stream, partials_bytes);
+    return launch_gemm_2sm<MN, 0, 0>(a, b, g, nonoise, stream, partials_bytes);
 }
 
 }  // namespace
@@ -910,26 +882,26 @@ size_t tc_tail_scratch_bytes() { return (size_t)(kNumSMs / 2 - 1) * 2 * 256 * BN
 
 int tc_gemm_nt(const void* a_planes, const void* b_planes, float* C, int M, int N, int K, const uint32_t* absmax_a,
                const uint32_t* absmax_b, cudaStream_t stream, int ldc, int a_exact, void* tail_scratch, size_t tail_scratch_bytes,
-               const FuseFwd* fuse, const FuseNoise* noise, int write_pad) {
+               const FuseNoise* noise, int write_pad) {
     if (ldc <= 0) ldc = N;
     const int kp = pitch_of(K);
     CUtensorMap ma, mb;
     if (int rc = make_map(&ma, a_planes, K, M, kp, 64, BM, a_exact ? 1 : 2)) return rc;
     if (int rc = make_map(&mb, b_planes, K, N, kp, 64, HB)) return rc;
     return launch_gemm<false>(ma, mb, C, M, N, K, ldc, absmax_a, absmax_b, stream, a_exact ? 1 : 0, static_cast<float*>(tail_scratch),
-                              tail_scratch_bytes, fuse, noise, nullptr, nullptr, 3, write_pad != 0);
+                              tail_scratch_bytes, noise, nullptr, nullptr, write_pad != 0);
 }
 
 int tc_gemm_tn(const void* a_planes, const void* b_planes, float* C, int M, int N1, int N2, const uint32_t* absmax_a,
                const uint32_t* absmax_b, cudaStream_t stream, int b_exact, void* tail_scratch, size_t tail_scratch_bytes,
-               int a_pitch, const FusePeer* peer, int* exchanged_tiles, int peer_mode) {
+               int a_pitch, const FusePeer* peer, int* exchanged_tiles) {
     // a_pitch > 0: A is a column range of wider planes (row slab of C): a_planes points at its first column
     const int p1 = a_pitch > 0 ? a_pitch : pitch_of(N1), p2 = pitch_of(N2);
     CUtensorMap ma, mb;
     if (int rc = make_map(&ma, a_planes, N1, M, p1, 64, 64)) return rc;
     if (int rc = make_map(&mb, b_planes, N2, M, p2, 64, 64, b_exact ? 1 : 2)) return rc;
     return launch_gemm<true>(ma, mb, C, N1, N2, M, N2, absmax_a, absmax_b, stream, b_exact ? 2 : 0, static_cast<float*>(tail_scratch),
-                             tail_scratch_bytes, nullptr, nullptr, peer, exchanged_tiles, peer_mode);
+                             tail_scratch_bytes, nullptr, peer, exchanged_tiles);
 }
 
 }  // namespace mpv

@@ -312,7 +312,7 @@ static void launch_reduce_w(const PeerCtx& ctx, size_t n, int ctas, int unroll, 
 }
 
 int launch_peer_reduce(const PeerCtx& ctx_in, size_t n, cudaStream_t stream, size_t first) {
-    // [first, first + n): a sub-range of the buffers (the rows the fused exchange left over); n == 0 still runs the two
+    // [first, first + n): a sub-range of the buffers (the rows the slab exchange left over); n == 0 still runs the two
     // flag phases, which is what tells every rank that all deliveries of this step are done
     PeerCtx ctx = ctx_in;
     for (int i = 0; i < ctx.world; ++i) { ctx.part[i] += first; ctx.g_r[i] += first; }

@@ -26,7 +26,6 @@
 //   pass B    probit_cond_predict_kernel  probit_predict_rows_kernel with the weights u_s
 // observed[b, l]: 0 or 1 = observed with that value, any other byte = unobserved.
 #include "common.cuh"
-#include "fused_rows.cuh"
 #include "probit_math.cuh"
 #include "rows.h"
 #include "sample_rows.cuh"   // kThreads, kChunk, kLL, for_sample_pairs, rows_grid

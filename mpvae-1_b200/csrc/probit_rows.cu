@@ -18,7 +18,6 @@
 #include <type_traits>
 
 #include "common.cuh"
-#include "fused_rows.cuh"
 #include "philox.cuh"
 #include "probit_math.cuh"
 #include "rows.h"
@@ -166,8 +165,8 @@ __device__ __forceinline__ void row_tail(const RowArgs& a, int b) {
     }
 }
 
-// Second half of the tiled forward: adds the per-(sample-row, chunk) partials the cell kernel (or the product kernel's
-// math warps, fused_rows.cuh) left, in a fixed order, and runs the per-row tail.  One CTA per batch row.
+// Second half of the tiled forward: adds the per-(sample-row, chunk) partials the cell kernel left, in a fixed order,
+// and runs the per-row tail.  One CTA per batch row.
 template <bool MASKED>
 __global__ void __launch_bounds__(kThreads, 4)
 probit_row_finalize_kernel(const RowArgs a) {

@@ -7,7 +7,12 @@
 
 namespace mpv {
 
-struct FusePart;   // fused_rows.cuh
+// partial sums of one sample-row over the labels of one chunk, both branches: what the row forward's cell kernel leaves
+// for the finalize kernel, and the conditional prediction's log-likelihood pass for its weights kernel (lp_x)
+struct __align__(16) FusePart {
+    double lp_l, lp_x;                      // sum_l ll            (label branch, feature branch)
+    float pos_l, neg_l, pos_x, neg_x;       // sum_l exp(-5E) [y = 1], sum_l exp(5E) [y = 0]
+};
 
 // Arguments of the per-row kernels (probit_rows.cu).  Pointers are device pointers.
 struct RowArgs {
@@ -22,8 +27,8 @@ struct RowArgs {
     const float *y, *fe_out, *fx_out, *fe_mu, *fe_logvar, *fx_mu, *fx_logvar;
     int ldn;           // row pitch (floats) of nr and gxs: L rounded up to a multiple of 4 (16-byte aligned rows)
     const float* nr;   // (S*B,ldn) noise.R^T
-    // fused forward (tensor engine): per-(sample-row, tile) partial sums left by the product kernel's math warps; the
-    // finalize kernel adds them over the part_tiles column tiles in a fixed order
+    // per-(sample-row, label chunk) partial sums left by the row forward's cell kernel; the finalize kernel adds them
+    // over the part_tiles chunks in a fixed order
     const FusePart* part;
     int part_tiles;
     // training forward: the clamped probabilities of both branches, (S*B, ldn) each, kept for the backward (which then
@@ -94,7 +99,7 @@ int launch_erf_probe(const float* in, float* out, float* ref, size_t n, cudaStre
 int launch_warp_sum_probe(const void* in, void* out, void* ref, int groups, bool fp64, cudaStream_t stream);   // test hook
 int row_chunks(int L);   // 64-label chunks of a row: launch_row_forward needs B * S * row_chunks(L) FusePart records in a.part
 int launch_row_forward(RowArgs a, cudaStream_t stream);
-// the tail of the forward when the product kernel has already done the cell work (a.part != nullptr)
+// the tail of the forward after its cell kernel: a.part holds a.part_tiles chunk partials per sample-row
 int launch_row_finalize(RowArgs a, cudaStream_t stream);
 int launch_row_backward(RowArgs a, cudaStream_t stream);
 // *out_bits = fp32 bits of an upper bound of max |gxs| over the whole batch (NaN for non-sanitised degenerate rows),

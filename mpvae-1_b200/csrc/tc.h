@@ -7,9 +7,8 @@
 
 namespace mpv {
 
-struct FuseFwd;     // fused_rows.cuh: the probit row forward carried by the nt product kernel (opt-in)
-struct FuseNoise;   // fused_rows.cuh: the A operand's Philox noise drawn by the nt product kernel itself
-struct FusePeer;    // fused_rows.cuh: the finished tiles of the tn product summed over the ranks through peer memory
+struct FuseNoise;   // tc_warps.cuh: the A operand's Philox noise drawn by the nt product kernel itself
+struct FusePeer;    // tc_warps.cuh: the finished tiles of the tn product published for the exchange over the ranks
 
 bool tc_available();
 
@@ -41,12 +40,11 @@ int tc_philox_planes(void* planes, int S, int B, int Z, int B_global, int row0, 
                      const uint64_t* offset_dev, cudaStream_t stream);
 // a_exact / b_exact: that operand lies exactly on the 11-bit piece grid and is stored as ONE plane (the library's own
 // Philox noise): two MMA passes instead of three.
-// fuse != nullptr: the kernel also runs the probit row forward on its finished tiles (fused_rows.cuh; no K-slicing).
 // Columns [N, ldc) of C are left alone unless write_pad != 0: then they are padding the caller owns, and the epilogue
 // may fill them (with zeros) to store whole 16-byte vectors.
 int tc_gemm_nt(const void* a_planes, const void* b_planes, float* C, int M, int N, int K, const uint32_t* absmax_a,
                const uint32_t* absmax_b, cudaStream_t stream, int ldc = 0, int a_exact = 0,   // ldc: pitch of C (0 = N)
-               void* tail_scratch = nullptr, size_t tail_scratch_bytes = 0, const FuseFwd* fuse = nullptr,
+               void* tail_scratch = nullptr, size_t tail_scratch_bytes = 0,
                const FuseNoise* noise = nullptr,    // noise != nullptr: a_planes is written by the kernel itself (a_exact)
                int write_pad = 0);
 // tail_scratch (optional, tc_tail_scratch_bytes()): lets the kernel cut the tiles of the last, partial wave of its
@@ -57,11 +55,10 @@ int tc_absmax(const float* src, size_t n, uint32_t* out_bits, cudaStream_t strea
 int tc_gemm_tn(const void* a_planes, const void* b_planes, float* C, int M, int N1, int N2, const uint32_t* absmax_a,
                const uint32_t* absmax_b, cudaStream_t stream, int b_exact = 0, void* tail_scratch = nullptr,
                size_t tail_scratch_bytes = 0, int a_pitch = 0,
-               // peer != nullptr: C is this rank's partial; tiles [0, *exchanged_tiles) are summed over the ranks inside the
-               // kernel (into every rank's g_r), the K-sliced tail tiles are left to the caller
-               // peer_mode 3: on the kernel's own math warps; 4: the kernel only PUBLISHES finished tiles (per-tile counters in
-               // peer memory) and leaves exchange_sms() SMs free for the exchange kernel the caller runs beside it
-               const FusePeer* peer = nullptr, int* exchanged_tiles = nullptr, int peer_mode = 3);
+               // peer != nullptr: C is this rank's partial; the kernel PUBLISHES its finished tiles [0, *exchanged_tiles) in
+               // per-tile counters in peer memory and leaves exchange_sms() SMs free for the exchange kernel the caller runs
+               // beside it; the K-sliced tail tiles are left to the caller
+               const FusePeer* peer = nullptr, int* exchanged_tiles = nullptr);
 // SMs the g_R product leaves to the exchange kernel running beside it (even; MPVAE_EXCHANGE_SMS overrides: experiments)
 int exchange_sms(int world);
 

@@ -33,10 +33,9 @@ def main():
         ring = (NvlsRing if os.environ.get("PEER_CHECK_RING") == "nvls" else PeerRing)(L, Z, dev)
 
         def run(use_ring, step):
-            # PEER_CHECK_FUSED=1: the sum runs tile by tile inside the g_R product kernel (MPVAE_FLAG_FUSED_EXCHANGE)
+            # PEER_CHECK_SERIAL=1: the sum runs after the g_R product at every shape (MPVAE_FLAG_SERIAL_EXCHANGE)
             args = synth.make_args(L, Z, n_train_sample=S, noise_seed=5, noise_offset=step,
-                                   mpvae_flags=(0x40 if os.environ.get("PEER_CHECK_FUSED") == "1" else
-                                                0x80 if os.environ.get("PEER_CHECK_SERIAL") == "1" else 0) if use_ring else 0)
+                                   mpvae_flags=(0x80 if os.environ.get("PEER_CHECK_SERIAL") == "1" else 0) if use_ring else 0)
             args.dp_global_batch, args.dp_row0 = B * world, rank * B
             args.peer_ring = ring if use_ring else None
             leaves = {k: (v if k in ("y", "r_sqrt_sigma") else v.clone().requires_grad_(True)) for k, v in t.items()}

@@ -1,5 +1,5 @@
 """Measurement helper (not a test): per-kernel device times of the loss step from the library's own CUDA-event records
-(mpvae_profile*), with the row forward fused into the product kernel and as a separate kernel.
+(mpvae_profile*), with the noise drawn by the product kernel's math warps and by a kernel of its own.
 
     python tests/step_breakdown.py [--workload eurlex] [--z Z] [--batch B] [--steps 20] [--external-noise]
 """
@@ -31,7 +31,7 @@ def main():
     r32 = t.pop("r_sqrt_sigma").float().requires_grad_(True)
     noise = torch.randn(S, B, Z, device=dev) if a.external_noise else None
     flush = torch.empty(64 * 1024 * 1024, dtype=torch.float32, device=dev)
-    for name, flags in (("default", 0), ("separate_noise_kernel", _lib.FLAG_SEPARATE_NOISE), ("fused_row_forward", _lib.FLAG_FUSED_FORWARD)):
+    for name, flags in (("default", 0), ("separate_noise_kernel", _lib.FLAG_SEPARATE_NOISE)):
         args = synth.make_args(L, Z, n_train_sample=S, n_test_sample=S, mode=sh.mode, mpvae_flags=flags, noise_seed=1)
 
         def step(i):

@@ -185,7 +185,7 @@ def test_full_size_properties(name, L, Z, B, library_noise):
       * the backward is linear in the upstream cotangent
       * predictions are probabilities inside the clamp [eps/2, 1 - eps/2]
     `eurlex_philox` is bench.py's headline configuration exactly: S10 B1024 L3993 Z3993, library Philox noise, two-pass
-    tensor product with the row forward fused into it."""
+    tensor product, then the row forward."""
     from mpvae_b200 import synth
     S = 10
     inp = synth.loss_inputs(L, Z, B, S, seed=3, label_rate=20.0 / L, with_noise=not library_noise)

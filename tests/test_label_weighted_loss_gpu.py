@@ -1,7 +1,7 @@
 """GPU: label-weighted training (compute_loss(..., pos_weight=, neg_weight=) -> mpvae_probit_forward_label_weighted /
 _backward_label_weighted) in every regime: small (yeast / mirflickr shapes), CUDA-core (L = 200, Z = 64), dense tensor
 (delicious shape, reduced B) and the stable-CDF backward.  All-ones weights against None (bits, with a mask, row weights,
-soft labels, FUSED_FORWARD), the label-weighted oracle (random, zero, negative weights and a mix with a mask and row
+soft labels), the label-weighted oracle (random, zero, negative weights and a mix with a mask and row
 weights), weights of 1e4 and 1e-4 against the g_R bar, zero-weight cells, predictions, repeatability,
 DataParallelStep and GraphedTrainStep, and a planted model with rare labels trained with pos_weight."""
 import copy
@@ -12,16 +12,16 @@ import torch
 
 from tests import helpers as H
 from tests import label_weighted_elbo_oracle as LO
-from tests.test_masked_loss_gpu import (DEV, FUSED, LEAVES, SANITIZE, STABLE, TENSOR, _args, _bits, _inputs, _random_mask,
+from tests.test_masked_loss_gpu import (DEV, LEAVES, SANITIZE, STABLE, TENSOR, _args, _bits, _inputs, _random_mask,
                                         _vae_args)
 from tests.test_weighted_loss_gpu import _UP_NAMES, _upstream
 
 pytestmark = pytest.mark.gpu
 
 # (S, B, L, Z, flags, external noise): small regime (yeast, mirflickr), CUDA-core (tiled forward + saved backward),
-# dense tensor (delicious shape, B reduced), the stable-CDF backward (small and dense shapes), SANITIZE
+# dense tensor (delicious shape, B reduced; a ragged label tile), the stable-CDF backward (small and dense shapes), SANITIZE
 REGIME_CASES = [(10, 16, 14, 14, 0, False), (3, 33, 38, 38, 0, True), (10, 40, 200, 64, 0, False), (7, 21, 200, 64, 0, True),
-                (10, 70, 983, 983, 0, False), (3, 19, 983, 983, TENSOR, True), (10, 16, 38, 38, STABLE, False),
+                (10, 70, 983, 983, 0, False), (3, 19, 983, 983, TENSOR, True), (3, 77, 130, 256, 0, True), (10, 16, 38, 38, STABLE, False),
                 (10, 40, 257, 300, STABLE, False), (10, 33, 983, 10, SANITIZE, False)]
 ORACLE_CASES = [(10, 16, 38, 38, 0), (1, 5, 14, 14, 0), (10, 20, 200, 64, 0), (10, 20, 983, 983, 0), (7, 19, 130, 64, TENSOR),
                 (10, 16, 38, 38, STABLE), (10, 12, 257, 300, STABLE)]
@@ -78,18 +78,6 @@ def test_all_ones_label_weights_equal_none(S, B, L, Z, flags, external, masked, 
             assert _bits(o0[i], o1[i]), i
         for k in LEAVES:
             assert _bits(g0[k], g1[k]), k
-
-
-@pytest.mark.parametrize("S,B,L,Z,external", [(10, 70, 983, 983, False), (3, 77, 130, 256, True)])
-def test_all_ones_label_weights_under_fused_forward(S, B, L, Z, external):
-    """A label-weighted forward takes the separate row kernel: bits as the separate row kernel without weights."""
-    t, noise = _inputs(S, B, L, Z, external, seed=S + B)
-    o0, g0 = _run(t, noise, _args(S, L, Z, TENSOR))
-    o1, g1 = _run(t, noise, _args(S, L, Z, FUSED | TENSOR), pos=torch.ones(L, device=DEV))
-    for i in range(8):
-        assert _bits(o0[i], o1[i]), i
-    for k in LEAVES:
-        assert _bits(g0[k], g1[k]), k
 
 
 def _check_against_oracle(t, noise, args, lw, w, mask, out, g, upstream=None):

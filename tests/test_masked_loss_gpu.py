@@ -17,7 +17,7 @@ from tests import masked_elbo_oracle as MO
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 
-SANITIZE, TENSOR, FMA, STABLE, FUSED, SEPARATE = 0x1, 0x2, 0x4, 0x8, 0x10, 0x20
+SANITIZE, TENSOR, FMA, STABLE, SEPARATE = 0x1, 0x2, 0x4, 0x8, 0x20
 LEAVES = ("fe_out", "fe_mu", "fe_logvar", "fx_out", "fx_mu", "fx_logvar", "r_sqrt_sigma")
 
 
@@ -66,7 +66,7 @@ ALL_ONES_CASES = [
     (10, 16, 38, 38, STABLE, False), (100, 7, 81, 81, STABLE, True), (10, 70, 983, 983, FMA, False), (3, 9, 130, 64, FMA, True),
     (10, 70, 983, 983, 0, False), (10, 70, 983, 983, 0, True), (3, 77, 130, 256, 0, True), (100, 12, 300, 128, SEPARATE, False),
     (1, 300, 256, 256, 0, False), (7, 5, 130, 64, TENSOR, False), (10, 40, 257, 300, STABLE, False),
-    (3, 19, 983, 983, SEPARATE, True), (100, 1024, 3993, 3993, 0, False),
+    (3, 19, 983, 983, SEPARATE, True), (100, 1024, 3993, 3993, 0, False), (10, 1024, 3993, 3993, 0, False),
     (10, 16, 38, 38, SANITIZE, False), (10, 33, 983, 10, SANITIZE, False), (10, 70, 983, 983, SANITIZE, False),
 ]
 
@@ -88,21 +88,6 @@ def test_all_ones_mask_equals_unmasked(S, B, L, Z, flags, external):
             assert _bits(o0[i], o1[i]), (mode, i)
         for k in LEAVES:
             assert _bits(g0[k], g1[k]), (mode, k)
-
-
-@pytest.mark.parametrize("S,B,L,Z,external", [(10, 70, 983, 983, False), (3, 77, 130, 256, True), (10, 1024, 3993, 3993, False)])
-def test_all_ones_mask_under_fused_forward(S, B, L, Z, external):
-    """A masked call takes the separate row kernel under FUSED_FORWARD: the fused-vs-separate bar of
-    test_parity_gpu (predictions bit-equal, scalars <= 5e-7 relative, gradients <= 2e-6)."""
-    t, noise = _inputs(S, B, L, Z, external, seed=S + B)
-    args = _args(S, L, Z, FUSED | TENSOR)
-    o0, g0 = _run(t, noise, args)
-    o1, g1 = _run(t, noise, args, mask=torch.ones(B, L, dtype=torch.uint8, device=DEV))
-    assert torch.equal(o0[6], o1[6]) and torch.equal(o0[7], o1[7])
-    for i in range(6):
-        assert H.rel_err(o1[i].cpu().numpy(), o0[i].cpu().numpy()) <= 5e-7, i
-    for k in LEAVES:
-        assert H.rel_err(g1[k].cpu().numpy(), g0[k].cpu().numpy()) <= 2e-6, k
 
 
 @pytest.mark.parametrize("S,B,L,Z,flags", [(10, 16, 38, 38, 0), (100, 37, 81, 81, 0), (10, 33, 983, 10, 0),

@@ -42,12 +42,6 @@ def test_peer_ring_equals_nccl_allreduce():
     assert r.returncode == 0 and "PEER_CHECK PASS" in r.stdout
 
 
-def test_fused_exchange_equals_nccl_allreduce():
-    """MPVAE_FLAG_FUSED_EXCHANGE: the g_R product kernel sums its finished tiles over the ranks on its math warps."""
-    r = _torchrun("peer_check.py", env={"PEER_CHECK_FUSED": "1"})
-    assert r.returncode == 0 and "PEER_CHECK PASS" in r.stdout
-
-
 def test_serial_exchange_equals_nccl_allreduce():
     """MPVAE_FLAG_SERIAL_EXCHANGE: the stand-alone reduce kernel after the product at every shape."""
     r = _torchrun("peer_check.py", env={"PEER_CHECK_SERIAL": "1"})

@@ -1,5 +1,5 @@
 """GPU: weighted training (compute_loss(..., row_weight=) -> mpvae_probit_forward_weighted / _backward_weighted).  All-ones
-weights against row_weight=None (bits, with and without a mask, under FUSED_FORWARD too), the weighted oracle (positive,
+weights against row_weight=None (bits, with and without a mask), the weighted oracle (positive,
 zero and negative weights, a mask, cotangents on all 8 outputs), duplicated rows, zero-weight rows, a large weight in
 the tensor regime, predictions, repeatability, DataParallelStep and GraphedTrainStep, and a planted model with noisy
 rows down-weighted."""
@@ -11,7 +11,7 @@ import torch
 
 from tests import helpers as H
 from tests import weighted_elbo_oracle as WO
-from tests.test_masked_loss_gpu import (ALL_ONES_CASES, DEV, FUSED, LEAVES, ORACLE_CASES, SANITIZE, STABLE, TENSOR, _args,
+from tests.test_masked_loss_gpu import (ALL_ONES_CASES, DEV, LEAVES, ORACLE_CASES, SANITIZE, STABLE, TENSOR, _args,
                                         _bits, _inputs, _planted, _random_mask, _vae_args)
 
 pytestmark = pytest.mark.gpu
@@ -68,19 +68,6 @@ def test_all_ones_weights_equal_unweighted(S, B, L, Z, flags, external, masked):
             assert _bits(o0[i], o1[i]), (mode, i)
         for k in LEAVES:
             assert _bits(g0[k], g1[k]), (mode, k)
-
-
-@pytest.mark.parametrize("S,B,L,Z,external", [(10, 70, 983, 983, False), (3, 77, 130, 256, True), (10, 1024, 3993, 3993, False)])
-def test_all_ones_weights_under_fused_forward(S, B, L, Z, external):
-    """A weighted call keeps the fused row forward (the weights enter its finalize kernel): bits as without weights."""
-    t, noise = _inputs(S, B, L, Z, external, seed=S + B)
-    args = _args(S, L, Z, FUSED | TENSOR)
-    o0, g0 = _run(t, noise, args)
-    o1, g1 = _run(t, noise, args, weight=torch.ones(B, dtype=torch.float64, device=DEV))
-    for i in range(8):
-        assert _bits(o0[i], o1[i]), i
-    for k in LEAVES:
-        assert _bits(g0[k], g1[k]), k
 
 
 def _upstream(B, L, seed):
