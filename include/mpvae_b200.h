@@ -75,13 +75,15 @@ typedef struct mpvae_probit_params {
                                NULL = draw them inside the library (Philox, fields at the end of this struct) */
 
     /* ---- forward outputs (device) ---- */
-    float *scalars[6];       /* six 1-element outputs: total, nll, nll_x, c, c_x, kl   mpvae.py:207-210
+    float *scalars[6];       /* six 1-element outputs (B elements each, mpvae_probit_forward_rows): total, nll,
+                                nll_x, c, c_x, kl   mpvae.py:207-210
                                 (separate buffers so the host can hand them out as independent 0-dim tensors) */
     float *indiv_prob;       /* (B,L) mean_s E_x                              mpvae.py:203 */
     float *indiv_prob_label; /* (B,L) mean_s E                                mpvae.py:204 */
 
     /* ---- backward: upstream cotangents (device; a NULL entry = zero cotangent) ---- */
-    const float *g_scalars[6];       /* d objective / d (total, nll, nll_x, c, c_x, kl), 1 element each */
+    const float *g_scalars[6];       /* d objective / d (total, nll, nll_x, c, c_x, kl), 1 element each
+                                        (B each, mpvae_probit_backward_rows) */
     const float *g_indiv_prob;       /* (B,L) or NULL */
     const float *g_indiv_prob_label; /* (B,L) or NULL */
 
@@ -321,6 +323,23 @@ int mpvae_probit_forward_label_weighted(const mpvae_probit_params *p, const uint
                                         const float *label_weight, void *cuda_stream);
 int mpvae_probit_backward_label_weighted(const mpvae_probit_params *p, const uint8_t *label_mask, const float *row_weight,
                                          const float *label_weight, void *cuda_stream);
+
+/* Per-row losses (reduction 'none'): the ELBO's terms of every row as outputs, forward and backward.  Arguments as
+ * mpvae_probit_forward_label_weighted (any of label_mask, row_weight, label_weight may be NULL), but each p->scalars[k]
+ * addresses B floats: total_b, nll_b, nll_x_b, c_b, c_x_b, kl_b.  With t_b the row's fp64 terms (above), the five terms
+ * are w_b t_b (w_b = 1 without row weights) rounded once to fp32 -- exactly 0 on all six outputs for w_b == 0, whatever
+ * t_b holds -- and total_b is formed from them with the operations of total_loss.  So the mean over the rows of each
+ * output is the batch output up to summation order, and for B = 1 the two calls give the same bits.  indiv_prob and
+ * indiv_prob_label are unchanged.  In the backward each p->g_scalars[k] addresses B floats (row b's cotangent) or is
+ * NULL (zero); row b's coefficients are those of the batch call with its own cotangents and the divisor 1 in place of
+ * B.  A row whose six cotangents are all 0 gets all-zero loss coefficients, as a zero-weight row does: a degenerate row
+ * left out of the objective gets no NaN, even without MPVAE_FLAG_SANITIZE_DEGENERATE.  The cotangents enter the bound
+ * that scales the fp16 operands of the g_R product.  The backward must receive the forward's mask and weights.  Same
+ * workspace size as the batch calls. */
+int mpvae_probit_forward_rows(const mpvae_probit_params *p, const uint8_t *label_mask, const float *row_weight,
+                              const float *label_weight, void *cuda_stream);
+int mpvae_probit_backward_rows(const mpvae_probit_params *p, const uint8_t *label_mask, const float *row_weight,
+                               const float *label_weight, void *cuda_stream);
 
 /* Counter-based standard-normal noise, replaces torch.normal(0,1,(S,B,Z)) of mpvae.py:162.
  * Element (s, b_global, z) depends only on (seed, offset, s, b_global, z): a rank holding rows

@@ -36,6 +36,7 @@ EXPORTS = (
     "mpvae_probit_predict_conditional", "mpvae_probit_forward_masked", "mpvae_probit_backward_masked",
     "mpvae_probit_forward_weighted", "mpvae_probit_backward_weighted",
     "mpvae_probit_forward_label_weighted", "mpvae_probit_backward_label_weighted",
+    "mpvae_probit_forward_rows", "mpvae_probit_backward_rows",
     "mpvae_ghk_workspace_bytes", "mpvae_probit_predict_conditional_ghk",
     "mpvae_probit_sample_labels", "mpvae_f1_sets_workspace_bytes", "mpvae_f1_sets",
     "mpvae_mode_workspace_bytes", "mpvae_probit_score_sets", "mpvae_probit_predict_mode",
@@ -126,7 +127,8 @@ def _load():
     for fn in (lib.mpvae_probit_forward_weighted, lib.mpvae_probit_backward_weighted):
         fn.restype = C.c_int
         fn.argtypes = [C.POINTER(ProbitParams), C.c_void_p, C.c_void_p, C.c_void_p]
-    for fn in (lib.mpvae_probit_forward_label_weighted, lib.mpvae_probit_backward_label_weighted):
+    for fn in (lib.mpvae_probit_forward_label_weighted, lib.mpvae_probit_backward_label_weighted,
+               lib.mpvae_probit_forward_rows, lib.mpvae_probit_backward_rows):
         fn.restype = C.c_int
         fn.argtypes = [C.POINTER(ProbitParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.mpvae_philox_normal.restype = C.c_int

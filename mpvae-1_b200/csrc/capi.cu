@@ -461,8 +461,9 @@ int mpvae_probit_forward_weighted(const mpvae_probit_params* p_in, const uint8_t
     return mpvae_probit_forward_label_weighted(p_in, label_mask, row_weight, nullptr, cuda_stream);
 }
 
-int mpvae_probit_forward_label_weighted(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
-                                        const float* label_weight, void* cuda_stream) {
+// per_row: each p->scalars[k] addresses B floats (one per row) instead of one
+static int probit_forward(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
+                          const float* label_weight, bool per_row, void* cuda_stream) {
     mpvae_probit_params tmp;
     const mpvae_probit_params* p = normalize(p_in, &tmp);
     if (!p) return 1;
@@ -481,6 +482,7 @@ int mpvae_probit_forward_label_weighted(const mpvae_probit_params* p_in, const u
     a.mask = label_mask;
     a.row_weight = row_weight;   // read by row_tail only
     a.label_weight = label_weight;
+    a.per_row = per_row ? 1 : 0;
     // a scratch block sized for the backward means a training call: the forward keeps E for it (same placement in
     // both layouts: the backward-only buffers follow everything the forward shares)
     const Workspace wb = carve(p->S, p->B, p->L, p->Z, true, p->flags);
@@ -509,6 +511,16 @@ int mpvae_probit_forward_label_weighted(const mpvae_probit_params* p_in, const u
     if ((rc = fma_nt_product(p, w, stream))) return rc;
     ProfScope ps(MPVAE_PROF_ROW_FORWARD, stream);
     return launch_row_forward(a, stream);
+}
+
+int mpvae_probit_forward_label_weighted(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
+                                        const float* label_weight, void* cuda_stream) {
+    return probit_forward(p_in, label_mask, row_weight, label_weight, false, cuda_stream);
+}
+
+int mpvae_probit_forward_rows(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
+                              const float* label_weight, void* cuda_stream) {
+    return probit_forward(p_in, label_mask, row_weight, label_weight, true, cuda_stream);
 }
 
 int mpvae_probit_predict(const mpvae_probit_params* p_in, void* cuda_stream) {
@@ -674,8 +686,9 @@ int mpvae_probit_backward_weighted(const mpvae_probit_params* p_in, const uint8_
     return mpvae_probit_backward_label_weighted(p_in, label_mask, row_weight, nullptr, cuda_stream);
 }
 
-int mpvae_probit_backward_label_weighted(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
-                                         const float* label_weight, void* cuda_stream) {
+// per_row: each p->g_scalars[k] addresses B floats (one cotangent per row) or is NULL
+static int probit_backward(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
+                           const float* label_weight, bool per_row, void* cuda_stream) {
     mpvae_probit_params tmp;
     const mpvae_probit_params* p = normalize(p_in, &tmp);
     if (!p) return 1;
@@ -689,6 +702,7 @@ int mpvae_probit_backward_label_weighted(const mpvae_probit_params* p_in, const 
     a.mask = label_mask;
     a.row_weight = row_weight;   // scales the per-row coefficients, and with them the gxs bound of the fp16 planes
     a.label_weight = label_weight;
+    a.per_row = per_row ? 1 : 0;   // row b's cotangents: they enter the gxs bound through row_coeffs as well
     a.E_l = reinterpret_cast<float*>(base + w.e_l);
     a.E_x = reinterpret_cast<float*>(base + w.e_x);
     const int M = p->S * p->B;
@@ -814,6 +828,16 @@ int mpvae_probit_backward_label_weighted(const mpvae_probit_params* p_in, const 
         return launch_peer_reduce_nvls(pctx, static_cast<const float*>(p->peer_mc_part), static_cast<float*>(p->peer_mc_g_r),
                                        (size_t)p->L * p->Z, stream);
     return launch_peer_reduce(pctx, (size_t)p->L * p->Z, stream);
+}
+
+int mpvae_probit_backward_label_weighted(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
+                                         const float* label_weight, void* cuda_stream) {
+    return probit_backward(p_in, label_mask, row_weight, label_weight, false, cuda_stream);
+}
+
+int mpvae_probit_backward_rows(const mpvae_probit_params* p_in, const uint8_t* label_mask, const float* row_weight,
+                               const float* label_weight, void* cuda_stream) {
+    return probit_backward(p_in, label_mask, row_weight, label_weight, true, cuda_stream);
 }
 
 int mpvae_test_log_normal(const float* in, float* out, float* ref, uint64_t n, void* cuda_stream) {

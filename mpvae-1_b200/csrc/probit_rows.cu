@@ -75,11 +75,21 @@ __device__ __forceinline__ BlockCounts count_labels(const float* __restrict__ yr
     return c;
 }
 
+// total_loss from the five terms (mpvae.py:207-208): the same operations for the batch means and for one row's terms
+__device__ __forceinline__ float loss_total(const RowArgs& a, float nll, float nllx, float c, float cx, float kl) {
+    return MPV_ADD(MPV_ADD(MPV_MUL(MPV_ADD(nll, nllx), a.nll_coeff), MPV_MUL(MPV_ADD(c, cx), a.c_coeff)), MPV_MUL(kl, 1.1f));
+}
+
+// The divisor of the batch means in the backward's coefficients: B, or 1 for per-row outputs
+__device__ __forceinline__ float mean_div(const RowArgs& a) { return a.per_row ? 1.0f : (float)a.B; }
+
 // The per-row tail of the forward, shared by every forward kernel: label counts, KL row term (mpvae.py:147-148), per-row
 // log-mean-exp over samples, softmax weights, ranking sums (mpvae.py:188-190,115-122), and -- in the last CTA to
 // arrive -- the batch means and the total (mpvae.py:190,122,147,207-208) in a fixed summation order.  Expects the
 // row's a.lp / a.stat entries to have been written by threads of this CTA (any of them); blockDim.x == NT.  MASKED: the
-// label counts run over the observed labels (a.mask); the rest is unchanged.
+// label counts run over the observed labels (a.mask); the rest is unchanged.  Per-row outputs (a.per_row): the row's
+// own six values instead of the batch means -- w_b t_b formed in fp64 and rounded once (exactly 0 for a zero weight),
+// then the total from them as for the means, so that B = 1 gives the bits of the means.
 template <int NT = kThreads, bool MASKED = false>
 __device__ __forceinline__ void row_tail(const RowArgs& a, int b) {
     constexpr int kWarps = NT / 32;
@@ -129,8 +139,21 @@ __device__ __forceinline__ void row_tail(const RowArgs& a, int b) {
             for (int q = 0; q < 5; ++q) a.rowout[(size_t)b * 8 + q] = outv[q];
             a.rowaux[(size_t)b * 2 + 0] = (float)cnt.npos;
             a.rowaux[(size_t)b * 2 + 1] = (float)cnt.nneg;
+            if (a.per_row) {
+                const double w = a.row_weight ? (double)a.row_weight[b] : 1.0, dS = (double)S;
+                float t[5] = {0.0f, 0.0f, 0.0f, 0.0f, 0.0f};   // a zero-weight row: 0 even where its terms are inf / NaN
+                if (w != 0.0) {
+                    t[0] = (float)(w * outv[0]); t[1] = (float)(w * outv[1]);
+                    t[2] = (float)(w * outv[2] / dS); t[3] = (float)(w * outv[3] / dS);
+                    t[4] = (float)(w * outv[4]);
+                }
+                a.scalars[0][b] = loss_total(a, t[0], t[1], t[2], t[3], t[4]);
+#pragma unroll
+                for (int q = 0; q < 5; ++q) a.scalars[q + 1][b] = t[q];
+            }
         }
     }
+    if (a.per_row) return;   // no batch means: the last-CTA counter is never touched and stays 0
     __threadfence();
     __syncthreads();
     if (tid == 0) s_last = (atomicAdd(a.counter, 1u) == gridDim.x - 1);
@@ -157,9 +180,7 @@ __device__ __forceinline__ void row_tail(const RowArgs& a, int b) {
         const float nll = (float)(s_fin[0] / dB), nllx = (float)(s_fin[1] / dB);
         const float c = (float)(s_fin[2] / dSB), cx = (float)(s_fin[3] / dSB);
         const float kl = (float)(s_fin[4] / dB);
-        const float total = MPV_ADD(MPV_ADD(MPV_MUL(MPV_ADD(nll, nllx), a.nll_coeff), MPV_MUL(MPV_ADD(c, cx), a.c_coeff)),
-                                    MPV_MUL(kl, 1.1f));
-        *a.scalars[0] = total; *a.scalars[1] = nll; *a.scalars[2] = nllx;
+        *a.scalars[0] = loss_total(a, nll, nllx, c, cx, kl); *a.scalars[1] = nll; *a.scalars[2] = nllx;
         *a.scalars[3] = c; *a.scalars[4] = cx; *a.scalars[5] = kl;
         *a.counter = 0u;   // ready for the next launch on this workspace
     }
@@ -307,12 +328,17 @@ probit_row_fwd_tiled_kernel(const RowArgs a, FusePart* __restrict__ part, int nc
 // (mpvae.py:207-208 + upstream cotangents), the ranking normaliser k_b and the log-likelihood factor -(a_nll / B).
 // Weighted rows: a_nll, a_c and a_kl are multiplied by w_b before the divisions (a weight of 1 keeps the unweighted
 // bits); a zero-weight row gets all-zero coefficients, returned before the 0/0 of a degenerate row.
+// Per-row outputs (a.per_row): row b's own cotangents and the divisor 1 (mean_div); a row whose six cotangents are all 0
+// gets all-zero coefficients as a zero-weight row does, so a degenerate row left out of the objective gets no NaN.
 struct RowCoeffs { float kb[2], cnb[2], a_kl; };
 
 __device__ __forceinline__ RowCoeffs row_coeffs(const RowArgs& a, int b) {
-    const float gt = a.g_scalars[0] ? *a.g_scalars[0] : 0.0f, g1 = a.g_scalars[1] ? *a.g_scalars[1] : 0.0f,
-                g2 = a.g_scalars[2] ? *a.g_scalars[2] : 0.0f, g3 = a.g_scalars[3] ? *a.g_scalars[3] : 0.0f,
-                g4 = a.g_scalars[4] ? *a.g_scalars[4] : 0.0f, g5 = a.g_scalars[5] ? *a.g_scalars[5] : 0.0f;
+    const int gi = a.per_row ? b : 0;
+    const float gt = a.g_scalars[0] ? a.g_scalars[0][gi] : 0.0f, g1 = a.g_scalars[1] ? a.g_scalars[1][gi] : 0.0f,
+                g2 = a.g_scalars[2] ? a.g_scalars[2][gi] : 0.0f, g3 = a.g_scalars[3] ? a.g_scalars[3][gi] : 0.0f,
+                g4 = a.g_scalars[4] ? a.g_scalars[4][gi] : 0.0f, g5 = a.g_scalars[5] ? a.g_scalars[5][gi] : 0.0f;
+    if (a.per_row && gt == 0.0f && g1 == 0.0f && g2 == 0.0f && g3 == 0.0f && g4 == 0.0f && g5 == 0.0f)
+        return RowCoeffs{{0.0f, 0.0f}, {0.0f, 0.0f}, 0.0f};
     float a_nll[2] = {gt * a.nll_coeff + g1, gt * a.nll_coeff + g2};
     float a_c[2] = {gt * a.c_coeff + g3, gt * a.c_coeff + g4};
     RowCoeffs rc;
@@ -326,7 +352,7 @@ __device__ __forceinline__ RowCoeffs row_coeffs(const RowArgs& a, int b) {
     }
     const float npos = a.rowaux[(size_t)b * 2], nneg = a.rowaux[(size_t)b * 2 + 1];
     const float norm5 = 5.0f * (npos * nneg);
-    const float fS = (float)a.S, fB = (float)a.B;
+    const float fS = (float)a.S, fB = mean_div(a);
 #pragma unroll
     for (int q = 0; q < 2; ++q) {
         if (norm5 == 0.0f) {
@@ -391,7 +417,7 @@ probit_row_bwd_kernel(const RowArgs a) {
     extern __shared__ float s_gacc[];   // [nws][2][L] logit-gradient partial sums
     const int b = blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int L = a.L, S = a.S, B = a.B;
+    const int L = a.L, S = a.S;
     const int nwl = a.nwl, nws = kWarps / nwl;
     const int wl = warp % nwl, ws = warp / nwl;
     const int nchunks = (L + 31) >> 5;
@@ -402,7 +428,7 @@ probit_row_bwd_kernel(const RowArgs a) {
     for (int i = tid; i < nws * 2 * L; i += kThreads) s_gacc[i] = 0.0f;
 
     const RowCoeffs rc = row_coeffs(a, b);
-    const float fS = (float)S, fB = (float)B;
+    const float fS = (float)S, fB = mean_div(a);
     const float a_kl = rc.a_kl;
     const float* kb = rc.kb;
     const float* cnb = rc.cnb;
@@ -495,7 +521,7 @@ probit_row_bwd_kernel(const RowArgs a) {
         a.g_fe_out[(size_t)b * L + l] = sl;
         a.g_fx_out[(size_t)b * L + l] = sx;
     }
-    // KL gradients (SURVEY 8a-12): c = a_kl * 0.5 / B
+    // KL gradients (SURVEY 8a-12): c = a_kl * 0.5 / B (1 per row)
     const float kc = a_kl * 0.5f / fB;
     const size_t o = (size_t)b * a.D;
     for (int d = tid; d < a.D; d += kThreads) {
@@ -532,7 +558,7 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
         c[4] = 5.0f * rc.kb[0] * st.x;    c[5] = 5.0f * rc.kb[1] * st.z;    // x pos sums
     }
     __syncthreads();
-    const float fS = (float)S, fB = (float)a.B;
+    const float fS = (float)S, fB = mean_div(a);
     const bool has_gp = a.g_indiv_prob != nullptr, has_gpl = a.g_indiv_prob_label != nullptr;
     const float gscale = a.gxs_planes ? scale_from_absmax_bits(*a.gxs_scale) : 1.0f;
     // chunks of 64 labels; with operand planes the chunks run to the plane pitch (a multiple of 64): pad columns get zeros
@@ -623,7 +649,7 @@ probit_row_bwd_saved_kernel(const RowArgs a) {
         if ((c + 1) * 64 <= L) chunk(c, std::true_type{});
         else chunk(c, std::false_type{});
     }
-    if (blockIdx.y == 0) {   // KL gradients (SURVEY 8a-12): c = a_kl * 0.5 / B
+    if (blockIdx.y == 0) {   // KL gradients (SURVEY 8a-12): c = a_kl * 0.5 / B (1 per row)
         const float kc = rc.a_kl * 0.5f / fB;
         const size_t o = (size_t)b * a.D;
         for (int d = tid; d < a.D; d += kThreads) {
@@ -780,7 +806,7 @@ probit_small_bwd_kernel(const SmallArgs p) {
     for (int i = tid; i < S * Z; i += kThreads) nzs[i] = nsrc[((size_t)(i / Z) * B + b) * Z + (i % Z)];
     for (int i = tid; i < kWarps * 2 * L; i += kThreads) gsum[i] = 0.f;
     __syncthreads();
-    const float fS = (float)S, fB = (float)B;
+    const float fS = (float)S, fB = mean_div(a);
     const int nch = (L + 31) >> 5;
     for (int pair = warp; pair < npairs; pair += kWarps) {
 #pragma unroll

@@ -70,6 +70,11 @@ struct RowArgs {
     // log-likelihood is multiplied by its weight (a zero weight drops it) before the log-mean-exp, and in the backward
     // its log-likelihood coefficient likewise.  The ranking terms, KL and predictions do not read it.
     const float* label_weight;
+    // per-row losses (reduction 'none'): scalars[k] and g_scalars[k] address B floats, one per row, instead of one; the
+    // divisor of the means (mean_div) is 1 instead of B.  row_tail writes each row's six outputs and no batch means;
+    // row_coeffs reads row b's cotangents and gives a row whose six cotangents are all 0 all-zero coefficients.  No
+    // kernel is instantiated for it: the code branches on the flag.
+    int per_row;
 };
 
 size_t row_smem_bytes(int L);

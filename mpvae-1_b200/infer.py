@@ -16,6 +16,9 @@ import torch.distributed as dist
 from .train import shard_rows
 
 
+_ROW_TERMS = ("total_loss", "nll_loss", "nll_loss_x", "c_loss", "c_loss_x", "kl_loss")
+
+
 def _fields(res):
     return (res,) if isinstance(res, torch.Tensor) else tuple(res)
 
@@ -79,7 +82,7 @@ def _score_rows(model, feats: torch.Tensor, args, batch_size: Optional[int], gat
 @torch.no_grad()
 def predict_proba(model, feats: torch.Tensor, labels: Optional[torch.Tensor], args, batch_size: Optional[int] = None,
                   loss_fn=None, gather: bool = True, group=None, predict_fn=None, label_mask=None, row_weight=None,
-                  pos_weight=None, neg_weight=None):
+                  pos_weight=None, neg_weight=None, reduction="mean"):
     """Returns (indiv_prob (N, L), summed-loss dict).  `feats` / `labels` are device tensors for ALL N rows.
 
     `labels=None` scores rows that have no labels: each batch runs only the feature branch (`model.feat_forward`) and
@@ -90,7 +93,15 @@ def predict_proba(model, feats: torch.Tensor, labels: Optional[torch.Tensor], ar
     then those of the observed labels, and the predictions do not change.  `row_weight` (N,), with labels: the row
     weights (`compute_loss`); the summed losses are then the weighted sums sum_n w_n t_n (importance-weighted
     validation), and the predictions do not change.  `pos_weight` / `neg_weight` (L,), with labels: the label weights
-    (`compute_loss`); the summed losses are then the label-weighted ones, and the predictions do not change."""
+    (`compute_loss`); the summed losses are then the label-weighted ones, and the predictions do not change.
+    `reduction='none'`, with labels: the second value is instead a dict of every row's terms, (N,) tensors named
+    total_loss, nll_loss, nll_loss_x, c_loss, c_loss_x and kl_loss (`compute_loss(..., reduction='none')`), gathered
+    across ranks like the predictions -- e.g. each row's held-out -log-likelihood nll_loss_x, to rank rows for review
+    or attach a bootstrap error to the mean; the predictions do not change."""
+    if reduction not in ("mean", "none"):
+        raise ValueError(f"reduction must be 'mean' or 'none', got {reduction!r}")
+    if reduction == "none" and labels is None:
+        raise ValueError("reduction='none' returns per-row losses, which need labels")
     if labels is None and predict_fn is None:
         from .mpvae import predict as predict_fn
     if labels is not None and loss_fn is None:
@@ -111,15 +122,21 @@ def predict_proba(model, feats: torch.Tensor, labels: Optional[torch.Tensor], ar
             kw["pos_weight"] = pos_weight
         if neg_weight is not None:
             kw["neg_weight"] = neg_weight
+        if reduction == "none":
+            kw["reduction"] = "none"
         out = loss_fn(y, label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar, model.r_sqrt_sigma, args, **kw)
+        if reduction == "none":
+            return (out[6], *out[:6])
         if b > a:           # the empty slice of a rank without rows has NaN losses, means over nothing
             sums["total_loss"] = sums["total_loss"] + out[0] * (b - a)               # test.py:67-70
             sums["nll_loss"] = sums["nll_loss"] + out[1] * (b - a)
             sums["c_loss"] = sums["c_loss"] + out[3] * (b - a)
         return out[6]
 
-    probs = _score_rows(model, feats, args, batch_size, gather, group, score)
-    return probs, (sums if labels is not None else None)
+    res = _score_rows(model, feats, args, batch_size, gather, group, score)
+    if reduction == "none":
+        return res[0], dict(zip(_ROW_TERMS, res[1:]))
+    return res, (sums if labels is not None else None)
 
 
 @torch.no_grad()

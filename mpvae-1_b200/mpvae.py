@@ -155,7 +155,7 @@ def draw_noise(args, n_sample, n_batch, device, noise=None):
 
 
 def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r_sqrt_sigma, args, noise=None,
-                 label_mask=None, row_weight=None, pos_weight=None, neg_weight=None):
+                 label_mask=None, row_weight=None, pos_weight=None, neg_weight=None, reduction="mean"):
     """Reference signature (mpvae.py:145) -> (total_loss, nll_loss, nll_loss_x, c_loss, c_loss_x, kl_loss,
     indiv_prob, indiv_prob_label) (mpvae.py:210).
 
@@ -201,8 +201,26 @@ def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar
       - a zero weight drops the cell's term (it is not multiplied by 0) and its log-likelihood gradient is exactly 0;
       - other values are used as given (negatives included); they are not checked on the host.
     The weights receive no gradient: a weight that requires grad is refused, as are a wrong shape, device or a
-    non-floating dtype, before any noise offset is consumed."""
+    non-floating dtype, before any noise offset is consumed.
+
+    `reduction` 'mean' (the default: the batch means above) or 'none': per-row losses, e.g. to select or reweight rows
+    by their own loss (small-loss selection, group DRO, CVaR) or to score rows one by one.  The same 8-tuple comes back,
+    with total_loss, nll_loss, nll_loss_x, c_loss, c_loss_x and kl_loss as (B,) fp32 tensors of every row's values:
+      - with t_b the row's fp64 terms (above; label_mask and the label weights act inside them), the five terms are
+        w_b t_b (w_b = 1 without row_weight), rounded once to fp32, and total_loss[b] is formed from them with the
+        operations of the batch total; so the mean over the rows of each output is the 'mean' output up to summation
+        order, and with B = 1 the two reductions give the same bits on all 8 outputs and every gradient;
+      - a zero-weight row returns exactly 0 on all six outputs, inf / NaN terms included;
+      - indiv_prob and indiv_prob_label are unchanged;
+      - backward: each of the six takes a (B,) cotangent; row b's gradients are those of the 'mean' call with row b's
+        cotangents and the divisor 1 in place of B, so `total.sum() / B` gives the 'mean' gradients up to rounding;
+      - a row whose six cotangents are all 0 gets no loss gradient at all, as a zero-weight row: selecting rows by
+        indexing (`total[keep].sum()`) leaves an unselected degenerate row without NaN, even without
+        MPVAE_FLAG_SANITIZE_DEGENERATE; a selected degenerate row gets NaN gradients as with 'mean'.
+    Any other value is refused before any noise offset is consumed."""
     device = input_label.device
+    if reduction not in ("mean", "none"):
+        raise ValueError(f"reduction must be 'mean' or 'none', got {reduction!r}")
     if row_weight is not None:
         row_weight = _check_row_weight(row_weight, fe_out.shape[0], device)
     label_weight = _check_label_weight(pos_weight, neg_weight, fe_out.shape[1], device)
@@ -215,6 +233,9 @@ def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar
         # train.py:102 runs int(N/bs)+1 steps, so an empty last batch reaches the loss: every mean is NaN
         nan = (fe_out.sum() + fx_out.sum() + fe_mu.sum() + fe_logvar.sum() + fx_mu.sum() + fx_logvar.sum()) * math.nan
         empty = fx_out.new_empty((0, fx_out.shape[1]))
+        if reduction == "none":     # no rows, no per-row values
+            z = (fe_out.sum() + fx_out.sum() + fe_mu.sum() + fe_logvar.sum() + fx_mu.sum() + fx_logvar.sum()).reshape(1)[:0]
+            return (z, z.clone(), z.clone(), z.clone(), z.clone(), z.clone(), empty, empty.clone())
         return (nan, nan.clone(), nan.clone(), nan.clone(), nan.clone(), nan.clone(), empty, empty.clone())
     r32 = r_sqrt_sigma.to(device).float()                # mpvae.py:165 -- outside the Function: grad returns as fp64
     noise, spec = noise_plan(args, n_sample, n_batch, device, noise)
@@ -222,7 +243,7 @@ def compute_loss(input_label, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar
     # args.peer_ring (peer.PeerRing, data-parallel runs): g_R comes back already summed over the ranks
     return ProbitELBO.apply(input_label.float(), fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise,
                             float(args.nll_coeff), float(args.c_coeff), flags, spec, getattr(args, "peer_ring", None),
-                            label_mask, row_weight, label_weight)
+                            label_mask, row_weight, label_weight, reduction == "none")
 
 
 def predict(fx_out, r_sqrt_sigma, args, noise=None):

@@ -163,11 +163,14 @@ class ProbitELBO(torch.autograd.Function):
 
     `label_weight` (2, L) fp32 on the batch's device (`_check_label_weight`: row 0 weighs the y == 0 cells, row 1 the
     y == 1 cells), or None: the label weights of the cell log-likelihoods (mpvae_probit_forward_label_weighted,
-    semantics in mpvae.compute_loss).  It receives no gradient."""
+    semantics in mpvae.compute_loss).  It receives no gradient.
+
+    `per_row` (reduction 'none'): the six loss outputs are (B,) tensors of every row's terms, and their cotangents are
+    (B,) per row (mpvae_probit_forward_rows / _backward_rows, semantics in mpvae.compute_loss)."""
 
     @staticmethod
     def forward(ctx, y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32, noise, nll_coeff, c_coeff, flags,
-                noise_spec=None, peer=None, label_mask=None, row_weight=None, label_weight=None):
+                noise_spec=None, peer=None, label_mask=None, row_weight=None, label_weight=None, per_row=False):
         lib = _lib.lib()
         y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32 = (
             t.contiguous() for t in (y, fe_out, fe_mu, fe_logvar, fx_out, fx_mu, fx_logvar, r32))
@@ -191,7 +194,7 @@ class ProbitELBO(torch.autograd.Function):
         with torch.cuda.device(dev):
             ws_bytes = int(lib.mpvae_workspace_bytes(S, B, L, Z, 1 if want_bwd else 0, flags))
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-            scalars = [torch.empty((), dtype=torch.float32, device=dev) for _ in range(6)]
+            scalars = [torch.empty((B,) if per_row else (), dtype=torch.float32, device=dev) for _ in range(6)]
             prob = torch.empty((B, L), dtype=torch.float32, device=dev)
             prob_label = torch.empty((B, L), dtype=torch.float32, device=dev)
             _poison(ws, prob, prob_label, *scalars)
@@ -209,7 +212,10 @@ class ProbitELBO(torch.autograd.Function):
             p.indiv_prob, p.indiv_prob_label = _ptr(prob), _ptr(prob_label)
             p.workspace, p.workspace_bytes = _ptr(ws), ws_bytes
             stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            if label_weight is not None:
+            if per_row:
+                _lib.check(lib.mpvae_probit_forward_rows(C.byref(p), _ptr(label_mask), _ptr(row_weight),
+                                                         _ptr(label_weight), stream), "mpvae_probit_forward_rows")
+            elif label_weight is not None:
                 _lib.check(lib.mpvae_probit_forward_label_weighted(C.byref(p), _ptr(label_mask), _ptr(row_weight),
                                                                    _ptr(label_weight), stream),
                            "mpvae_probit_forward_label_weighted")
@@ -236,6 +242,7 @@ class ProbitELBO(torch.autograd.Function):
                                   *([label_weight] if label_weight is not None else []))
             ctx.dims = (S, B, L, Z, D)
             ctx.coeffs = (float(nll_coeff), float(c_coeff), int(flags))
+            ctx.per_row = bool(per_row)
             ctx.set_materialize_grads(False)
         return (*scalars, prob, prob_label)
 
@@ -261,7 +268,7 @@ class ProbitELBO(torch.autograd.Function):
                 g = g.expand(shape)
             return g.contiguous()
 
-        g_scal = [as_f32(g) for g in (g_total, g_nll, g_nll_x, g_c, g_c_x, g_kl)]
+        g_scal = [as_f32(g, (B,) if ctx.per_row else None) for g in (g_total, g_nll, g_nll_x, g_c, g_c_x, g_kl)]
         g_prob = as_f32(g_prob, (B, L))
         g_prob_label = as_f32(g_prob_label, (B, L))
         with torch.cuda.device(dev):
@@ -290,7 +297,10 @@ class ProbitELBO(torch.autograd.Function):
             p.g_r = _ptr(g_r)
             p.workspace, p.workspace_bytes = _ptr(ws), ws.numel()
             stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            if label_weight is not None:
+            if ctx.per_row:
+                _lib.check(lib.mpvae_probit_backward_rows(C.byref(p), _ptr(label_mask), _ptr(row_weight),
+                                                          _ptr(label_weight), stream), "mpvae_probit_backward_rows")
+            elif label_weight is not None:
                 _lib.check(lib.mpvae_probit_backward_label_weighted(C.byref(p), _ptr(label_mask), _ptr(row_weight),
                                                                     _ptr(label_weight), stream),
                            "mpvae_probit_backward_label_weighted")
@@ -304,7 +314,7 @@ class ProbitELBO(torch.autograd.Function):
                            "mpvae_probit_backward_masked")
         #       y     fe_out    fe_mu      fe_logvar  fx_out    fx_mu      fx_logvar  r32  noise nll_c c_c flags spec
         return (None, g_fe_out, g_mulv[0], g_mulv[1], g_fx_out, g_mulv[2], g_mulv[3], g_r, None, None, None, None, None,
-                None, None, None, None)   # peer, label_mask, row_weight, label_weight
+                None, None, None, None, None)   # peer, label_mask, row_weight, label_weight, per_row
 
 
 def _predict_dims(name, fx_out, r32, S, noise, noise_spec):

@@ -91,7 +91,10 @@ class DataParallelStep:
     def __init__(self, model: nn.Module, optimizer, scheduler, args, *, clip_norm: float = 100.0,
                  skip_nonfinite: bool = False, group=None, loss_fn: Optional[Callable] = None,
                  regulariser: Optional[Callable] = None, distributed: bool = True, peer_g_r: bool = False,
-                 peer_all: bool = False):
+                 peer_all: bool = False, row_objective: Optional[Callable] = None):
+        if row_objective is not None and regulariser is not None:
+            raise ValueError("DataParallelStep takes row_objective or regulariser, not both: fold the regulariser into "
+                             "the row objective")
         self.model, self.optimizer, self.scheduler = model, optimizer, scheduler
         self.args = copy.copy(args)
         self.clip_norm = clip_norm                 # 100 in train.py:126, 10 in fairsoft_train.py:141
@@ -111,6 +114,9 @@ class DataParallelStep:
             from .mpvae import compute_loss as loss_fn
         self.loss_fn = loss_fn
         self.regulariser = regulariser             # callable(StepOutput-like 8-tuple, row slice) -> scalar tensor
+        # callable(8-tuple of compute_loss(..., reduction='none'), row slice) -> (rows,) tensor phi: the step minimises
+        # sum_b phi_b / B over the global batch (see step)
+        self.row_objective = row_objective
         self.step_no = 0
         r = getattr(model, "r_sqrt_sigma", None)
         self.r_param = r if (r is not None and r.requires_grad) else None
@@ -218,7 +224,14 @@ class DataParallelStep:
         `row_weight`, if given, is the global (B,) row weight (`compute_loss`), sliced and passed as `row_weight=` in the
         same way.  Each rank's terms are sum_b w_b t_b / (its rows) and the shard weighting below makes the global loss
         sum over all rows of w_b t_b / B, as in one process.  `pos_weight` / `neg_weight`, if given, are the (L,) label
-        weights (`compute_loss`): they weigh labels, not rows, so every rank passes them whole, again only when given."""
+        weights (`compute_loss`): they weigh labels, not rows, so every rank passes them whole, again only when given.
+
+        With `row_objective=f` (constructor), the loss is called with `reduction='none'` and `f(out, slice(lo, hi))`
+        returns the shard's (hi - lo,) per-row values phi_b (e.g. `out[0] * keep`, or a group-DRO mixture of out[2]).  The
+        step minimises sum_b phi_b / B over the global batch: each rank backpropagates phi.sum() * world / B, and the
+        gradient average divides by world.  A selection over the global batch (a quantile of all rows' losses) is f's
+        business: it may all-gather the detached terms itself.  The returned scalars stay the batch means of the per-row
+        terms, so logging is unchanged."""
         args = self.args
         n_rows = input_label.shape[0]
         lo, hi = shard_rows(n_rows, self.rank, self.world)
@@ -250,15 +263,25 @@ class DataParallelStep:
                 kw["pos_weight"] = pos_weight
             if neg_weight is not None:
                 kw["neg_weight"] = neg_weight
+            if self.row_objective is not None:
+                kw["reduction"] = "none"
             out = self.loss_fn(y, label_out, label_mu, label_logvar, feat_out, feat_mu, feat_logvar, r, args, **kw)
-            total = out[0]
-            if self.regulariser is not None:
-                extra = self.regulariser(out, slice(lo, hi))
-                if extra is not None:
-                    total = total + extra
-            # every term is a mean over this rank's rows; weight by the shard size so unequal shards still average right
-            weight = (hi - lo) * self.world / max(n_rows, 1)
-            (total * weight if weight != 1.0 else total).backward()
+            if self.row_objective is not None:
+                phi = self.row_objective(out, slice(lo, hi))
+                if not isinstance(phi, torch.Tensor) or phi.shape != (hi - lo,):
+                    raise ValueError(f"row_objective must return a ({hi - lo},) tensor (one value per row of the shard), "
+                                     f"got {getattr(phi, 'shape', type(phi))}")
+                (phi.sum() * (self.world / max(n_rows, 1))).backward()
+                out = tuple(t.detach().mean() for t in out[:6]) + tuple(out[6:])
+            else:
+                total = out[0]
+                if self.regulariser is not None:
+                    extra = self.regulariser(out, slice(lo, hi))
+                    if extra is not None:
+                        total = total + extra
+                # every term is a mean over this rank's rows; weight by the shard size so unequal shards still average
+                weight = (hi - lo) * self.world / max(n_rows, 1)
+                (total * weight if weight != 1.0 else total).backward()
         else:
             # a ragged last batch with fewer rows than ranks leaves this rank without a row: it contributes zero
             # gradients (the bucket was just zeroed) and zero-weighted scalars, and still joins every collective below
